@@ -13,6 +13,10 @@ pinned HOST numpy buffers (H2D of the batch and D2H of the loss inside the timed
 object is the ThreadPredictor path (Network.predict_p_and_v) at B=4096, measured the same two ways.
 
 One JSON line on stdout (rank 0).  Everything else goes to stderr.
+
+--dump-outputs DIR writes what the timed paths computed in their last step as DIR/<name>.npy (float32): the weights after
+the last timed train step (train_<variable>.npy) and p / v of the last timed predict call (predict_p.npy, predict_v.npy).
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -254,7 +258,7 @@ def run_mlp_section(args, dev, stream, pk, clocks):
             dx, dyr, da = (torch.from_numpy(t).to(dev) for t in (x, y_r, act))
             p_out = torch.empty((b, a), dtype=torch.float32, device=dev)
             v_out = torch.empty((b,), dtype=torch.float32, device=dev)
-            steps = 20 if b > 4096 else 100
+            steps = args.steps
 
             def timed(fn):
                 for _ in range(3):
@@ -275,13 +279,13 @@ def run_mlp_section(args, dev, stream, pk, clocks):
             kt = {k: round(t / c * 1e3, 2) for k, (t, c) in net.kernel_times().items()}
             net.kernel_timing(0)
             t0 = time.perf_counter()
-            for _ in range(5):
+            for _ in range(steps):
                 net.train(x, y_r, act, None, None, 0, fetch_losses=True)
-            s_e2e_t = (time.perf_counter() - t0) / 5
+            s_e2e_t = (time.perf_counter() - t0) / steps
             t0 = time.perf_counter()
-            for _ in range(5):
+            for _ in range(steps):
                 net.predict_p_and_v(x)
-            s_e2e_p = (time.perf_counter() - t0) / 5
+            s_e2e_p = (time.perf_counter() - t0) / steps
             row = {"train_samples_per_s": b / (ms_t / 1e3), "train_ms": round(ms_t, 4),
                    "predictions_per_s": b / (ms_p / 1e3), "predict_ms": round(ms_p, 4),
                    "e2e_train_samples_per_s": b / s_e2e_t, "e2e_predictions_per_s": b / s_e2e_p,
@@ -395,6 +399,16 @@ def dp_check(net, rank, local_rank, world, B):
     return rep
 
 
+def dump_outputs(out_dir, variables, p_dev, v_dev):
+    """--dump-outputs: 4 MB of weights plus 28 bytes per predicted row, below 64 MB for any predict batch that fits in HBM."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"train_" + k.replace(":0", "").replace("/", "_"): v for k, v in variables.items()}
+    arrays.update(predict_p=p_dev.cpu().numpy(), predict_v=v_dev.cpu().numpy())
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float32))
+    log(f"[bench] wrote {len(arrays)} arrays ({sum(a.nbytes for a in arrays.values()) / 2 ** 20:.1f} MB) to {out_dir}")
+
+
 def run_ours(args, rank, local_rank, world):
     import torch
     import torch.distributed as dist
@@ -484,6 +498,8 @@ def run_ours(args, rank, local_rank, world):
     ms_train = timed(train_step, K)
     launches = net.launch_count() - l0
     ms_pred = timed(predict_step, K)
+    if args.dump_outputs and rank == 0:         # before the legs below train further
+        dump_outputs(args.dump_outputs, net.get_variables(), p_out, v_out)
 
     # spread: the same K steps timed in blocks of <= 10 (SURVEY 8d asks for median and best next to the mean)
     blocks = []
@@ -560,7 +576,7 @@ def run_ours(args, rank, local_rank, world):
         hx, hyr, ha = host[i % len(host)]
         net.train(hx.numpy(), hyr.numpy(), ha.numpy(), None, None, t, fetch_losses=True)
 
-    k_e2e = max(4, min(K, 20))
+    k_e2e = K
     for i in range(2):
         train_e2e(i); predict_e2e(i); train_e2e_t(i, 1)
     s_train_e2e = e2e(train_e2e, k_e2e)
@@ -781,7 +797,11 @@ def main():
     ap.add_argument("--cpu-steps", type=int, default=10)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-mlp", action="store_true", help="skip the configs[3] low-dimensional MLP section")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed train and predict steps as "
+                                                          "DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -15,7 +15,7 @@ predictions per second whatever the network costs (SURVEY 0.5).  These classes k
                           block (blocking while the ring is full = Queue(maxsize) back-pressure) and posts it.
 
 The reference's own `ThreadPredictor` / `ThreadTrainer` / `ProcessAgent` run unmodified over these objects (duck-typed
-queues; tests/test_transport.py does exactly that where /root/reference is present).  `ga3c_b200.ThreadPredictor` also uses
+queues; tests/test_transport.py does exactly that when GA3C_REFERENCE is set).  `ga3c_b200.ThreadPredictor` also uses
 the batch calls (`get_batch`, `reply_batch`): one gather into a pinned buffer and one reply scatter per batch instead of
 128 queue operations.  Blocking uses OS semaphores (no busy-waiting: 256 agents share the host's cores).
 
@@ -296,8 +296,13 @@ class SlabTrainingQueue:
         if not self._free[aid].acquire(block, timeout):     # ring full: Queue(maxsize) back-pressure
             import queue
             raise queue.Full
-        b = aid * self.blocks + self._next[aid]
-        self._next[aid] = (self._next[aid] + 1) % self.blocks
+        # the consumer takes blocks in slab order from its cursor, not in this producer's order: the block after the last one
+        # written may still be posted while an earlier one was taken (the permit guarantees that one block is free)
+        k = self._next[aid]
+        while self._posted.array[aid * self.blocks + k]:
+            k = (k + 1) % self.blocks
+        b = aid * self.blocks + k
+        self._next[aid] = (k + 1) % self.blocks
         self._x.array[b, :n] = np.asarray(x).reshape(n, -1)
         if self.ship_next_state:
             self._x2.array[b, :n] = np.asarray(x2).reshape(n, -1)

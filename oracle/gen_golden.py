@@ -1,7 +1,7 @@
-"""Generates tests/golden/*.npz|json.  Run in the BUILD container only (it imports the reference's
-own host-side Python from /root/reference, which does not exist on the GPU box):
+"""Generates tests/golden/*.npz|json.  Imports the reference's own host-side Python from the original GA3C's ga3c/
+directory, which is not part of this repository:
 
-    python -m oracle.gen_golden
+    GA3C_REFERENCE=/path/to/GA3C/ga3c python -m oracle.gen_golden
 
 Pinned against the REAL reference (imported, unmodified):
   returns.json      ProcessAgent._accumulate_rewards  (ProcessAgent.py:70-84) under the default
@@ -27,12 +27,14 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = os.path.join(os.path.dirname(HERE), "tests", "golden")
-REF = "/root/reference/ga3c"
+REF = os.environ.get("GA3C_REFERENCE", "")
 
 
 def import_reference_agent():
     """ProcessAgent imports gym/matplotlib/skimage transitively (EnvironmentPend ->
     PyperEnvironment -> pyper_env); stub them so the *unmodified* module imports."""
+    if not os.path.isdir(REF):
+        raise RuntimeError("GA3C_REFERENCE must name the original GA3C's ga3c/ directory")
     sys.dont_write_bytecode = True
     if REF not in sys.path:
         sys.path.insert(0, REF)

@@ -1,6 +1,6 @@
 """CPU tests (`-m "not gpu"`) of the boundary and the host logic: the C-ABI library loads and exports
 every symbol include/ga3c_b200.h declares (no compute calls), the batching threads keep the
-reference's queue contracts, and -- where /root/reference exists -- behave like the reference's
+reference's queue contracts, and -- where $GA3C_REFERENCE is set -- behave like the reference's
 own ThreadPredictor / ThreadTrainer on the same queue traffic."""
 import ctypes
 import os

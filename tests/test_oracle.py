@@ -1,7 +1,7 @@
 """CPU tests pinning the oracle (`-m "not gpu"`).
 
  * host-side functions: bit-exact against golden vectors produced by the REAL reference code
-   (oracle/gen_golden.py), and live against /root/reference where it exists;
+   (oracle/gen_golden.py), and live against $GA3C_REFERENCE where it is set;
  * network arithmetic (parity unpinned by the reference): finite differences, torch autograd as
    an independent second opinion, and a frozen self-pin.
 """

@@ -212,6 +212,35 @@ def test_training_queue_get_batch_follows_the_reference_stop_rule():
         tq.close()
 
 
+def test_training_queue_loses_no_item_when_the_consumer_wraps_past_a_producer():
+    """The consumer's cursor runs over the whole slab, so it can take a producer's newer block before an older one; the
+    producer's next put must then go to the block that was freed, not overwrite the older item that is still posted."""
+    tq = SlabTrainingQueue(2, max_rows=1, state_dim=S, num_actions=A, blocks_per_agent=2, ctx=CTX)
+    try:
+        x = np.zeros((1, S), np.float32); r = np.zeros(1); a = np.zeros((1, A), np.float32); d = np.zeros(1, bool)
+
+        def put(aid, v):
+            tq.for_agent(aid).put((np.full((1, S), v, np.float32), np.full(1, v, np.float64), np.zeros((1, A), np.float32),
+                                   None, np.zeros(1, bool)), timeout=1)
+
+        def take():
+            n = tq.get_batch(0, x, r, a, d, timeout=0.05)
+            return None if n is None else float(r[0])
+
+        put(0, 1.0); assert take() == 1.0              # agent 0's block 0; the cursor moves to block 1
+        put(1, 10.0); assert take() == 10.0            # agent 1's block 2; the cursor moves to block 3
+        put(0, 2.0); put(0, 3.0)                       # agent 0: item 2 in block 1, item 3 in block 0
+        assert take() == 3.0                           # the cursor wraps to block 0 first
+        put(0, 4.0)                                    # must not land on block 1, which still holds item 2
+        rest = []
+        while (v := take()) is not None:
+            rest.append(v)
+        assert sorted(rest) == [2.0, 4.0]
+        assert np.array_equal(x[0], np.full(S, rest[-1], np.float32))
+    finally:
+        tq.close()
+
+
 def _agent_proc(aid, pq, tq, n_steps, t_max, out):
     """A ProcessAgent-shaped loop (ProcessAgent.py:102-107, :117-176): predict every step, ship experiences every t_max."""
     rng = np.random.default_rng(aid)
@@ -308,7 +337,7 @@ def test_trainer_batches_equal_over_queue_and_slab():
 
 @pytest.mark.reference
 def test_reference_threads_run_unmodified_over_the_slab_queues():
-    """The reference's own ThreadPredictor / ThreadTrainer (imported from /root/reference) over the slab objects."""
+    """The reference's own ThreadPredictor / ThreadTrainer (imported from $GA3C_REFERENCE) over the slab objects."""
     sys.dont_write_bytecode = True
     sys.path.insert(0, REFERENCE)
     try:
