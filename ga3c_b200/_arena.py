@@ -36,7 +36,9 @@ class ArenaNetworkMixin:
         """NetworkVP.py:259-265 writes TensorBoard summaries from a second forward pass.  Here the same
         scalars (Pcost_advantage, Pcost_entropy, Pcost, Vcost, LearningRate, Beta) are appended to
         logs/<model_name>/scalars.csv."""
-        l = self.losses(x, y_r, a)
+        self._log_csv(self.losses(x, y_r, a), training_step)
+
+    def _log_csv(self, l: dict, training_step):
         os.makedirs(os.path.join("logs", self.model_name), exist_ok=True)
         with open(os.path.join("logs", self.model_name, "scalars.csv"), "a") as f:
             f.write(f"{training_step},{l['cost_p_1']},{l['cost_p_2']},{l['cost_p']},{l['cost_v']},"

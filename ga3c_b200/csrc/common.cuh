@@ -206,7 +206,8 @@ __device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.
 // serialise the PDL chain, ncu serialises and flushes the caches).  One pointer per translation unit, set by
 // trace_attach_<file>(); detached (the default) it costs one predicated load per CTA.
 enum KernelId { K_CONV_FWD = 0, K_DENSE_FWD, K_HEADS, K_DENSE_WGRAD, K_DENSE_DGRAD, K_CONV12_BWD, K_CONV11_WGRAD, K_RMSPROP,
-                K_GRAD_REDUCE, K_MLP_FUSED, K_MLP_WGRAD, K_MLP_REDUCE, K_DP_BIG, K_MLP_TC, K_COUNT };
+                K_GRAD_REDUCE, K_MLP_FUSED, K_MLP_WGRAD, K_MLP_REDUCE, K_DP_BIG, K_MLP_TC, K_HISTO,
+                K_COUNT };
 constexpr int TRACE_SLOTS = 6;
 static __device__ unsigned long long* g_trace = nullptr;
 __device__ __forceinline__ void trace_mark(int kid, int what) {      // what: 0 launched, 1 started, 2 ended

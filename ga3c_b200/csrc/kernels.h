@@ -211,4 +211,29 @@ int launch_returns(const double* rewards, const int64_t* seg_offsets, int n_segm
 int launch_select_actions(const float* p, const double* u, int batch, int num_actions, int32_t* action,
                           cudaStream_t stream);
 
+// histo.cu -- TF's histogram::Histogram of each source (the TensorBoard summaries of Network.log): output row s of `out` is
+// {min, max, num, sum, sum_squares, 1551 bucket counts} in fp64, bad[s] != 0 if source s holds a NaN / Inf.  histo_zero clears
+// out / bad, launch_histo counts (integer atomics into the count slots) and leaves fp64 partial moments in part[block][4],
+// launch_histo_merge sums them in block order: bit-identical output from call to call.
+constexpr int HISTO_MAX_SRC = 15;
+struct HistoSrc {
+  const void* p;                  // 16-byte aligned
+  long long n;                    // values in storage (Blk2: frames x B2_BYTES / 2, borders included)
+  int bf16;                       // 0 fp32, 1 bf16
+  int blk2;                       // bf16 n1 in the Blk2 layout (common.cuh): only the live 441 x 16 values of a frame count
+};
+struct HistoArgs {
+  HistoSrc src[HISTO_MAX_SRC];
+  int blk_end[HISTO_MAX_SRC];     // histo_plan: prefix sums of the blocks per source
+  int n_src;
+  double* out;                    // [n_src][5 + 1551]
+  int32_t* bad;                   // [n_src]
+  double* part;                   // [histo_blocks()][4] scratch
+};
+int histo_plan(HistoArgs& a);     // validates the sources and fills blk_end
+int histo_blocks(const HistoArgs& a);
+int histo_zero(const HistoArgs& a, cudaStream_t stream);
+int launch_histo(const HistoArgs& a, cudaStream_t stream);
+int launch_histo_merge(const HistoArgs& a, cudaStream_t stream);
+
 }  // namespace ga3c

@@ -102,6 +102,8 @@ struct ga3c_net {
   int last_batch = 0;
   unsigned long long* evt = nullptr;       // pipeline event log of CTA 0 (ga3c_evt_*), device memory
   unsigned long long* trace = nullptr;     // [K_COUNT][TRACE_SLOTS] globaltimer stamps (ga3c_trace_*), device memory
+  double* histo_part = nullptr;            // ga3c_histograms: fp64 partial moments per block
+  size_t histo_part_bytes = 0;
 
   int64_t off(int i) const { return params[i].offset; }
 };
@@ -109,7 +111,8 @@ struct ga3c_net {
 
 static const char* const kKernelNames[K_COUNT] = {"conv_fwd", "dense_fwd", "heads", "dense_wgrad", "dense_bwd",
                                                   "conv_bwd", "conv11_wgrad", "rmsprop", "grad_reduce",
-                                                  "mlp_fused", "mlp_wgrad", "mlp_reduce", "dp_big", "mlp_tc"};
+                                                  "mlp_fused", "mlp_wgrad", "mlp_reduce", "dp_big", "mlp_tc",
+                                                  "histograms"};
 
 enum { P_C11W = 0, P_C11B, P_C12W, P_C12B, P_D1W, P_D1B, P_VW, P_VB, P_PW, P_PB, P_COUNT };
 
@@ -122,7 +125,7 @@ int set_error(const std::string& m) { g_err = m; return -1; }     // for the oth
 const char* kernel_name(int kid) { return (kid >= 0 && kid < K_COUNT) ? kKernelNames[kid] : nullptr; }
 }
 extern "C" const char* ga3c_last_error(void) { return g_err.c_str(); }
-extern "C" int ga3c_abi_version(void) { return 6; }
+extern "C" int ga3c_abi_version(void) { return 7; }
 
 extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
   if (!cfg || !out) return fail_msg("ga3c_create: null argument");
@@ -266,6 +269,7 @@ extern "C" int ga3c_destroy(ga3c_net* n) {
   cudaFree(n->clip_ss); cudaFree(n->clip_scale); cudaFree(n->clip_ss2); cudaFree(n->clip_scale2);
   cudaFree(n->g2); cudaFree(n->ms2); cudaFree(n->mom2);
   if (n->trace) { trace_attach_all(nullptr); cudaFree(n->trace); }
+  cudaFree(n->histo_part);
   free_workspace(n);
   n->log.clear();
   delete n;
@@ -984,6 +988,42 @@ extern "C" int ga3c_workspace_ptr(ga3c_net* n, int which, void** ptr, int64_t* b
     case 7: *ptr = n->xblk; if (bytes) *bytes = b * XB_FRAME_BYTES; break;
     default: return fail_msg("ga3c_workspace_ptr: bad id");
   }
+  return 0;
+}
+
+extern "C" int ga3c_histograms(ga3c_net* n, int32_t batch, const float* p, const float* v, double* out, int32_t* bad,
+                               void* stream) {
+  if (int r = check_batch(n, batch, "ga3c_histograms")) return r;
+  if (!p || !v || !out || !bad) return fail_msg("ga3c_histograms: null buffer");
+  if (batch != n->last_batch) return fail_msg("ga3c_histograms: batch differs from the last forward on this handle");
+  if (n->dp_world > 1) return fail_msg("ga3c_histograms: not available on a peer-memory data-parallel handle");
+  CK(cudaSetDevice(n->cfg.device));
+  static_assert(GA3C_HISTO_SOURCES == P_COUNT + 5, "sources: the variables, n1, n2, d1, v, p");
+  HistoArgs a{};
+  for (int i = 0; i < P_COUNT; ++i) a.src[i] = HistoSrc{n->w + n->off(i), n->params[i].count, 0, 0};
+  const long long b = batch;
+  a.src[P_COUNT + 0] = HistoSrc{n->n1, b * B2_BYTES / 2, 1, 1};
+  a.src[P_COUNT + 1] = HistoSrc{n->n2, b * FLAT, 1, 0};
+  a.src[P_COUNT + 2] = HistoSrc{n->d1, b * FC, 0, 0};
+  a.src[P_COUNT + 3] = HistoSrc{v, b, 0, 0};
+  a.src[P_COUNT + 4] = HistoSrc{p, b * n->cfg.num_actions, 0, 0};
+  a.n_src = GA3C_HISTO_SOURCES;
+  a.out = out;
+  a.bad = bad;
+  if (int r = histo_plan(a)) return r;
+  const size_t part_bytes = sizeof(double) * 4 * histo_blocks(a);
+  if (part_bytes > n->histo_part_bytes) {
+    CK(cudaFree(n->histo_part));
+    n->histo_part = nullptr;
+    n->histo_part_bytes = 0;
+    CK(cudaMalloc((void**)&n->histo_part, part_bytes));
+    n->histo_part_bytes = part_bytes;
+  }
+  a.part = n->histo_part;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int r = histo_zero(a, st)) return r;
+  LAUNCH(n, K_HISTO, st, launch_histo(a, st));
+  LAUNCH(n, K_HISTO, st, launch_histo_merge(a, st));
   return 0;
 }
 

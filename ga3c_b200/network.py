@@ -7,7 +7,7 @@ Same constructor, attributes and methods as the reference class:
     .learning_rate, .beta          mutable, read at every train() (NetworkVP.py:230-231; Server.py:174-175)
     predict_p_and_v(x) -> [p, v]   (NetworkVP.py:248-252)
     train(x, y_r, a, x2, done, trainer_id)   (NetworkVP.py:254-257)
-    log / save / load / predict_single / predict_p / predict_v / get_global_step /
+    log / histograms / save / load / predict_single / predict_p / predict_v / get_global_step /
     get_variables_names / get_variable_value
 
 PyTorch is used for pinned host staging, device buffers, streams and torch.distributed only; every
@@ -19,11 +19,12 @@ import ctypes as C
 import os
 import re
 import threading
+import warnings
 
 import numpy as np
 import torch
 
-from . import _capi
+from . import _capi, summaries
 from ._arena import ArenaNetworkMixin
 from .config import Config as _DefaultConfig
 
@@ -199,6 +200,8 @@ class Network(ArenaNetworkMixin):
             dist.barrier(device_ids=[self._ordinal])      # every rank has mapped every slab before the first step
         self._dp = self.dp_mode == "nccl"
         self.last_losses = None
+        self._summ_dev = self._summ_host = None     # Network.log / histograms: device results and their pinned copy
+        self._events = None                         # the TensorBoard event file, opened by the first log()
 
     # ------------------------------------------------------------------ buffers
     def _alloc_io(self, rows: int):
@@ -291,6 +294,8 @@ class Network(ArenaNetworkMixin):
 
     def __del__(self):
         try:
+            if getattr(self, "_events", None) is not None:
+                self._events.close()
             if getattr(self, "_h", None):
                 self._lib.ga3c_dp_detach(self._h)
                 self._lib.ga3c_destroy(self._h)
@@ -463,6 +468,94 @@ class Network(ArenaNetworkMixin):
             st.synchronize()
         c1, c2, cv = (float(v) for v in l[:3])
         return dict(cost_p_1=c1, cost_p_2=c2, cost_p=-(c1 + c2), cost_v=cv, cost_all=-(c1 + c2) + cv)
+
+    # ------------------------------------------------------------------ TensorBoard summaries (NetworkVP.py:152-173, :259-265)
+    _HROW = 5 + summaries.BUCKETS
+
+    def _summaries(self, x, y_r, a):
+        """predict, forward_backward and ga3c_histograms on the same frames as ONE critical section of the handle (no trainer
+        thread can overwrite the activation workspace in between), then one device -> host copy.  predict goes first: it
+        rewrites n2 / d1 of the workspace, which forward_backward then leaves as the training forward computes them.  Weights,
+        slots and the step counter are not touched.  Returns (losses, {tag: (min, max, num, sum, sum_squares, counts)},
+        [tags of the histograms holding a NaN / Inf])."""
+        x = self._frames(x, self.state_dim)
+        b = x.shape[0]
+        if b == 0:
+            raise ValueError("the summaries need at least one row")
+        y_r = np.asarray(y_r, dtype=np.float32).reshape(b)
+        a = np.asarray(a, dtype=np.float32).reshape(b, self.num_actions)
+        u8 = x.dtype == np.uint8
+        tags = summaries.histogram_tags(self._table)
+        n_hist = len(tags) * self._HROW
+        if self._summ_dev is None:
+            # [histogram rows | 16 int32 non-finite flags | 4 fp32 loss sums] as doubles, so that one copy brings it all back
+            with torch.cuda.device(self._tdev):
+                self._summ_dev = torch.empty(n_hist + 10, dtype=torch.float64, device=self._tdev)
+                self._summ_host = torch.empty(n_hist + 10, dtype=torch.float64, pin_memory=True)
+        base = self._summ_dev.data_ptr()
+        bad_ptr, loss_ptr = base + 8 * n_hist, base + 8 * n_hist + 64
+        with self._lock:
+            self._ensure(b)
+            hx, dx = self._io_u8() if u8 else (self._hx, self._dx)
+            st = self._stream
+            with torch.cuda.stream(st):
+                self._h2d(x, hx, dx, b)
+                self._h2d(y_r, self._hyr, self._dyr, b)
+                self._h2d(a, self._ha, self._da, b)
+                pred = self._lib.ga3c_predict_u8 if u8 else self._lib.ga3c_predict
+                _capi.check(pred(self._h, dx.data_ptr(), b, self._dp_out.data_ptr(), self._dv_out.data_ptr(), st.cuda_stream),
+                            "ga3c_predict")
+                fb = self._lib.ga3c_forward_backward_u8 if u8 else self._lib.ga3c_forward_backward
+                _capi.check(fb(self._h, dx.data_ptr(), self._dyr.data_ptr(), self._da.data_ptr(), b, float(self.beta), loss_ptr,
+                               st.cuda_stream), "ga3c_forward_backward")
+                _capi.check(self._lib.ga3c_histograms(self._h, b, self._dp_out.data_ptr(), self._dv_out.data_ptr(), base, bad_ptr,
+                                                      st.cuda_stream), "ga3c_histograms")
+                self._summ_host.copy_(self._summ_dev, non_blocking=True)
+            st.synchronize()
+            host = self._summ_host.numpy().copy()
+        rows = host[:n_hist].reshape(len(tags), self._HROW)
+        stats = {t: (r[0], r[1], r[2], r[3], r[4], r[5:]) for t, r in zip(tags, rows)}
+        bad = host[n_hist:n_hist + 8].view(np.int32)[:len(tags)]
+        c1, c2, cv = (float(v) for v in host[n_hist + 8:].view(np.float32)[:3])
+        l = dict(cost_p_1=c1, cost_p_2=c2, cost_p=-(c1 + c2), cost_v=cv, cost_all=-(c1 + c2) + cv)
+        return l, stats, [t for t, f in zip(tags, bad) if f]
+
+    @staticmethod
+    def _nonfinite(tags):
+        # HistogramSummary's InvalidArgument: "Nan in summary histogram for: <tag>" (or "Infinity ...")
+        return ValueError("NaN or Infinity in summary histogram for: " + ", ".join(tags))
+
+    def histograms(self, x, y_r, a) -> dict:
+        """The 15 histograms `log` writes, for frames x (float32 or uint8) and targets y_r, a:
+        {tag: (min, max, num, sum, sum_squares, counts)}, TF's histogram::Histogram with its 1551 default buckets
+        (ga3c_b200.summaries.LIMITS), computed on the GPU.  Tags: weights_<variable name> (tf.summary's tag cleaning, e.g.
+        weights_conv11/w_0) in TF creation order, then activation_n1, activation_n2, activation_d2 (dense1), activation_v and
+        activation_p.  n1 and n2 are histogrammed as the network stores them (bf16).  Raises ValueError on a NaN / Inf."""
+        _, stats, bad = self._summaries(x, y_r, a)
+        if bad:
+            raise self._nonfinite(bad)
+        return stats
+
+    def log(self, x, y_r, a, training_step, feed_dict=None):
+        """NetworkVP.py:259-265: appends the six scalars to logs/<model_name>/scalars.csv (as the MLP networks do) and writes
+        them with the 15 histograms of `histograms` at step `training_step` to a TensorBoard event file in logs/<model_name>
+        (needs the optional tensorboard package; without it: the CSV line and one warning).  A NaN / Inf in a histogram raises
+        ValueError naming its tag after the CSV line is written; no event is written for that call.  With the peer-memory
+        data-parallel exchange (dp_mode 'fused') the dense1/w slices live on their owners: CSV only, one warning."""
+        if self.dp_mode == "fused":
+            if not getattr(self, "_warned_fused_log", False):
+                self._warned_fused_log = True
+                warnings.warn("Network.log: no TensorBoard histograms with dp_mode 'fused'; writing scalars.csv only",
+                              RuntimeWarning, stacklevel=2)
+            return super().log(x, y_r, a, training_step, feed_dict)
+        l, stats, bad = self._summaries(x, y_r, a)
+        self._log_csv(l, training_step)
+        if bad:
+            raise self._nonfinite(bad)
+        if self._events is None:
+            self._events = summaries.EventLog(os.path.join("logs", self.model_name))
+        values = (l["cost_p_1"], l["cost_p_2"], l["cost_p"], l["cost_v"], self.learning_rate, self.beta)
+        self._events.write(int(training_step), dict(zip(summaries.SCALAR_TAGS, values)), stats)
 
     # ------------------------------------------------------------------ variables / checkpoints
     def get_global_step(self):              # NetworkVP.py:233-235

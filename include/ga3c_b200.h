@@ -300,7 +300,26 @@ int ga3c_keep_dn1(ga3c_net* net, int32_t on);
 int64_t ga3c_launch_count(const ga3c_net* net);
 
 
-/* ---- per-kernel device timing (bench.py's roofline leg) -------------------------------------
+/* ---- TensorBoard histograms (NetworkVP.py:152-173, written by Network.log every TENSORBOARD_UPDATE_FREQUENCY steps) ----
+ * TensorFlow's histogram::Histogram of each source, computed on the device: {min, max, num, sum, sum_squares} in fp64 and the
+ * counts of its 1551 default buckets (bucket i holds limit[i-1] <= x < limit[i]; limits: +-1e-12 * 1.1^k up to 1e20, +-DBL_MAX
+ * and 0.0).  Deterministic: the same inputs give bit-identical output.  Non-finite values are left out of the statistics and
+ * flagged (TF's HistogramSummary refuses them).
+ * ga3c_histograms sources, in this order: the 10 variables (TF creation order), then n1, n2, d1 of the last
+ * ga3c_forward_backward[_u8] on this handle (`batch` must be its batch; n1 and n2 as stored, bf16), then v_dev [B] and
+ * p_dev [B, A] (fp32, 16-byte aligned: what ga3c_predict wrote for the same frames).  Not available once ga3c_dp_attach* has
+ * run: dense1/w slices then live on their owners.  Launches two kernels, both under kernel id "histograms".
+ * out_dev: GA3C_HISTO_SOURCES x (5 + GA3C_HISTO_BUCKETS) doubles {min, max, num, sum, sum_squares, counts...}
+ * bad_dev: GA3C_HISTO_SOURCES int32, non-zero if that source holds a NaN / Inf */
+#define GA3C_HISTO_BUCKETS 1551
+#define GA3C_HISTO_SOURCES 15
+int ga3c_histograms(ga3c_net* net, int32_t batch, const float* p_dev, const float* v_dev, double* out_dev, int32_t* bad_dev,
+                    void* stream);
+/* kernel-level test entry: one flat, 16-byte aligned array of n >= 1 fp32 (dtype 0) or bf16 (dtype 1) values; out_dev holds
+ * 5 + GA3C_HISTO_BUCKETS doubles, bad_dev one int32 */
+int ga3c_debug_histogram(const void* x_dev, int32_t dtype, int64_t n, double* out_dev, int32_t* bad_dev, void* stream);
+
+/* ---- per-kernel device timing (bench.py's roofline leg)-------------------------------------
  * ga3c_timing_enable(net, R) pre-creates events for R kernel records (R = 0 switches timing off).
  * While enabled, every kernel the hot path launches is bracketed by cudaEventRecord on the launch
  * stream -- no synchronisation is added.  ga3c_timing_collect synchronises the device, sums the
