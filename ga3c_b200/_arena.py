@@ -1,5 +1,6 @@
 """What the conv `Network` and the low-dimensional MLP networks share on the host side: the reference's small accessors, the
-flat parameter arena seen as a dict of TF-named tensors, RMSProp slots, checkpoints and the scalar log.
+flat parameter arena seen as a dict of TF-named tensors, RMSProp slots, checkpoints, the scalar log and the writing of
+`log`'s TensorBoard event file.
 
 A subclass provides `_table` ({TF variable name: (offset, shape)} into the fp32 arena, in TF creation order), `_download(which)`
 / `_upload(which, arena)` (arena ids: 0 weights, 1 gradients, 2 / 3 ms / mom of the first optimizer, 5 / 6 of the second),
@@ -12,6 +13,8 @@ import os
 import re
 
 import numpy as np
+
+from . import summaries
 
 
 class ArenaNetworkMixin:
@@ -43,6 +46,22 @@ class ArenaNetworkMixin:
         with open(os.path.join("logs", self.model_name, "scalars.csv"), "a") as f:
             f.write(f"{training_step},{l['cost_p_1']},{l['cost_p_2']},{l['cost_p']},{l['cost_v']},"
                     f"{self.learning_rate},{self.beta}\n")
+
+    @staticmethod
+    def _nonfinite(tags):
+        # HistogramSummary's InvalidArgument: "Nan in summary histogram for: <tag>" (or "Infinity ...")
+        return ValueError("NaN or Infinity in summary histogram for: " + ", ".join(tags))
+
+    def _log_summaries(self, l: dict, stats: dict, bad: list, training_step):
+        """`log` of a network with TensorBoard histograms: the CSV line, then ValueError if a histogram holds a NaN / Inf (no
+        event written), else the six scalars and `stats` at step training_step in the event file of logs/<model_name>."""
+        self._log_csv(l, training_step)
+        if bad:
+            raise self._nonfinite(bad)
+        if getattr(self, "_events", None) is None:
+            self._events = summaries.EventLog(os.path.join("logs", self.model_name))
+        values = (l["cost_p_1"], l["cost_p_2"], l["cost_p"], l["cost_v"], self.learning_rate, self.beta)
+        self._events.write(int(training_step), dict(zip(summaries.SCALAR_TAGS, values)), stats)
 
     # ------------------------------------------------------------------ the arena as named tensors
     def _split(self, arena: np.ndarray):

@@ -119,6 +119,8 @@ SIGNATURES = {
                                          C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "ga3c_histograms": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ga3c_debug_histogram": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "ga3c_mlp_histogram_count": (C.c_int, [C.c_void_p]),
+    "ga3c_mlp_histograms": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ga3c_mlp_timing_enable": (C.c_int, [C.c_void_p, C.c_int32]),
     "ga3c_mlp_timing_collect": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int64), C.c_int32]),
 }

@@ -215,7 +215,7 @@ int launch_select_actions(const float* p, const double* u, int batch, int num_ac
 // {min, max, num, sum, sum_squares, 1551 bucket counts} in fp64, bad[s] != 0 if source s holds a NaN / Inf.  histo_zero clears
 // out / bad, launch_histo counts (integer atomics into the count slots) and leaves fp64 partial moments in part[block][4],
 // launch_histo_merge sums them in block order: bit-identical output from call to call.
-constexpr int HISTO_MAX_SRC = 15;
+constexpr int HISTO_MAX_SRC = 23;     // conv net 15; MLP nets: variables + live hidden layers + 2, at most 23
 struct HistoSrc {
   const void* p;                  // 16-byte aligned
   long long n;                    // values in storage (Blk2: frames x B2_BYTES / 2, borders included)

@@ -46,6 +46,9 @@ struct ga3c_mlp {
   float* dz[MLP_MAX_LAYERS] = {};
   float* dlogits = nullptr;
   float* loss_part = nullptr;
+  int last_batch = 0;                    // rows of act[] written by the last forward (0: none since the workspace was allocated)
+  double* histo_part = nullptr;          // ga3c_mlp_histograms: fp64 partial moments per block
+  size_t histo_part_bytes = 0;
   int64_t global_step = 0;
   // tensor-core mode (mlp_tc.cu): the run of wide layers [tc_lo, tc_hi) as 3xTF32 GEMMs for training batches >= tc_min_batch
   int tc_lo = 0, tc_hi = 0, tc_min_batch = 4096;
@@ -78,6 +81,7 @@ extern "C" int ga3c_mlp_destroy(ga3c_mlp* n) {
   cudaFree(n->w); cudaFree(n->g); cudaFree(n->ms); cudaFree(n->mom); cudaFree(n->part);
   cudaFree(n->clip_ss); cudaFree(n->clip_scale); cudaFree(n->clip_ss2); cudaFree(n->clip_scale2);
   cudaFree(n->g2); cudaFree(n->ms2); cudaFree(n->mom2);
+  cudaFree(n->histo_part);
   free_workspace(n);
   n->log.clear();
   delete n;
@@ -243,6 +247,7 @@ extern "C" int ga3c_mlp_reserve(ga3c_mlp* n, int32_t max_batch) {
   CK(cudaSetDevice(n->cfg.device));
   CK(cudaDeviceSynchronize());
   free_workspace(n);
+  n->last_batch = 0;
   if (int r = alloc_workspace(n, max_batch)) { n->cfg.max_batch = 0; return r; }
   return 0;
 }
@@ -329,6 +334,47 @@ static int check_batch(ga3c_mlp* n, int batch, const char* who) {
   return 0;
 }
 
+extern "C" int ga3c_mlp_histogram_count(const ga3c_mlp* n) {
+  return n ? (int)n->params.size() + n->net.n_layers + 2 : 0;
+}
+
+extern "C" int ga3c_mlp_histograms(ga3c_mlp* n, int32_t batch, const float* p, const float* v, double* out, int32_t* bad,
+                                   void* stream) {
+  if (int r = check_batch(n, batch, "ga3c_mlp_histograms")) return r;
+  if (!p || !v || !out || !bad) return set_error("ga3c_mlp_histograms: null buffer");
+  if (batch != n->last_batch) return set_error("ga3c_mlp_histograms: batch differs from the last forward on this handle");
+  const int n_src = ga3c_mlp_histogram_count(n);
+  if (n_src > HISTO_MAX_SRC) return set_error("ga3c_mlp_histograms: more than " + std::to_string(HISTO_MAX_SRC) + " sources");
+  CK(cudaSetDevice(n->cfg.device));
+  // the variables (gradient-less ones included: they are trainable variables of the graph), act[] of every live hidden layer,
+  // v, p.  Arena offsets are multiples of ALIGN_FLOATS and each act[l] is its own allocation: every source is 16-byte aligned.
+  HistoArgs a{};
+  int s = 0;
+  for (const MlpParam& q : n->params) a.src[s++] = HistoSrc{n->w + q.offset, q.count, 0, 0};
+  const long long b = batch;
+  for (int l = 0; l < n->net.n_layers; ++l) a.src[s++] = HistoSrc{n->act[l], b * n->net.L[l].n, 0, 0};
+  a.src[s++] = HistoSrc{v, b, 0, 0};
+  a.src[s++] = HistoSrc{p, b * n->cfg.num_actions, 0, 0};
+  a.n_src = n_src;
+  a.out = out;
+  a.bad = bad;
+  if (int r = histo_plan(a)) return r;
+  const size_t part_bytes = sizeof(double) * 4 * histo_blocks(a);
+  if (part_bytes > n->histo_part_bytes) {
+    CK(cudaFree(n->histo_part));
+    n->histo_part = nullptr;
+    n->histo_part_bytes = 0;
+    CK(cudaMalloc((void**)&n->histo_part, part_bytes));
+    n->histo_part_bytes = part_bytes;
+  }
+  a.part = n->histo_part;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int r = histo_zero(a, st)) return r;
+  LAUNCH(n, K_HISTO, st, launch_histo(a, st));
+  LAUNCH(n, K_HISTO, st, launch_histo_merge(a, st));
+  return 0;
+}
+
 static MlpStepArgs step_args(ga3c_mlp* n, const float* x, int batch) {
   MlpStepArgs s{};
   s.w = n->w; s.x = x; s.batch = batch;
@@ -353,9 +399,10 @@ extern "C" int ga3c_mlp_predict(ga3c_mlp* n, const float* x, int32_t batch, floa
       LAUNCH(n, K_MLP_TC, st, launch_mlp_tc_fwd(n->w + net.L[l].w_off, n->w + net.L[l].b_off, net.L[l].k, net.L[l].n, net.L[l].act,
                                                 n->act[l - 1], n->act[l], batch, st));
     LAUNCH(n, K_MLP_FUSED, st, launch_mlp_heads(net, s, n->num_sms, st));
+    n->last_batch = batch;
     return 0;
   }
-  LAUNCH(n, K_MLP_FUSED, st, launch_mlp_fused(n->net, s, n->num_sms, st));
+  LAUNCH(n, K_MLP_FUSED, st, launch_mlp_fused(n->net, s, n->num_sms, st));     // writes no act[]: last_batch stays
   return 0;
 }
 
@@ -367,6 +414,7 @@ static int mlp_fb_impl(ga3c_mlp* n, const float* x, const float* yr, const float
   cudaStream_t st = (cudaStream_t)stream;
   MlpStepArgs s = step_args(n, x, batch);
   s.yr = yr; s.a = a; s.beta = beta; s.train = 1; s.part = part;
+  n->last_batch = batch;
   const int tm = mlp_tile_rows(batch, n->num_sms);
   if (n->tc_hi > n->tc_lo && batch >= n->tc_min_batch) {
     // the wide layers as 3xTF32 tensor-core GEMMs over the activations the fused kernel keeps in HBM anyway

@@ -125,7 +125,7 @@ int set_error(const std::string& m) { g_err = m; return -1; }     // for the oth
 const char* kernel_name(int kid) { return (kid >= 0 && kid < K_COUNT) ? kKernelNames[kid] : nullptr; }
 }
 extern "C" const char* ga3c_last_error(void) { return g_err.c_str(); }
-extern "C" int ga3c_abi_version(void) { return 7; }
+extern "C" int ga3c_abi_version(void) { return 8; }
 
 extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
   if (!cfg || !out) return fail_msg("ga3c_create: null argument");

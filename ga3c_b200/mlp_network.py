@@ -19,7 +19,7 @@ import threading
 import numpy as np
 import torch
 
-from . import _capi
+from . import _capi, summaries
 from ._arena import ArenaNetworkMixin
 from .config import Config as _DefaultConfig
 from .network import _parse_device
@@ -81,6 +81,11 @@ class _MlpNetwork(ArenaNetworkMixin):
         rng = np.random.default_rng(seed)
         self.set_variables({k: rng.uniform(-0.3, 0.3, size=s).astype(np.float32) for k, (_, s) in self._table.items()})
         self.last_losses = None
+        self._hist_tags = summaries.mlp_histogram_tags([(k, self._live[k]) for k in self._table])
+        if len(self._hist_tags) != self._lib.ga3c_mlp_histogram_count(self._h):
+            raise _capi.Ga3cError("ga3c_mlp_histogram_count disagrees with the variable table")
+        self._summ_dev = self._summ_host = None     # log / histograms: device results and their pinned copy
+        self._events = None                         # the TensorBoard event file, opened by the first log()
 
     # ------------------------------------------------------------------ buffers
     def _alloc_io(self, rows: int):
@@ -107,6 +112,8 @@ class _MlpNetwork(ArenaNetworkMixin):
 
     def __del__(self):
         try:
+            if getattr(self, "_events", None) is not None:
+                self._events.close()
             if getattr(self, "_h", None):
                 self._lib.ga3c_mlp_destroy(self._h)
                 self._h = None
@@ -211,6 +218,68 @@ class _MlpNetwork(ArenaNetworkMixin):
                 l = self._loss_dev.cpu()
             self._stream.synchronize()
         return self._loss_dict(l)
+
+    # ------------------------------------------------------------------ TensorBoard summaries (NetworkVP.py:152-173, :259-265)
+    _HROW = 5 + summaries.BUCKETS
+
+    def _summaries(self, x, y_r, a):
+        """predict, forward_backward and ga3c_mlp_histograms on the same rows as ONE critical section of the handle (no trainer
+        thread can overwrite the layer outputs in between), then one device -> host copy.  predict goes first: for a
+        tensor-core batch it writes its layer outputs through the training workspace, which forward_backward then rewrites.
+        Weights, slots and the step counter are not touched.  Returns (losses, {tag: (min, max, num, sum, sum_squares,
+        counts)}, [tags of the histograms holding a NaN / Inf])."""
+        x = self._rows(x)
+        if x.shape[0] == 0:
+            raise ValueError("the summaries need at least one row")
+        tags = self._hist_tags
+        n_hist = len(tags) * self._HROW
+        n_bad = (len(tags) + 1) // 2
+        if self._summ_dev is None:
+            # [histogram rows | int32 non-finite flags | 4 fp32 loss sums] as doubles, so that one copy brings it all back
+            with torch.cuda.device(self._tdev):
+                self._summ_dev = torch.empty(n_hist + n_bad + 2, dtype=torch.float64, device=self._tdev)
+                self._summ_host = torch.empty(n_hist + n_bad + 2, dtype=torch.float64, pin_memory=True)
+        base = self._summ_dev.data_ptr()
+        bad_ptr, loss_ptr = base + 8 * n_hist, base + 8 * (n_hist + n_bad)
+        with self._lock:
+            st = self._stream
+            with torch.cuda.stream(st):
+                b = self._stage_train(x, y_r, a)
+                dx, dp, dv = self._dx[:b], self._dp_out[:b], self._dv_out[:b]
+                self.predict_device(dx, dp, dv, stream=st)
+                _capi.check(self._lib.ga3c_mlp_forward_backward(self._h, dx.data_ptr(), self._dyr.data_ptr(), self._da.data_ptr(),
+                                                                b, float(self.beta), loss_ptr, st.cuda_stream),
+                            "ga3c_mlp_forward_backward")
+                _capi.check(self._lib.ga3c_mlp_histograms(self._h, b, dp.data_ptr(), dv.data_ptr(), base, bad_ptr,
+                                                          st.cuda_stream), "ga3c_mlp_histograms")
+                self._summ_host.copy_(self._summ_dev, non_blocking=True)
+            st.synchronize()
+            host = self._summ_host.numpy().copy()
+        rows = host[:n_hist].reshape(len(tags), self._HROW)
+        stats = {t: (r[0], r[1], r[2], r[3], r[4], r[5:]) for t, r in zip(tags, rows)}
+        bad = host[n_hist:n_hist + n_bad].view(np.int32)[:len(tags)]
+        l = self._loss_dict(host[n_hist + n_bad:].view(np.float32))
+        return l, stats, [t for t, f in zip(tags, bad) if f]
+
+    def histograms(self, x, y_r, a) -> dict:
+        """The histograms `log` writes, for rows x [B, S] and targets y_r, a: {tag: (min, max, num, sum, sum_squares, counts)},
+        TF's histogram::Histogram with its 1551 default buckets (ga3c_b200.summaries.LIMITS), computed on the GPU.  Tags
+        (summaries.mlp_histogram_tags): weights_<variable name> (tf.summary's tag cleaning, e.g. weights_dense1/w_0) for every
+        variable in TF creation order, gradient-less ones included; activation_<layer scope> for every live hidden layer in
+        forward order (fork NetworkVP: activation_dense11_p ... activation_dense14_p, activation_dense1; NetworkVP_discrate:
+        activation_dense1_<n>_p); then activation_v (logits_v) and activation_p (softmax_p: for the fork NetworkVP the atan2
+        output).  Raises ValueError on a NaN / Inf."""
+        _, stats, bad = self._summaries(x, y_r, a)
+        if bad:
+            raise self._nonfinite(bad)
+        return stats
+
+    def log(self, x, y_r, a, training_step, feed_dict=None):
+        """NetworkVP.py:259-265: appends the six scalars to logs/<model_name>/scalars.csv and writes them with the histograms
+        of `histograms` at step `training_step` to a TensorBoard event file in logs/<model_name> (needs the optional
+        tensorboard package; without it: the CSV line and one warning).  A NaN / Inf in a histogram raises ValueError naming
+        its tag after the CSV line is written; no event is written for that call."""
+        self._log_summaries(*self._summaries(x, y_r, a), training_step)
 
     # ------------------------------------------------------------------ variables / checkpoints
     def get_global_step(self):

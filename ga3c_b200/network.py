@@ -520,11 +520,6 @@ class Network(ArenaNetworkMixin):
         l = dict(cost_p_1=c1, cost_p_2=c2, cost_p=-(c1 + c2), cost_v=cv, cost_all=-(c1 + c2) + cv)
         return l, stats, [t for t, f in zip(tags, bad) if f]
 
-    @staticmethod
-    def _nonfinite(tags):
-        # HistogramSummary's InvalidArgument: "Nan in summary histogram for: <tag>" (or "Infinity ...")
-        return ValueError("NaN or Infinity in summary histogram for: " + ", ".join(tags))
-
     def histograms(self, x, y_r, a) -> dict:
         """The 15 histograms `log` writes, for frames x (float32 or uint8) and targets y_r, a:
         {tag: (min, max, num, sum, sum_squares, counts)}, TF's histogram::Histogram with its 1551 default buckets
@@ -548,14 +543,7 @@ class Network(ArenaNetworkMixin):
                 warnings.warn("Network.log: no TensorBoard histograms with dp_mode 'fused'; writing scalars.csv only",
                               RuntimeWarning, stacklevel=2)
             return super().log(x, y_r, a, training_step, feed_dict)
-        l, stats, bad = self._summaries(x, y_r, a)
-        self._log_csv(l, training_step)
-        if bad:
-            raise self._nonfinite(bad)
-        if self._events is None:
-            self._events = summaries.EventLog(os.path.join("logs", self.model_name))
-        values = (l["cost_p_1"], l["cost_p_2"], l["cost_p"], l["cost_v"], self.learning_rate, self.beta)
-        self._events.write(int(training_step), dict(zip(summaries.SCALAR_TAGS, values)), stats)
+        self._log_summaries(*self._summaries(x, y_r, a), training_step)
 
     # ------------------------------------------------------------------ variables / checkpoints
     def get_global_step(self):              # NetworkVP.py:233-235

@@ -1,7 +1,7 @@
 """TensorBoard summaries of `Network.log` (NetworkVP.py:152-173, :259-265): the six scalars and the weight / activation
 histograms, written to an event file under logs/<model_name> as the reference's `tf.summary.FileWriter` does.
 
-The histogram statistics come from the device (ga3c_histograms); this module only turns them into TF's histogram encoding and
+The histogram statistics come from the device (ga3c_histograms, ga3c_mlp_histograms); this module only turns them into TF's histogram encoding and
 writes them with `torch.utils.tensorboard.SummaryWriter`, which needs the optional `tensorboard` package.
 """
 from __future__ import annotations
@@ -37,10 +37,21 @@ def clean_tag(name: str) -> str:
     return re.sub(r"[^-/\w\.]", "_", name)
 
 
-def histogram_tags(variable_names) -> list:
-    """The tags of the 15 histograms in the order of ga3c_histograms' sources: weights_<var.name> per variable, then the
-    activations as upstream NetworkVP._create_tensor_board names them (n1, n2, d1, logits_v, softmax_p)."""
-    return [clean_tag("weights_" + n) for n in variable_names] + list(ACTIVATION_TAGS)
+def histogram_tags(variable_names, activation_tags=ACTIVATION_TAGS) -> list:
+    """The histogram tags in the order of ga3c_histograms' sources: weights_<var.name> per variable, then the activations,
+    by default the conv net's as upstream NetworkVP._create_tensor_board names them (n1, n2, d1, logits_v, softmax_p)."""
+    return [clean_tag("weights_" + n) for n in variable_names] + list(activation_tags)
+
+
+def mlp_histogram_tags(variables) -> list:
+    """The histogram tags of an MLP network in the order of ga3c_mlp_histograms' sources.  variables: (TF name, live) pairs in
+    creation order (ga3c_mlp_param_info).  weights_<var.name> for every variable, the gradient-less ones included; then
+    activation_<layer scope> for every live hidden layer in forward order (the scope of a live variable outside the heads
+    logits_v / logits_p: dense11_p ... dense1 for the fork NetworkVP, dense1_<n>_p for NetworkVP_discrate); then activation_v
+    (logits_v) and activation_p (softmax_p; for the fork NetworkVP the atan2 output it aliases)."""
+    names = [n for n, _ in variables]
+    scopes = dict.fromkeys(n.split("/")[0] for n, live in variables if live and not n.startswith("logits_"))
+    return histogram_tags(names, [clean_tag("activation_" + s) for s in scopes] + ["activation_v", "activation_p"])
 
 
 def collapse(counts):
@@ -71,7 +82,7 @@ class EventLog:
             except ImportError as e:
                 self._missing = True
                 warnings.warn(f"Network.log writes logs/<model_name>/scalars.csv only: no TensorBoard event file without the "
-                              f"tensorboard package ({e})", RuntimeWarning, stacklevel=3)
+                              f"tensorboard package ({e})", RuntimeWarning, stacklevel=4)   # the caller of log()
             else:
                 self._writer = SummaryWriter(self.logdir)
         if self._writer is None:

@@ -239,6 +239,17 @@ int ga3c_debug_tf32x3_gemm(int32_t mode, const float* a, const float* b, const f
 /* per-kernel event timing, as ga3c_timing_* (kernel ids are shared: ga3c_kernel_name) */
 int ga3c_mlp_timing_enable(ga3c_mlp* net, int32_t max_records);
 int ga3c_mlp_timing_collect(ga3c_mlp* net, double* total_ms, int64_t* counts, int32_t n_kernels);
+/* TensorBoard histograms of an MLP handle (Network.log; the histogram itself is described with ga3c_histograms below).
+ * ga3c_mlp_histogram_count: the number of sources, variables + live hidden layers + 2 (at most 23: fork NetworkVP 16 + 5 + 2,
+ * DISCRATE with 8 DENSE_LAYERS 20 + 1 + 2).  ga3c_mlp_histograms sources, in this order: every variable in ga3c_mlp_param_info
+ * order (the gradient-less DISCRATE ones included), the output of every live hidden layer in forward order as the last forward
+ * on this handle left it (ga3c_mlp_forward_backward / ga3c_mlp_train_step, or a ga3c_mlp_predict of a tensor-core batch,
+ * which writes the same workspace; `batch` must be that forward's batch), then v_dev [B] and p_dev [B, A] (fp32, 16-byte
+ * aligned: what ga3c_mlp_predict wrote for the same rows).  out_dev: ga3c_mlp_histogram_count(net) x (5 + GA3C_HISTO_BUCKETS)
+ * doubles, bad_dev: as many int32.  Launches two kernels, both under kernel id "histograms". */
+int ga3c_mlp_histogram_count(const ga3c_mlp* net);
+int ga3c_mlp_histograms(ga3c_mlp* net, int32_t batch, const float* p_dev, const float* v_dev, double* out_dev,
+                        int32_t* bad_dev, void* stream);
 
 /* ---- serialisation ---------------------------------------------------------------------------------
  * A handle is not re-entrant (one activation workspace).  Whoever drives it from several threads -- the reference calls
@@ -304,7 +315,7 @@ int64_t ga3c_launch_count(const ga3c_net* net);
  * TensorFlow's histogram::Histogram of each source, computed on the device: {min, max, num, sum, sum_squares} in fp64 and the
  * counts of its 1551 default buckets (bucket i holds limit[i-1] <= x < limit[i]; limits: +-1e-12 * 1.1^k up to 1e20, +-DBL_MAX
  * and 0.0).  Deterministic: the same inputs give bit-identical output.  Non-finite values are left out of the statistics and
- * flagged (TF's HistogramSummary refuses them).
+ * flagged (TF's HistogramSummary refuses them).  The MLP networks' entry is ga3c_mlp_histograms (above).
  * ga3c_histograms sources, in this order: the 10 variables (TF creation order), then n1, n2, d1 of the last
  * ga3c_forward_backward[_u8] on this handle (`batch` must be its batch; n1 and n2 as stored, bf16), then v_dev [B] and
  * p_dev [B, A] (fp32, 16-byte aligned: what ga3c_predict wrote for the same frames).  Not available once ga3c_dp_attach* has
