@@ -5,7 +5,7 @@
 //     g_w12 = patches(n1)^T dn2 , g_b12 = colsum(dn2)
 //     g_w11 = patches(x)^T dn1  , g_b11 = colsum(dn1)                  (conv11 has no data-gradient: x is the input)
 // bf16 operands, fp32 accumulation in TMEM; the weight-gradient accumulators stay in TMEM for all frames of the CTA and are
-// stored once into the CTA's slab of the gradient-partial workspace (rmsprop_reduce / dp_tail add the slabs in a fixed order).
+// stored once into the CTA's slab of the gradient-partial workspace (rmsprop_reduce / dp_small add the slabs in a fixed order).
 //
 // Every input arrives in HBM already in the no-swizzle UMMA operand layout it is consumed in (common.cuh): xblk (the bf16
 // block matrix of the frame, written by conv_fwd next to n1), n1 as Blk2, dn2 as G (written by the dense1 data-gradient
@@ -40,20 +40,16 @@
 //                conv11; final store of the TMEM weight-gradient accumulators
 //   warp  11     the 28 live rows of the second data-gradient tile (it shares TMEM lane quarter 3 with warp 7)
 //   warps 3,8-10 bias gradient of conv12 (column sums of G: warp = chunk plane, lane = row phase)
-//   warps 12-15  the optimizer of dense1/w, whose gradient is final since dense_bwd (98.6 % of the parameters): RMSProp + bf16
-//                shadow refresh on a single GPU, the reduce-scatter / RMSProp / all-gather over peer memory when data parallel
-//                (dp_exchange.cuh) -- pure load/store work that rides on issue slots and HBM bandwidth this kernel leaves idle,
-//                so the launch at the end of the step is left with the 58 KB of small tensors
+//   warps 12-15  no work: they go straight to the final block barrier
 #include "common.cuh"
 #include "kernels.h"
 #include "tcgen05.cuh"
 #include "conv_blk.cuh"
-#include "dp_exchange.cuh"
 
 namespace ga3c {
 
 constexpr int FB_THREADS = 512, FB_LOAD_WARP = 0, FB_ISSUE_WARP = 1, FB_C12_WARP = 2, FB_EPI_WARP0 = 4, FB_T1_WARP = 11,
-              FB_OPT_WARP0 = 12, FB_OPT_THREADS = FB_THREADS - 32 * FB_OPT_WARP0;
+              FB_IDLE_WARP0 = 12;
 static_assert(FB_EPI_WARP0 % 4 == 0 && FB_T1_WARP % 4 == 3, "an epilogue warp may only read TMEM lane quarter warp % 4");
 constexpr int FB_RING = 4;                                        // Blk quarter slots: one frame
 constexpr int W11_KSTEPS = 31;                                    // 496 >= 484 block rows
@@ -85,31 +81,18 @@ constexpr int FB_DONE = 15;       //     every UMMA of the kernel retired       
 constexpr int FB_W12DRDY = 16;    //     data-gradient weights laid out, 9 arrivals                        (-> issuer)
 constexpr int FB_NBAR = 17;
 constexpr int FB_OFF_TSLOT = FB_OFF_BAR + FB_NBAR * 8;
-constexpr int FB_OFF_LAST = FB_OFF_TSLOT + 16;                    // one int: "this CTA's optimizer warps finished last" (data parallel)
-constexpr int FB_SMEM = FB_OFF_LAST + 16 + 128;                   // incl. slack to align the base to 128 B
+constexpr int FB_SMEM = FB_OFF_TSLOT + 16 + 128;                  // incl. slack to align the base to 128 B
 static_assert(FB_SMEM <= 232448, "shared memory budget of one CTA per SM");
 constexpr int FB_TMEM_COLS = 512, TM_W11 = 0, TM_W12 = 64, TM_D12 = 192;   // 64 | 2x64 | 2x64 columns
 
-// DPM: 0 single GPU; 1 data parallel, exchange at the end of the step (the default): CTA 0 publishes "dense1/w gradient final" and
-// that is all; 2 data parallel with the exchange inside this launch (exchange CTAs, or the optimizer warps in mode 2).  Separate
-// instantiations: the exchange code costs the conv path 20 registers and a few spills.  EVT: the instantiation with the pipeline
-// event log of CTA 0 (ga3c_evt_*, tools/evt_timeline.py); the production instantiations carry none of it.
-template <int DPM, bool EVT>
+// EVT: the instantiation with the pipeline event log of CTA 0 (ga3c_evt_*, tools/evt_timeline.py); the production
+// instantiation carries none of it.
+template <bool EVT>
 __global__ void __launch_bounds__(FB_THREADS, 1)
 conv_bwd_kernel(const uint8_t* __restrict__ xblk, const uint8_t* __restrict__ n1b2, const uint8_t* __restrict__ dn2g,
                 const float* __restrict__ w12, uint16_t* __restrict__ dn1_out, float* __restrict__ g_w11,
                 float* __restrict__ g_b11, float* __restrict__ g_w12, float* __restrict__ g_b12, int64_t gp_stride, int batch,
-                int n_conv, int hints, const ConvBwdOpt opt, const DpBigArgs dp) {
-  // data parallel, overlapped exchange: CTAs [n_conv, gridDim.x) are exchange CTAs -- they move dense1/w (final since
-  // dense_bwd, the launch this one depends on) between the ranks while CTAs [0, n_conv) compute the conv gradients
-  constexpr bool DP = DPM != 0;
-  if (DPM == 2 && (int)blockIdx.x >= n_conv) {
-    griddep_launch();
-    griddep_wait(K_DP_BIG);
-    dp_big_exchange(dp, (int)blockIdx.x - n_conv, (int)gridDim.x - n_conv);
-    trace_mark(K_DP_BIG, 2);
-    return;
-  }
+                int hints) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t sbase = (smem_u32(smem_raw) + 127u) & ~127u;
   uint8_t* const smem = smem_raw + (sbase - smem_u32(smem_raw));
@@ -119,7 +102,7 @@ conv_bwd_kernel(const uint8_t* __restrict__ xblk, const uint8_t* __restrict__ n1
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   EvtLog evt_i = EVT ? evt_open() : EvtLog{nullptr, 0};
   auto mark = [&](int id, int arg) { if (EVT) evt_mark(evt_i, id, arg); };
-  const int stride = DPM == 2 ? (int)gridDim.x - dp.n_exch : (int)gridDim.x;
+  const int stride = (int)gridDim.x;
   const int n_frames = ((int)blockIdx.x < batch) ? (batch - 1 - (int)blockIdx.x) / stride + 1 : 0;
   auto frame_of = [&](int k) { return (size_t)(blockIdx.x + k * stride); };
   auto bar = [&](int i) { return bars + i * 8; };
@@ -189,13 +172,6 @@ conv_bwd_kernel(const uint8_t* __restrict__ xblk, const uint8_t* __restrict__ n1
   mark(50, 0);
   griddep_wait(K_CONV12_BWD);   // every input comes from the kernels that precede this one
   mark(53, 0);
-  if (DP && opt.mode != 2 && blockIdx.x == 0 && tid < dp.world) {
-    // data parallel: dense_bwd of this rank is complete, i.e. its dense1/w gradient is final -- tell every rank now, a whole
-    // conv backward before the exchange at the end of the step needs it (dp_tail_kernel)
-    __threadfence_system();
-    dp_st_flag(dp.peer[tid] + dp.comm_offset + DPC_BIGREADY + 64 * dp.rank, dp.step);
-  }
-
 
   // Data-gradient epilogue of one 128-row tile for TMEM lane quarter `qt`: rows of the first tile go to warps 4-7, the 28
   // live rows of the second tile (lanes 100..127) to warp 11.
@@ -382,50 +358,8 @@ conv_bwd_kernel(const uint8_t* __restrict__ xblk, const uint8_t* __restrict__ n1
     }
     if (elect_one()) tc_commit(bar(FB_DONE));
     __syncwarp();
-  } else if (warp >= FB_OPT_WARP0) {
-    // =========================== optimizer of dense1/w ===========================
-    const int t = tid - 32 * FB_OPT_WARP0;
-    if (opt.mode == 1) {
-      // single GPU: RMSProp (NetworkVP_discrate.py:101-105 for this variable) + bf16 shadow, float4 i of the tensor on thread
-      // (CTA, t) strided over all conv CTAs; 4 elements (12 loads) in flight per thread
-      const long long stride4 = (long long)n_conv * FB_OPT_THREADS;
-      const float one_m_rho = 1.f - opt.decay;
-      const bool has_mom = opt.momentum != 0.f;
-      const float4* g4 = reinterpret_cast<const float4*>(opt.g);
-      float4* w4 = reinterpret_cast<float4*>(opt.w);
-      float4* ms4 = reinterpret_cast<float4*>(opt.ms);
-      float4* mom4 = reinterpret_cast<float4*>(opt.mom);
-      uint2* sh = reinterpret_cast<uint2*>(opt.shadow);
-      constexpr int U = 4;
-#pragma unroll 1
-      for (long long i0 = (long long)blockIdx.x * FB_OPT_THREADS + t; i0 < opt.n4; i0 += U * stride4) {
-        float4 gv[U], wv[U], mv[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-          const long long i = i0 + u * stride4;
-          if (i < opt.n4) { gv[u] = __ldcg(g4 + i); wv[u] = w4[i]; mv[u] = ms4[i]; }
-        }
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-          const long long i = i0 + u * stride4;
-          if (i >= opt.n4) continue;
-          float4 mo = has_mom ? mom4[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-#define GA3C_RMS(c)                                                          \
-  mv[u].c = opt.decay * mv[u].c + one_m_rho * gv[u].c * gv[u].c;             \
-  mo.c = opt.momentum * mo.c + opt.lr * gv[u].c / sqrtf(mv[u].c + opt.eps);  \
-  wv[u].c -= mo.c;
-          GA3C_RMS(x) GA3C_RMS(y) GA3C_RMS(z) GA3C_RMS(w)
-#undef GA3C_RMS
-          w4[i] = wv[u];
-          ms4[i] = mv[u];
-          if (has_mom) mom4[i] = mo;
-          sh[i] = make_uint2(pack_bf16(wv[u].x, wv[u].y), pack_bf16(wv[u].z, wv[u].w));
-        }
-      }
-    } else if (DPM == 2 && opt.mode == 2) {
-      // data parallel: CTA 0's group publishes "dense_bwd done on this rank", then every group takes its share of the exchange
-      dp_big_group(dp, t, FB_OPT_THREADS, (int)blockIdx.x, n_conv, 4, reinterpret_cast<int*>(smem + FB_OFF_LAST), true);
-    }
+  } else if (warp >= FB_IDLE_WARP0) {
+    // no role: straight to the final barrier (kept out of the "warp >= 8" bias branch below)
   } else if (warp == FB_T1_WARP) {
     // =========================== second data-gradient tile ===========================
     if (!w12d_early) build_w12d();
@@ -534,31 +468,22 @@ int evt_attach_conv_bwd(unsigned long long* buf) {
   return (int)cudaMemcpyToSymbol(g_evt, &buf, sizeof(buf));
 }
 
-int conv_bwd_grid(int batch, int num_sms, int n_exch) { return min(batch, num_sms - n_exch); }
+int conv_bwd_grid(int batch, int num_sms) { return min(batch, num_sms); }
 
 int configure_conv_bwd_fused() {
-  cudaError_t e = cudaFuncSetAttribute(conv_bwd_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FB_SMEM);
+  cudaError_t e = cudaFuncSetAttribute(conv_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FB_SMEM);
   if (e != cudaSuccess) return (int)e;
-  e = cudaFuncSetAttribute(conv_bwd_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FB_SMEM);
-  if (e != cudaSuccess) return (int)e;
-  e = cudaFuncSetAttribute(conv_bwd_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FB_SMEM);
-  if (e != cudaSuccess) return (int)e;
-  return (int)cudaFuncSetAttribute(conv_bwd_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FB_SMEM);
+  return (int)cudaFuncSetAttribute(conv_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FB_SMEM);
 }
 
 int launch_conv_bwd(const uint8_t* xblk, const uint8_t* n1b2, const uint8_t* dn2g, const float* w12, uint16_t* dn1_out,
                     float* g_w11, float* g_b11, float* g_w12, float* g_b12, int64_t gp_stride, int batch, int num_sms, bool x_u8,
-                    const ConvBwdOpt& opt, const DpBigArgs* dp, cudaStream_t stream) {
-  DpBigArgs d{};
-  if (dp != nullptr) d = *dp;
-  const int n_conv = conv_bwd_grid(batch, num_sms, d.n_exch);
-  const dim3 grid(n_conv + d.n_exch);
+                    cudaStream_t stream) {
+  const dim3 grid(conv_bwd_grid(batch, num_sms));
   if (grid.x == 0) return 0;
-  if (opt.mode == 2 && (dp == nullptr || n_conv == 0)) return (int)cudaErrorInvalidValue;
-  auto kernel = dp != nullptr ? ((d.n_exch > 0 || opt.mode == 2) ? conv_bwd_kernel<2, false> : conv_bwd_kernel<1, false>)
-                              : (g_evt_attached ? conv_bwd_kernel<0, true> : conv_bwd_kernel<0, false>);
+  auto kernel = g_evt_attached ? conv_bwd_kernel<true> : conv_bwd_kernel<false>;
   return launch_pdl(kernel, grid, dim3(FB_THREADS), FB_SMEM, stream, xblk, n1b2, dn2g, w12, dn1_out, g_w11, g_b11, g_w12, g_b12,
-                    gp_stride, batch, n_conv, l2_hints(true, x_u8) | (batch >= num_sms ? 8 : 0), opt, d);
+                    gp_stride, batch, l2_hints(true, x_u8) | (batch >= num_sms ? 8 : 0));
 }
 
 }  // namespace ga3c

@@ -58,43 +58,6 @@ struct EpiPartialF32 {      // raw fp32 tile into part[split][M][N]  (bias + rel
                            __uint_as_float(r[4 * i + 3]));
   }
 };
-// The dense1/w gradient tile of the fused backward launch (one thread = one row of dense1/w, 32 consecutive columns).  Data parallel
-// (push.world > 1): a float4 of a slice this rank does not own is PUSHED into the owner's receive buffer in the LL wire format
-// (dp_exchange.cuh) instead of being stored locally -- a whole conv backward before the owner needs it, so the exchange at the end
-// of the step finds every contribution in its own HBM and never waits for a load across NVLink.
-struct EpiWgradPush {
-  float* out; int ldc;
-  WgradPush push;
-  struct Pre {};
-  __device__ __forceinline__ void prefetch(Pre&, int, int, bool) const {}
-  __device__ __forceinline__ void operator()(const Pre&, int, int m, int n, const uint32_t (&r)[32]) const {
-    const size_t e0 = (size_t)m * ldc + n;
-    if (push.world <= 1) {
-      float4* dst = reinterpret_cast<float4*>(out + e0);
-#pragma unroll
-      for (int i = 0; i < 8; ++i)
-        dst[i] = make_float4(__uint_as_float(r[4 * i]), __uint_as_float(r[4 * i + 1]), __uint_as_float(r[4 * i + 2]),
-                             __uint_as_float(r[4 * i + 3]));
-      return;
-    }
-    const long long i4 = (long long)(e0 >> 2);
-    const int q0 = (int)(i4 / push.per4), q1 = (int)((i4 + 7) / push.per4);       // 8 float4: at most two owners
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      const float4 gv = make_float4(__uint_as_float(r[4 * i]), __uint_as_float(r[4 * i + 1]), __uint_as_float(r[4 * i + 2]),
-                                    __uint_as_float(r[4 * i + 3]));
-      const int q = (q0 == q1 || i4 + i < (long long)q1 * push.per4) ? q0 : q1;
-      if (q == push.rank) {
-        reinterpret_cast<float4*>(out + e0)[i] = gv;             // this rank owns the slice: its own contribution stays local
-      } else {
-        uint8_t* dst = push.peer[q] + push.recv_off +
-                       (((long long)(push.flag & 1u) * push.world + push.rank) * push.per4 + (i4 + i - (long long)q * push.per4)) * 32;
-        dp_ll_store(dst, gv, push.flag);
-      }
-    }
-  }
-};
-
 struct EpiReluMaskBf16Tc {  // dn2 = acc where n2 > 0 else 0, bf16, stored in the G operand layout the conv backward consumes (common.cuh)
   uint8_t* out; const uint16_t* act; int ldc;
   struct Pre { uint4 a[4]; };     // this thread's 32 activations: fetched while the MMAs are still running
@@ -274,7 +237,7 @@ constexpr int WGM_ST = 3;                   // wgrad inside the merged launch: 3
 struct DenseBwdArgs {
   int batch, dg_mtiles, n_dg, wg_mtiles, wg_kblocks;
   EpiReluMaskBf16Tc epi_dg;
-  EpiWgradPush epi_wg;
+  EpiPartialF32 epi_wg;
 };
 __global__ void __launch_bounds__(TC_THREADS, 3)     // <= 96 registers: 18 warps fit the four 16K register files
 dense_bwd_kernel(const __grid_constant__ CUtensorMap dg_a, const __grid_constant__ CUtensorMap dg_b,
@@ -285,8 +248,8 @@ dense_bwd_kernel(const __grid_constant__ CUtensorMap dg_a, const __grid_constant
                                                                 p.epi_dg, b % p.dg_mtiles, b / p.dg_mtiles, 0);
   } else {
     const int t = b - p.n_dg;
-    gemm_tc_body<WG_BN, WGM_ST, true, true, EpiWgradPush>(wg_a, wg_b, (int)FLAT, (int)FC, p.wg_kblocks, p.wg_kblocks,
-                                                          p.epi_wg, t % p.wg_mtiles, t / p.wg_mtiles, 0);
+    gemm_tc_body<WG_BN, WGM_ST, true, true, EpiPartialF32>(wg_a, wg_b, (int)FLAT, (int)FC, p.wg_kblocks, p.wg_kblocks,
+                                                           p.epi_wg, t % p.wg_mtiles, t / p.wg_mtiles, 0);
   }
 }
 
@@ -324,10 +287,6 @@ static int make_tmap(CUtensorMap* map, const void* base, uint64_t rows, uint64_t
                                       estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? 0 : (int)cudaErrorInvalidValue;
-}
-
-int make_tmap_bf16(CUtensorMap* map, const void* base, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows) {
-  return make_tmap(map, base, rows, cols, ld, box_rows);       // for dense_heads.cu
 }
 
 template <int BN, int STAGES>
@@ -420,7 +379,7 @@ int launch_dense_wgrad_tc(const uint16_t* n2, const uint16_t* dd1, float* g_w1, 
 }
 
 int launch_dense_bwd_tc(const uint16_t* dd1, const uint16_t* w1bf, const uint16_t* n2, uint8_t* dn2, float* g_w1, int batch,
-                        const WgradPush* push, cudaStream_t stream) {
+                        cudaStream_t stream) {
   CUtensorMap da, db, wa, wb;
   if (make_tmap(&da, dd1, batch, FC, FC, TC_BM)) return (int)cudaErrorInvalidValue;           // dgrad A: [B][256], K inner
   if (make_tmap(&db, w1bf, FLAT, FC, FC, DG_BN)) return (int)cudaErrorInvalidValue;           // dgrad B: [3872][256] = [N][K]
@@ -433,9 +392,7 @@ int launch_dense_bwd_tc(const uint16_t* dd1, const uint16_t* w1bf, const uint16_
   p.wg_mtiles = (FLAT + TC_BM - 1) / TC_BM;
   p.wg_kblocks = (batch + TC_BK - 1) / TC_BK;
   p.epi_dg = EpiReluMaskBf16Tc{dn2, n2, FLAT};
-  p.epi_wg.out = g_w1; p.epi_wg.ldc = FC;
-  if (push) p.epi_wg.push = *push;
-  else p.epi_wg.push.world = 1;
+  p.epi_wg = EpiPartialF32{g_w1, FC, 0};
   const int grid = p.n_dg + p.wg_mtiles * (FC / WG_BN);
   return launch_pdl(dense_bwd_kernel, dim3(grid), dim3(TC_THREADS), DBW_SMEM, stream, da, db, wa, wb, p);
 }

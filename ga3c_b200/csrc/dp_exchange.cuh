@@ -1,17 +1,17 @@
 // Data-parallel exchange over CUDA-IPC peer memory (one process per GPU, NVLink / NVSwitch loads and stores).
 //
 // The step's gradients become final in two instalments, and so does the exchange:
-//   dense1/w (98.6 % of the bytes) is final after dense_bwd.  A few extra CTAs of the conv backward launch ("exchange
-//       CTAs", dp_big_exchange below) reduce-scatter it, apply RMSProp to the owned slice and all-gather the new fp32
-//       weights + bf16 shadow into every rank's slab WHILE the other CTAs of the same launch compute the conv gradients.
-//       Only the bf16 shadow (what dense_fwd / dense_bwd read) travels: the fp32 master copy and the ms slot of a slice
-//       live on its owner, and ga3c_arena_download collects the owners' slices when the host asks for the weights.
+//   dense1/w (98.6 % of the bytes) is final after dense_bwd.  dp_big_side_kernel (elementwise.cu), launched on a side stream
+//       behind dense_bwd, reduce-scatters it, applies RMSProp to the owned slice and all-gathers the bf16 shadow into every
+//       rank's slab WHILE the conv backward of this step and the conv forward of the next run on the main stream.  Only the
+//       bf16 shadow (what dense_fwd / dense_bwd read) travels: the fp32 master copy and the ms slot of a slice live on its
+//       owner, and ga3c_arena_download collects the owners' slices when the host asks for the weights.  dense_fwd of the next
+//       step waits for every rank's "slice landed" flag before it reads the shadow (DpGate, dense_tc.cu).
 //   the small tensors (conv11 / conv12 / dense1 bias / heads, 58 KB) are final after the conv backward.  dp_small_kernel
 //       (elementwise.cu) sums this rank's per-CTA slabs and PUSHES the sums into every rank's receive buffer with the
 //       step number packed into every 8 bytes ({value, flag} pairs, the "LL" wire format: an 8-byte store lands whole,
 //       so data that carries the expected flag is valid -- no fence, no separate flag, one NVLink one-way trip).  Every
 //       rank adds the contributions in rank order and applies the identical update locally; nothing is written back.
-//       The kernel then holds the launch open until every rank's dense1/w slice has landed.
 // Flags are monotonically increasing step numbers PUSHED into every rank's comm block; a waiter only polls its own HBM.
 #pragma once
 #include "common.cuh"
@@ -20,17 +20,12 @@ namespace ga3c {
 
 constexpr int DP_WORLD_MAX = 8;
 // comm block layout (bytes from comm_offset)
-constexpr int DPC_READY = 0;          // [8] x 64 B   single-kernel exchange (rmsprop_dp_kernel): gradients final
-constexpr int DPC_DONE = 512;         // [8] x 64 B   single-kernel exchange: slice stored everywhere
-constexpr int DPC_CTR_DONE = 1024;    // u32 block counters of this rank's own grids
-constexpr int DPC_CTR_RED = 1028;
-constexpr int DPC_CTR_BIG = 1032;
+constexpr int DPC_CTR_BIG = 1032;     // u32 block counter of this rank's own dense1/w exchange grid
 constexpr int DPC_ERR = 1040;         // u32: set when a wait gave up (a rank died or fell out of step): ga3c_dp_error
 constexpr int DPC_BIGREADY = 2048;    // [8] x 64 B   dense_bwd of the step complete on rank r
 constexpr int DPC_BIGDONE = 2560;     // [8] x 64 B   rank r's dense1/w slice stored everywhere
-constexpr int DPC_CB = 4096;          // [8][DP_MAX_CB] u64: column block cb of rank r's small gradients published
-constexpr int DP_MAX_CB = 256;
-constexpr int DP_COMM_BYTES = DPC_CB + DP_WORLD_MAX * DP_MAX_CB * 8;
+constexpr int DP_COMM_BYTES = DPC_BIGDONE + DP_WORLD_MAX * 64;
+constexpr int DP_MAX_CB = 256;        // column blocks of the small tensors (blocks of dp_small_kernel)
 
 __device__ __forceinline__ uint64_t dp_ld_flag(const void* p) {
   uint64_t v;
@@ -45,8 +40,7 @@ __device__ __forceinline__ void dp_st_flag(void* p, uint64_t v) {
 // number of times must not hold the others' GPUs for ever.  On expiry the waiter raises the error word of its own comm block and carries on;
 // the host sees it through ga3c_dp_error (results of that step are garbage).
 constexpr unsigned int DP_SPIN_LIMIT = 1u << 25;
-// error bits: 1 "gradients ready" (single-kernel exchange), 2 "done" (single-kernel), 4 dense_bwd-done flags of the
-// exchange CTAs, 8 small-tensor LL data, 16 dense1/w slices landed
+// error bits: 4 dense_bwd-done flags of the dense1/w exchange, 8 small-tensor LL data, 16 dense1/w slices landed
 __device__ __forceinline__ void dp_wait_flag(const void* p, unsigned long long want, void* err, unsigned int bit) {
   for (unsigned int i = 0; dp_ld_flag(p) < want; ++i)
     if (i > DP_SPIN_LIMIT) { atomicOr(static_cast<unsigned int*>(err), bit); break; }
@@ -86,16 +80,10 @@ __device__ __forceinline__ float4 dp_ld_f4(const float4* p) {      // L2 (the ow
 struct DpBigArgs {
   uint8_t* peer[DP_WORLD_MAX];      // slab bases: [params | grads | ms | mom | shadow | LL receive buffers | comm]
   int rank, world;
-  int n_exch;                       // exchange CTAs appended to the conv backward grid (0: data parallel off)
   unsigned long long step;
   long long arena_bytes, shadow_off, comm_offset;
   long long w1_offset, w1_count;    // dense1/w inside the arena, in floats (multiples of 4)
   float lr, decay, momentum, eps;
-  // pushed != 0: the peers' gradient slices were pushed into this rank's receive buffers by their dense1 wgrad epilogues
-  // (dense_tc.cu EpiWgradPush): [2 parities][world][per float4 in LL format] at bigrecv_off of the slab.  The reduce reads
-  // local memory only and needs no "gradient final" flags.
-  int pushed;
-  long long bigrecv_off;
 };
 
 // reduce-scatter + RMSProp + all-gather over float4 indices [lo, hi) of dense1/w, strided over the exchange CTAs.  The loop is
@@ -149,97 +137,18 @@ __device__ __forceinline__ void dp_big_loop(const DpBigArgs& d, long long lo, lo
   }
 }
 
-// one attempt at an LL float4: true when all four flags carry `flag`
-__device__ __forceinline__ bool dp_ll_try(const void* src, uint32_t flag, float4& v) {
-  uint32_t a0, f0, a1, f1, a2, f2, a3, f3;
-  asm volatile("ld.relaxed.sys.global.v4.b32 {%0,%1,%2,%3}, [%4];\n" : "=r"(a0), "=r"(f0), "=r"(a1), "=r"(f1) : "l"(src) : "memory");
-  asm volatile("ld.relaxed.sys.global.v4.b32 {%0,%1,%2,%3}, [%4];\n" : "=r"(a2), "=r"(f2), "=r"(a3), "=r"(f3)
-               : "l"(static_cast<const uint8_t*>(src) + 16) : "memory");
-  v = make_float4(__uint_as_float(a0), __uint_as_float(a1), __uint_as_float(a2), __uint_as_float(a3));
-  return f0 == flag && f1 == flag && f2 == flag && f3 == flag;
-}
-
-// dp_big_loop with the peers' contributions taken from the LOCAL receive buffers they were pushed into (DpBigArgs::pushed)
-template <int W, int U>
-__device__ __forceinline__ void dp_big_loop_pushed(const DpBigArgs& d, long long lo, long long hi, long long first, long long stride) {
-  const long long base4 = d.w1_offset >> 2;
-  const float one_m_rho = 1.f - d.decay;
-  uint8_t* mine = d.peer[d.rank];
-  float4* w_own = reinterpret_cast<float4*>(mine) + base4;
-  float4* g_own = reinterpret_cast<float4*>(mine + d.arena_bytes) + base4;
-  float4* ms_own = reinterpret_cast<float4*>(mine + 2 * d.arena_bytes) + base4;
-  float4* mom_own = reinterpret_cast<float4*>(mine + 3 * d.arena_bytes) + base4;
-  const bool has_mom = d.momentum != 0.f;
-  constexpr int NW = W > 0 ? W : DP_WORLD_MAX;
-  const long long per = hi - lo > 0 ? ((d.w1_count >> 2) + d.world - 1) / d.world : 1;
-  const uint32_t flag = (uint32_t)d.step;
-  const uint8_t* recv = mine + d.bigrecv_off + (long long)(d.step & 1) * d.world * per * 32;
-  for (long long i0 = lo + first; i0 < hi; i0 += U * stride) {
-    float4 q[U][NW], w[U], ms[U];
-    bool ok[U][NW];
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      const long long i = i0 + u * stride;
-#pragma unroll
-      for (int r = 0; r < NW; ++r) {
-        ok[u][r] = true;
-        q[u][r] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (i < hi && (W > 0 || r < d.world)) {
-          if (r == d.rank) q[u][r] = dp_ld_f4(g_own + i);
-          else ok[u][r] = dp_ll_try(recv + ((long long)r * per + (i - lo)) * 32, flag, q[u][r]);
-        }
-      }
-      if (i < hi) { w[u] = w_own[i]; ms[u] = ms_own[i]; }
-    }
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      const long long i = i0 + u * stride;
-      if (i >= hi) continue;
-#pragma unroll
-      for (int r = 0; r < NW; ++r)            // normally every contribution arrived long ago; otherwise wait for it (bounded)
-        if (!ok[u][r]) q[u][r] = dp_ll_load(recv + ((long long)r * per + (i - lo)) * 32, flag, mine + d.comm_offset + DPC_ERR);
-      float4 g = q[u][0];
-#pragma unroll
-      for (int r = 1; r < NW; ++r) { g.x += q[u][r].x; g.y += q[u][r].y; g.z += q[u][r].z; g.w += q[u][r].w; }   // rank order
-      float4 mo = has_mom ? mom_own[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-#define GA3C_RMS(c)                                                          \
-  ms[u].c = d.decay * ms[u].c + one_m_rho * g.c * g.c;                       \
-  mo.c = d.momentum * mo.c + d.lr * g.c / sqrtf(ms[u].c + d.eps);            \
-  w[u].c -= mo.c;
-      GA3C_RMS(x) GA3C_RMS(y) GA3C_RMS(z) GA3C_RMS(w)
-#undef GA3C_RMS
-      ms_own[i] = ms[u];
-      if (has_mom) mom_own[i] = mo;
-      g_own[i] = g;                    // the reduced gradient of the owned slice (introspection)
-      const uint2 sh = make_uint2(pack_bf16(w[u].x, w[u].y), pack_bf16(w[u].z, w[u].w));
-      w_own[i] = w[u];
-#pragma unroll
-      for (int r = 0; r < NW; ++r)
-        if (W > 0 || r < d.world) reinterpret_cast<uint2*>(d.peer[r] + d.shadow_off)[i] = sh;
-    }
-  }
-}
-
-// The same exchange on a GROUP of `nthreads` threads of a block (thread t of the group, named barrier `bar_id`): the spare warps
-// of every conv backward CTA (conv_bwd_fused.cu) or half of every block of the tail kernel (dp_tail_kernel).  `cta` / `n_cta`:
-// index and number of the groups that share the work; last_smem: one int of shared memory.  Ends with the rank's "slice landed
-// everywhere" flag pushed by the last group to finish.  Waits with acquire loads, no fence between the two flag hops.
-template <bool PUSH_CAPABLE = true>      // false: compiled without the pushed-slices variant (leaner: the side-stream kernel)
-__device__ __forceinline__ void dp_big_group(const DpBigArgs& d, int t, int nthreads, int cta, int n_cta, int bar_id, int* last_smem,
-                                             bool push_ready) {
+// The whole exchange on a GROUP of `nthreads` threads (thread t of the group, named barrier `bar_id`).  `cta` / `n_cta`: index and
+// number of the groups that share the work; last_smem: one int that only thread 0 uses.  Group 0 publishes "dense_bwd done on
+// this rank" (the dense1/w gradient is final by stream order), every group waits for every rank's, takes its share of the loop,
+// and the last group to finish pushes the rank's "slice landed everywhere" flag.  Waits with acquire loads, no fence between the
+// two flag hops.
+__device__ __forceinline__ void dp_big_group(const DpBigArgs& d, int t, int nthreads, int cta, int n_cta, int bar_id, int* last_smem) {
   uint8_t* my_comm = d.peer[d.rank] + d.comm_offset;
   const long long n4 = d.w1_count >> 2;
   const long long per = (n4 + d.world - 1) / d.world;
   const long long lo = per * d.rank, hi = lo + per < n4 ? lo + per : n4;
   const long long stride = (long long)n_cta * nthreads, first = (long long)cta * nthreads + t;
-  if (PUSH_CAPABLE && d.pushed) {
-    // the peers' slices sit in this rank's receive buffers, every float4 carrying the step number: nothing to wait for here
-    if (d.world == 2) dp_big_loop_pushed<2, 4>(d, lo, hi, first, stride);
-    else if (d.world == 4) dp_big_loop_pushed<4, 2>(d, lo, hi, first, stride);
-    else if (d.world == 8) dp_big_loop_pushed<8, 1>(d, lo, hi, first, stride);
-    else dp_big_loop_pushed<0, 1>(d, lo, hi, first, stride);
-  } else {
-  if (push_ready && cta == 0 && t < d.world) {
+  if (cta == 0 && t < d.world) {
     __threadfence_system();
     dp_st_flag(d.peer[t] + d.comm_offset + DPC_BIGREADY + 64 * d.rank, d.step);
   }
@@ -249,7 +158,6 @@ __device__ __forceinline__ void dp_big_group(const DpBigArgs& d, int t, int nthr
   else if (d.world == 4) dp_big_loop<4, 2>(d, lo, hi, first, stride);
   else if (d.world == 8) dp_big_loop<8, 1>(d, lo, hi, first, stride);
   else dp_big_loop<0, 1>(d, lo, hi, first, stride);
-  }
   asm volatile("bar.sync %0, %1;\n" ::"r"(bar_id), "r"(nthreads) : "memory");
   if (t == 0) {
     __threadfence_system();            // cumulative over the group's peer stores (observed through the barrier)
@@ -261,43 +169,6 @@ __device__ __forceinline__ void dp_big_group(const DpBigArgs& d, int t, int nthr
       for (int r = 0; r < d.world; ++r) dp_st_flag(d.peer[r] + d.comm_offset + DPC_BIGDONE + 64 * d.rank, d.step);
     }
   }
-}
-
-// Body of an exchange CTA (512 threads).  Called after griddepcontrol.wait: dense_bwd of this rank is complete, i.e. its
-// dense1/w gradient is final and nothing on this rank reads dense1/w or its shadow again before the next forward.
-__device__ __forceinline__ void dp_big_exchange(const DpBigArgs& d, int cta, int n_cta, EvtLog* evt = nullptr) {
-  __shared__ int dp_last;
-  const int tid = threadIdx.x;
-  uint8_t* my_comm = d.peer[d.rank] + d.comm_offset;
-  if (cta == 0 && tid < d.world) dp_st_flag(d.peer[tid] + d.comm_offset + DPC_BIGREADY + 64 * d.rank, d.step);
-  if (tid < d.world) {
-    dp_wait_flag(my_comm + DPC_BIGREADY + 64 * tid, d.step, my_comm + DPC_ERR, 4u);
-    __threadfence_system();
-  }
-  __syncthreads();
-  if (evt) evt_mark(*evt, 70, 0);
-
-  const long long n4 = d.w1_count >> 2;
-  const long long per = (n4 + d.world - 1) / d.world;
-  const long long lo = per * d.rank, hi = lo + per < n4 ? lo + per : n4;
-  const long long stride = (long long)n_cta * blockDim.x, first = (long long)cta * blockDim.x + tid;
-  if (d.world == 2) dp_big_loop<2, 4>(d, lo, hi, first, stride);
-  else if (d.world == 4) dp_big_loop<4, 2>(d, lo, hi, first, stride);
-  else if (d.world == 8) dp_big_loop<8, 1>(d, lo, hi, first, stride);
-  else dp_big_loop<0, 1>(d, lo, hi, first, stride);
-  if (evt) evt_mark(*evt, 71, 0);
-  __syncthreads();
-  if (tid == 0) {
-    __threadfence_system();            // cumulative over the block's peer stores (observed through the barrier)
-    unsigned int* ctr = reinterpret_cast<unsigned int*>(my_comm + DPC_CTR_BIG);
-    dp_last = atomicAdd(ctr, 1u) == (unsigned int)n_cta - 1;
-    if (dp_last) {
-      *ctr = 0;
-      __threadfence_system();
-      for (int r = 0; r < d.world; ++r) dp_st_flag(d.peer[r] + d.comm_offset + DPC_BIGDONE + 64 * d.rank, d.step);
-    }
-  }
-  if (evt) evt_mark(*evt, 72, 0);
 }
 
 }  // namespace ga3c

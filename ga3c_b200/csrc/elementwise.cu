@@ -8,10 +8,6 @@
 
 namespace ga3c {
 
-__device__ __forceinline__ void named_bar_sync_ew(int id, int nthreads) {
-  asm volatile("bar.sync %0, %1;\n" ::"r"(id), "r"(nthreads) : "memory");
-}
-
 // ---- gradient-partial reduction ---------------------------------------------------------------------
 // The heads / conv12_bwd / conv11_wgrad kernels leave one slab of partial sums per CTA (a mirror of the small-tensor
 // prefix of the gradient arena + the loss sums).  512 threads = 16 slab lanes x 32 float4 columns: lane l adds slabs
@@ -391,216 +387,44 @@ int launch_rmsprop_reduce(const RmsPropArgs& a, const GradReduceArgs& r, cudaStr
   return launch_pdl(rmsprop_reduce_kernel<false>, dim3(grid), dim3(T), 0, stream, a, r, n_red);
 }
 
-// ---- data-parallel RMSProp over peer memory ---------------------------------------------------------
-// reduce-scatter(gradients) -> RMSProp on the owned slice -> all-gather(weights), fused in ONE kernel:
-// the gradient slice is read from every rank's slab with plain loads through NVLink (P2P mappings), the
-// updated fp32 weights and the bf16 shadow of dense1/w are stored into every rank's slab.  Cross-rank
-// ordering uses two monotonically increasing step flags per rank, PUSHED into every rank's slab (a waiter polls its own
-// HBM; polling a peer's slab costs an NVLink round trip per probe):
-//   ready[r] = s  "rank r's gradients of step s are final"        stored when r's kernel starts (it is stream-ordered
-//                                                                   after r's backward); every block waits for all ranks
-//   done[r]  = s  "rank r's slice of step s is stored everywhere"  stored by the LAST block of r's grid to finish, which
-//                                                                   then waits for every rank's done before the kernel ends,
-//                                                                   so the next forward (stream-ordered) sees all slices
-// No block waits on another block of its own grid, so progress does not depend on co-residency.
-// comm block layout (bytes): [64 r] ready[r] u64, [512 + 64 r] done[r] u64, [1024] finished-block counter u32, [1028] the
-// slab-reduction phase's counter
-__device__ __forceinline__ uint64_t ld_flag(const uint64_t* p) {
-  uint64_t v;
-  asm volatile("ld.relaxed.sys.global.u64 %0, [%1];\n" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void st_flag(uint64_t* p, uint64_t v) {
-  asm volatile("st.relaxed.sys.global.u64 [%0], %1;\n" ::"l"(p), "l"(v) : "memory");
-}
-
-template <bool HAS_MOM>
-__global__ void __launch_bounds__(512) rmsprop_dp_kernel(RmsPropDpArgs d) {
-  const RmsPropArgs& a = d.base;
-  EvtLog evt_i = evt_open();                                      // pipeline event log of CTA 0 (ga3c_evt_*), off unless attached
-  griddep_launch();
-  evt_mark(evt_i, 60, 0);
-  griddep_wait(K_RMSPROP);      // the gradients come from the backward kernels that precede this one
-  evt_mark(evt_i, 61, 0);
-  uint8_t* my_comm = d.peer[d.rank] + d.comm_offset;
-  if (d.has_red) {
-    // phase 0: this rank's slabs -> its gradient arena (same order and bits as grad_reduce_kernel); the block that
-    // finishes last publishes "ready"
-    __shared__ float4 part[GR_LANES][GR_COLS];
-    __shared__ int last_red;
-    const GradReduceArgs& r = d.red;
-    const int col = threadIdx.x & (GR_COLS - 1), sl = threadIdx.x / GR_COLS;
-    const int n_cb = (r.n_floats / 4 + GR_COLS - 1) / GR_COLS;
-    for (int cb = blockIdx.x; cb < n_cb; cb += gridDim.x) {
-      const int j = (cb * GR_COLS + col) * 4;
-      int count = 0;
-      if (j < r.n_floats) {
-#pragma unroll
-        for (int s = GR_MAX_SEG - 1; s >= 0; --s)
-          if (j < r.seg_end[s]) count = r.seg_count[s];
-      }
-      float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-      const float* src = r.part + j;
-      for (int i0 = sl; i0 < count; i0 += GR_UNROLL * GR_LANES) {
-        float4 q[GR_UNROLL];
-#pragma unroll
-        for (int u = 0; u < GR_UNROLL; ++u) {
-          const int i = i0 + u * GR_LANES;
-          q[u] = i < count ? __ldcg(reinterpret_cast<const float4*>(src + (int64_t)i * r.stride)) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-#pragma unroll
-        for (int u = 0; u < GR_UNROLL; ++u) { acc.x += q[u].x; acc.y += q[u].y; acc.z += q[u].z; acc.w += q[u].w; }
-      }
-      part[sl][col] = acc;
-      __syncthreads();
-      if (sl == 0 && j < r.n_floats) {
-#pragma unroll
-        for (int l = 1; l < GR_LANES; ++l) {
-          const float4 q = part[l][col];
-          acc.x += q.x; acc.y += q.y; acc.z += q.z; acc.w += q.w;
-        }
-        if (j < r.out_floats) *reinterpret_cast<float4*>(r.out + j) = acc;
-        else if (r.out_tail != nullptr) {
-          float* t = r.out_tail + (j - r.out_floats);
-          t[0] = acc.x; t[1] = acc.y; t[2] = acc.z; t[3] = acc.w;
-        }
-      }
-      __syncthreads();
-    }
-    if (threadIdx.x == 0) {
-      __threadfence_system();          // the reduced gradients are read by the peers
-      unsigned int* ctr = reinterpret_cast<unsigned int*>(my_comm + DPC_CTR_RED);
-      last_red = atomicAdd(ctr, 1u) == gridDim.x - 1;
-      if (last_red) {
-        *ctr = 0;
-        __threadfence_system();
-        for (int r = 0; r < d.world; ++r)                            // my gradients are final
-          st_flag(reinterpret_cast<uint64_t*>(d.peer[r] + d.comm_offset + 64 * d.rank), d.step);
-      }
-    }
-  } else if (blockIdx.x == 0 && (int)threadIdx.x < d.world) {
-    st_flag(reinterpret_cast<uint64_t*>(d.peer[threadIdx.x] + d.comm_offset + 64 * d.rank), d.step);   // my gradients are final
-  }
-  if ((int)threadIdx.x < d.world) {
-    dp_wait_flag(my_comm + DPC_READY + 64 * threadIdx.x, d.step, my_comm + DPC_ERR, 1u);
-    __threadfence_system();
-  }
-  __syncthreads();
-  evt_mark(evt_i, 62, 0);
-
-  const int64_t n4 = a.n_floats >> 2;
-  const int64_t per = (n4 + d.world - 1) / d.world;
-  const int64_t lo = per * d.rank, hi = lo + per < n4 ? lo + per : n4;
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  const float one_m_rho = 1.f - a.decay;
-  const int64_t g_off = d.arena_bytes, shadow_off = 4 * d.arena_bytes;
-  for (int64_t i = lo + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < hi; i += stride) {
-    float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-    for (int r = 0; r < DP_MAX_WORLD; ++r) {
-      if (r < d.world) {
-        const float4 q = reinterpret_cast<const float4*>(d.peer[r] + g_off)[i];
-        g.x += q.x; g.y += q.y; g.z += q.z; g.w += q.w;
-      }
-    }
-    float4 w = reinterpret_cast<float4*>(a.w)[i];
-    float4 ms = reinterpret_cast<float4*>(a.ms)[i];
-    float4 mo = HAS_MOM ? reinterpret_cast<float4*>(a.mom)[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-#define GA3C_RMS(c)                                                          \
-  ms.c = a.decay * ms.c + one_m_rho * g.c * g.c;                             \
-  mo.c = a.momentum * mo.c + a.lr * g.c / sqrtf(ms.c + a.eps);              \
-  w.c -= mo.c;
-    GA3C_RMS(x) GA3C_RMS(y) GA3C_RMS(z) GA3C_RMS(w)
-#undef GA3C_RMS
-    reinterpret_cast<float4*>(a.ms)[i] = ms;
-    if (HAS_MOM) reinterpret_cast<float4*>(a.mom)[i] = mo;
-    reinterpret_cast<float4*>(const_cast<float*>(a.g))[i] = g;       // the reduced gradient of the owned slice (introspection)
-    const int64_t e = i << 2;
-    const bool in_w1 = e >= a.w1_offset && e < a.w1_offset + a.w1_count;
-    const uint2 sh = make_uint2(pack_bf16(w.x, w.y), pack_bf16(w.z, w.w));
-#pragma unroll
-    for (int r = 0; r < DP_MAX_WORLD; ++r) {
-      if (r < d.world) {
-        reinterpret_cast<float4*>(d.peer[r])[i] = w;
-        if (in_w1) reinterpret_cast<uint2*>(d.peer[r] + shadow_off)[(e - a.w1_offset) >> 2] = sh;
-      }
-    }
-  }
-
-  // publish "done" once the whole grid has stored its part, then hold the kernel open until every rank is done
-  __shared__ int last;
-  evt_mark(evt_i, 63, 0);
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    __threadfence_system();            // cumulative: orders the block's peer stores (observed through the barrier)
-    evt_mark(evt_i, 64, 0);
-    unsigned int* ctr = reinterpret_cast<unsigned int*>(my_comm + DPC_CTR_DONE);
-    last = atomicAdd(ctr, 1u) == gridDim.x - 1;
-    if (last) {
-      *ctr = 0;
-      __threadfence_system();
-      for (int r = 0; r < d.world; ++r)
-        st_flag(reinterpret_cast<uint64_t*>(d.peer[r] + d.comm_offset + DPC_DONE + 64 * d.rank), d.step);
-    }
-  }
-  __syncthreads();
-  if (last && (int)threadIdx.x < d.world) {
-    dp_wait_flag(my_comm + DPC_DONE + 64 * threadIdx.x, d.step, my_comm + DPC_ERR, 2u);
-    __threadfence_system();
-  }
-  if (last) evt_mark(evt_i, 65, blockIdx.x);
-  trace_mark(K_RMSPROP, 2);
-}
-
 GA3C_EVT_ATTACH(evt_attach_elementwise)
 
-// ---- overlapped data-parallel exchange, second instalment (dp_exchange.cuh) ---------------------------------
+// ---- data-parallel exchange, small tensors (dp_exchange.cuh) ---------------------------------------------
 // One block per 32-float4 column block of the small-tensor prefix (+ the loss sums).  Block cb sums this rank's per-CTA
 // slabs for its columns (same order and bits as grad_reduce_kernel); its 32 owner threads push the sums into every peer's
 // receive buffer in the LL wire format, collect the peers' contributions from this rank's own receive buffer, add them in
 // rank order (every rank computes the identical sum) and apply RMSProp to the local copy.  Receive buffers alternate with
 // the step parity: a peer pushes step s + 2 only after it has seen this rank's step s + 1, i.e. after this rank's step-s
-// launch has ended.  Block 0 keeps the launch open until every rank's dense1/w slice (exchange CTAs of the conv backward
-// launch) has landed.
-// The small-tensor instalment in two phases, shared by dp_small_kernel (overlapped exchange) and dp_tail_kernel (exchange at the
-// end of the step).  Phase 1: slab sums of this block's 32 float4 columns, LL push of the sums to every peer.  Phase 2: collect
-// the peers' sums (they have had the time in between to arrive), add in rank order, RMSProp on the local copy.
-struct DpSmallState {
-  float4 w, ms, mo, acc;
-  int j;
-  bool owner;
-};
+// launch has ended.
 template <bool HAS_MOM>
-__device__ __forceinline__ void dp_small_phase1(const RmsPropDpArgs& d, int64_t recv_offset, int cb, bool pre_wait_loads, int kid,
-                                                EvtLog& evt_i, DpSmallState& st, float4 (*part)[GR_COLS]) {
+__global__ void __launch_bounds__(GR_LANES * GR_COLS) dp_small_kernel(RmsPropDpArgs d, int64_t recv_offset) {
+  __shared__ float4 part[GR_LANES][GR_COLS];
+  EvtLog evt_i = evt_open();
   const RmsPropArgs& a = d.base;
   const GradReduceArgs& r = d.red;
   const int col = threadIdx.x & (GR_COLS - 1), sl = threadIdx.x / GR_COLS;
-  const int j = (cb * GR_COLS + col) * 4;
-  st.j = j;
-  st.owner = sl == 0 && j < r.out_floats;
+  const int j = (blockIdx.x * GR_COLS + col) * 4;
+  const bool owner = sl == 0 && j < r.out_floats;
   int count = 0;
   if (j < r.n_floats) {
 #pragma unroll
     for (int s = GR_MAX_SEG - 1; s >= 0; --s)
       if (j < r.seg_end[s]) count = r.seg_count[s];
   }
-  st.w = make_float4(0.f, 0.f, 0.f, 0.f); st.ms = st.w; st.mo = st.w;
+  float4 w = make_float4(0.f, 0.f, 0.f, 0.f), ms = w, mo = w;
   auto load_state = [&]() {
-    st.w = *reinterpret_cast<const float4*>(a.w + j);
-    st.ms = *reinterpret_cast<const float4*>(a.ms + j);
-    if (HAS_MOM) st.mo = *reinterpret_cast<const float4*>(a.mom + j);
+    w = *reinterpret_cast<const float4*>(a.w + j);
+    ms = *reinterpret_cast<const float4*>(a.ms + j);
+    if (HAS_MOM) mo = *reinterpret_cast<const float4*>(a.mom + j);
   };
   // w / ms of the small prefix were last written by this kernel one step ago; see rmsprop_reduce_kernel for when the early
   // loads are safe
-  if (pre_wait_loads) {
-    if (st.owner && a.preload) load_state();
-    griddep_launch();
-    evt_mark(evt_i, 60, 0);
-    griddep_wait(kid);            // the slabs come from the conv backward launch that precedes this one
-    evt_mark(evt_i, 61, 0);
-    if (st.owner && !a.preload) load_state();
-  }
+  if (owner && a.preload) load_state();
+  griddep_launch();
+  evt_mark(evt_i, 60, 0);
+  griddep_wait(K_RMSPROP);        // the slabs come from the conv backward launch that precedes this one
+  evt_mark(evt_i, 61, 0);
+  if (owner && !a.preload) load_state();
   float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
   const float* src = r.part + j;
   for (int i0 = sl; i0 < count; i0 += GR_UNROLL * GR_LANES) {
@@ -626,10 +450,10 @@ __device__ __forceinline__ void dp_small_phase1(const RmsPropDpArgs& d, int64_t 
       t[0] = acc.x; t[1] = acc.y; t[2] = acc.z; t[3] = acc.w;
     }
   }
-  st.acc = acc;
   evt_mark(evt_i, 62, 0);
-  if (st.owner) {
+  if (owner) {
     // receive buffers: [parity][source rank][small prefix in LL format: 8 bytes per float]
+    uint8_t* my_comm = d.peer[d.rank] + d.comm_offset;
     const uint32_t flag = (uint32_t)d.step;
     const int64_t slot = recv_offset + ((int64_t)(d.step & 1) * DP_WORLD_MAX + d.rank) * r.out_floats * 8 + (int64_t)j * 8;
 #pragma unroll
@@ -637,179 +461,39 @@ __device__ __forceinline__ void dp_small_phase1(const RmsPropDpArgs& d, int64_t 
       if (q < d.world && q != d.rank) dp_ll_store(d.peer[q] + slot, acc, flag);
     *reinterpret_cast<float4*>(r.out + j) = acc;                     // this rank's own gradient (introspection)
     evt_mark(evt_i, 66, 0);
-  }
-}
-template <bool HAS_MOM>
-__device__ __forceinline__ void dp_small_phase2(const RmsPropDpArgs& d, int64_t recv_offset, EvtLog& evt_i, DpSmallState& st,
-                                                bool load) {
-  const RmsPropArgs& a = d.base;
-  const GradReduceArgs& r = d.red;
-  if (!st.owner) return;
-  uint8_t* my_comm = d.peer[d.rank] + d.comm_offset;
-  const uint32_t flag = (uint32_t)d.step;
-  const int j = st.j;
-  if (load) {                     // phase 1 ran without the state loads (a block that serves several column blocks)
-    st.w = *reinterpret_cast<const float4*>(a.w + j);
-    st.ms = *reinterpret_cast<const float4*>(a.ms + j);
-    if (HAS_MOM) st.mo = *reinterpret_cast<const float4*>(a.mom + j);
-  }
-  float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
-  for (int q = 0; q < DP_WORLD_MAX; ++q)
-    if (q < d.world) {
-      const float4 v = q == d.rank ? st.acc
-                                   : dp_ll_load(d.peer[d.rank] + recv_offset +
-                                                    ((int64_t)(d.step & 1) * DP_WORLD_MAX + q) * r.out_floats * 8 + (int64_t)j * 8,
-                                                flag, my_comm + DPC_ERR);
-      g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
-    }
-  evt_mark(evt_i, 63, 0);
-  rms_update<HAS_MOM>(a, g, st.w, st.ms, st.mo);
-  *reinterpret_cast<float4*>(a.w + j) = st.w;
-  *reinterpret_cast<float4*>(a.ms + j) = st.ms;
-  if (HAS_MOM) *reinterpret_cast<float4*>(a.mom + j) = st.mo;
-}
-
-template <bool HAS_MOM>
-__global__ void __launch_bounds__(GR_LANES * GR_COLS) dp_small_kernel(RmsPropDpArgs d, int64_t recv_offset, int wait_big) {
-  __shared__ float4 part[GR_LANES][GR_COLS];
-  EvtLog evt_i = evt_open();
-  DpSmallState st;
-  uint8_t* my_comm = d.peer[d.rank] + d.comm_offset;
-  dp_small_phase1<HAS_MOM>(d, recv_offset, blockIdx.x, true, K_RMSPROP, evt_i, st, part);
-  dp_small_phase2<HAS_MOM>(d, recv_offset, evt_i, st, false);
+    for (int q = 0; q < DP_WORLD_MAX; ++q)
+      if (q < d.world) {
+        const float4 v = q == d.rank ? acc
+                                     : dp_ll_load(d.peer[d.rank] + recv_offset +
+                                                      ((int64_t)(d.step & 1) * DP_WORLD_MAX + q) * r.out_floats * 8 + (int64_t)j * 8,
+                                                  flag, my_comm + DPC_ERR);
+        g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
+      }
+    evt_mark(evt_i, 63, 0);
+    rms_update<HAS_MOM>(a, g, w, ms, mo);
+    *reinterpret_cast<float4*>(a.w + j) = w;
+    *reinterpret_cast<float4*>(a.ms + j) = ms;
+    if (HAS_MOM) *reinterpret_cast<float4*>(a.mom + j) = mo;
+  }
   evt_mark(evt_i, 64, 0);
-  if (wait_big && blockIdx.x == 0 && (int)threadIdx.x < d.world) {     // (the side-stream exchange waits for the slices itself)
-    dp_wait_flag(my_comm + DPC_BIGDONE + 64 * threadIdx.x, d.step, my_comm + DPC_ERR, 16u);
-    __threadfence_system();
-  }
-  evt_mark(evt_i, 65, 0);
   trace_mark(K_RMSPROP, 2);
 }
 
-// ---- data-parallel exchange at the END of the step (default) -----------------------------------------------------------
-// One launch on every SM after the conv backward: blocks [0, n_cb) first sum this rank's slabs for their columns and push the
-// sums to the peers (phase 1 above); then EVERY block takes its share of the dense1/w exchange (dp_big_exchange: reduce-scatter
-// with peer loads, RMSProp on the owned slice, all-gather of the bf16 shadow with peer stores); then the small-tensor blocks
-// collect the peers' sums -- which arrived while the big loop ran -- and update (phase 2).  Block 0 holds the launch open
-// until every rank's dense1/w slice has landed.  Every rank's "dense_bwd done" flag was pushed by CTA 0 of its conv backward
-// launch, a whole conv backward ago, so nobody waits for a peer's gradient; the conv backward itself keeps all the SMs
-// (the overlapped variant gives up 20 of them and pays a whole extra round of frames at B = 1024).
-// Both instalments run CONCURRENTLY on different warps of every block (each is a chain of NVLink latencies, not bandwidth):
-//   threads   0-255  small tensors: slab sums of a 32-float4 column block (8 slab lanes), LL push to every peer, collect the
-//                    peers' sums, identical RMSProp update on every rank
-//   threads 256-511  dense1/w: wait (acquire) for every rank's "dense_bwd done" flag -- pushed a whole conv backward ago --, then
-//                    reduce-scatter with peer loads, RMSProp on the owned slice, all-gather of the bf16 shadow with peer stores
-// No fence sits between the two flag hops of the step: the only fence.sys is the one that orders a block's peer stores before
-// the rank's "slice landed" flag (measured at 2 ranks, profiles/r2i_dp_tail_timeline.txt: the first version of this kernel
-// spent 2.7 us in a fence after the flag wait and 3.1 us in the one before the counter, one after the other).
-constexpr int DPT_SMALL = 256, DPT_LANES = DPT_SMALL / GR_COLS;
-template <bool HAS_MOM>
-__global__ void __launch_bounds__(512) dp_tail_kernel(RmsPropDpArgs d, DpBigArgs big, int64_t recv_offset, int n_cb) {
-  __shared__ float4 part[DPT_LANES][GR_COLS];
-  __shared__ int dp_last;
-  const RmsPropArgs& a = d.base;
-  const GradReduceArgs& r = d.red;
-  EvtLog evt_i = evt_open();
-  const int tid = threadIdx.x;
-  uint8_t* my_comm = d.peer[d.rank] + d.comm_offset;
-  griddep_launch();
-  evt_mark(evt_i, 60, 0);
-  griddep_wait(K_RMSPROP);            // the slabs come from the conv backward launch that precedes this one
-  evt_mark(evt_i, 61, 0);
-  if (tid >= DPT_SMALL) {
-    // ---------------- dense1/w ----------------
-    const int t = tid - DPT_SMALL;
-    // (CTA 0 of the conv backward has published "dense_bwd done" already, unless this step had no rows: publish again)
-    dp_big_group(big, t, 512 - DPT_SMALL, (int)blockIdx.x, (int)gridDim.x, 1, &dp_last, true);
-    if (t == 0) evt_mark(evt_i, 72, 0);
-  } else {
-    // ---------------- small tensors ----------------
-    const int col = tid & (GR_COLS - 1), sl = tid / GR_COLS;
-    const uint32_t flag = (uint32_t)d.step;
-    for (int cb = blockIdx.x; cb < n_cb; cb += gridDim.x) {
-      const int j = (cb * GR_COLS + col) * 4;
-      const bool owner = sl == 0 && j < r.out_floats;
-      int count = 0;
-      if (j < r.n_floats) {
-#pragma unroll
-        for (int s = GR_MAX_SEG - 1; s >= 0; --s)
-          if (j < r.seg_end[s]) count = r.seg_count[s];
-      }
-      float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-      const float* src = r.part + j;
-      for (int i0 = sl; i0 < count; i0 += GR_UNROLL * DPT_LANES) {
-        float4 q[GR_UNROLL];
-#pragma unroll
-        for (int u = 0; u < GR_UNROLL; ++u) {
-          const int i = i0 + u * DPT_LANES;
-          q[u] = i < count ? __ldcg(reinterpret_cast<const float4*>(src + (int64_t)i * r.stride)) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-#pragma unroll
-        for (int u = 0; u < GR_UNROLL; ++u) { acc.x += q[u].x; acc.y += q[u].y; acc.z += q[u].z; acc.w += q[u].w; }
-      }
-      part[sl][col] = acc;
-      named_bar_sync_ew(2, DPT_SMALL);
-      if (sl == 0 && j < r.n_floats) {
-#pragma unroll
-        for (int l = 1; l < DPT_LANES; ++l) {
-          const float4 q = part[l][col];
-          acc.x += q.x; acc.y += q.y; acc.z += q.z; acc.w += q.w;
-        }
-        if (j >= r.out_floats && r.out_tail != nullptr) {
-          float* tl = r.out_tail + (j - r.out_floats);
-          tl[0] = acc.x; tl[1] = acc.y; tl[2] = acc.z; tl[3] = acc.w;
-        }
-      }
-      if (tid == 0) evt_mark(evt_i, 62, cb);
-      if (owner) {
-        // receive buffers: [parity][source rank][small prefix in LL format: 8 bytes per float]
-        const int64_t slot = recv_offset + ((int64_t)(d.step & 1) * DP_WORLD_MAX + d.rank) * r.out_floats * 8 + (int64_t)j * 8;
-#pragma unroll
-        for (int q = 0; q < DP_WORLD_MAX; ++q)
-          if (q < d.world && q != d.rank) dp_ll_store(d.peer[q] + slot, acc, flag);
-        *reinterpret_cast<float4*>(r.out + j) = acc;                     // this rank's own gradient (introspection)
-        float4 w = *reinterpret_cast<const float4*>(a.w + j);
-        float4 ms = *reinterpret_cast<const float4*>(a.ms + j);
-        float4 mo = HAS_MOM ? *reinterpret_cast<const float4*>(a.mom + j) : make_float4(0.f, 0.f, 0.f, 0.f);
-        float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-        for (int q = 0; q < DP_WORLD_MAX; ++q)
-          if (q < d.world) {
-            const float4 v = q == d.rank ? acc
-                                         : dp_ll_load(d.peer[d.rank] + recv_offset +
-                                                          ((int64_t)(d.step & 1) * DP_WORLD_MAX + q) * r.out_floats * 8 + (int64_t)j * 8,
-                                                      flag, my_comm + DPC_ERR);
-            g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
-          }
-        rms_update<HAS_MOM>(a, g, w, ms, mo);
-        *reinterpret_cast<float4*>(a.w + j) = w;
-        *reinterpret_cast<float4*>(a.ms + j) = ms;
-        if (HAS_MOM) *reinterpret_cast<float4*>(a.mom + j) = mo;
-      }
-      if (tid == 0) evt_mark(evt_i, 64, cb);
-      named_bar_sync_ew(2, DPT_SMALL);                                   // `part` is reused by the next column block
-    }
-  }
-  __syncthreads();
-  if (blockIdx.x == 0 && tid < d.world) dp_wait_flag_acquire(my_comm + DPC_BIGDONE + 64 * tid, d.step, my_comm + DPC_ERR, 16u);
-  evt_mark(evt_i, 65, 0);
-  trace_mark(K_RMSPROP, 2);
-}
-
-// ---- the dense1/w exchange as a kernel of its own, on a side stream (GA3C_DP_EXCHANGE=side, the default) -------------------------
+// ---- data-parallel exchange, dense1/w: a kernel of its own on a side stream -----------------------------------------------
 // 128-thread blocks without shared memory: small enough to be resident NEXT TO the conv backward CTAs of this step and the conv
 // forward CTAs of the next one (both leave ~12 K registers and 1,500 thread slots per SM), so the whole chain of NVLink latencies
 // -- wait for every rank's "dense_bwd done" flag, pull the slices, RMSProp, push the bf16 shadow, fence, "slice landed" flags, wait
 // for every rank's -- runs under kernels that do not depend on it.  The next launch that reads the shadow (dense_fwd) waits for
-// this kernel's completion event; block 0 ends only when every rank's slice has landed in THIS rank's slab.
-// By default it is launched behind an event recorded after dense_bwd (its own gradient is final by stream order) and publishes
+// every rank's "slice landed" flag (DpGate, dense_tc.cu); block 0 ends only when every rank's slice has landed in THIS rank's slab.
+// It is launched behind an event recorded after dense_bwd (its own gradient is final by stream order) and publishes
 // that to the peers itself: it then only ever waits for OTHER GPUs, never for a kernel of its own GPU that might not find room
 // on an SM next to it (a spinning kernel that waits for a kernel it keeps from being resident is a deadlock).
-__global__ void __launch_bounds__(128, 6) dp_big_side_kernel(DpBigArgs big, int push_ready) {      // <= 85 registers: 11 K per block
+__global__ void __launch_bounds__(128, 6) dp_big_side_kernel(DpBigArgs big) {      // <= 85 registers: 11 K per block
   trace_mark(K_DP_BIG, 0);
   int dp_last = 0;      // thread 0's only.  NO shared memory: next to a conv CTA an SM has room for the reserved 1 KB of a block and no more
-  dp_big_group<false>(big, (int)threadIdx.x, 128, (int)blockIdx.x, (int)gridDim.x, 1, &dp_last, push_ready != 0);
+  dp_big_group(big, (int)threadIdx.x, 128, (int)blockIdx.x, (int)gridDim.x, 1, &dp_last);
   __syncthreads();
   trace_mark(K_DP_BIG, 1);             // (trace row of this kernel: first/last block started, own slice done, all slices landed)
   uint8_t* my_comm = big.peer[big.rank] + big.comm_offset;
@@ -820,30 +504,13 @@ __global__ void __launch_bounds__(128, 6) dp_big_side_kernel(DpBigArgs big, int 
     trace_mark(K_DP_BIG, 2);
   }
 }
-int launch_dp_big_side(const DpBigArgs& big, bool push_ready, int num_sms, cudaStream_t side_stream) {
+int launch_dp_big_side(const DpBigArgs& big, int num_sms, cudaStream_t side_stream) {
   int grid = num_sms;
   if (const char* e = getenv("GA3C_DP_SIDE_CTAS")) {     // tests with several ranks on one GPU leave room for the other ranks' kernels
     const int g = atoi(e);
     if (g >= 1 && g <= grid) grid = g;
   }
-  dp_big_side_kernel<<<grid, 128, 0, side_stream>>>(big, push_ready ? 1 : 0);
-  return (int)cudaGetLastError();
-}
-
-// a rank with no rows this step (ga3c_train_step with batch 0) pushes ZERO gradient slices, so that the owners' reduce finds a
-// contribution from every rank in its receive buffers
-__global__ void __launch_bounds__(256) dp_push_zero_kernel(WgradPush push, long long n4) {
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
-  for (long long i4 = (long long)blockIdx.x * blockDim.x + threadIdx.x; i4 < n4; i4 += stride) {
-    const int q = (int)(i4 / push.per4);
-    if (q == push.rank) continue;
-    dp_ll_store(push.peer[q] + push.recv_off + (((long long)(push.flag & 1u) * push.world + push.rank) * push.per4 + (i4 - (long long)q * push.per4)) * 32,
-                zero, push.flag);
-  }
-}
-int launch_dp_push_zero(const WgradPush& push, long long n4, cudaStream_t stream) {
-  dp_push_zero_kernel<<<148, 256, 0, stream>>>(push, n4);
+  dp_big_side_kernel<<<grid, 128, 0, side_stream>>>(big);
   return (int)cudaGetLastError();
 }
 
@@ -855,38 +522,15 @@ int configure_dp() {
   int r;
   if ((r = (int)cudaFuncGetAttributes(&a, dp_small_kernel<false>))) return r;
   if ((r = (int)cudaFuncGetAttributes(&a, dp_small_kernel<true>))) return r;
-  if ((r = (int)cudaFuncGetAttributes(&a, dp_big_side_kernel))) return r;
-  if ((r = (int)cudaFuncGetAttributes(&a, dp_tail_kernel<false>))) return r;
-  if ((r = (int)cudaFuncGetAttributes(&a, dp_tail_kernel<true>))) return r;
-  if ((r = (int)cudaFuncGetAttributes(&a, rmsprop_dp_kernel<false>))) return r;
-  return (int)cudaFuncGetAttributes(&a, rmsprop_dp_kernel<true>);
+  return (int)cudaFuncGetAttributes(&a, dp_big_side_kernel);
 }
 
-int launch_dp_small(const RmsPropDpArgs& d, int64_t recv_offset, cudaStream_t stream, bool wait_big) {
+int launch_dp_small(const RmsPropDpArgs& d, int64_t recv_offset, cudaStream_t stream) {
   const int n_cb = (d.red.n_floats / 4 + GR_COLS - 1) / GR_COLS;
-  if (n_cb > DP_MAX_CB || !d.has_red) return (int)cudaErrorInvalidValue;
+  if (n_cb > DP_MAX_CB) return (int)cudaErrorInvalidValue;
   if (d.base.momentum != 0.f)
-    return launch_pdl(dp_small_kernel<true>, dim3(n_cb), dim3(GR_LANES * GR_COLS), 0, stream, d, recv_offset, wait_big ? 1 : 0);
-  return launch_pdl(dp_small_kernel<false>, dim3(n_cb), dim3(GR_LANES * GR_COLS), 0, stream, d, recv_offset, wait_big ? 1 : 0);
-}
-
-
-int launch_dp_tail(const RmsPropDpArgs& d, const DpBigArgs& big, int64_t recv_offset, int num_sms, cudaStream_t stream) {
-  const int n_cb = (d.red.n_floats / 4 + GR_COLS - 1) / GR_COLS;
-  if (n_cb > DP_MAX_CB || !d.has_red) return (int)cudaErrorInvalidValue;
-  int grid = n_cb > num_sms ? n_cb : num_sms;
-  if (const char* e = getenv("GA3C_DP_TAIL_CTAS")) {     // tests with several ranks on one GPU leave SMs to the other ranks' kernels
-    const int g = atoi(e);
-    if (g >= 1 && g <= grid) grid = g;
-  }
-  if (d.base.momentum != 0.f)
-    return launch_pdl(dp_tail_kernel<true>, dim3(grid), dim3(GR_LANES * GR_COLS), 0, stream, d, big, recv_offset, n_cb);
-  return launch_pdl(dp_tail_kernel<false>, dim3(grid), dim3(GR_LANES * GR_COLS), 0, stream, d, big, recv_offset, n_cb);
-}
-
-int launch_rmsprop_dp(const RmsPropDpArgs& d, int num_sms, cudaStream_t stream) {
-  if (d.base.momentum != 0.f) return launch_pdl(rmsprop_dp_kernel<true>, dim3(num_sms), dim3(512), 0, stream, d);
-  return launch_pdl(rmsprop_dp_kernel<false>, dim3(num_sms), dim3(512), 0, stream, d);
+    return launch_pdl(dp_small_kernel<true>, dim3(n_cb), dim3(GR_LANES * GR_COLS), 0, stream, d, recv_offset);
+  return launch_pdl(dp_small_kernel<false>, dim3(n_cb), dim3(GR_LANES * GR_COLS), 0, stream, d, recv_offset);
 }
 
 __global__ void __launch_bounds__(256) f32_to_bf16_kernel(const float* __restrict__ src, uint16_t* __restrict__ dst, int64_t n4) {

@@ -1,7 +1,5 @@
 // The fused value / policy heads, softmax, A3C loss and its backward (NetworkVP_discrate.py:60-85, :100; SURVEY A.3 / A.4) as device
-// functions shared by the two kernels that run them: heads_kernel (heads.cu: behind the split-K dense1 GEMM, summing its partial
-// tiles from L2) and dense_heads_kernel (dense_heads.cu: as the epilogue of the cluster split-K dense1 GEMM, summing the partial
-// tiles over distributed shared memory).  All fp32.
+// functions, run by heads_kernel (heads.cu: behind the split-K dense1 GEMM, summing its partial tiles from L2).  All fp32.
 #pragma once
 #include "common.cuh"
 #include "kernels.h"

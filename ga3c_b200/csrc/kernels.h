@@ -12,13 +12,11 @@ int trace_attach_conv_bwd_fused(unsigned long long* buf);
 int trace_attach_dense_tc(unsigned long long* buf);
 int trace_attach_heads(unsigned long long* buf);
 int trace_attach_elementwise(unsigned long long* buf);
-int trace_attach_dense_heads(unsigned long long* buf);
 
 // pipeline event log of CTA 0 (debug): attach a zeroed [16 warps][1024][2] uint64 buffer (or nullptr)
 int evt_attach_conv_fwd(unsigned long long* buf);
 int evt_attach_conv_bwd(unsigned long long* buf);
 int evt_attach_elementwise(unsigned long long* buf);
-int evt_attach_dense_heads(unsigned long long* buf);
 int evt_attach_dense_tc(unsigned long long* buf);      // records only in a -DGA3C_DENSE_EVT build
 
 // L2 residency hints on the conv kernels' loads and stores (common.cuh); GA3C_L2_HINTS=0 switches them off (evict_normal)
@@ -57,17 +55,9 @@ int launch_dense_fwd_tc(const uint16_t* n2, const uint16_t* w1bf, float* d1_part
 int launch_dense_dgrad_tc(const uint16_t* dd1, const uint16_t* w1bf, const uint16_t* n2, uint8_t* dn2, int batch,
                           cudaStream_t stream);       // dn2 in the G operand layout (common.cuh), borders untouched
 int launch_dense_wgrad_tc(const uint16_t* n2, const uint16_t* dd1, float* g_w1, int batch, cudaStream_t stream);
-// dgrad + wgrad tiles in one grid (both only need dd1): the single-GPU / fused-DP step uses this one
-// data parallel, exchange at the end of the step: where the dense1/w gradient tiles push the slices this rank does not own
-// (dense_tc.cu EpiWgradPush; receive buffers [2 parities][world][per4 float4 in LL format] at recv_off of every slab)
-struct WgradPush {
-  uint8_t* peer[8];
-  int rank, world;
-  long long per4, recv_off;
-  unsigned int flag;         // the step number; parity = flag & 1
-};
+// dgrad + wgrad tiles in one grid (both only need dd1): the train step uses this one
 int launch_dense_bwd_tc(const uint16_t* dd1, const uint16_t* w1bf, const uint16_t* n2, uint8_t* dn2, float* g_w1, int batch,
-                        const WgradPush* push, cudaStream_t stream);
+                        cudaStream_t stream);
 
 // heads.cu -- value / policy heads, softmax, A3C loss and its backward (NetworkVP_discrate.py:60-85)
 struct HeadsArgs {
@@ -94,35 +84,16 @@ struct HeadsArgs {
 int heads_grid(int batch, int num_sms);          // CTAs (= slabs written) of a training launch
 int launch_heads(const HeadsArgs& args, int num_sms, cudaStream_t stream);
 
-// dense_heads.cu -- dense1 forward (cluster split-K, partial tiles reduced over distributed shared memory) with the heads, the
-// loss and its backward as its epilogue: replaces launch_dense_fwd_tc + launch_heads (args.d1_part / n_split are not used).
-// In training it writes dense_heads_ctas(batch) slabs.
-int configure_dense_heads();
-int dense_heads_ctas(int batch);
-int launch_dense_heads(const uint16_t* n2, const uint16_t* w1bf, const HeadsArgs& args, cudaStream_t stream);
-
 // conv_bwd_fused.cu
 // Weight / bias gradients are per-CTA partial sums: CTA i stores into slab i (g_* point into slab 0, slabs are
 // gp_stride floats apart) and launch_grad_reduce adds the slabs in a fixed order.  No contended atomics, and the
 // step is bit-reproducible.
-struct DpBigArgs;                                // dp_exchange.cuh
-int conv_bwd_grid(int batch, int num_sms, int n_exch = 0);   // conv CTAs (= slabs written); n_exch SMs are left to the exchange CTAs
+int conv_bwd_grid(int batch, int num_sms);       // conv CTAs (= slabs written)
 // conv_bwd_fused.cu -- conv12 data gradient (dn1, kept on chip; dn1_out: optional copy for tests), conv12 and conv11
 // weight / bias gradients in one kernel on tcgen05
-// what warps 12-15 of every conv backward CTA do with dense1/w, whose gradient is final when that kernel starts:
-//   mode 0 nothing; mode 1 RMSProp + bf16 shadow refresh over the whole tensor (single GPU; the pointers are the dense1/w ranges
-//   of the arenas, n4 its size in float4); mode 2 the data-parallel exchange described by the DpBigArgs of the launch
-struct ConvBwdOpt {
-  int mode;
-  const float* g;
-  float *w, *ms, *mom;
-  uint16_t* shadow;
-  long long n4;
-  float lr, decay, momentum, eps;
-};
 int launch_conv_bwd(const uint8_t* xblk, const uint8_t* n1b2, const uint8_t* dn2g, const float* w12, uint16_t* dn1_out,
                     float* g_w11, float* g_b11, float* g_w12, float* g_b12, int64_t gp_stride, int batch, int num_sms, bool x_u8,
-                    const ConvBwdOpt& opt, const DpBigArgs* dp, cudaStream_t stream);   // dp != null: data parallel (+ dp->n_exch exchange CTAs)
+                    cudaStream_t stream);
 
 // elementwise.cu
 // out[j] = sum over slabs i < count(j) of part[i * stride + j], j in [0, n_floats): the per-CTA gradient partials of
@@ -181,29 +152,23 @@ int launch_rmsprop_dual(const RmsPropDualArgs& d, cudaStream_t stream);
 int launch_rmsprop_dual_clipped(RmsPropDualArgs d, const ClipArgs& c1, const ClipArgs& c2, cudaStream_t stream);
 // grad_reduce + RMSProp in one launch (single-GPU step; r.out must be a.g, r.out_floats the small-tensor prefix)
 int launch_rmsprop_reduce(const RmsPropArgs& a, const GradReduceArgs& r, cudaStream_t stream);
-// data-parallel RMSProp over peer memory: rank r owns arena slice r; it sums that slice of every rank's gradient
-// arena (fixed rank order), applies RMSProp, and stores the new weights (+ bf16 shadow) into every rank's slab.
+// data-parallel exchange over peer memory (dp_exchange.cuh), in two instalments.
 constexpr int DP_MAX_WORLD = 8;
+struct DpBigArgs;
+// dense1/w on a side stream, resident next to the conv kernels (elementwise.cu dp_big_side_kernel): rank r owns slice r, sums that
+// slice of every rank's gradient (fixed rank order), applies RMSProp and stores the bf16 shadow into every rank's slab
+int launch_dp_big_side(const DpBigArgs& big, int num_sms, cudaStream_t side_stream);
+// the small tensors behind the conv backward: slab reduction, LL push into every rank's receive buffer, identical RMSProp on
+// every rank.  recv_offset: byte offset in the slab of the receive buffers [2][DP_MAX_WORLD][small prefix * 8 B].
 struct RmsPropDpArgs {
   RmsPropArgs base;                 // this rank's own arenas
-  uint8_t* peer[DP_MAX_WORLD];      // slab bases: [params | grads | ms | mom | shadow | comm]
+  uint8_t* peer[DP_MAX_WORLD];      // slab bases: [params | grads | ms | mom | shadow | LL receive buffers | comm]
   int rank, world;
-  uint64_t step;                    // 1, 2, ... : value the ready / done flags reach in this step
+  uint64_t step;                    // 1, 2, ... : the flag value of this step
   int64_t arena_bytes, comm_offset;
-  GradReduceArgs red;               // has_red: first sum this rank's gradient-partial slabs into its gradient arena
-  int has_red;                      // (saves the separate grad_reduce launch in front of the exchange)
+  GradReduceArgs red;               // this rank's gradient-partial slabs
 };
-int launch_rmsprop_dp(const RmsPropDpArgs& a, int num_sms, cudaStream_t stream);
-// second instalment of the overlapped exchange (dp_exchange.cuh): slab reduction of the small tensors, LL push into every
-// rank's receive buffer, identical RMSProp on every rank; returns only when every rank's dense1/w slice has landed.
-// a.red is required; recv_offset: byte offset in the slab of the receive buffers [2][DP_MAX_WORLD][small prefix * 8 B].
-// wait_big: block 0 also holds the launch open until every rank's dense1/w slice has landed (the overlapped modes)
-int launch_dp_small(const RmsPropDpArgs& a, int64_t recv_offset, cudaStream_t stream, bool wait_big);
-// the whole exchange in one launch at the end of the step (default): small tensors as launch_dp_small, dense1/w on every SM
-int launch_dp_tail(const RmsPropDpArgs& a, const DpBigArgs& big, int64_t recv_offset, int num_sms, cudaStream_t stream);
-// the dense1/w exchange alone, on a side stream, resident next to the conv kernels (elementwise.cu dp_big_side_kernel)
-int launch_dp_big_side(const DpBigArgs& big, bool push_ready, int num_sms, cudaStream_t side_stream);
-int launch_dp_push_zero(const WgradPush& push, long long n4, cudaStream_t stream);   // a rank without rows: zero slices to the owners
+int launch_dp_small(const RmsPropDpArgs& a, int64_t recv_offset, cudaStream_t stream);
 int configure_dp();     // load the exchange kernels now (not lazily at their first launch)
 int launch_f32_to_bf16(const float* src, uint16_t* dst, int64_t n, cudaStream_t stream);
 int launch_returns(const double* rewards, const int64_t* seg_offsets, int n_segments, const double* terminal,

@@ -53,32 +53,10 @@ struct ga3c_net {
   uint8_t* dp_peer[DP_MAX_WORLD] = {};   // slab base of every rank as mapped in this process (own slab at dp_rank)
   bool dp_ipc[DP_MAX_WORLD] = {};        // mapped with cudaIpcOpenMemHandle (to be closed on detach)
   uint64_t dp_step = 0;
-  int dp_exch = 20;                // overlapped exchange: exchange CTAs appended to the conv backward launch (GA3C_DP_EXCH_CTAS)
-  int dp_exchange = 4;             // GA3C_DP_EXCHANGE: 4 "side" (default: dense1/w exchanged by a small-footprint kernel on a side stream
-                                   // that is resident next to the conv backward of this step and the conv forward of the next;
-                                   // small tensors in dp_small), 0 "tail" (one launch on every SM at the end of the step), 3 "warps" (the
-                                   // dense1/w exchange on the optimizer warps of every conv backward CTA, small tensors + completion
-                                   // in dp_small), 1 "overlap" (exchange CTAs inside the conv backward launch + dp_small), 2
-                                   // "single" (the first version: one kernel that also broadcasts the fp32 weights).  Measured at 2
-                                   // GPUs, B = 1024 per GPU (profiles/r2l_*): tail 0.1196 ms, warps 0.1205, overlap 0.1403
-  int fuse_heads = 0;              // GA3C_FUSE_HEADS=1: dense1 forward + heads as ONE cluster launch (dense_heads.cu: split-K over a
-                                   // thread-block cluster, partial tiles reduced over distributed shared memory).  Parity-green, but
-                                   // measured slower at B = 1024 (step 0.1015 -> 0.1077 ms, profiles/r2r_*): 64 CTAs run the heads of
-                                   // 16 samples each in two serial rounds where the separate kernel runs 128 CTAs of one round
-  int fuse_opt = 0;                // GA3C_FUSE_OPT=1: single GPU, dense1/w updated by the optimizer warps of the conv backward CTAs
-                                   // instead of the launch at the end.  Measured: conv_bwd 26.3 -> 30.6 us, rmsprop 8.9 -> 5.0 us,
-                                   // step 0.1015 -> 0.1032 ms: the conv backward is HBM-bound, the 22 MB cost what they cost alone
-  int cur_exch = 0;                // ... of the step being enqueued (0 outside the overlapped data-parallel step)
   int64_t xbuf_off = 0, comm_off = 0;    // byte offsets in the slab: LL receive buffers [2][8][small prefix * 8 B], comm block
-  int64_t bigrecv_off = 0;               // ... and the LL receive buffers of the pushed dense1/w gradient slices [2][(n4 + 8) * 32 B]
-  int dp_push = 0;                       // GA3C_DP_PUSH=1 (with GA3C_DP_EXCHANGE=tail): slices pushed by the dense1 wgrad epilogues in the
-                                         // LL format instead of pulled by their owners.  Measured at 2 GPUs: 0.1463 vs 0.1181 ms per
-                                         // step -- scattered 16-byte stores across NVLink from the GEMM epilogue triple its time
-  cudaStream_t dp_stream = nullptr;      // GA3C_DP_EXCHANGE=side: the dense1/w exchange runs here, next to the conv kernels
-  cudaEvent_t dp_big_done = nullptr;     // ... and whatever reads the dense1/w shadow next waits for this
-  bool dp_big_pending = false;
+  cudaStream_t dp_stream = nullptr;      // the dense1/w exchange runs here, next to the conv kernels
+  bool dp_big_pending = false;           // an exchange was launched since the ranks attached: dense_fwd waits for its flags (dp_gate)
   cudaEvent_t dp_grad_ready = nullptr;   // recorded behind dense_bwd: the side stream waits for it
-  const DpBigArgs* dp_side = nullptr;    // set while a side-mode step is enqueued: fb_tail_impl launches the exchange behind dense_bwd
   // workspace
   uint16_t *n2 = nullptr, *dd1 = nullptr, *dn1 = nullptr;
   // training-only activations, stored in the UMMA operand layouts the conv backward consumes (common.cuh); their zero borders /
@@ -125,7 +103,7 @@ int set_error(const std::string& m) { g_err = m; return -1; }     // for the oth
 const char* kernel_name(int kid) { return (kid >= 0 && kid < K_COUNT) ? kKernelNames[kid] : nullptr; }
 }
 extern "C" const char* ga3c_last_error(void) { return g_err.c_str(); }
-extern "C" int ga3c_abi_version(void) { return 8; }
+extern "C" int ga3c_abi_version(void) { return 9; }
 
 extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
   if (!cfg || !out) return fail_msg("ga3c_create: null argument");
@@ -178,8 +156,7 @@ extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
   const size_t shadow_bytes = (size_t)FLAT * FC * 2;
   n->xbuf_off = (int64_t)(4 * ab + shadow_bytes);
   n->comm_off = n->xbuf_off + 2 * (int64_t)DP_MAX_WORLD * n->small_floats * 8;
-  n->bigrecv_off = (n->comm_off + DP_COMM_BYTES + 127) / 128 * 128;
-  n->slab_bytes = (size_t)n->bigrecv_off + 2 * ((size_t)FLAT * FC / 4 + DP_MAX_WORLD) * 32;
+  n->slab_bytes = (size_t)n->comm_off + DP_COMM_BYTES;
   GA3C_ALLOC(n->slab, n->slab_bytes);
 #undef GA3C_ALLOC
   n->w = reinterpret_cast<float*>(n->slab);
@@ -212,8 +189,6 @@ extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
     if (e != cudaSuccess) { ga3c_destroy(n); return fail("cudaMalloc", e); }
   }
   if (int r = alloc_workspace(n, cfg->max_batch)) { ga3c_destroy(n); return r; }
-  if (const char* f = getenv("GA3C_FUSE_OPT")) n->fuse_opt = atoi(f) != 0;
-  if (const char* f = getenv("GA3C_FUSE_HEADS")) n->fuse_heads = atoi(f) != 0;
   cudaMemset(n->w, 0, ab); cudaMemset(n->g, 0, ab); cudaMemset(n->mom, 0, ab);
   cudaMemset(n->w1_shadow, 0, (size_t)FLAT * FC * 2);
   {  // ms slot starts at 1.0 [TF-SEMANTICS]
@@ -221,7 +196,7 @@ extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
     cudaMemcpy(n->ms, ones.data(), ab, cudaMemcpyHostToDevice);
   }
   int r;
-  if ((r = configure_conv_fwd()) || (r = configure_conv_bwd_fused()) || (r = configure_dense_tc()) || (r = configure_dense_heads())) {
+  if ((r = configure_conv_fwd()) || (r = configure_conv_bwd_fused()) || (r = configure_dense_tc())) {
     ga3c_destroy(n);
     return fail("cudaFuncSetAttribute", (cudaError_t)r);
   }
@@ -348,7 +323,7 @@ extern "C" int ga3c_arena_download(ga3c_net* n, int which, float* host, int64_t 
   CK(cudaDeviceSynchronize());
   CK(cudaMemcpy(host, src, (size_t)nf * 4, cudaMemcpyDeviceToHost));
   if (n->dp_world > 1 && (which == 0 || which == 2 || which == 3)) {
-    // overlapped exchange: the fp32 master copy and the RMSProp slots of a dense1/w slice live on its owner (only the bf16
+    // peer-memory exchange: the fp32 master copy and the RMSProp slots of a dense1/w slice live on its owner (only the bf16
     // shadow travels).  A peer's slice is stable here: it changes only inside a step this rank takes part in.
     const int64_t n4 = (int64_t)FLAT * FC / 4, per = (n4 + n->dp_world - 1) / n->dp_world;
     for (int q = 0; q < n->dp_world; ++q) {
@@ -384,31 +359,17 @@ static HeadsArgs heads_args(ga3c_net* n, int batch, int splits) {
   return h;
 }
 
-// data parallel, side-stream exchange: the bf16 shadow of dense1/w is complete when the exchange kernel of the previous step is
-static int wait_dp_big(ga3c_net* n, cudaStream_t st) {
-  // (not cleared: predict and train may come on different streams, and each of them has to see the exchange complete)
-  if (n->dp_big_pending) CK(cudaStreamWaitEvent(st, n->dp_big_done, 0));
-  return 0;
-}
-// ... or, by default (GA3C_DP_GATE=0 brings the event wait back), when dense_fwd's TMA producer has seen every rank's "slice
-// landed everywhere" flag of the last exchanged step in this rank's comm block (DpGate, dense_tc.cu): no stream operation between
-// conv_fwd and dense_fwd, so the launch chain stays programmatic
-static bool dp_gated(const ga3c_net* n) {
-  static const bool on = [] { const char* e = getenv("GA3C_DP_GATE"); return !e || atoi(e) != 0; }();
-  return on && n->dp_big_pending && n->dp_world > 1;
-}
+// data parallel: the bf16 shadow of dense1/w is complete when dense_fwd's TMA producer has seen every rank's "slice landed
+// everywhere" flag of the last exchanged step in this rank's comm block (DpGate, dense_tc.cu): no stream operation between
+// conv_fwd and dense_fwd, so the launch chain stays programmatic.  (dp_big_pending is cleared by ga3c_dp_detach, so it implies
+// dp_world > 1.)
 static DpGate dp_gate(const ga3c_net* n) {
   DpGate g{};
-  if (dp_gated(n)) {
+  if (n->dp_big_pending) {
     uint8_t* comm = n->dp_peer[n->dp_rank] + n->comm_off;
     g.flags = comm + DPC_BIGDONE; g.err = comm + DPC_ERR; g.step = n->dp_step; g.world = n->dp_world;
   }
   return g;
-}
-
-// dense1 forward + heads in one cluster launch (dense_heads.cu) while its slabs fit the gradient-partial workspace
-static bool fused_heads(const ga3c_net* n, int batch) {
-  return n->fuse_heads && !n->cfg.dual_rmsprop && dense_heads_ctas(batch) <= 2 * n->num_sms;
 }
 
 static int predict_impl(ga3c_net* n, const void* x, bool x_u8, int32_t batch, float* p_out, float* v_out, void* stream) {
@@ -419,19 +380,12 @@ static int predict_impl(ga3c_net* n, const void* x, bool x_u8, int32_t batch, fl
   const float* w = n->w;
   LAUNCH(n, K_CONV_FWD, st, launch_conv_fwd(x, x_u8, w + n->off(P_C11W), w + n->off(P_C11B), w + n->off(P_C12W),
                                             w + n->off(P_C12B), nullptr, nullptr, n->n2, batch, n->num_sms, st));
-  const bool fused_p = fused_heads(n, batch);
-  const DpGate gate = fused_p ? DpGate{} : dp_gate(n);
-  if (gate.flags == nullptr)
-    if (int r = wait_dp_big(n, st)) return r;
+  const DpGate gate = dp_gate(n);
   const int splits = dense_fwd_splits(batch, n->num_sms);
   HeadsArgs h = heads_args(n, batch, splits);
   h.p_out = p_out; h.v_out = v_out; h.train = 0;
-  if (fused_p) {
-    LAUNCH(n, K_DENSE_FWD, st, launch_dense_heads(n->n2, n->w1_shadow, h, st));
-  } else {
-    LAUNCH(n, K_DENSE_FWD, st, launch_dense_fwd_tc(n->n2, n->w1_shadow, n->d1_part, batch, splits, st, &gate));
-    LAUNCH(n, K_HEADS, st, launch_heads(h, n->num_sms, st));
-  }
+  LAUNCH(n, K_DENSE_FWD, st, launch_dense_fwd_tc(n->n2, n->w1_shadow, n->d1_part, batch, splits, st, &gate));
+  LAUNCH(n, K_HEADS, st, launch_heads(h, n->num_sms, st));
   n->last_batch = batch;
   return 0;
 }
@@ -456,23 +410,19 @@ static int fb_head_impl(ga3c_net* n, const void* x, bool x_u8, const float* yr, 
   float* g = n->g;
   float* gp = n->gpart;       // small-tensor gradients: per-CTA partial slabs, summed at the end of ga3c_fb_tail
   const int splits = dense_fwd_splits(batch, n->num_sms);
-  const bool fused = fused_heads(n, batch);
   if (!skip_forward) {        // the second DUAL_RMSPROP pass reuses n1 / n2 / the dense1 partials of the first
     LAUNCH(n, K_CONV_FWD, st, launch_conv_fwd(x, x_u8, w + n->off(P_C11W), w + n->off(P_C11B), w + n->off(P_C12W),
                                               w + n->off(P_C12B), n->n1, n->xblk, n->n2, batch, n->num_sms, st));
-    const DpGate gate = fused ? DpGate{} : dp_gate(n);
-    if (gate.flags == nullptr)
-      if (int r = wait_dp_big(n, st)) return r;
-    if (!fused) LAUNCH(n, K_DENSE_FWD, st, launch_dense_fwd_tc(n->n2, n->w1_shadow, n->d1_part, batch, splits, st, &gate));
+    const DpGate gate = dp_gate(n);
+    LAUNCH(n, K_DENSE_FWD, st, launch_dense_fwd_tc(n->n2, n->w1_shadow, n->d1_part, batch, splits, st, &gate));
   }
   HeadsArgs h = heads_args(n, batch, splits);
   h.yr = yr; h.a = a; h.beta = beta; h.train = 1; h.dd1 = n->dd1; h.part = part;
   h.g_wp = gp + n->off(P_PW); h.g_bp = gp + n->off(P_PB); h.g_wv = gp + n->off(P_VW); h.g_bv = gp + n->off(P_VB);
   h.g_b1 = gp + n->off(P_D1B); h.loss = gp + n->small_floats; h.gp_stride = n->gp_stride;
-  n->gp_heads_grid = fused ? dense_heads_ctas(batch) : heads_grid(batch, n->num_sms);
+  n->gp_heads_grid = heads_grid(batch, n->num_sms);
   n->loss_out = loss;
-  if (fused) LAUNCH(n, K_DENSE_FWD, st, launch_dense_heads(n->n2, n->w1_shadow, h, st));
-  else LAUNCH(n, K_HEADS, st, launch_heads(h, n->num_sms, st));
+  LAUNCH(n, K_HEADS, st, launch_heads(h, n->num_sms, st));
   (void)g;
   if (with_wgrad) LAUNCH(n, K_DENSE_WGRAD, st, launch_dense_wgrad_tc(n->n2, n->dd1, n->g + n->off(P_D1W), batch, st));
   n->last_batch = batch;
@@ -491,24 +441,25 @@ static GradReduceArgs reduce_args(ga3c_net* n, int batch, float* g_dst = nullptr
   r.part = n->gpart; r.stride = n->gp_stride; r.out = g_dst ? g_dst : n->g; r.out_tail = n->loss_out;
   r.out_floats = (int)n->small_floats; r.n_floats = (int)n->small_floats + 4;
   for (int s = 0; s < GR_MAX_SEG; ++s) { r.seg_end[s] = r.n_floats; r.seg_count[s] = n->gp_heads_grid; }
-  r.seg_end[0] = (int)n->off(P_D1B); r.seg_count[0] = conv_bwd_grid(batch, n->num_sms, n->cur_exch);
+  r.seg_end[0] = (int)n->off(P_D1B); r.seg_count[0] = conv_bwd_grid(batch, n->num_sms);
   return r;
 }
 
-// dense1 data gradient and the two conv backward kernels; with `reduce` the slabs are summed into the gradient arena
-// (conv11/*, conv12/*, dense1/b, heads, loss sums), otherwise the caller does it (fused with RMSProp).
-static WgradPush wgrad_push(const ga3c_net* n, uint64_t step) {
-  WgradPush p{};
-  for (int r = 0; r < n->dp_world; ++r) p.peer[r] = n->dp_peer[r];
-  p.rank = n->dp_rank; p.world = n->dp_world;
-  p.per4 = ((long long)FLAT * FC / 4 + n->dp_world - 1) / n->dp_world;
-  p.recv_off = n->bigrecv_off;
-  p.flag = (unsigned int)step;
-  return p;
+// the dense1/w exchange on the side stream, behind everything enqueued on `st` so far (dense1/w's gradient is final there)
+static int enqueue_dp_big(ga3c_net* n, const DpBigArgs& b, cudaStream_t st) {
+  CK(cudaEventRecord(n->dp_grad_ready, st));
+  CK(cudaStreamWaitEvent(n->dp_stream, n->dp_grad_ready, 0));
+  CKL(launch_dp_big_side(b, n->num_sms, n->dp_stream));
+  n->log.launches++;
+  n->dp_big_pending = true;
+  return 0;
 }
 
+// dense1 data gradient and the two conv backward kernels; with `reduce` the slabs are summed into the gradient arena
+// (conv11/*, conv12/*, dense1/b, heads, loss sums), otherwise the caller does it (fused with RMSProp).  With `dp` the dense1/w
+// exchange of the data-parallel step is launched on the side stream as soon as dense1/w's gradient is final.
 static int fb_tail_impl(ga3c_net* n, const void* x, bool x_u8, int32_t batch, void* stream, bool with_wgrad, bool reduce,
-                        const DpBigArgs* dp = nullptr, float* g_dst = nullptr, const ConvBwdOpt* opt = nullptr) {
+                        const DpBigArgs* dp = nullptr, float* g_dst = nullptr) {
   if (int r = check_batch(n, batch, "ga3c_fb_tail")) return r;
   if (!x) return fail_msg("ga3c_fb_tail: null buffer");
   if (batch != n->last_batch) return fail_msg("ga3c_fb_tail: batch differs from the preceding ga3c_fb_head");
@@ -516,26 +467,15 @@ static int fb_tail_impl(ga3c_net* n, const void* x, bool x_u8, int32_t batch, vo
   cudaStream_t st = (cudaStream_t)stream;
   const float* w = n->w;
   float* gp = n->gpart;
-  if (with_wgrad) {   // dgrad + wgrad tiles of dense1 in one grid
-    WgradPush push{};
-    const bool pushed = dp != nullptr && dp->pushed;
-    if (pushed) push = wgrad_push(n, dp->step);
-    LAUNCH(n, K_DENSE_DGRAD, st, launch_dense_bwd_tc(n->dd1, n->w1_shadow, n->n2, n->dn2, (g_dst ? g_dst : n->g) + n->off(P_D1W), batch,
-                                                     pushed ? &push : nullptr, st));
-  } else
+  if (with_wgrad)   // dgrad + wgrad tiles of dense1 in one grid
+    LAUNCH(n, K_DENSE_DGRAD, st, launch_dense_bwd_tc(n->dd1, n->w1_shadow, n->n2, n->dn2, (g_dst ? g_dst : n->g) + n->off(P_D1W), batch, st));
+  else
     LAUNCH(n, K_DENSE_DGRAD, st, launch_dense_dgrad_tc(n->dd1, n->w1_shadow, n->n2, n->dn2, batch, st));
-  if (n->dp_side != nullptr) {
-    // side-stream exchange of dense1/w: its gradient is final behind this point of the stream
-    CK(cudaEventRecord(n->dp_grad_ready, st));
-    CK(cudaStreamWaitEvent(n->dp_stream, n->dp_grad_ready, 0));
-    CKL(launch_dp_big_side(*n->dp_side, true, n->num_sms, n->dp_stream));
-    n->log.launches++;
-    CK(cudaEventRecord(n->dp_big_done, n->dp_stream));
-    n->dp_big_pending = true;
-  }
+  if (dp != nullptr)
+    if (int r = enqueue_dp_big(n, *dp, st)) return r;
   LAUNCH(n, K_CONV12_BWD, st, launch_conv_bwd(n->xblk, n->n1, n->dn2, w + n->off(P_C12W), n->keep_dn1 ? n->dn1 : nullptr,
                                               gp + n->off(P_C11W), gp + n->off(P_C11B), gp + n->off(P_C12W),
-                                              gp + n->off(P_C12B), n->gp_stride, batch, n->num_sms, x_u8, opt ? *opt : ConvBwdOpt{}, dp, st));
+                                              gp + n->off(P_C12B), n->gp_stride, batch, n->num_sms, x_u8, st));
   if (reduce) LAUNCH(n, K_GRAD_REDUCE, st, launch_grad_reduce(reduce_args(n, batch, g_dst), st));
   return 0;
 }
@@ -581,7 +521,7 @@ static ClipArgs clip_args(ga3c_net* n, int which = 0) {        // which: 0 the (
   return c;
 }
 
-static int apply_rmsprop_impl(ga3c_net* n, float lr, void* stream, const GradReduceArgs* red) {
+static int apply_rmsprop_impl(ga3c_net* n, float lr, void* stream) {
   if (!n) return fail_msg("ga3c_apply_rmsprop: null handle");
   CK(cudaSetDevice(n->cfg.device));
   RmsPropArgs a = rmsprop_args(n, lr);
@@ -594,25 +534,14 @@ static int apply_rmsprop_impl(ga3c_net* n, float lr, void* stream, const GradRed
     n->log.launches += 2;
     return 0;          // NetworkVP_discrate.py:121: apply_gradients without global_step -- the step counter stays put
   }
-  if (n->dp_world > 1) {
-    // fused reduce-scatter(grads) -> RMSProp on this rank's slice -> all-gather(weights) over peer memory
-    RmsPropDpArgs d{};
-    d.base = a;
-    for (int r = 0; r < n->dp_world; ++r) d.peer[r] = n->dp_peer[r];
-    d.rank = n->dp_rank; d.world = n->dp_world; d.step = ++n->dp_step;
-    d.arena_bytes = (int64_t)n->arena_floats * 4;
-    d.comm_offset = n->comm_off;
-    d.has_red = red != nullptr;
-    if (red) d.red = *red;
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_dp(d, n->num_sms, (cudaStream_t)stream));
-  } else {
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop(a, (cudaStream_t)stream));
-  }
+  // the peer-memory exchange is part of the train step (its dense1/w half starts behind dense_bwd, on a side stream)
+  if (n->dp_world > 1) return fail_msg("ga3c_apply_rmsprop: not available on a peer-memory data-parallel handle; use ga3c_train_step");
+  LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop(a, (cudaStream_t)stream));
   n->global_step += 1;   // opt.minimize(..., global_step=self.global_step), NetworkVP_discrate.py:130
   return 0;
 }
 
-extern "C" int ga3c_apply_rmsprop(ga3c_net* n, float lr, void* stream) { return apply_rmsprop_impl(n, lr, stream, nullptr); }
+extern "C" int ga3c_apply_rmsprop(ga3c_net* n, float lr, void* stream) { return apply_rmsprop_impl(n, lr, stream); }
 
 // ---- data parallel over CUDA IPC peer memory ---------------------------------------------------------
 extern "C" int ga3c_dp_handle_bytes(void) { return (int)sizeof(cudaIpcMemHandle_t); }
@@ -631,9 +560,8 @@ extern "C" int ga3c_dp_detach(ga3c_net* n) {
   if (n->dp_stream) {
     cudaStreamSynchronize(n->dp_stream);
     cudaStreamDestroy(n->dp_stream);
-    cudaEventDestroy(n->dp_big_done);
     cudaEventDestroy(n->dp_grad_ready);
-    n->dp_stream = nullptr; n->dp_big_done = nullptr; n->dp_big_pending = false;
+    n->dp_stream = nullptr; n->dp_big_pending = false;
   }
   for (int r = 0; r < DP_MAX_WORLD; ++r)
     if (n->dp_peer[r] && n->dp_ipc[r]) cudaIpcCloseMemHandle(n->dp_peer[r]);
@@ -690,26 +618,12 @@ extern "C" int ga3c_dp_attach_local(ga3c_net* n, int32_t rank, int32_t world, ga
 
 static int dp_attach_finish(ga3c_net* n, int32_t rank, int32_t world) {
   n->dp_rank = rank; n->dp_world = world; n->dp_step = 0;
-  n->dp_exchange = 4;
-  if (const char* e = getenv("GA3C_DP_EXCHANGE")) {
-    const std::string m(e);
-    if (m == "side") n->dp_exchange = 4;
-    else if (m == "warps") n->dp_exchange = 3;
-    else if (m == "tail") n->dp_exchange = 0;
-    else if (m == "overlap") n->dp_exchange = 1;
-    else if (m == "single") n->dp_exchange = 2;
-    else return fail_msg("GA3C_DP_EXCHANGE must be side, warps, tail, overlap or single");
-  }
-  if (const char* e = getenv("GA3C_DP_PUSH")) n->dp_push = atoi(e) != 0;
-  if (const char* e = getenv("GA3C_DP_EXCH_CTAS")) n->dp_exch = atoi(e);
-  if (n->dp_exch < 1 || n->dp_exch > n->num_sms / 2) n->dp_exch = 20;
   CK(cudaMemset(n->slab + n->xbuf_off, 0, n->slab_bytes - (size_t)n->xbuf_off));
   CKL(configure_dp());
   if (!n->dp_stream) {
     int lo = 0, hi = 0;
     cudaDeviceGetStreamPriorityRange(&lo, &hi);
     CK(cudaStreamCreateWithPriority(&n->dp_stream, cudaStreamNonBlocking, hi));
-    CK(cudaEventCreateWithFlags(&n->dp_big_done, cudaEventDisableTiming));
     CK(cudaEventCreateWithFlags(&n->dp_grad_ready, cudaEventDisableTiming));
   }
   n->dp_big_pending = false;
@@ -770,15 +684,13 @@ extern "C" int ga3c_dual_forward_backward_u8(ga3c_net* n, const uint8_t* x, cons
 }
 extern "C" int ga3c_dual_apply(ga3c_net* n, float lr, void* stream) { return dual_apply_impl(n, lr, stream); }
 
-static DpBigArgs dp_big_args(ga3c_net* n, float lr, int n_exch) {
+static DpBigArgs dp_big_args(ga3c_net* n, float lr) {
   DpBigArgs b{};
   for (int r = 0; r < n->dp_world; ++r) b.peer[r] = n->dp_peer[r];
-  b.rank = n->dp_rank; b.world = n->dp_world; b.n_exch = n_exch; b.step = ++n->dp_step;
+  b.rank = n->dp_rank; b.world = n->dp_world; b.step = ++n->dp_step;
   b.arena_bytes = (int64_t)n->arena_floats * 4; b.shadow_off = 4 * b.arena_bytes; b.comm_offset = n->comm_off;
   b.w1_offset = n->off(P_D1W); b.w1_count = (int64_t)FLAT * FC;
   b.lr = lr; b.decay = n->cfg.rmsprop_decay; b.momentum = n->cfg.rmsprop_momentum; b.eps = n->cfg.rmsprop_epsilon;
-  b.pushed = n->dp_exchange == 0 && n->dp_push;       // exchange at the end of the step: slices pushed by the wgrad epilogues
-  b.bigrecv_off = n->bigrecv_off;
   return b;
 }
 static RmsPropDpArgs dp_small_args(ga3c_net* n, float lr, int batch, const DpBigArgs& b) {
@@ -788,7 +700,7 @@ static RmsPropDpArgs dp_small_args(ga3c_net* n, float lr, int batch, const DpBig
   for (int q = 0; q < n->dp_world; ++q) d.peer[q] = n->dp_peer[q];
   d.rank = n->dp_rank; d.world = n->dp_world; d.step = b.step;
   d.arena_bytes = b.arena_bytes; d.comm_offset = n->comm_off;
-  d.has_red = 1; d.red = reduce_args(n, batch);
+  d.red = reduce_args(n, batch);
   return d;
 }
 
@@ -803,52 +715,13 @@ static int train_step_empty(ga3c_net* n, float lr, float* loss, void* stream) {
   n->gp_heads_grid = 0;
   n->loss_out = loss;
   n->last_batch = 0;
-  if (n->dp_exchange == 4) {          // side-stream exchange: it publishes "gradient final" itself; dp_small with zero slabs
-    CK(cudaMemsetAsync(n->g + n->off(P_D1W), 0, (size_t)FLAT * FC * 4, st));
-    DpBigArgs b = dp_big_args(n, lr, 0);
-    b.pushed = 0;
-    n->cur_exch = 0;
-    CK(cudaEventRecord(n->dp_grad_ready, st));                    // the zeroed gradient is in place
-    CK(cudaStreamWaitEvent(n->dp_stream, n->dp_grad_ready, 0));
-    CKL(launch_dp_big_side(b, true, n->num_sms, n->dp_stream));
-    n->log.launches++;
-    CK(cudaEventRecord(n->dp_big_done, n->dp_stream));
-    n->dp_big_pending = true;
-    const RmsPropDpArgs d = dp_small_args(n, lr, 0, b);
-    LAUNCH(n, K_RMSPROP, st, launch_dp_small(d, n->xbuf_off, st, false));
-    n->global_step += 1;
-    return 0;
-  }
-  if (n->dp_exchange == 0 || n->dp_exchange == 3) {   // nothing but the exchange launch (dp_tail: both instalments); it publishes "gradient final"
-    CK(cudaMemsetAsync(n->g + n->off(P_D1W), 0, (size_t)FLAT * FC * 4, st));
-    const DpBigArgs b = dp_big_args(n, lr, 0);
-    n->cur_exch = 0;
-    if (b.pushed) {
-      CKL(launch_dp_push_zero(wgrad_push(n, b.step), (long long)FLAT * FC / 4, st));
-      n->log.launches++;
-    }
-    const RmsPropDpArgs d = dp_small_args(n, lr, 0, b);    // zero slabs in every segment: the sums are 0
-    LAUNCH(n, K_RMSPROP, st, launch_dp_tail(d, b, n->xbuf_off, n->num_sms, st));
-    n->global_step += 1;
-    return 0;
-  }
-  if (n->dp_exchange == 1) {
-    CK(cudaMemsetAsync(n->g + n->off(P_D1W), 0, (size_t)FLAT * FC * 4, st));
-    const DpBigArgs b = dp_big_args(n, lr, n->dp_exch);
-    n->cur_exch = b.n_exch;
-    float* gp = n->gpart;
-    LAUNCH(n, K_CONV12_BWD, st, launch_conv_bwd(n->xblk, n->n1, n->dn2, n->w + n->off(P_C12W), nullptr,
-                                                gp + n->off(P_C11W), gp + n->off(P_C11B), gp + n->off(P_C12W),
-                                                gp + n->off(P_C12B), n->gp_stride, 0, n->num_sms, false, ConvBwdOpt{}, &b, st));
-    const RmsPropDpArgs d = dp_small_args(n, lr, 0, b);
-    n->cur_exch = 0;
-    LAUNCH(n, K_RMSPROP, st, launch_dp_small(d, n->xbuf_off, st, true));
-    n->global_step += 1;
-    return 0;
-  }
-  CK(cudaMemsetAsync(n->g, 0, (size_t)n->arena_floats * 4, st));
-  if (loss) CK(cudaMemsetAsync(loss, 0, 16, st));
-  return apply_rmsprop_impl(n, lr, stream, nullptr);
+  // the exchange publishes "gradient final" itself; dp_small sums zero slabs
+  CK(cudaMemsetAsync(n->g + n->off(P_D1W), 0, (size_t)FLAT * FC * 4, st));
+  const DpBigArgs b = dp_big_args(n, lr);
+  if (int r = enqueue_dp_big(n, b, st)) return r;                  // behind the zeroed gradient
+  LAUNCH(n, K_RMSPROP, st, launch_dp_small(dp_small_args(n, lr, 0, b), n->xbuf_off, st));
+  n->global_step += 1;
+  return 0;
 }
 
 static int train_step_impl(ga3c_net* n, const void* x, bool x_u8, const float* yr, const float* a, int32_t batch, float lr,
@@ -862,87 +735,25 @@ static int train_step_impl(ga3c_net* n, const void* x, bool x_u8, const float* y
   if (int r = fb_head_impl(n, x, x_u8, yr, a, batch, beta, loss, stream, false)) return r;
   if (n->cfg.use_grad_clip) {
     if (int r = fb_tail_impl(n, x, x_u8, batch, stream, true, true)) return r;
-    return apply_rmsprop_impl(n, lr, stream, nullptr);
+    return apply_rmsprop_impl(n, lr, stream);
   }
-  if (n->dp_world > 1 && n->dp_exchange == 4) {
-    // default: the conv backward keeps every SM; the exchange of dense1/w is launched behind dense_bwd on the side stream and
-    // runs next to it (and next to the conv forward of the following step); dp_small follows the conv
-    // backward on this stream with the small tensors.  dense_fwd of the next call waits for the exchange's completion event.
-    DpBigArgs b = dp_big_args(n, lr, 0);
-    b.pushed = 0;
-    n->cur_exch = 0;
+  if (n->dp_world > 1) {
+    // the conv backward keeps every SM; the exchange of dense1/w is launched behind dense_bwd on the side stream and runs next
+    // to it (and next to the conv forward of the following step); dp_small follows the conv backward on this stream with the
+    // small tensors.  dense_fwd of the next call waits for the exchange's flags (dp_gate).
     // (launched behind an event after dense_bwd, NOT on a flag the conv backward would publish: at batch >= 148 a spinning side
     //  grid that got its blocks resident first kept conv_bwd CTA 0 -- the publisher -- off its SM, and the step timed out)
-    n->dp_side = &b;
-    const int r = fb_tail_impl(n, x, x_u8, batch, stream, true, false);
-    n->dp_side = nullptr;
-    if (r) return r;
-    RmsPropDpArgs d = dp_small_args(n, lr, batch, b);
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_dp_small(d, n->xbuf_off, (cudaStream_t)stream, false));
-    n->global_step += 1;
-    return 0;
-  }
-  if (n->dp_world > 1 && n->dp_exchange == 3) {
-    // default: the dense1/w exchange rides on the optimizer warps of the conv backward CTAs (all SMs keep computing conv
-    // gradients); dp_small follows with the small tensors and holds the step open until every rank's slice has landed
-    const DpBigArgs b = dp_big_args(n, lr, 0);
-    n->cur_exch = 0;
-    ConvBwdOpt opt{};
-    opt.mode = 2;
-    if (int r = fb_tail_impl(n, x, x_u8, batch, stream, true, false, &b, nullptr, &opt)) return r;
-    const RmsPropDpArgs d = dp_small_args(n, lr, batch, b);
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_dp_small(d, n->xbuf_off, (cudaStream_t)stream, true));
-    n->global_step += 1;
-    return 0;
-  }
-  if (n->dp_world > 1 && n->dp_exchange == 0) {
-    // exchange at the end of the step (dp_tail_kernel): the conv backward keeps every SM; its CTA 0 publishes "dense1/w gradient
-    // final" to the peers as soon as dense_bwd is complete, so that no rank waits for another rank's gradient at the tail
-    const DpBigArgs b = dp_big_args(n, lr, 0);
-    n->cur_exch = 0;
+    const DpBigArgs b = dp_big_args(n, lr);
     if (int r = fb_tail_impl(n, x, x_u8, batch, stream, true, false, &b)) return r;
-    const RmsPropDpArgs d = dp_small_args(n, lr, batch, b);
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_dp_tail(d, b, n->xbuf_off, n->num_sms, (cudaStream_t)stream));
+    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_dp_small(dp_small_args(n, lr, batch, b), n->xbuf_off, (cudaStream_t)stream));
     n->global_step += 1;
     return 0;
   }
-  if (n->dp_world > 1 && n->dp_exchange == 1) {
-    // overlapped exchange (dp_exchange.cuh): dense1/w moves between the ranks on exchange CTAs of the conv backward
-    // launch; the small tensors follow in dp_small, which also holds the step open until every slice has landed
-    const DpBigArgs b = dp_big_args(n, lr, n->dp_exch);
-    n->cur_exch = b.n_exch;
-    int r = fb_tail_impl(n, x, x_u8, batch, stream, true, false, &b);
-    const RmsPropDpArgs d = dp_small_args(n, lr, batch, b);
-    n->cur_exch = 0;
-    if (r) return r;
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_dp_small(d, n->xbuf_off, (cudaStream_t)stream, true));
-    n->global_step += 1;
-    return 0;
-  }
-  if (n->dp_world == 1 && n->fuse_opt) {
-    // single GPU: dense1/w is updated by the optimizer warps of the conv backward CTAs; the launch at the end of the step sums the
-    // slabs and updates the small tensors
-    ConvBwdOpt opt{};
-    opt.mode = 1;
-    opt.g = n->g + n->off(P_D1W); opt.w = n->w + n->off(P_D1W); opt.ms = n->ms + n->off(P_D1W); opt.mom = n->mom + n->off(P_D1W);
-    opt.shadow = n->w1_shadow; opt.n4 = (long long)FLAT * FC / 4;
-    opt.lr = lr; opt.decay = n->cfg.rmsprop_decay; opt.momentum = n->cfg.rmsprop_momentum; opt.eps = n->cfg.rmsprop_epsilon;
-    if (int r = fb_tail_impl(n, x, x_u8, batch, stream, true, false, nullptr, nullptr, &opt)) return r;
-    RmsPropArgs ra = rmsprop_args(n, lr);
-    ra.n_floats = n->small_floats;                  // dense1/w is done
-    ra.preload = batch >= n->num_sms;
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_reduce(ra, reduce_args(n, batch), (cudaStream_t)stream));
-    n->global_step += 1;
-    return 0;
-  }
-  if (int r = fb_tail_impl(n, x, x_u8, batch, stream, true, false)) return r;
-  const GradReduceArgs red = reduce_args(n, batch);
-  if (n->dp_world > 1)            // peers read this rank's gradient arena: the exchange kernel first sums the slabs into it
-    return apply_rmsprop_impl(n, lr, stream, &red);
   // single GPU: the slab reduction rides in the optimizer launch
+  if (int r = fb_tail_impl(n, x, x_u8, batch, stream, true, false)) return r;
   RmsPropArgs ra = rmsprop_args(n, lr);
   ra.preload = batch >= n->num_sms;               // see rmsprop_reduce_kernel
-  LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_reduce(ra, red, (cudaStream_t)stream));
+  LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_reduce(ra, reduce_args(n, batch), (cudaStream_t)stream));
   n->global_step += 1;   // opt.minimize(..., global_step=self.global_step), NetworkVP_discrate.py:130
   return 0;
 }
@@ -1042,7 +853,7 @@ extern "C" const char* ga3c_kernel_name(int kid) { return (kid >= 0 && kid < K_C
 static int trace_attach_all(unsigned long long* buf) {
   int r;
   if ((r = trace_attach_conv_fwd(buf)) || (r = trace_attach_conv_bwd_fused(buf)) || (r = trace_attach_dense_tc(buf)) ||
-      (r = trace_attach_heads(buf)) || (r = trace_attach_dense_heads(buf)) || (r = trace_attach_elementwise(buf)) || (r = trace_attach_mlp(buf)) || (r = trace_attach_mlp_tc(buf)) || (r = trace_attach_mlp_stream(buf)))
+      (r = trace_attach_heads(buf)) || (r = trace_attach_elementwise(buf)) || (r = trace_attach_mlp(buf)) || (r = trace_attach_mlp_tc(buf)) || (r = trace_attach_mlp_stream(buf)))
     return r;
   return 0;
 }
@@ -1083,7 +894,6 @@ extern "C" int ga3c_evt_begin(ga3c_net* n) {
     CKL(evt_attach_conv_fwd(n->evt));
     CKL(evt_attach_conv_bwd(n->evt));
     CKL(evt_attach_elementwise(n->evt));
-    CKL(evt_attach_dense_heads(n->evt));
   } else {
     CKL(evt_attach_dense_tc(n->evt));
   }
@@ -1097,7 +907,6 @@ extern "C" int ga3c_evt_end(ga3c_net* n, uint64_t* records, int32_t cap, int32_t
   CKL(evt_attach_conv_fwd(nullptr));
   CKL(evt_attach_conv_bwd(nullptr));
   CKL(evt_attach_elementwise(nullptr));
-  CKL(evt_attach_dense_heads(nullptr));
   CKL(evt_attach_dense_tc(nullptr));
   std::vector<uint64_t> all((size_t)2 * 16384);
   CK(cudaMemcpy(all.data(), n->evt, all.size() * 8, cudaMemcpyDeviceToHost));

@@ -134,11 +134,16 @@ int ga3c_dual_forward_backward_u8(ga3c_net* net, const uint8_t* x8_dev, const fl
 /* ---- data parallel over peer memory (one process per GPU, one node, <= 8 ranks) ---------------------
  * Every rank exports a CUDA IPC handle of its state slab (ga3c_dp_export), the host exchanges the handles
  * (torch.distributed all_gather in ga3c_b200.Network) and attaches them in rank order (ga3c_dp_attach).  From
- * then on ga3c_apply_rmsprop is ONE fused kernel per rank: wait until every rank's gradients of this step are
- * final, sum this rank's slice of all gradient arenas over NVLink (fixed rank order => replicas bit-identical),
- * apply RMSProp to the slice, store the new weights into every rank's slab; the last block to finish publishes
- * "done" and holds the kernel open until every rank is done, so the next forward sees all slices.  SUM, no averaging:
- * every loss term is a reduce_sum (NetworkVP_discrate.py:61,:83-85).  All ranks must call train the same number
+ * then on ga3c_train_step exchanges the gradients and updates the weights inside the step, in two instalments
+ * (dp_exchange.cuh).  dense1/w: as soon as its gradient is final, a kernel on a side stream of the handle sums this
+ * rank's slice of every rank's gradient over NVLink, applies RMSProp to the slice and stores its bf16 copy into every
+ * rank's slab, while the conv backward runs; the fp32 weights and slots of a slice stay on the rank that owns it
+ * (ga3c_arena_download collects them).  The other variables: after the conv backward every rank pushes its gradient
+ * to every rank, and every rank applies the identical update to its own copy.  Sums in fixed rank order, so the
+ * replicas stay bit-identical; the next forward waits until every rank's dense1/w slice has landed.  SUM, no averaging:
+ * every loss term is a reduce_sum (NetworkVP_discrate.py:61,:83-85).  ga3c_apply_rmsprop refuses an attached handle
+ * (use ga3c_train_step), and ga3c_train_step refuses one created with use_grad_clip or dual_rmsprop.  All ranks must call
+ * train the same number
  * of times; a rank with nothing to train on calls ga3c_train_step with batch = 0 (buffers may be NULL): it contributes a
  * zero gradient and applies the same update as everybody else (the host-side lock step that makes the reference's
  * asynchronous trainer loop, ThreadTrainer.py:42-62, fit this rule is ga3c_b200.threads.LockstepTrainer). */

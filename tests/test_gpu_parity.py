@@ -158,23 +158,18 @@ def test_log_softmax_knob(ga3c):
     assert np.allclose(p.sum(axis=1), 1.0, atol=1e-5)
 
 
-@pytest.mark.parametrize("exchange", ["side", "tail", "warps", "overlap"])
-def test_data_parallel_exchange_two_ranks_on_one_gpu(ga3c, monkeypatch, exchange):
-    """The fused data-parallel step (dp_exchange.cuh; "side", the default: dense1/w exchanged by a small-footprint kernel on a
-    side stream next to the conv kernels, LL push of the small tensors after the conv backward; "tail": the whole exchange in
-    one launch at the end of the step; "warps": dense1/w on the optimizer warps of every conv backward CTA; "overlap": on extra
-    exchange CTAs of the conv backward launch) with BOTH ranks on one device: two handles attached to each other with ga3c_dp_attach_local, each on its
-    own stream, each training on its row shard.  After 3 steps the replicas are bit-identical and equal the oracle's
-    single-process steps on the concatenated batch (what a single ThreadTrainer would have computed).  The grids are small
-    (12 rows per rank), so both ranks' kernels are resident together; every cross-rank wait is bounded, so a scheduling
-    surprise fails the test instead of hanging the GPU."""
+def test_data_parallel_exchange_two_ranks_on_one_gpu(ga3c, monkeypatch):
+    """The fused data-parallel step (dp_exchange.cuh: dense1/w exchanged by a small-footprint kernel on a side stream next to
+    the conv kernels, LL push of the small tensors after the conv backward) with BOTH ranks on one device: two handles attached
+    to each other with ga3c_dp_attach_local, each on its own stream, each training on its row shard.  After 3 steps the replicas
+    are bit-identical and equal the oracle's single-process steps on the concatenated batch (what a single ThreadTrainer would
+    have computed).  The grids are small (12 rows per rank), so both ranks' kernels are resident together; every cross-rank
+    wait is bounded, so a scheduling surprise fails the test instead of hanging the GPU.  ga3c_apply_rmsprop refuses an
+    attached handle: its exchange is part of ga3c_train_step."""
     import ctypes as C
     import torch
     from ga3c_b200 import _capi
-    monkeypatch.setenv("GA3C_DP_EXCHANGE", exchange)
-    monkeypatch.setenv("GA3C_DP_EXCH_CTAS", "4")
-    monkeypatch.setenv("GA3C_DP_TAIL_CTAS", "8")      # both ranks share this GPU: leave SMs for the other rank's conv kernels
-    monkeypatch.setenv("GA3C_DP_SIDE_CTAS", "8")
+    monkeypatch.setenv("GA3C_DP_SIDE_CTAS", "8")      # both ranks share this GPU: leave room for the other rank's conv kernels
     world, b = 2, 12
     rng = np.random.default_rng(17)
     params = onp.init_params(rng, 6)
@@ -221,6 +216,8 @@ def test_data_parallel_exchange_two_ranks_on_one_gpu(ga3c, monkeypatch, exchange
             assert np.array_equal(w[0][k], w[1][k]) and np.array_equal(m[0][k], m[1][k]), k     # replicas bit-identical
             assert np.abs(w[0][k] - ref[k]).max() <= 4 * TOL_W_ABS, (k, np.abs(w[0][k] - ref[k]).max())
         assert nets[0].get_global_step() == 4 and nets[1].get_global_step() == 4
+        assert lib.ga3c_apply_rmsprop(nets[0]._h, C.c_float(1e-3), None) != 0
+        assert b"ga3c_train_step" in lib.ga3c_last_error()
     finally:
         for n in nets:
             lib.ga3c_dp_detach(n._h)

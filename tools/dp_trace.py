@@ -50,9 +50,8 @@ buf = (C.c_uint64 * (2 * 16384))(); cnt = C.c_int32()
 _capi.check(lib.ga3c_evt_end(net._h, buf, 16384, C.byref(cnt)), "evt_end")
 if rank == 0:
     recs = sorted((buf[2 * i], buf[2 * i + 1] >> 32, (buf[2 * i + 1] >> 16) & 0xFFFF, buf[2 * i + 1] & 0xFFFF) for i in range(cnt.value))
-    names = {60: "dp: launched", 61: "dp: dependency satisfied", 62: "dp: all ranks ready | dp_small: slabs summed", 66: "dp_small: fence + flags pushed",
-             63: "dp: loop done | dp_small: every rank's column block arrived", 64: "dp: fence done | dp_small: updated", 65: "dp: last block saw all done | dp_small: every dense1/w slice landed",
-             70: "big: every rank's dense_bwd-done flag seen", 71: "big: loop done (thread 0)", 72: "big: block fenced + counted", 67: "big: exchange returned"}
+    names = {60: "dp_small: launched", 61: "dp_small: dependency satisfied", 62: "dp_small: slabs summed", 66: "dp_small: sums pushed",
+             63: "dp_small: every rank's column block arrived", 64: "dp_small: updated"}
     t0 = recs[0][0]
     for t, w, e, arg in recs:
         if e >= 60 and w == 0: print(f"{(t - t0) / 1e3:9.2f} us  {names.get(e, e)} {arg}")
