@@ -4,6 +4,7 @@ from __future__ import annotations
 
 import numpy as np
 
+from oracle import oracle_mlp as om
 from oracle import oracle_np as onp
 
 
@@ -13,6 +14,48 @@ def make_case(batch: int, num_actions: int = 6, seed: int = 12345):
     x = onp.synth_frames(rng, batch)
     y_r, a = onp.synth_targets(rng, batch, num_actions)
     return params, x, y_r, a
+
+
+def make_mlp_net(mlp, kind: str, s: int, a: int, **kw):
+    """The MLP network of `kind` ('fork_vp': NetworkVP, 'discrate': NetworkVP_discrate) for state size s and a actions; kw go to
+    the constructor (config=, max_batch=, seed=)."""
+    cls = mlp.NetworkVP if kind == "fork_vp" else mlp.NetworkVP_discrate
+    return cls("gpu:0", "test" + kind.replace("_", ""), a, s, **kw)   # no "_": the reference parses the episode out of the name
+
+
+# fork_vp: least distance of (sigmoid(out_x), sigmoid(out_y)) from (0.5, 0.5), where p = atan2(Y, X) / pi is singular
+ANGLE_R_MIN = 0.01
+
+
+def near_angle_singularity(params, x):
+    """fork_vp: which rows of x have an angle closer than ANGLE_R_MIN to the singular point of the angle head under `params`."""
+    _, _, f = om.forward(params, x, "fork_vp", keep=True)
+    return (np.hypot(f["ox"] - 0.5, f["oy"] - 0.5) < ANGLE_R_MIN).any(axis=1)
+
+
+def make_mlp_case(kind: str, s: int, a: int, b: int, seed: int = 12345, dense_layers=om.DISCRATE_DENSE_LAYERS):
+    """Seeded MLP weights (dense_layers = Config.DENSE_LAYERS, 'discrate' only) and b rows of x, y_r and actions.
+
+    fork_vp: rows with an angle closer than ANGLE_R_MIN to the singular point of the angle head are redrawn.  There X = sigmoid(z_x)
+    - 0.5 and Y carry the fp32 rounding of sigmoid near 0.5 (delta = 2^-23, one ulp), which p amplifies by up to sqrt(2) / (pi r)
+    and the out_x / out_y gradients by 1 / r^2: any fp32 implementation differs from the fp64 oracle there, TF's included.  Measured
+    on a B200 for (256, 18) at 5,000 rows, with an angle at r = 7.3e-4: |dp| = 5.55e-5 (the oracle itself run in fp32: 4.5e-5) and
+    1.15e-3 relative in logits_p/out_y/w (2.9e-5 with the 42 rows that hold an angle at r < 5e-3 removed).  At r >= ANGLE_R_MIN
+    the bound is sqrt(2) 2^-23 / (pi r) <= 5.4e-6 for p, a quarter of the p, v tolerance.  The rows drawn for state_dim 3 and 4
+    lie at r > 0.05 and are never redrawn.  Training moves the angles: a test that trains checks them at every step's weights."""
+    rng = np.random.default_rng(seed)
+    params = om.init_params(rng, kind, s, a, dense_layers)
+    x = rng.uniform(-1, 1, size=(b, s)).astype(np.float32)
+    y_r = rng.uniform(-1, 1, size=b).astype(np.float32)
+    if kind == "fork_vp":
+        act = rng.uniform(-1, 1, size=(b, a)).astype(np.float32)      # continuous action (ProcessAgent.py:92-93)
+        rows = np.arange(b)
+        while rows.size:
+            rows = rows[near_angle_singularity(params, x[rows])]
+            x[rows] = rng.uniform(-1, 1, size=(rows.size, s)).astype(np.float32)
+    else:
+        act = np.eye(a, dtype=np.float32)[rng.integers(0, a, size=b)]
+    return params, x, y_r, act
 
 
 def err(got, ref):

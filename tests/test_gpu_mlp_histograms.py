@@ -7,6 +7,7 @@ import pytest
 
 from oracle import histogram_np as oh
 from oracle import oracle_mlp as om
+from _parity import make_mlp_case, make_mlp_net
 
 pytestmark = pytest.mark.gpu
 
@@ -20,23 +21,6 @@ def mlp():
         pytest.fail("GPU tests need a CUDA device; there is no CPU fallback")
     from ga3c_b200 import mlp_network
     return mlp_network
-
-
-def make_net(mlp, kind, s, a, **kw):
-    cls = mlp.NetworkVP if kind == "fork_vp" else mlp.NetworkVP_discrate
-    return cls("gpu:0", "hist" + kind.replace("_", ""), a, s, **kw)
-
-
-def make_case(kind, s, a, b, seed=12345, dense_layers=om.DISCRATE_DENSE_LAYERS):
-    rng = np.random.default_rng(seed)
-    params = om.init_params(rng, kind, s, a, dense_layers)
-    x = rng.uniform(-1, 1, size=(b, s)).astype(np.float32)
-    y_r = rng.uniform(-1, 1, size=b).astype(np.float32)
-    if kind == "fork_vp":
-        act = rng.uniform(-1, 1, size=(b, a)).astype(np.float32)
-    else:
-        act = np.eye(a, dtype=np.float32)[rng.integers(0, a, size=b)]
-    return params, x, y_r, act
 
 
 def assert_matches(got, x, tag=""):
@@ -71,8 +55,8 @@ def check_against_the_network(net, kind, x, y_r, act, dense_layers=om.DISCRATE_D
 @pytest.mark.parametrize("kind,s,a", CASES)
 @pytest.mark.parametrize("b", [1, 63, 1000, 4097])
 def test_histograms_match_the_oracle(mlp, kind, s, a, b):
-    params, x, y_r, act = make_case(kind, s, a, b)
-    net = make_net(mlp, kind, s, a, max_batch=b)
+    params, x, y_r, act = make_mlp_case(kind, s, a, b)
+    net = make_mlp_net(mlp, kind, s, a, max_batch=b)
     net.set_variables(params)
     check_against_the_network(net, kind, x, y_r, act)
 
@@ -84,8 +68,8 @@ def test_histograms_on_the_tensor_core_path(mlp, monkeypatch, stream):
     monkeypatch.setenv("GA3C_MLP_TC", "1")
     monkeypatch.setenv("GA3C_MLP_STREAM", stream)
     kind, s, a, b = "fork_vp", 3, 1, 1000
-    params, x, y_r, act = make_case(kind, s, a, b, seed=3)
-    net = make_net(mlp, kind, s, a, max_batch=b)
+    params, x, y_r, act = make_mlp_case(kind, s, a, b, seed=3)
+    net = make_mlp_net(mlp, kind, s, a, max_batch=b)
     net.set_variables(params)
     n0 = net.launch_count()
     net.predict_p_and_v(x)
@@ -101,8 +85,8 @@ def test_discrate_with_eight_dense_layers_uses_every_source(mlp):
     class Cfg(mlp._DefaultConfig):
         DENSE_LAYERS = dense
     kind, s, a, b = "discrate", 4, 2, 777
-    params, x, y_r, act = make_case(kind, s, a, b, seed=5, dense_layers=dense)
-    net = make_net(mlp, kind, s, a, config=Cfg, max_batch=b)
+    params, x, y_r, act = make_mlp_case(kind, s, a, b, seed=5, dense_layers=dense)
+    net = make_mlp_net(mlp, kind, s, a, config=Cfg, max_batch=b)
     net.set_variables(params)
     assert net._lib.ga3c_mlp_histogram_count(net._h) == 23
     for _ in range(3):
@@ -117,8 +101,8 @@ def test_discrate_with_eight_dense_layers_uses_every_source(mlp):
 
 def test_histograms_are_bit_identical_from_call_to_call(mlp):
     kind, s, a, b = "fork_vp", 3, 1, 65536           # multi-block sources: the fp64 moments are merged in block order
-    params, x, y_r, act = make_case(kind, s, a, b, seed=9)
-    net = make_net(mlp, kind, s, a, max_batch=b)
+    params, x, y_r, act = make_mlp_case(kind, s, a, b, seed=9)
+    net = make_mlp_net(mlp, kind, s, a, max_batch=b)
     net.set_variables(params)
     first = net.histograms(x, y_r, act)
     again = net.histograms(x, y_r, act)
@@ -129,8 +113,8 @@ def test_histograms_are_bit_identical_from_call_to_call(mlp):
 
 def test_kernel_times_report_the_histograms(mlp):
     kind, s, a, b = "discrate", 4, 2, 100
-    params, x, y_r, act = make_case(kind, s, a, b)
-    net = make_net(mlp, kind, s, a)
+    params, x, y_r, act = make_mlp_case(kind, s, a, b)
+    net = make_mlp_net(mlp, kind, s, a)
     net.set_variables(params)
     net.kernel_timing(64)
     net.kernel_times()
@@ -146,8 +130,8 @@ def test_log_writes_events_and_leaves_the_state_alone(mlp, tmp_path, monkeypatch
     from tensorboard.backend.event_processing import event_accumulator
     from ga3c_b200 import summaries
     monkeypatch.chdir(tmp_path)
-    params, x, y_r, act = make_case(kind, s, a, 300, seed=17)
-    net = make_net(mlp, kind, s, a)
+    params, x, y_r, act = make_mlp_case(kind, s, a, 300, seed=17)
+    net = make_mlp_net(mlp, kind, s, a)
     net.set_variables(params)
     net.learning_rate, net.beta = 1e-4, 0.02
     ms0, mom0 = net.get_slots()
@@ -193,8 +177,8 @@ def test_histograms_refuse_a_batch_other_than_the_last_forward(mlp):
     import torch
     from ga3c_b200 import _capi
     kind, s, a = "fork_vp", 3, 1
-    params, x, y_r, act = make_case(kind, s, a, 64)
-    net = make_net(mlp, kind, s, a)
+    params, x, y_r, act = make_mlp_case(kind, s, a, 64)
+    net = make_mlp_net(mlp, kind, s, a)
     net.set_variables(params)
     lib, n_src = net._lib, net._lib.ga3c_mlp_histogram_count(net._h)
     out = torch.empty(n_src * (5 + 1551), dtype=torch.float64, device="cuda:0")
