@@ -8,19 +8,19 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GA3C_LIB") or os.path.join(_HERE, "_lib", "libga3c_b200.so")     # GA3C_LIB: A/B runs of two builds on one box
 
 
-class ga3c_config(C.Structure):
-    _fields_ = [("device", C.c_int32), ("num_actions", C.c_int32), ("max_batch", C.c_int32),
-                ("rmsprop_decay", C.c_float), ("rmsprop_momentum", C.c_float), ("rmsprop_epsilon", C.c_float),
+# the optimizer and loss fields both network configs end with
+_CONFIG_TAIL = [("rmsprop_decay", C.c_float), ("rmsprop_momentum", C.c_float), ("rmsprop_epsilon", C.c_float),
                 ("log_epsilon", C.c_float), ("min_policy", C.c_float), ("use_log_softmax", C.c_int32),
                 ("use_grad_clip", C.c_int32), ("grad_clip_norm", C.c_float), ("dual_rmsprop", C.c_int32)]
+
+
+class ga3c_config(C.Structure):
+    _fields_ = [("device", C.c_int32), ("num_actions", C.c_int32), ("max_batch", C.c_int32)] + _CONFIG_TAIL
 
 
 class ga3c_mlp_config(C.Structure):
     _fields_ = [("device", C.c_int32), ("kind", C.c_int32), ("state_dim", C.c_int32), ("num_actions", C.c_int32),
-                ("max_batch", C.c_int32), ("n_dense", C.c_int32), ("dense_width", C.c_int32 * 8),
-                ("rmsprop_decay", C.c_float), ("rmsprop_momentum", C.c_float), ("rmsprop_epsilon", C.c_float),
-                ("log_epsilon", C.c_float), ("min_policy", C.c_float), ("use_log_softmax", C.c_int32),
-                ("use_grad_clip", C.c_int32), ("grad_clip_norm", C.c_float), ("dual_rmsprop", C.c_int32)]
+                ("max_batch", C.c_int32), ("n_dense", C.c_int32), ("dense_width", C.c_int32 * 8)] + _CONFIG_TAIL
 
 
 class ga3c_batcher_config(C.Structure):

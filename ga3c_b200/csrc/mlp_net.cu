@@ -4,56 +4,24 @@
 #include <algorithm>
 #include <vector>
 
-#include "../../include/ga3c_b200.h"
-#include "common.cuh"
-#include "kernels.h"
-#include "host_util.h"
+#include "handle.h"
 #include "mlp.cuh"
 
 using namespace ga3c;
 
-namespace {
-
-int fail(const char* where, cudaError_t e) { return fail_cuda(where, e); }
-
-struct MlpParam {
-  std::string name;
-  int64_t offset, count;
-  int32_t ndim;
-  int64_t shape[4];
-  int32_t live;
-};
-
-constexpr int64_t ALIGN_FLOATS = 64;
-int64_t align_up(int64_t v) { return (v + ALIGN_FLOATS - 1) / ALIGN_FLOATS * ALIGN_FLOATS; }
-
-}  // namespace
-
-struct ga3c_mlp {
-  ga3c_mlp_config cfg;
-  int num_sms = 148;
+struct ga3c_mlp : Handle<ga3c_mlp_config> {
   MlpNet net{};
-  std::vector<MlpParam> params;          // TF creation order
-  int64_t arena_floats = 0, live_floats = 0;   // live tensors are packed first; [live_floats, arena_floats) is never updated
-  float *w = nullptr, *g = nullptr, *ms = nullptr, *mom = nullptr;
+  int64_t live_floats = 0;               // live tensors are packed first; [live_floats, arena_floats) is never updated
   float* part = nullptr;                 // [MLP_MAX_SPLITS][live_floats] weight-gradient partial arenas
-  float *clip_ss = nullptr, *clip_scale = nullptr;   // Config.USE_GRAD_CLIP scratch
-  float *clip_ss2 = nullptr, *clip_scale2 = nullptr; // ... of the second optimizer's gradient (DUAL_RMSPROP + USE_GRAD_CLIP)
-  float *g2 = nullptr, *ms2 = nullptr, *mom2 = nullptr;   // Config.DUAL_RMSPROP: gradient of cost_v, second optimizer's slots
   int64_t skip_lo[2] = {}, skip_hi[2] = {};          // arena ranges of logits_v/* and of the policy head
-  // workspace for max_batch rows
+  // workspace for max_batch rows; last_batch: rows of act[] written by the last forward (0: none since it was allocated)
   float* act[MLP_MAX_LAYERS] = {};
   float* dz[MLP_MAX_LAYERS] = {};
   float* dlogits = nullptr;
   float* loss_part = nullptr;
-  int last_batch = 0;                    // rows of act[] written by the last forward (0: none since the workspace was allocated)
-  double* histo_part = nullptr;          // ga3c_mlp_histograms: fp64 partial moments per block
-  size_t histo_part_bytes = 0;
-  int64_t global_step = 0;
   // tensor-core mode (mlp_tc.cu): the run of wide layers [tc_lo, tc_hi) as 3xTF32 GEMMs for training batches >= tc_min_batch
   int tc_lo = 0, tc_hi = 0, tc_min_batch = 4096;
-  bool stream_ok = false, stream_ok_pending = false;                // ... with the narrow ends as streaming passes (mlp_stream.cu; GA3C_MLP_STREAM=0: fused-kernel phases)
-  LaunchLog log;                         // launch counter + per-kernel CUDA-event timing (ga3c_mlp_timing_*)
+  bool stream_ok = false;                // ... with the narrow ends as streaming passes (mlp_stream.cu)
 };
 
 static void free_workspace(ga3c_mlp* n) {
@@ -78,12 +46,9 @@ static int alloc_workspace(ga3c_mlp* n, int max_batch) {
 
 extern "C" int ga3c_mlp_destroy(ga3c_mlp* n) {
   if (!n) return 0;
-  cudaFree(n->w); cudaFree(n->g); cudaFree(n->ms); cudaFree(n->mom); cudaFree(n->part);
-  cudaFree(n->clip_ss); cudaFree(n->clip_scale); cudaFree(n->clip_ss2); cudaFree(n->clip_scale2);
-  cudaFree(n->g2); cudaFree(n->ms2); cudaFree(n->mom2);
-  cudaFree(n->histo_part);
+  free_arenas(n);
+  cudaFree(n->part);
   free_workspace(n);
-  n->log.clear();
   delete n;
   return 0;
 }
@@ -102,26 +67,20 @@ extern "C" int ga3c_mlp_create(const ga3c_mlp_config* cfg, ga3c_mlp** out) {
         return set_error("ga3c_mlp_create: dense widths must be 1..256");
     if (cfg->dense_width[cfg->n_dense - 1] > MLP_MAX_HID) return set_error("ga3c_mlp_create: the last dense width must be <= 128");
   }
-  int ndev = 0;
-  cudaError_t e = cudaGetDeviceCount(&ndev);
-  if (e != cudaSuccess || ndev == 0) return set_error("ga3c_mlp_create: no CUDA device (there is no CPU fallback)");
-  if (cfg->device < 0 || cfg->device >= ndev) return set_error("ga3c_mlp_create: device ordinal out of range");
-  CK(cudaSetDevice(cfg->device));
-  cudaDeviceProp prop;
-  CK(cudaGetDeviceProperties(&prop, cfg->device));
-  if (prop.major != 10) return set_error("ga3c_mlp_create: kernels are built for sm_100a only");
+  int num_sms = 0;
+  if (int r = open_device(cfg->device, "ga3c_mlp_create", &num_sms)) return r;
 
   ga3c_mlp* n = new ga3c_mlp();
   n->cfg = *cfg;
-  n->num_sms = prop.multiProcessorCount;
+  n->num_sms = num_sms;
   const int S = cfg->state_dim, A = cfg->num_actions;
   MlpNet& net = n->net;
   net.kind = cfg->kind; net.state_dim = S; net.num_actions = A;
   net.log_eps = cfg->log_epsilon; net.min_policy = cfg->min_policy; net.log_softmax = cfg->use_log_softmax != 0;
 
   auto add = [&](const std::string& scope, int k, int width, int live) {    // dense_layer: 'w' [k, width] then 'b' [width]
-    MlpParam w{scope + "/w:0", 0, (int64_t)k * width, 2, {k, width, 0, 0}, live};
-    MlpParam b{scope + "/b:0", 0, (int64_t)width, 1, {width, 0, 0, 0}, live};
+    Param w{scope + "/w:0", 0, (int64_t)k * width, 2, {k, width, 0, 0}, live};
+    Param b{scope + "/b:0", 0, (int64_t)width, 1, {width, 0, 0, 0}, live};
     n->params.push_back(w); n->params.push_back(b);
     return (int)n->params.size() - 2;
   };
@@ -157,8 +116,6 @@ extern "C" int ga3c_mlp_create(const ga3c_mlp_config* cfg, ga3c_mlp** out) {
       const int v = atoi(e);
       if (v <= 0) n->tc_lo = n->tc_hi = 0; else n->tc_min_batch = v;
     }
-    const char* es = getenv("GA3C_MLP_STREAM");
-    n->stream_ok_pending = !(es && atoi(es) == 0);
   }
   const int pv = add("logits_v", net.hid, 1, 1);
   int px, py = -1;
@@ -173,7 +130,7 @@ extern "C" int ga3c_mlp_create(const ga3c_mlp_config* cfg, ga3c_mlp** out) {
   net.n_out_ld = (net.n_out + 3) & ~3;
   int64_t cur = 0;
   for (int pass = 1; pass >= 0; --pass) {          // live tensors first, then the gradient-less ones
-    for (MlpParam& p : n->params)
+    for (Param& p : n->params)
       if (p.live == pass) { p.offset = cur; cur = align_up(cur + p.count); }
     if (pass == 1) n->live_floats = cur;
   }
@@ -188,34 +145,10 @@ extern "C" int ga3c_mlp_create(const ga3c_mlp_config* cfg, ga3c_mlp** out) {
   n->skip_lo[0] = n->params[pv].offset; n->skip_hi[0] = n->params[pv + 1].offset + n->params[pv + 1].count;
   const int plast = py >= 0 ? py + 1 : px + 1;      // the policy head's variables are consecutive in the arena
   n->skip_lo[1] = n->params[px].offset; n->skip_hi[1] = n->params[plast].offset + n->params[plast].count;
-  n->stream_ok = n->stream_ok_pending && n->tc_hi > n->tc_lo && mlp_stream_ok(net, n->tc_lo, n->tc_hi);
+  n->stream_ok = n->tc_hi > n->tc_lo && mlp_stream_ok(net, n->tc_lo, n->tc_hi);
 
-  const size_t ab = (size_t)n->arena_floats * 4;
-  float** arenas[4] = {&n->w, &n->g, &n->ms, &n->mom};
-  for (float** a : arenas) {
-    e = cudaMalloc((void**)a, ab);
-    if (e != cudaSuccess) { ga3c_mlp_destroy(n); return fail("cudaMalloc", e); }
-    cudaMemset(*a, 0, ab);
-  }
-  {  // ms slot starts at 1.0 [TF-SEMANTICS]
-    std::vector<float> ones((size_t)n->arena_floats, 1.0f);
-    cudaMemcpy(n->ms, ones.data(), ab, cudaMemcpyHostToDevice);
-  }
-  e = cudaMalloc((void**)&n->part, (size_t)MLP_MAX_SPLITS * n->live_floats * 4);
-  if (e != cudaSuccess) { ga3c_mlp_destroy(n); return fail("cudaMalloc", e); }
-  cudaMemset(n->part, 0, (size_t)MLP_MAX_SPLITS * n->live_floats * 4);
-  if (cfg->dual_rmsprop) {
-    float** extra[3] = {&n->g2, &n->ms2, &n->mom2};
-    for (float** a : extra) {
-      e = cudaMalloc((void**)a, ab);
-      if (e != cudaSuccess) { ga3c_mlp_destroy(n); return fail("cudaMalloc", e); }
-      cudaMemset(*a, 0, ab);
-    }
-    std::vector<float> ones((size_t)n->arena_floats, 1.0f);
-    cudaMemcpy(n->ms2, ones.data(), ab, cudaMemcpyHostToDevice);
-  }
   if (cfg->use_grad_clip) {
-    for (const MlpParam& p : n->params)
+    for (const Param& p : n->params)
       if (!p.live && !cfg->dual_rmsprop) {     // opt.compute_gradients yields (None, var) and tf.clip_by_average_norm(None, ..) raises;
                                                // the DUAL_RMSPROP branch filters `if not g is None` (NetworkVP_discrate.py:110,:115)
         ga3c_mlp_destroy(n);
@@ -223,20 +156,15 @@ extern "C" int ga3c_mlp_create(const ga3c_mlp_config* cfg, ga3c_mlp** out) {
                          "DENSE_LAYERS entry from x): the reference graph cannot be built either");
       }
     if ((int)n->params.size() > CLIP_MAX_TENSORS) { ga3c_mlp_destroy(n); return set_error("ga3c_mlp_create: too many variables for USE_GRAD_CLIP"); }
-    int64_t mx = 0;
-    for (const MlpParam& p : n->params) mx = p.count > mx ? p.count : mx;
-    e = cudaMalloc((void**)&n->clip_ss, n->params.size() * clip_chunks(mx) * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc((void**)&n->clip_scale, n->params.size() * sizeof(float));
-    if (e == cudaSuccess && cfg->dual_rmsprop) {
-      e = cudaMalloc((void**)&n->clip_ss2, n->params.size() * clip_chunks(mx) * sizeof(float));
-      if (e == cudaSuccess) e = cudaMalloc((void**)&n->clip_scale2, n->params.size() * sizeof(float));
-    }
-    if (e != cudaSuccess) { ga3c_mlp_destroy(n); return fail("cudaMalloc", e); }
   }
+  if (int r = alloc_arenas(n, 0)) { ga3c_mlp_destroy(n); return r; }
+  cudaError_t e = cudaMalloc((void**)&n->part, (size_t)MLP_MAX_SPLITS * n->live_floats * 4);
+  if (e != cudaSuccess) { ga3c_mlp_destroy(n); return fail_cuda("cudaMalloc", e); }
+  cudaMemset(n->part, 0, (size_t)MLP_MAX_SPLITS * n->live_floats * 4);
   if (int r = alloc_workspace(n, cfg->max_batch)) { ga3c_mlp_destroy(n); return r; }
-  if (int r = configure_mlp()) { ga3c_mlp_destroy(n); return fail("cudaFuncSetAttribute", (cudaError_t)r); }
+  if (int r = configure_mlp()) { ga3c_mlp_destroy(n); return fail_cuda("cudaFuncSetAttribute", (cudaError_t)r); }
   e = cudaDeviceSynchronize();
-  if (e != cudaSuccess) { ga3c_mlp_destroy(n); return fail("ga3c_mlp_create sync", e); }
+  if (e != cudaSuccess) { ga3c_mlp_destroy(n); return fail_cuda("ga3c_mlp_create sync", e); }
   *out = n;
   return 0;
 }
@@ -256,44 +184,17 @@ extern "C" int ga3c_mlp_param_count(const ga3c_mlp* n) { return n ? (int)n->para
 
 extern "C" int ga3c_mlp_param_info(const ga3c_mlp* n, int i, const char** name, int64_t* offset, int32_t* ndim,
                                    int64_t shape[4], int32_t* live) {
-  if (!n || i < 0 || i >= (int)n->params.size()) return set_error("ga3c_mlp_param_info: bad index");
-  const MlpParam& d = n->params[i];
-  if (name) *name = d.name.c_str();
-  if (offset) *offset = d.offset;
-  if (ndim) *ndim = d.ndim;
-  if (shape) for (int k = 0; k < 4; ++k) shape[k] = d.shape[k];
-  if (live) *live = d.live;
-  return 0;
+  return param_info(n, i, name, offset, ndim, shape, live, "ga3c_mlp_param_info");
 }
 
 extern "C" int64_t ga3c_mlp_arena_floats(const ga3c_mlp* n) { return n ? n->arena_floats : 0; }
 
-static float* arena_of(ga3c_mlp* n, int which) {
-  switch (which) {
-    case 0: return n->w; case 1: return n->g; case 2: return n->ms; case 3: return n->mom;
-    case 4: return n->g2; case 5: return n->ms2; case 6: return n->mom2;      // null unless dual_rmsprop
-  }
-  return nullptr;
-}
-
 extern "C" int ga3c_mlp_arena_upload(ga3c_mlp* n, int which, const float* host, int64_t nf) {
-  if (!n || !host) return set_error("ga3c_mlp_arena_upload: null argument");
-  float* dst = arena_of(n, which);
-  if (!dst || nf != n->arena_floats) return set_error("ga3c_mlp_arena_upload: bad arena id or size");
-  CK(cudaSetDevice(n->cfg.device));
-  CK(cudaDeviceSynchronize());
-  CK(cudaMemcpy(dst, host, (size_t)nf * 4, cudaMemcpyHostToDevice));
-  return 0;
+  return arena_upload(n, which, host, nf, "ga3c_mlp_arena_upload");
 }
 
 extern "C" int ga3c_mlp_arena_download(ga3c_mlp* n, int which, float* host, int64_t nf) {
-  if (!n || !host) return set_error("ga3c_mlp_arena_download: null argument");
-  float* src = arena_of(n, which);
-  if (!src || nf != n->arena_floats) return set_error("ga3c_mlp_arena_download: bad arena id or size");
-  CK(cudaSetDevice(n->cfg.device));
-  CK(cudaDeviceSynchronize());
-  CK(cudaMemcpy(host, src, (size_t)nf * 4, cudaMemcpyDeviceToHost));
-  return 0;
+  return arena_download(n, which, host, nf, "ga3c_mlp_arena_download");
 }
 
 extern "C" int64_t ga3c_mlp_global_step(const ga3c_mlp* n) { return n ? n->global_step : -1; }
@@ -316,7 +217,7 @@ extern "C" int ga3c_debug_tf32x3_gemm(int32_t mode, const float* a, const float*
     if (splits < 1 || rows_per_split < 32 || rows_per_split % 32) return set_error("ga3c_debug_tf32x3_gemm: rows_per_split must be a multiple of 32");
     r = launch_mlp_tc_wgrad(k, nn, a, b, m, splits, rows_per_split, out, nullptr, (int64_t)k * nn, st);
   } else return set_error("ga3c_debug_tf32x3_gemm: mode must be 0, 1 or 2");
-  if (r) return fail("ga3c_debug_tf32x3_gemm", (cudaError_t)r);
+  if (r) return fail_cuda("ga3c_debug_tf32x3_gemm", (cudaError_t)r);
   return 0;
 }
 extern "C" int ga3c_mlp_workspace_ptr(ga3c_mlp* n, int32_t which, int32_t layer, void** ptr, int32_t* width) {
@@ -324,13 +225,6 @@ extern "C" int ga3c_mlp_workspace_ptr(ga3c_mlp* n, int32_t which, int32_t layer,
   if (which < 0 || which > 1 || layer < 0 || layer >= n->net.n_layers) return set_error("ga3c_mlp_workspace_ptr: bad matrix id");
   *ptr = which == 0 ? n->act[layer] : n->dz[layer];
   *width = n->net.L[layer].n;
-  return 0;
-}
-
-static int check_batch(ga3c_mlp* n, int batch, const char* who) {
-  if (!n) return set_error(std::string(who) + ": null handle");
-  if (batch < 1 || batch > n->cfg.max_batch)
-    return set_error(std::string(who) + ": batch " + std::to_string(batch) + " outside 1.." + std::to_string(n->cfg.max_batch));
   return 0;
 }
 
@@ -350,7 +244,7 @@ extern "C" int ga3c_mlp_histograms(ga3c_mlp* n, int32_t batch, const float* p, c
   // v, p.  Arena offsets are multiples of ALIGN_FLOATS and each act[l] is its own allocation: every source is 16-byte aligned.
   HistoArgs a{};
   int s = 0;
-  for (const MlpParam& q : n->params) a.src[s++] = HistoSrc{n->w + q.offset, q.count, 0, 0};
+  for (const Param& q : n->params) a.src[s++] = HistoSrc{n->w + q.offset, q.count, 0, 0};
   const long long b = batch;
   for (int l = 0; l < n->net.n_layers; ++l) a.src[s++] = HistoSrc{n->act[l], b * n->net.L[l].n, 0, 0};
   a.src[s++] = HistoSrc{v, b, 0, 0};
@@ -358,21 +252,14 @@ extern "C" int ga3c_mlp_histograms(ga3c_mlp* n, int32_t batch, const float* p, c
   a.n_src = n_src;
   a.out = out;
   a.bad = bad;
-  if (int r = histo_plan(a)) return r;
-  const size_t part_bytes = sizeof(double) * 4 * histo_blocks(a);
-  if (part_bytes > n->histo_part_bytes) {
-    CK(cudaFree(n->histo_part));
-    n->histo_part = nullptr;
-    n->histo_part_bytes = 0;
-    CK(cudaMalloc((void**)&n->histo_part, part_bytes));
-    n->histo_part_bytes = part_bytes;
-  }
-  a.part = n->histo_part;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (int r = histo_zero(a, st)) return r;
-  LAUNCH(n, K_HISTO, st, launch_histo(a, st));
-  LAUNCH(n, K_HISTO, st, launch_histo_merge(a, st));
-  return 0;
+  return launch_histograms(n, a, (cudaStream_t)stream);
+}
+
+// the first optimizer over the live prefix; no bf16 shadow
+static RmsPropArgs rmsprop_args(ga3c_mlp* n, float lr) {
+  RmsPropArgs a = rmsprop_base(n, lr, n->live_floats);
+  a.w1_offset = n->live_floats;
+  return a;
 }
 
 static MlpStepArgs step_args(ga3c_mlp* n, const float* x, int batch) {
@@ -421,7 +308,7 @@ static int mlp_fb_impl(ga3c_mlp* n, const float* x, const float* yr, const float
     const MlpNet& net = n->net;
     const int lo = n->tc_lo, hi = n->tc_hi;
     s.tc_lo = lo; s.tc_hi = hi;
-    const bool streamed = n->stream_ok;       // narrow ends as streaming passes (mlp_stream.cu) instead of fused-kernel phases
+    const bool streamed = n->stream_ok;       // narrow ends as streaming passes (mlp_stream.cu), else as fused-kernel phases
     s.phase = 1;
     if (streamed) LAUNCH(n, K_MLP_FUSED, st, launch_mlp_front_fwd(net, s, n->num_sms, st));
     else LAUNCH(n, K_MLP_FUSED, st, launch_mlp_fused(net, s, n->num_sms, st));
@@ -483,22 +370,11 @@ extern "C" int ga3c_mlp_forward_backward(ga3c_mlp* n, const float* x, const floa
 extern "C" int ga3c_mlp_apply_rmsprop(ga3c_mlp* n, float lr, void* stream) {
   if (!n) return set_error("ga3c_mlp_apply_rmsprop: null handle");
   CK(cudaSetDevice(n->cfg.device));
-  RmsPropArgs a{};
-  a.w = n->w; a.ms = n->ms; a.mom = n->mom; a.g = n->g; a.w1_shadow = nullptr;
-  a.n_floats = n->live_floats;           // the gradient-less variables behind the live prefix are never touched
-  a.w1_offset = n->live_floats; a.w1_count = 0;
-  a.lr = lr; a.decay = n->cfg.rmsprop_decay; a.momentum = n->cfg.rmsprop_momentum; a.eps = n->cfg.rmsprop_epsilon;
+  const RmsPropArgs a = rmsprop_args(n, lr);
   if (n->cfg.dual_rmsprop) return set_error("ga3c_mlp_apply_rmsprop: with DUAL_RMSPROP use ga3c_mlp_train_step (two backward passes)");
   if (n->cfg.use_grad_clip) {            // tf.clip_by_average_norm per variable (NetworkVP.py:138-141, NetworkVP_discrate.py:118-121)
-    ClipArgs c{};
-    c.g = n->g; c.n_tensors = (int)n->params.size();
-    int64_t mx = 0;
-    for (int i = 0; i < c.n_tensors; ++i) {
-      c.offset[i] = n->params[i].offset; c.count[i] = n->params[i].count;
-      mx = c.count[i] > mx ? c.count[i] : mx;
-    }
-    c.max_chunks = clip_chunks(mx); c.clip = n->cfg.grad_clip_norm; c.chunk_ss = n->clip_ss; c.scale = n->clip_scale;
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_clipped(a, c, (cudaStream_t)stream));
+    // every variable is live here (checked at create)
+    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_clipped(a, clip_args(n, 0), (cudaStream_t)stream));
     n->log.launches += 2;
     if (n->cfg.kind == GA3C_MLP_FORK_VP) n->global_step += 1;     // the fork's NetworkVP passes global_step, _discrate does not
     return 0;
@@ -515,30 +391,17 @@ extern "C" int ga3c_mlp_train_step(ga3c_mlp* n, const float* x, const float* yr,
     if (int r = mlp_fb_impl(n, x, yr, a, batch, beta, loss, stream, 1, n->g)) return r;
     if (int r = mlp_fb_impl(n, x, yr, a, batch, beta, nullptr, stream, 2, n->g2)) return r;
     RmsPropDualArgs d{};
-    d.a.w = n->w; d.a.ms = n->ms; d.a.mom = n->mom; d.a.g = n->g; d.a.w1_shadow = nullptr;
-    d.a.n_floats = n->live_floats; d.a.w1_offset = n->live_floats; d.a.w1_count = 0;
-    d.a.lr = lr; d.a.decay = n->cfg.rmsprop_decay; d.a.momentum = n->cfg.rmsprop_momentum; d.a.eps = n->cfg.rmsprop_epsilon;
+    d.a = rmsprop_args(n, lr);
     d.g2 = n->g2; d.ms2 = n->ms2; d.mom2 = n->mom2;
     d.skip_lo[0] = n->skip_lo[0]; d.skip_hi[0] = n->skip_hi[0];        // cost_p: not logits_v
     d.skip_lo[2] = n->skip_lo[1]; d.skip_hi[2] = n->skip_hi[1];        // cost_v: not the policy head
     if (n->cfg.use_grad_clip) {
       // tf.clip_by_norm per variable and optimizer (NetworkVP.py:127-137, NetworkVP_discrate.py:107-117); the fork's NetworkVP
       // hands global_step to both apply_gradients calls, NetworkVP_discrate to neither
-      ClipArgs c[2] = {};
-      int64_t mx = 0;
-      for (int w = 0; w < 2; ++w) {
-        c[w].g = w ? n->g2 : n->g;
-        c[w].n_tensors = 0;
-        for (const MlpParam& p : n->params) {
-          if (!p.live) continue;                                       // gradient is None: filtered by the reference
-          c[w].offset[c[w].n_tensors] = p.offset; c[w].count[c[w].n_tensors] = p.count; ++c[w].n_tensors;
-          mx = p.count > mx ? p.count : mx;
-        }
-        c[w].clip = n->cfg.grad_clip_norm; c[w].by_norm = 1;
-        c[w].chunk_ss = w ? n->clip_ss2 : n->clip_ss; c[w].scale = w ? n->clip_scale2 : n->clip_scale;
-      }
-      c[0].max_chunks = c[1].max_chunks = clip_chunks(mx);
-      LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_dual_clipped(d, c[0], c[1], (cudaStream_t)stream));
+      // (the gradient-less variables' gradient is None: the reference filters them, clip_args leaves them out)
+      ClipArgs c1 = clip_args(n, 0), c2 = clip_args(n, 1);
+      c1.by_norm = c2.by_norm = 1;
+      LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_dual_clipped(d, c1, c2, (cudaStream_t)stream));
       n->log.launches += 4;
       if (n->cfg.kind == GA3C_MLP_FORK_VP) n->global_step += 2;
       return 0;
@@ -552,15 +415,9 @@ extern "C" int ga3c_mlp_train_step(ga3c_mlp* n, const float* x, const float* yr,
 }
 
 extern "C" int ga3c_mlp_timing_enable(ga3c_mlp* n, int32_t max_records) {
-  if (!n || max_records < 0) return set_error("ga3c_mlp_timing_enable: bad argument");
-  CK(cudaSetDevice(n->cfg.device));
-  CK(cudaDeviceSynchronize());
-  return n->log.enable(max_records);
+  return timing_enable(n, max_records, "ga3c_mlp_timing_enable");
 }
 
 extern "C" int ga3c_mlp_timing_collect(ga3c_mlp* n, double* total_ms, int64_t* counts, int32_t n_kernels) {
-  if (!n || !total_ms || !counts || n_kernels < K_COUNT) return set_error("ga3c_mlp_timing_collect: bad argument");
-  CK(cudaSetDevice(n->cfg.device));
-  CK(cudaDeviceSynchronize());
-  return n->log.collect(total_ms, reinterpret_cast<long long*>(counts), n_kernels);
+  return timing_collect(n, total_ms, counts, n_kernels, "ga3c_mlp_timing_collect");
 }

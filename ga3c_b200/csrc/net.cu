@@ -10,43 +10,18 @@
 #include "../../include/ga3c_b200.h"
 #include "common.cuh"
 #include "kernels.h"
-#include "host_util.h"
+#include "handle.h"
 #include "mlp.cuh"
 #include "dp_exchange.cuh"
 
 using namespace ga3c;
 
-namespace {
+static thread_local std::string g_err;
 
-thread_local std::string g_err;
-
-int fail(const char* where, cudaError_t e) { return fail_cuda(where, e); }
-int fail_msg(const std::string& m) { g_err = m; return -1; }
-
-struct ParamDesc {
-  std::string name;
-  int64_t offset;
-  int32_t ndim;
-  int64_t shape[4];
-  int64_t count;
-};
-
-constexpr int64_t ALIGN_FLOATS = 64;
-int64_t align_up(int64_t v) { return (v + ALIGN_FLOATS - 1) / ALIGN_FLOATS * ALIGN_FLOATS; }
-
-}  // namespace
-
-struct ga3c_net {
-  ga3c_config cfg;
-  int num_sms = 148;
-  std::vector<ParamDesc> params;   // TF creation order
-  int64_t arena_floats = 0;
+struct ga3c_net : Handle<ga3c_config> {
   int64_t small_floats = 0;        // prefix holding every tensor except dense1/w (grads zeroed per step)
-  // one slab holds [params | grads | ms | mom | bf16 shadow of dense1/w | LL receive buffers | comm flags]: a single CUDA IPC handle
-  // exposes everything a data-parallel peer needs (ga3c_dp_*)
-  uint8_t* slab = nullptr;
-  size_t slab_bytes = 0;
-  float *w = nullptr, *g = nullptr, *ms = nullptr, *mom = nullptr;
+  // the arena slab holds [params | grads | ms | mom | bf16 shadow of dense1/w | LL receive buffers | comm flags]: a single CUDA
+  // IPC handle exposes everything a data-parallel peer needs (ga3c_dp_*)
   uint16_t* w1_shadow = nullptr;   // bf16 [3872,256]
   // data parallel over peer memory (single node, <= 8 ranks)
   int dp_rank = 0, dp_world = 1;
@@ -70,18 +45,10 @@ struct ga3c_net {
   int64_t gp_stride = 0;
   int gp_heads_grid = 0;           // slabs the heads kernel of the current step wrote
   float* loss_out = nullptr;       // caller's loss buffer of the current step (may be null)
-  float *clip_ss = nullptr, *clip_scale = nullptr;   // Config.USE_GRAD_CLIP scratch: chunk sums of squares, per-tensor scale
-  float *clip_ss2 = nullptr, *clip_scale2 = nullptr; // ... of the second optimizer's gradient (DUAL_RMSPROP + USE_GRAD_CLIP)
-  float *g2 = nullptr, *ms2 = nullptr, *mom2 = nullptr;   // Config.DUAL_RMSPROP: gradient of cost_v and the second optimizer's slots
   bool keep_dn1 = false;           // tests: also store dn1 (which otherwise never leaves the SM) to the workspace
-  int64_t global_step = 0;
   std::mutex mtx;                  // ga3c_lock / ga3c_unlock
-  LaunchLog log;                   // launch counter + per-kernel CUDA-event timing (ga3c_timing_*)
-  int last_batch = 0;
   unsigned long long* evt = nullptr;       // pipeline event log of CTA 0 (ga3c_evt_*), device memory
   unsigned long long* trace = nullptr;     // [K_COUNT][TRACE_SLOTS] globaltimer stamps (ga3c_trace_*), device memory
-  double* histo_part = nullptr;            // ga3c_histograms: fp64 partial moments per block
-  size_t histo_part_bytes = 0;
 
   int64_t off(int i) const { return params[i].offset; }
 };
@@ -106,22 +73,15 @@ extern "C" const char* ga3c_last_error(void) { return g_err.c_str(); }
 extern "C" int ga3c_abi_version(void) { return 9; }
 
 extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
-  if (!cfg || !out) return fail_msg("ga3c_create: null argument");
+  if (!cfg || !out) return set_error("ga3c_create: null argument");
   *out = nullptr;
-  if (cfg->num_actions < 1 || cfg->num_actions > MAX_ACTIONS) return fail_msg("ga3c_create: num_actions must be 1..18");
-  if (cfg->max_batch < 1) return fail_msg("ga3c_create: max_batch must be >= 1");
-  int ndev = 0;
-  cudaError_t e = cudaGetDeviceCount(&ndev);
-  if (e != cudaSuccess || ndev == 0) return fail_msg("ga3c_create: no CUDA device (there is no CPU fallback)");
-  if (cfg->device < 0 || cfg->device >= ndev) return fail_msg("ga3c_create: device ordinal out of range");
-  CK(cudaSetDevice(cfg->device));
-  cudaDeviceProp prop;
-  CK(cudaGetDeviceProperties(&prop, cfg->device));
-  if (prop.major != 10) return fail_msg("ga3c_create: kernels are built for sm_100a only; device is sm_" +
-                                        std::to_string(prop.major) + std::to_string(prop.minor));
+  if (cfg->num_actions < 1 || cfg->num_actions > MAX_ACTIONS) return set_error("ga3c_create: num_actions must be 1..18");
+  if (cfg->max_batch < 1) return set_error("ga3c_create: max_batch must be >= 1");
+  int num_sms = 0;
+  if (int r = open_device(cfg->device, "ga3c_create", &num_sms)) return r;
   ga3c_net* n = new ga3c_net();
   n->cfg = *cfg;
-  n->num_sms = prop.multiProcessorCount;
+  n->num_sms = num_sms;
   const int A = cfg->num_actions;
   // TF creation order (NetworkVP.py:284-285 would list them so); offsets pack the small tensors first
   struct { const char* name; int nd; int64_t s[4]; } spec[P_COUNT] = {
@@ -132,9 +92,10 @@ extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
       {"logits_p/w:0", 2, {FC, A, 0, 0}}, {"logits_p/b:0", 1, {A, 0, 0, 0}}};
   n->params.resize(P_COUNT);
   for (int i = 0; i < P_COUNT; ++i) {
-    ParamDesc& d = n->params[i];
+    Param& d = n->params[i];
     d.name = spec[i].name;
     d.ndim = spec[i].nd;
+    d.live = 1;
     d.count = 1;
     for (int k = 0; k < 4; ++k) { d.shape[k] = spec[i].s[k]; if (k < d.ndim) d.count *= d.shape[k]; }
   }
@@ -148,60 +109,23 @@ extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
   n->arena_floats = cur;
 
   const size_t ab = (size_t)n->arena_floats * sizeof(float);
-#define GA3C_ALLOC(ptr, bytes)                                                   \
-  do {                                                                           \
-    cudaError_t _e = cudaMalloc((void**)&(ptr), (bytes));                        \
-    if (_e != cudaSuccess) { ga3c_destroy(n); return fail("cudaMalloc", _e); }   \
-  } while (0)
   const size_t shadow_bytes = (size_t)FLAT * FC * 2;
   n->xbuf_off = (int64_t)(4 * ab + shadow_bytes);
   n->comm_off = n->xbuf_off + 2 * (int64_t)DP_MAX_WORLD * n->small_floats * 8;
-  n->slab_bytes = (size_t)n->comm_off + DP_COMM_BYTES;
-  GA3C_ALLOC(n->slab, n->slab_bytes);
-#undef GA3C_ALLOC
-  n->w = reinterpret_cast<float*>(n->slab);
-  n->g = reinterpret_cast<float*>(n->slab + ab);
-  n->ms = reinterpret_cast<float*>(n->slab + 2 * ab);
-  n->mom = reinterpret_cast<float*>(n->slab + 3 * ab);
+  if (int r = alloc_arenas(n, (size_t)n->comm_off + DP_COMM_BYTES - 4 * ab)) { ga3c_destroy(n); return r; }
   n->w1_shadow = reinterpret_cast<uint16_t*>(n->slab + 4 * ab);
-  cudaMemset(n->slab + n->xbuf_off, 0, n->slab_bytes - (size_t)n->xbuf_off);
   n->gp_stride = n->small_floats + 64;
-  e = cudaMalloc((void**)&n->gpart, (size_t)2 * n->num_sms * n->gp_stride * sizeof(float));
-  if (e != cudaSuccess) { ga3c_destroy(n); return fail("cudaMalloc", e); }
+  cudaError_t e = cudaMalloc((void**)&n->gpart, (size_t)2 * n->num_sms * n->gp_stride * sizeof(float));
+  if (e != cudaSuccess) { ga3c_destroy(n); return fail_cuda("cudaMalloc", e); }
   cudaMemset(n->gpart, 0, (size_t)2 * n->num_sms * n->gp_stride * sizeof(float));
-  if (cfg->dual_rmsprop) {
-    float** extra[3] = {&n->g2, &n->ms2, &n->mom2};
-    for (float** a : extra) {
-      e = cudaMalloc((void**)a, ab);
-      if (e != cudaSuccess) { ga3c_destroy(n); return fail("cudaMalloc", e); }
-      cudaMemset(*a, 0, ab);
-    }
-    std::vector<float> ones((size_t)n->arena_floats, 1.0f);
-    cudaMemcpy(n->ms2, ones.data(), ab, cudaMemcpyHostToDevice);
-  }
-  if (cfg->use_grad_clip) {
-    e = cudaMalloc((void**)&n->clip_ss, (size_t)P_COUNT * clip_chunks((int64_t)FLAT * FC) * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc((void**)&n->clip_scale, P_COUNT * sizeof(float));
-    if (e == cudaSuccess && cfg->dual_rmsprop) {
-      e = cudaMalloc((void**)&n->clip_ss2, (size_t)P_COUNT * clip_chunks((int64_t)FLAT * FC) * sizeof(float));
-      if (e == cudaSuccess) e = cudaMalloc((void**)&n->clip_scale2, P_COUNT * sizeof(float));
-    }
-    if (e != cudaSuccess) { ga3c_destroy(n); return fail("cudaMalloc", e); }
-  }
   if (int r = alloc_workspace(n, cfg->max_batch)) { ga3c_destroy(n); return r; }
-  cudaMemset(n->w, 0, ab); cudaMemset(n->g, 0, ab); cudaMemset(n->mom, 0, ab);
-  cudaMemset(n->w1_shadow, 0, (size_t)FLAT * FC * 2);
-  {  // ms slot starts at 1.0 [TF-SEMANTICS]
-    std::vector<float> ones((size_t)n->arena_floats, 1.0f);
-    cudaMemcpy(n->ms, ones.data(), ab, cudaMemcpyHostToDevice);
-  }
   int r;
   if ((r = configure_conv_fwd()) || (r = configure_conv_bwd_fused()) || (r = configure_dense_tc())) {
     ga3c_destroy(n);
-    return fail("cudaFuncSetAttribute", (cudaError_t)r);
+    return fail_cuda("cudaFuncSetAttribute", (cudaError_t)r);
   }
   e = cudaDeviceSynchronize();
-  if (e != cudaSuccess) { ga3c_destroy(n); return fail("ga3c_create sync", e); }
+  if (e != cudaSuccess) { ga3c_destroy(n); return fail_cuda("ga3c_create sync", e); }
   *out = n;
   return 0;
 }
@@ -227,7 +151,7 @@ static int alloc_workspace(ga3c_net* n, int max_batch) {
 }
 
 extern "C" int ga3c_reserve(ga3c_net* n, int32_t max_batch) {
-  if (!n) return fail_msg("ga3c_reserve: null handle");
+  if (!n) return set_error("ga3c_reserve: null handle");
   if (max_batch <= n->cfg.max_batch) return 0;
   CK(cudaSetDevice(n->cfg.device));
   CK(cudaDeviceSynchronize());
@@ -239,25 +163,21 @@ extern "C" int ga3c_reserve(ga3c_net* n, int32_t max_batch) {
 extern "C" int ga3c_destroy(ga3c_net* n) {
   if (!n) return 0;
   ga3c_dp_detach(n);
-  cudaFree(n->slab);
+  free_arenas(n);
   cudaFree(n->gpart);
-  cudaFree(n->clip_ss); cudaFree(n->clip_scale); cudaFree(n->clip_ss2); cudaFree(n->clip_scale2);
-  cudaFree(n->g2); cudaFree(n->ms2); cudaFree(n->mom2);
   if (n->trace) { trace_attach_all(nullptr); cudaFree(n->trace); }
-  cudaFree(n->histo_part);
   free_workspace(n);
-  n->log.clear();
   delete n;
   return 0;
 }
 
 extern "C" int ga3c_lock(ga3c_net* n) {
-  if (!n) return fail_msg("ga3c_lock: null handle");
+  if (!n) return set_error("ga3c_lock: null handle");
   n->mtx.lock();
   return 0;
 }
 extern "C" int ga3c_unlock(ga3c_net* n) {
-  if (!n) return fail_msg("ga3c_unlock: null handle");
+  if (!n) return set_error("ga3c_unlock: null handle");
   n->mtx.unlock();
   return 0;
 }
@@ -266,19 +186,13 @@ extern "C" int ga3c_param_count(const ga3c_net* n) { return n ? (int)n->params.s
 
 extern "C" int ga3c_param_info(const ga3c_net* n, int i, const char** name, int64_t* offset, int32_t* ndim,
                                int64_t shape[4]) {
-  if (!n || i < 0 || i >= (int)n->params.size()) return fail_msg("ga3c_param_info: bad index");
-  const ParamDesc& d = n->params[i];
-  if (name) *name = d.name.c_str();
-  if (offset) *offset = d.offset;
-  if (ndim) *ndim = d.ndim;
-  if (shape) for (int k = 0; k < 4; ++k) shape[k] = d.shape[k];
-  return 0;
+  return param_info(n, i, name, offset, ndim, shape, nullptr, "ga3c_param_info");
 }
 
 extern "C" int64_t ga3c_arena_floats(const ga3c_net* n) { return n ? n->arena_floats : 0; }
 
 extern "C" int ga3c_arena_ptrs(ga3c_net* n, float** p, float** g, float** ms, float** mom) {
-  if (!n) return fail_msg("ga3c_arena_ptrs: null handle");
+  if (!n) return set_error("ga3c_arena_ptrs: null handle");
   if (p) *p = n->w;
   if (g) *g = n->g;
   if (ms) *ms = n->ms;
@@ -286,27 +200,15 @@ extern "C" int ga3c_arena_ptrs(ga3c_net* n, float** p, float** g, float** ms, fl
   return 0;
 }
 
-static float* arena_of(ga3c_net* n, int which) {
-  switch (which) {
-    case 0: return n->w; case 1: return n->g; case 2: return n->ms; case 3: return n->mom;
-    case 4: return n->g2; case 5: return n->ms2; case 6: return n->mom2;      // null unless dual_rmsprop
-  }
-  return nullptr;
-}
-
 extern "C" int ga3c_arena_ptr(ga3c_net* n, int which, float** ptr_dev) {
-  if (!n || !ptr_dev) return fail_msg("ga3c_arena_ptr: null argument");
+  if (!n || !ptr_dev) return set_error("ga3c_arena_ptr: null argument");
   *ptr_dev = arena_of(n, which);
-  if (!*ptr_dev) return fail_msg("ga3c_arena_ptr: bad arena id");
+  if (!*ptr_dev) return set_error("ga3c_arena_ptr: bad arena id");
   return 0;
 }
 
 extern "C" int ga3c_arena_upload(ga3c_net* n, int which, const float* host, int64_t nf) {
-  if (!n || !host) return fail_msg("ga3c_arena_upload: null argument");
-  float* dst = arena_of(n, which);
-  if (!dst || nf != n->arena_floats) return fail_msg("ga3c_arena_upload: bad arena id or size");
-  CK(cudaSetDevice(n->cfg.device));
-  CK(cudaMemcpy(dst, host, (size_t)nf * 4, cudaMemcpyHostToDevice));
+  if (int r = arena_upload(n, which, host, nf, "ga3c_arena_upload")) return r;
   if (which == 0) {
     CKL(launch_f32_to_bf16(n->w + n->off(P_D1W), n->w1_shadow, (int64_t)FLAT * FC, 0));
     n->log.launches++;
@@ -316,12 +218,7 @@ extern "C" int ga3c_arena_upload(ga3c_net* n, int which, const float* host, int6
 }
 
 extern "C" int ga3c_arena_download(ga3c_net* n, int which, float* host, int64_t nf) {
-  if (!n || !host) return fail_msg("ga3c_arena_download: null argument");
-  float* src = arena_of(n, which);
-  if (!src || nf != n->arena_floats) return fail_msg("ga3c_arena_download: bad arena id or size");
-  CK(cudaSetDevice(n->cfg.device));
-  CK(cudaDeviceSynchronize());
-  CK(cudaMemcpy(host, src, (size_t)nf * 4, cudaMemcpyDeviceToHost));
+  if (int r = arena_download(n, which, host, nf, "ga3c_arena_download")) return r;
   if (n->dp_world > 1 && (which == 0 || which == 2 || which == 3)) {
     // peer-memory exchange: the fp32 master copy and the RMSProp slots of a dense1/w slice live on its owner (only the bf16
     // shadow travels).  A peer's slice is stable here: it changes only inside a step this rank takes part in.
@@ -340,13 +237,6 @@ extern "C" int ga3c_arena_download(ga3c_net* n, int which, float* host, int64_t 
 
 extern "C" int64_t ga3c_global_step(const ga3c_net* n) { return n ? n->global_step : -1; }
 extern "C" int ga3c_set_global_step(ga3c_net* n, int64_t s) { if (!n) return -1; n->global_step = s; return 0; }
-
-static int check_batch(ga3c_net* n, int batch, const char* who) {
-  if (!n) return fail_msg(std::string(who) + ": null handle");
-  if (batch < 1 || batch > n->cfg.max_batch)
-    return fail_msg(std::string(who) + ": batch " + std::to_string(batch) + " outside 1.." + std::to_string(n->cfg.max_batch));
-  return 0;
-}
 
 static HeadsArgs heads_args(ga3c_net* n, int batch, int splits) {
   HeadsArgs h{};
@@ -374,7 +264,7 @@ static DpGate dp_gate(const ga3c_net* n) {
 
 static int predict_impl(ga3c_net* n, const void* x, bool x_u8, int32_t batch, float* p_out, float* v_out, void* stream) {
   if (int r = check_batch(n, batch, "ga3c_predict")) return r;
-  if (!x || !p_out || !v_out) return fail_msg("ga3c_predict: null buffer");
+  if (!x || !p_out || !v_out) return set_error("ga3c_predict: null buffer");
   CK(cudaSetDevice(n->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
   const float* w = n->w;
@@ -403,7 +293,7 @@ extern "C" int ga3c_predict_u8(ga3c_net* n, const uint8_t* x, int32_t batch, flo
 static int fb_head_impl(ga3c_net* n, const void* x, bool x_u8, const float* yr, const float* a, int32_t batch, float beta,
                         float* loss, void* stream, bool with_wgrad, int part = 0, bool skip_forward = false) {
   if (int r = check_batch(n, batch, "ga3c_fb_head")) return r;
-  if (!x || !yr || !a) return fail_msg("ga3c_fb_head: null buffer");
+  if (!x || !yr || !a) return set_error("ga3c_fb_head: null buffer");
   CK(cudaSetDevice(n->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
   const float* w = n->w;
@@ -461,8 +351,8 @@ static int enqueue_dp_big(ga3c_net* n, const DpBigArgs& b, cudaStream_t st) {
 static int fb_tail_impl(ga3c_net* n, const void* x, bool x_u8, int32_t batch, void* stream, bool with_wgrad, bool reduce,
                         const DpBigArgs* dp = nullptr, float* g_dst = nullptr) {
   if (int r = check_batch(n, batch, "ga3c_fb_tail")) return r;
-  if (!x) return fail_msg("ga3c_fb_tail: null buffer");
-  if (batch != n->last_batch) return fail_msg("ga3c_fb_tail: batch differs from the preceding ga3c_fb_head");
+  if (!x) return set_error("ga3c_fb_tail: null buffer");
+  if (batch != n->last_batch) return set_error("ga3c_fb_tail: batch differs from the preceding ga3c_fb_head");
   CK(cudaSetDevice(n->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
   const float* w = n->w;
@@ -506,36 +396,26 @@ extern "C" int ga3c_fb_tail_u8(ga3c_net* n, const uint8_t* x, int32_t batch, voi
 }
 
 static RmsPropArgs rmsprop_args(ga3c_net* n, float lr) {
-  RmsPropArgs a{};
-  a.w = n->w; a.ms = n->ms; a.mom = n->mom; a.g = n->g; a.w1_shadow = n->w1_shadow;
-  a.n_floats = n->arena_floats; a.w1_offset = n->off(P_D1W); a.w1_count = (int64_t)FLAT * FC;
-  a.lr = lr; a.decay = n->cfg.rmsprop_decay; a.momentum = n->cfg.rmsprop_momentum; a.eps = n->cfg.rmsprop_epsilon;
+  RmsPropArgs a = rmsprop_base(n, lr, n->arena_floats);
+  a.w1_shadow = n->w1_shadow; a.w1_offset = n->off(P_D1W); a.w1_count = (int64_t)FLAT * FC;
   return a;
 }
 
-static ClipArgs clip_args(ga3c_net* n, int which = 0) {        // which: 0 the (first) optimizer's gradient, 1 the second one's
-  ClipArgs c{};
-  c.g = which ? n->g2 : n->g; c.n_tensors = P_COUNT; c.max_chunks = clip_chunks((int64_t)FLAT * FC);
-  for (int i = 0; i < P_COUNT; ++i) { c.offset[i] = n->params[i].offset; c.count[i] = n->params[i].count; }
-  c.clip = n->cfg.grad_clip_norm; c.chunk_ss = which ? n->clip_ss2 : n->clip_ss; c.scale = which ? n->clip_scale2 : n->clip_scale;
-  return c;
-}
-
 static int apply_rmsprop_impl(ga3c_net* n, float lr, void* stream) {
-  if (!n) return fail_msg("ga3c_apply_rmsprop: null handle");
+  if (!n) return set_error("ga3c_apply_rmsprop: null handle");
   CK(cudaSetDevice(n->cfg.device));
   RmsPropArgs a = rmsprop_args(n, lr);
-  if (n->cfg.dual_rmsprop) return fail_msg("ga3c_apply_rmsprop: with DUAL_RMSPROP use ga3c_train_step (two backward passes)");
+  if (n->cfg.dual_rmsprop) return set_error("ga3c_apply_rmsprop: with DUAL_RMSPROP use ga3c_train_step (two backward passes)");
   if (n->cfg.use_grad_clip) {
     // clip_by_average_norm needs the whole (reduced) gradient of a variable: local arena only (single GPU, or after the
     // host's NCCL allreduce in dp_mode 'nccl')
-    if (n->dp_world > 1) return fail_msg("ga3c_apply_rmsprop: USE_GRAD_CLIP is not available with the peer-memory exchange");
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_clipped(a, clip_args(n), (cudaStream_t)stream));
+    if (n->dp_world > 1) return set_error("ga3c_apply_rmsprop: USE_GRAD_CLIP is not available with the peer-memory exchange");
+    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_clipped(a, clip_args(n, 0), (cudaStream_t)stream));
     n->log.launches += 2;
     return 0;          // NetworkVP_discrate.py:121: apply_gradients without global_step -- the step counter stays put
   }
   // the peer-memory exchange is part of the train step (its dense1/w half starts behind dense_bwd, on a side stream)
-  if (n->dp_world > 1) return fail_msg("ga3c_apply_rmsprop: not available on a peer-memory data-parallel handle; use ga3c_train_step");
+  if (n->dp_world > 1) return set_error("ga3c_apply_rmsprop: not available on a peer-memory data-parallel handle; use ga3c_train_step");
   LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop(a, (cudaStream_t)stream));
   n->global_step += 1;   // opt.minimize(..., global_step=self.global_step), NetworkVP_discrate.py:130
   return 0;
@@ -547,7 +427,7 @@ extern "C" int ga3c_apply_rmsprop(ga3c_net* n, float lr, void* stream) { return 
 extern "C" int ga3c_dp_handle_bytes(void) { return (int)sizeof(cudaIpcMemHandle_t); }
 
 extern "C" int ga3c_dp_export(ga3c_net* n, void* handle_out) {
-  if (!n || !handle_out) return fail_msg("ga3c_dp_export: null argument");
+  if (!n || !handle_out) return set_error("ga3c_dp_export: null argument");
   CK(cudaSetDevice(n->cfg.device));
   cudaIpcMemHandle_t h;
   CK(cudaIpcGetMemHandle(&h, n->slab));
@@ -571,9 +451,9 @@ extern "C" int ga3c_dp_detach(ga3c_net* n) {
 }
 
 extern "C" int ga3c_dp_attach(ga3c_net* n, int32_t rank, int32_t world, const void* handles) {
-  if (!n || !handles) return fail_msg("ga3c_dp_attach: null argument");
+  if (!n || !handles) return set_error("ga3c_dp_attach: null argument");
   if (world < 1 || world > DP_MAX_WORLD || rank < 0 || rank >= world)
-    return fail_msg("ga3c_dp_attach: world must be 1.." + std::to_string(DP_MAX_WORLD) + " and 0 <= rank < world");
+    return set_error("ga3c_dp_attach: world must be 1.." + std::to_string(DP_MAX_WORLD) + " and 0 <= rank < world");
   CK(cudaSetDevice(n->cfg.device));
   CK(cudaDeviceSynchronize());
   ga3c_dp_detach(n);
@@ -584,7 +464,7 @@ extern "C" int ga3c_dp_attach(ga3c_net* n, int32_t rank, int32_t world, const vo
     cudaError_t e = cudaIpcOpenMemHandle(&p, hs[r], cudaIpcMemLazyEnablePeerAccess);
     if (e != cudaSuccess) {
       ga3c_dp_detach(n);
-      return fail("cudaIpcOpenMemHandle (peer-to-peer access between the ranks' GPUs is required)", e);
+      return fail_cuda("cudaIpcOpenMemHandle (peer-to-peer access between the ranks' GPUs is required)", e);
     }
     n->dp_peer[r] = static_cast<uint8_t*>(p);
     n->dp_ipc[r] = true;
@@ -595,20 +475,20 @@ extern "C" int ga3c_dp_attach(ga3c_net* n, int32_t rank, int32_t world, const vo
 // ranks that live in ONE process (tests; a host that drives several GPUs from one process): the peers' slabs are ordinary
 // device pointers, no IPC handles involved.  peers[r] is rank r's handle (peers[rank] == net).
 extern "C" int ga3c_dp_attach_local(ga3c_net* n, int32_t rank, int32_t world, ga3c_net* const* peers) {
-  if (!n || !peers) return fail_msg("ga3c_dp_attach_local: null argument");
+  if (!n || !peers) return set_error("ga3c_dp_attach_local: null argument");
   if (world < 1 || world > DP_MAX_WORLD || rank < 0 || rank >= world || peers[rank] != n)
-    return fail_msg("ga3c_dp_attach_local: need 0 <= rank < world <= 8 and peers[rank] == net");
+    return set_error("ga3c_dp_attach_local: need 0 <= rank < world <= 8 and peers[rank] == net");
   CK(cudaSetDevice(n->cfg.device));
   CK(cudaDeviceSynchronize());
   ga3c_dp_detach(n);
   for (int r = 0; r < world; ++r) {
-    if (!peers[r] || peers[r]->arena_floats != n->arena_floats) { ga3c_dp_detach(n); return fail_msg("ga3c_dp_attach_local: peers must be handles of the same network"); }
+    if (!peers[r] || peers[r]->arena_floats != n->arena_floats) { ga3c_dp_detach(n); return set_error("ga3c_dp_attach_local: peers must be handles of the same network"); }
     if (peers[r]->cfg.device != n->cfg.device) {
       int can = 0;
       cudaDeviceCanAccessPeer(&can, n->cfg.device, peers[r]->cfg.device);
-      if (!can) { ga3c_dp_detach(n); return fail_msg("ga3c_dp_attach_local: no peer access between the devices"); }
+      if (!can) { ga3c_dp_detach(n); return set_error("ga3c_dp_attach_local: no peer access between the devices"); }
       cudaError_t e = cudaDeviceEnablePeerAccess(peers[r]->cfg.device, 0);
-      if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) { ga3c_dp_detach(n); return fail("cudaDeviceEnablePeerAccess", e); }
+      if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) { ga3c_dp_detach(n); return fail_cuda("cudaDeviceEnablePeerAccess", e); }
       cudaGetLastError();
     }
     n->dp_peer[r] = peers[r]->slab;
@@ -633,7 +513,7 @@ static int dp_attach_finish(ga3c_net* n, int32_t rank, int32_t world) {
 // 0: every cross-rank wait of the exchange kernels completed; 1: one gave up (a rank died, or the ranks' train calls fell out
 // of step) and the weights can no longer be trusted.  Synchronises the device.
 extern "C" int ga3c_dp_error(ga3c_net* n, int32_t* error_out) {
-  if (!n || !error_out) return fail_msg("ga3c_dp_error: null argument");
+  if (!n || !error_out) return set_error("ga3c_dp_error: null argument");
   *error_out = 0;
   if (n->dp_world <= 1) return 0;
   CK(cudaSetDevice(n->cfg.device));
@@ -647,7 +527,7 @@ extern "C" int ga3c_dp_error(ga3c_net* n, int32_t* error_out) {
 // Config.DUAL_RMSPROP: one forward, two backward passes (cost_p into g, cost_v into g2) ...
 static int dual_forward_backward_impl(ga3c_net* n, const void* x, bool x_u8, const float* yr, const float* a, int32_t batch,
                                       float beta, float* loss, void* stream) {
-  if (!n || !n->cfg.dual_rmsprop) return fail_msg("ga3c_dual_forward_backward: the handle was not created with dual_rmsprop");
+  if (!n || !n->cfg.dual_rmsprop) return set_error("ga3c_dual_forward_backward: the handle was not created with dual_rmsprop");
   if (int r = fb_head_impl(n, x, x_u8, yr, a, batch, beta, loss, stream, false, 1)) return r;
   if (int r = fb_tail_impl(n, x, x_u8, batch, stream, true, true)) return r;
   if (int r = fb_head_impl(n, x, x_u8, yr, a, batch, beta, nullptr, stream, false, 2, true)) return r;
@@ -655,7 +535,7 @@ static int dual_forward_backward_impl(ga3c_net* n, const void* x, bool x_u8, con
 }
 // ... and one update that subtracts both optimizers' steps, each taken at the weights the call started with
 static int dual_apply_impl(ga3c_net* n, float lr, void* stream) {
-  if (!n || !n->cfg.dual_rmsprop) return fail_msg("ga3c_dual_apply: the handle was not created with dual_rmsprop");
+  if (!n || !n->cfg.dual_rmsprop) return set_error("ga3c_dual_apply: the handle was not created with dual_rmsprop");
   CK(cudaSetDevice(n->cfg.device));
   RmsPropDualArgs d{};
   d.a = rmsprop_args(n, lr);
@@ -711,7 +591,7 @@ static int train_step_empty(ga3c_net* n, float lr, float* loss, void* stream) {
   CK(cudaSetDevice(n->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
   if (n->cfg.dual_rmsprop || n->cfg.use_grad_clip)
-    return fail_msg("ga3c_train_step: batch 0 is only defined for the peer-memory data-parallel step");
+    return set_error("ga3c_train_step: batch 0 is only defined for the peer-memory data-parallel step");
   n->gp_heads_grid = 0;
   n->loss_out = loss;
   n->last_batch = 0;
@@ -728,7 +608,7 @@ static int train_step_impl(ga3c_net* n, const void* x, bool x_u8, const float* y
                            float beta, float* loss, void* stream) {
   if (n && batch == 0 && n->dp_world > 1) return train_step_empty(n, lr, loss, stream);
   if (n->cfg.dual_rmsprop) {
-    if (n->dp_world > 1) return fail_msg("ga3c_train_step: DUAL_RMSPROP is not available with the peer-memory exchange (dp_mode 'nccl' is)");
+    if (n->dp_world > 1) return set_error("ga3c_train_step: DUAL_RMSPROP is not available with the peer-memory exchange (dp_mode 'nccl' is)");
     if (int r = dual_forward_backward_impl(n, x, x_u8, yr, a, batch, beta, loss, stream)) return r;
     return dual_apply_impl(n, lr, stream);
   }
@@ -768,25 +648,25 @@ extern "C" int ga3c_train_step_u8(ga3c_net* n, const uint8_t* x, const float* yr
 
 extern "C" int ga3c_returns(const double* rewards, const int64_t* seg, int32_t n_segments, const double* terminal,
                             double discount, int32_t flags, double rmin, double rmax, double* out, void* stream) {
-  if (n_segments < 0) return fail_msg("ga3c_returns: negative segment count");
+  if (n_segments < 0) return set_error("ga3c_returns: negative segment count");
   if (n_segments == 0) return 0;
-  if (!rewards || !seg || !terminal || !out) return fail_msg("ga3c_returns: null buffer");
+  if (!rewards || !seg || !terminal || !out) return set_error("ga3c_returns: null buffer");
   CKL(launch_returns(rewards, seg, n_segments, terminal, discount, flags, rmin, rmax, out, (cudaStream_t)stream));
   return 0;
 }
 
 extern "C" int ga3c_select_actions(const float* p, const double* u, int32_t batch, int32_t na, int32_t* action,
                                    void* stream) {
-  if (batch < 0) return fail_msg("ga3c_select_actions: negative batch");
+  if (batch < 0) return set_error("ga3c_select_actions: negative batch");
   if (batch == 0) return 0;
-  if (!p || !u || !action) return fail_msg("ga3c_select_actions: null buffer");
-  if (na < 1 || na > MAX_ACTIONS) return fail_msg("ga3c_select_actions: num_actions must be 1..18");
+  if (!p || !u || !action) return set_error("ga3c_select_actions: null buffer");
+  if (na < 1 || na > MAX_ACTIONS) return set_error("ga3c_select_actions: num_actions must be 1..18");
   CKL(launch_select_actions(p, u, batch, na, action, (cudaStream_t)stream));
   return 0;
 }
 
 extern "C" int ga3c_workspace_ptr(ga3c_net* n, int which, void** ptr, int64_t* bytes) {
-  if (!n || !ptr) return fail_msg("ga3c_workspace_ptr: null argument");
+  if (!n || !ptr) return set_error("ga3c_workspace_ptr: null argument");
   const int64_t b = n->last_batch;
   switch (which) {
     case 0: *ptr = n->n1; if (bytes) *bytes = b * B2_BYTES; break;
@@ -797,7 +677,7 @@ extern "C" int ga3c_workspace_ptr(ga3c_net* n, int which, void** ptr, int64_t* b
     case 5: *ptr = n->dn1; if (bytes) *bytes = b * N1_POS * C1_OUT * 2; break;
     case 6: *ptr = n->w1_shadow; if (bytes) *bytes = (int64_t)FLAT * FC * 2; break;
     case 7: *ptr = n->xblk; if (bytes) *bytes = b * XB_FRAME_BYTES; break;
-    default: return fail_msg("ga3c_workspace_ptr: bad id");
+    default: return set_error("ga3c_workspace_ptr: bad id");
   }
   return 0;
 }
@@ -805,9 +685,9 @@ extern "C" int ga3c_workspace_ptr(ga3c_net* n, int which, void** ptr, int64_t* b
 extern "C" int ga3c_histograms(ga3c_net* n, int32_t batch, const float* p, const float* v, double* out, int32_t* bad,
                                void* stream) {
   if (int r = check_batch(n, batch, "ga3c_histograms")) return r;
-  if (!p || !v || !out || !bad) return fail_msg("ga3c_histograms: null buffer");
-  if (batch != n->last_batch) return fail_msg("ga3c_histograms: batch differs from the last forward on this handle");
-  if (n->dp_world > 1) return fail_msg("ga3c_histograms: not available on a peer-memory data-parallel handle");
+  if (!p || !v || !out || !bad) return set_error("ga3c_histograms: null buffer");
+  if (batch != n->last_batch) return set_error("ga3c_histograms: batch differs from the last forward on this handle");
+  if (n->dp_world > 1) return set_error("ga3c_histograms: not available on a peer-memory data-parallel handle");
   CK(cudaSetDevice(n->cfg.device));
   static_assert(GA3C_HISTO_SOURCES == P_COUNT + 5, "sources: the variables, n1, n2, d1, v, p");
   HistoArgs a{};
@@ -821,25 +701,11 @@ extern "C" int ga3c_histograms(ga3c_net* n, int32_t batch, const float* p, const
   a.n_src = GA3C_HISTO_SOURCES;
   a.out = out;
   a.bad = bad;
-  if (int r = histo_plan(a)) return r;
-  const size_t part_bytes = sizeof(double) * 4 * histo_blocks(a);
-  if (part_bytes > n->histo_part_bytes) {
-    CK(cudaFree(n->histo_part));
-    n->histo_part = nullptr;
-    n->histo_part_bytes = 0;
-    CK(cudaMalloc((void**)&n->histo_part, part_bytes));
-    n->histo_part_bytes = part_bytes;
-  }
-  a.part = n->histo_part;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (int r = histo_zero(a, st)) return r;
-  LAUNCH(n, K_HISTO, st, launch_histo(a, st));
-  LAUNCH(n, K_HISTO, st, launch_histo_merge(a, st));
-  return 0;
+  return launch_histograms(n, a, (cudaStream_t)stream);
 }
 
 extern "C" int ga3c_keep_dn1(ga3c_net* n, int32_t on) {
-  if (!n) return fail_msg("ga3c_keep_dn1: null handle");
+  if (!n) return set_error("ga3c_keep_dn1: null handle");
   n->keep_dn1 = on != 0;
   return 0;
 }
@@ -859,7 +725,7 @@ static int trace_attach_all(unsigned long long* buf) {
 }
 
 extern "C" int ga3c_trace_begin(ga3c_net* n, void* stream) {
-  if (!n) return fail_msg("ga3c_trace_begin: null handle");
+  if (!n) return set_error("ga3c_trace_begin: null handle");
   CK(cudaSetDevice(n->cfg.device));
   const size_t words = (size_t)K_COUNT * TRACE_SLOTS;
   if (!n->trace) CK(cudaMalloc((void**)&n->trace, words * 8));
@@ -872,8 +738,8 @@ extern "C" int ga3c_trace_begin(ga3c_net* n, void* stream) {
 }
 
 extern "C" int ga3c_trace_end(ga3c_net* n, uint64_t* stamps, int32_t n_kernels) {
-  if (!n || !stamps || n_kernels < K_COUNT) return fail_msg("ga3c_trace_end: bad argument");
-  if (!n->trace) return fail_msg("ga3c_trace_end: no trace in progress");
+  if (!n || !stamps || n_kernels < K_COUNT) return set_error("ga3c_trace_end: bad argument");
+  if (!n->trace) return set_error("ga3c_trace_end: no trace in progress");
   CK(cudaSetDevice(n->cfg.device));
   CK(cudaDeviceSynchronize());
   CKL(trace_attach_all(nullptr));
@@ -883,7 +749,7 @@ extern "C" int ga3c_trace_end(ga3c_net* n, uint64_t* stamps, int32_t n_kernels) 
 
 // ---- pipeline event log (debug) ----------------------------------------------------------------------
 extern "C" int ga3c_evt_begin(ga3c_net* n) {
-  if (!n) return fail_msg("ga3c_evt_begin: null handle");
+  if (!n) return set_error("ga3c_evt_begin: null handle");
   CK(cudaSetDevice(n->cfg.device));
   CK(cudaDeviceSynchronize());
   if (!n->evt) CK(cudaMalloc((void**)&n->evt, (size_t)2 * 16384 * 8));
@@ -901,7 +767,7 @@ extern "C" int ga3c_evt_begin(ga3c_net* n) {
 }
 
 extern "C" int ga3c_evt_end(ga3c_net* n, uint64_t* records, int32_t cap, int32_t* count) {
-  if (!n || !records || !count || !n->evt || cap < 16384) return fail_msg("ga3c_evt_end: bad argument");
+  if (!n || !records || !count || !n->evt || cap < 16384) return set_error("ga3c_evt_end: bad argument");
   CK(cudaSetDevice(n->cfg.device));
   CK(cudaDeviceSynchronize());
   CKL(evt_attach_conv_fwd(nullptr));
@@ -918,15 +784,9 @@ extern "C" int ga3c_evt_end(ga3c_net* n, uint64_t* records, int32_t cap, int32_t
 }
 
 extern "C" int ga3c_timing_enable(ga3c_net* n, int32_t max_records) {
-  if (!n || max_records < 0) return fail_msg("ga3c_timing_enable: bad argument");
-  CK(cudaSetDevice(n->cfg.device));
-  CK(cudaDeviceSynchronize());
-  return n->log.enable(max_records);
+  return timing_enable(n, max_records, "ga3c_timing_enable");
 }
 
 extern "C" int ga3c_timing_collect(ga3c_net* n, double* total_ms, int64_t* counts, int32_t n_kernels) {
-  if (!n || !total_ms || !counts || n_kernels < K_COUNT) return fail_msg("ga3c_timing_collect: bad argument");
-  CK(cudaSetDevice(n->cfg.device));
-  CK(cudaDeviceSynchronize());
-  return n->log.collect(total_ms, reinterpret_cast<long long*>(counts), n_kernels);
+  return timing_collect(n, total_ms, counts, n_kernels, "ga3c_timing_collect");
 }

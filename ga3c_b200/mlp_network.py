@@ -12,8 +12,6 @@ CPU fallback.
 from __future__ import annotations
 
 import ctypes as C
-import os
-import re
 import threading
 
 import numpy as np
@@ -22,41 +20,20 @@ import torch
 from . import _capi, summaries
 from ._arena import ArenaNetworkMixin
 from .config import Config as _DefaultConfig
-from .network import _parse_device
 
 
 class _MlpNetwork(ArenaNetworkMixin):
     KIND = None
+    _PREFIX = "ga3c_mlp_"
 
     def __init__(self, device, model_name, num_actions, state_dim, *, config=None, max_batch=None, seed=None):
         cfg = config or _DefaultConfig
-        self.config = cfg
-        self.device = device
-        self.model_name = model_name
-        self.num_actions = int(num_actions)
-        self.state_dim = int(np.prod(state_dim)) if not isinstance(state_dim, int) else state_dim
-        self._dual = bool(getattr(cfg, "DUAL_RMSPROP", False))
-        self.learning_rate = cfg.LEARNING_RATE_START
-        self.beta = cfg.BETA_START
-        self.log_epsilon = cfg.LOG_EPSILON
-
-        self._lib = _capi.load()
-        if not torch.cuda.is_available():
-            raise _capi.Ga3cError("no CUDA device visible: ga3c_b200 has no CPU fallback")
-        self._ordinal = _parse_device(device)
-        self._tdev = torch.device("cuda", self._ordinal)
+        fields = self._setup(device, model_name, num_actions, state_dim, cfg, max_batch)
         self._lock = threading.Lock()
-        self._max_batch = int(max_batch or max(getattr(cfg, "PREDICTION_BATCH_SIZE", 128), 128))
         dense = tuple(getattr(cfg, "DENSE_LAYERS", (10, 10, 10, 10)))          # Config.py:107
         c = _capi.ga3c_mlp_config(device=self._ordinal, kind=self.KIND, state_dim=self.state_dim,
                                   num_actions=self.num_actions, max_batch=self._max_batch, n_dense=len(dense),
-                                  dense_width=(C.c_int32 * 8)(*dense[:8]),
-                                  rmsprop_decay=cfg.RMSPROP_DECAY, rmsprop_momentum=cfg.RMSPROP_MOMENTUM,
-                                  rmsprop_epsilon=cfg.RMSPROP_EPSILON, log_epsilon=cfg.LOG_EPSILON,
-                                  min_policy=cfg.MIN_POLICY,
-                                  use_log_softmax=int(bool(getattr(cfg, 'USE_LOG_SOFTMAX', False))),
-                              use_grad_clip=int(bool(getattr(cfg, 'USE_GRAD_CLIP', False))),
-                              grad_clip_norm=float(getattr(cfg, 'GRAD_CLIP_NORM', 40.0)), dual_rmsprop=int(self._dual))
+                                  dense_width=(C.c_int32 * 8)(*dense[:8]), **fields)
         if self.KIND == _capi.MLP_DISCRATE and len(dense) > 8:
             raise ValueError("Config.DENSE_LAYERS: at most 8 entries")
         h = C.c_void_p()
@@ -80,45 +57,9 @@ class _MlpNetwork(ArenaNetworkMixin):
         # every variable: U(-0.3, 0.3)  (dense_layer, NetworkVP.py:199-202)
         rng = np.random.default_rng(seed)
         self.set_variables({k: rng.uniform(-0.3, 0.3, size=s).astype(np.float32) for k, (_, s) in self._table.items()})
-        self.last_losses = None
         self._hist_tags = summaries.mlp_histogram_tags([(k, self._live[k]) for k in self._table])
         if len(self._hist_tags) != self._lib.ga3c_mlp_histogram_count(self._h):
             raise _capi.Ga3cError("ga3c_mlp_histogram_count disagrees with the variable table")
-        self._summ_dev = self._summ_host = None     # log / histograms: device results and their pinned copy
-        self._events = None                         # the TensorBoard event file, opened by the first log()
-
-    # ------------------------------------------------------------------ buffers
-    def _alloc_io(self, rows: int):
-        a, s = self.num_actions, self.state_dim
-        with torch.cuda.device(self._tdev):
-            self._hx = torch.empty((rows, s), dtype=torch.float32, pin_memory=True)
-            self._hyr = torch.empty((rows,), dtype=torch.float32, pin_memory=True)
-            self._ha = torch.empty((rows, a), dtype=torch.float32, pin_memory=True)
-            self._hp = torch.empty((rows, a), dtype=torch.float32, pin_memory=True)
-            self._hv = torch.empty((rows,), dtype=torch.float32, pin_memory=True)
-            self._dx = torch.empty((rows, s), dtype=torch.float32, device=self._tdev)
-            self._dyr = torch.empty((rows,), dtype=torch.float32, device=self._tdev)
-            self._da = torch.empty((rows, a), dtype=torch.float32, device=self._tdev)
-            self._dp_out = torch.empty((rows, a), dtype=torch.float32, device=self._tdev)
-            self._dv_out = torch.empty((rows,), dtype=torch.float32, device=self._tdev)
-        self._io_rows = rows
-
-    def _ensure(self, rows: int):
-        if rows > self._max_batch:
-            _capi.check(self._lib.ga3c_mlp_reserve(self._h, rows), "ga3c_mlp_reserve")
-            self._max_batch = rows
-        if rows > self._io_rows:
-            self._alloc_io(rows)
-
-    def __del__(self):
-        try:
-            if getattr(self, "_events", None) is not None:
-                self._events.close()
-            if getattr(self, "_h", None):
-                self._lib.ga3c_mlp_destroy(self._h)
-                self._h = None
-        except Exception:
-            pass
 
     # ------------------------------------------------------------------ device-resident API
     def predict_device(self, x_dev, p_out=None, v_out=None, stream=None):
@@ -187,11 +128,6 @@ class _MlpNetwork(ArenaNetworkMixin):
         self._da[:b].copy_(self._ha[:b], non_blocking=True)
         return b
 
-    @staticmethod
-    def _loss_dict(l):
-        c1, c2, cv = (float(v) for v in l[:3])
-        return dict(cost_p_1=c1, cost_p_2=c2, cost_p=-(c1 + c2), cost_v=cv, cost_all=-(c1 + c2) + cv)
-
     def train(self, x, y_r, a, x2=None, done=None, trainer_id=0, *, fetch_losses=False):
         """NetworkVP.py:254-257; x2, done, trainer_id are ignored as in the reference."""
         if np.asarray(x).shape[0] == 0:
@@ -220,59 +156,19 @@ class _MlpNetwork(ArenaNetworkMixin):
         return self._loss_dict(l)
 
     # ------------------------------------------------------------------ TensorBoard summaries (NetworkVP.py:152-173, :259-265)
-    _HROW = 5 + summaries.BUCKETS
-
-    def _summaries(self, x, y_r, a):
-        """predict, forward_backward and ga3c_mlp_histograms on the same rows as ONE critical section of the handle (no trainer
-        thread can overwrite the layer outputs in between), then one device -> host copy.  predict goes first: for a
+    def _summary_pass(self, x, y_r, a, loss_ptr, st):
+        """predict, then forward_backward with the loss sums to loss_ptr, on st; returns the rows.  predict goes first: for a
         tensor-core batch it writes its layer outputs through the training workspace, which forward_backward then rewrites.
-        Weights, slots and the step counter are not touched.  Returns (losses, {tag: (min, max, num, sum, sum_squares,
-        counts)}, [tags of the histograms holding a NaN / Inf])."""
-        x = self._rows(x)
-        if x.shape[0] == 0:
-            raise ValueError("the summaries need at least one row")
-        tags = self._hist_tags
-        n_hist = len(tags) * self._HROW
-        n_bad = (len(tags) + 1) // 2
-        if self._summ_dev is None:
-            # [histogram rows | int32 non-finite flags | 4 fp32 loss sums] as doubles, so that one copy brings it all back
-            with torch.cuda.device(self._tdev):
-                self._summ_dev = torch.empty(n_hist + n_bad + 2, dtype=torch.float64, device=self._tdev)
-                self._summ_host = torch.empty(n_hist + n_bad + 2, dtype=torch.float64, pin_memory=True)
-        base = self._summ_dev.data_ptr()
-        bad_ptr, loss_ptr = base + 8 * n_hist, base + 8 * (n_hist + n_bad)
-        with self._lock:
-            st = self._stream
-            with torch.cuda.stream(st):
-                b = self._stage_train(x, y_r, a)
-                dx, dp, dv = self._dx[:b], self._dp_out[:b], self._dv_out[:b]
-                self.predict_device(dx, dp, dv, stream=st)
-                _capi.check(self._lib.ga3c_mlp_forward_backward(self._h, dx.data_ptr(), self._dyr.data_ptr(), self._da.data_ptr(),
-                                                                b, float(self.beta), loss_ptr, st.cuda_stream),
-                            "ga3c_mlp_forward_backward")
-                _capi.check(self._lib.ga3c_mlp_histograms(self._h, b, dp.data_ptr(), dv.data_ptr(), base, bad_ptr,
-                                                          st.cuda_stream), "ga3c_mlp_histograms")
-                self._summ_host.copy_(self._summ_dev, non_blocking=True)
-            st.synchronize()
-            host = self._summ_host.numpy().copy()
-        rows = host[:n_hist].reshape(len(tags), self._HROW)
-        stats = {t: (r[0], r[1], r[2], r[3], r[4], r[5:]) for t, r in zip(tags, rows)}
-        bad = host[n_hist:n_hist + n_bad].view(np.int32)[:len(tags)]
-        l = self._loss_dict(host[n_hist + n_bad:].view(np.float32))
-        return l, stats, [t for t, f in zip(tags, bad) if f]
-
-    def histograms(self, x, y_r, a) -> dict:
-        """The histograms `log` writes, for rows x [B, S] and targets y_r, a: {tag: (min, max, num, sum, sum_squares, counts)},
-        TF's histogram::Histogram with its 1551 default buckets (ga3c_b200.summaries.LIMITS), computed on the GPU.  Tags
-        (summaries.mlp_histogram_tags): weights_<variable name> (tf.summary's tag cleaning, e.g. weights_dense1/w_0) for every
-        variable in TF creation order, gradient-less ones included; activation_<layer scope> for every live hidden layer in
-        forward order (fork NetworkVP: activation_dense11_p ... activation_dense14_p, activation_dense1; NetworkVP_discrate:
-        activation_dense1_<n>_p); then activation_v (logits_v) and activation_p (softmax_p: for the fork NetworkVP the atan2
-        output).  Raises ValueError on a NaN / Inf."""
-        _, stats, bad = self._summaries(x, y_r, a)
-        if bad:
-            raise self._nonfinite(bad)
-        return stats
+        Histogram tags (summaries.mlp_histogram_tags): every variable, gradient-less ones included; activation_<layer scope>
+        for every live hidden layer in forward order (fork NetworkVP: activation_dense11_p ... activation_dense14_p,
+        activation_dense1; NetworkVP_discrate: activation_dense1_<n>_p); activation_v (logits_v) and activation_p (softmax_p:
+        for the fork NetworkVP the atan2 output)."""
+        b = self._stage_train(x, y_r, a)
+        dx = self._dx[:b]
+        self.predict_device(dx, self._dp_out[:b], self._dv_out[:b], stream=st)
+        self._call("forward_backward", dx.data_ptr(), self._dyr.data_ptr(), self._da.data_ptr(), b, float(self.beta),
+                   loss_ptr, st.cuda_stream)
+        return b
 
     def log(self, x, y_r, a, training_step, feed_dict=None):
         """NetworkVP.py:259-265: appends the six scalars to logs/<model_name>/scalars.csv and writes them with the histograms
@@ -282,30 +178,13 @@ class _MlpNetwork(ArenaNetworkMixin):
         self._log_summaries(*self._summaries(x, y_r, a), training_step)
 
     # ------------------------------------------------------------------ variables / checkpoints
-    def get_global_step(self):
-        return int(self._lib.ga3c_mlp_global_step(self._h))
-
     def live_variables(self):
         return [k for k in self._table if self._live[k]]
-
-    def _download(self, which: int) -> np.ndarray:
-        out = np.empty(self._arena_floats, dtype=np.float32)
-        with self._lock:
-            _capi.check(self._lib.ga3c_mlp_arena_download(self._h, which, out.ctypes.data, out.size), "ga3c_mlp_arena_download")
-        return out
-
-    def _upload(self, which: int, arena: np.ndarray):
-        arena = np.ascontiguousarray(arena, dtype=np.float32)
-        with self._lock:
-            _capi.check(self._lib.ga3c_mlp_arena_upload(self._h, which, arena.ctypes.data, arena.size), "ga3c_mlp_arena_upload")
 
     def get_gradients(self):
         """Gradients of the last forward_backward; live variables only (the others have none)."""
         g = self._split(self._download(1))
         return {k: v for k, v in g.items() if self._live[k]}
-
-    def _set_global_step(self, step: int):
-        self._lib.ga3c_mlp_set_global_step(self._h, int(step))
 
     # ------------------------------------------------------------------ introspection
     def workspace(self, which: int, layer: int, batch: int) -> np.ndarray:
@@ -318,18 +197,6 @@ class _MlpNetwork(ArenaNetworkMixin):
         iface = {"shape": (int(batch) * width.value,), "typestr": "<f4", "data": (ptr.value, False), "version": 2}
         holder = type("H", (), {"__cuda_array_interface__": iface})()
         return torch.as_tensor(holder, device=self._tdev).cpu().numpy().reshape(int(batch), width.value).copy()
-
-    def launch_count(self) -> int:
-        return int(self._lib.ga3c_mlp_launch_count(self._h))
-
-    def kernel_timing(self, max_records: int):
-        _capi.check(self._lib.ga3c_mlp_timing_enable(self._h, int(max_records)), "ga3c_mlp_timing_enable")
-
-    def kernel_times(self) -> dict:
-        n = self._lib.ga3c_kernel_count()
-        tot, cnt = (C.c_double * n)(), (C.c_int64 * n)()
-        _capi.check(self._lib.ga3c_mlp_timing_collect(self._h, tot, cnt, n), "ga3c_mlp_timing_collect")
-        return {self._lib.ga3c_kernel_name(k).decode(): (tot[k], cnt[k]) for k in range(n) if cnt[k]}
 
 
 class NetworkVP(_MlpNetwork):

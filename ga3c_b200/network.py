@@ -17,7 +17,6 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-import re
 import threading
 import warnings
 
@@ -25,20 +24,10 @@ import numpy as np
 import torch
 
 from . import _capi, summaries
-from ._arena import ArenaNetworkMixin
+from ._arena import ArenaNetworkMixin, _parse_device  # noqa: F401  (_parse_device: part of this module's interface)
 from .config import Config as _DefaultConfig
 
 STATE_DIM = 84 * 84 * 4
-
-
-def _parse_device(device) -> int:
-    """Config.DEVICE is a TF-style string 'gpu:0' (Config.py:62); 'cuda:0' and ints are accepted too."""
-    if isinstance(device, int):
-        return device
-    m = re.fullmatch(r"/?(?:device:)?(gpu|cuda)(?::(\d+))?", str(device).strip().lower())
-    if not m:
-        raise ValueError(f"unsupported device {device!r}: this implementation is GPU-only ('gpu:N')")
-    return int(m.group(2) or 0)
 
 
 class _DevArray:
@@ -101,32 +90,11 @@ class Network(ArenaNetworkMixin):
     def __init__(self, device, model_name, num_actions, state_dim=STATE_DIM, *, config=None, max_batch=None,
                  seed=None, data_parallel=None, dp_mode=None):
         cfg = config or _DefaultConfig
-        self.config = cfg
-        self.device = device
-        self.model_name = model_name
-        self.num_actions = int(num_actions)
-        self.state_dim = int(np.prod(state_dim)) if not isinstance(state_dim, int) else state_dim
-        if self.state_dim != STATE_DIM:
-            raise ValueError(f"conv NetworkVP expects state_dim = 84*84*4 = {STATE_DIM}, got {self.state_dim}")
-        self._dual = bool(getattr(cfg, "DUAL_RMSPROP", False))
-
-        self.learning_rate = cfg.LEARNING_RATE_START      # NetworkVP.py:44
-        self.beta = cfg.BETA_START                        # NetworkVP.py:45
-        self.log_epsilon = cfg.LOG_EPSILON                # NetworkVP.py:46
-
-        self._lib = _capi.load()
-        if not torch.cuda.is_available():
-            raise _capi.Ga3cError("no CUDA device visible: ga3c_b200 has no CPU fallback")
-        self._ordinal = _parse_device(device)
-        self._tdev = torch.device("cuda", self._ordinal)
-        self._max_batch = int(max_batch or max(getattr(cfg, "PREDICTION_BATCH_SIZE", 128), 128))
-
-        c = _capi.ga3c_config(device=self._ordinal, num_actions=self.num_actions, max_batch=self._max_batch,
-                              rmsprop_decay=cfg.RMSPROP_DECAY, rmsprop_momentum=cfg.RMSPROP_MOMENTUM,
-                              rmsprop_epsilon=cfg.RMSPROP_EPSILON, log_epsilon=cfg.LOG_EPSILON,
-                              min_policy=cfg.MIN_POLICY, use_log_softmax=int(bool(getattr(cfg, 'USE_LOG_SOFTMAX', False))),
-                              use_grad_clip=int(bool(getattr(cfg, 'USE_GRAD_CLIP', False))),
-                              grad_clip_norm=float(getattr(cfg, 'GRAD_CLIP_NORM', 40.0)), dual_rmsprop=int(self._dual))
+        sd = int(np.prod(state_dim)) if not isinstance(state_dim, int) else state_dim
+        if sd != STATE_DIM:
+            raise ValueError(f"conv NetworkVP expects state_dim = 84*84*4 = {STATE_DIM}, got {sd}")
+        fields = self._setup(device, model_name, num_actions, sd, cfg, max_batch)
+        c = _capi.ga3c_config(device=self._ordinal, num_actions=self.num_actions, max_batch=self._max_batch, **fields)
         h = C.c_void_p()
         _capi.check(self._lib.ga3c_create(C.byref(c), C.byref(h)), "ga3c_create")
         self._h = h
@@ -199,25 +167,11 @@ class Network(ArenaNetworkMixin):
                         "ga3c_dp_attach")
             dist.barrier(device_ids=[self._ordinal])      # every rank has mapped every slab before the first step
         self._dp = self.dp_mode == "nccl"
-        self.last_losses = None
-        self._summ_dev = self._summ_host = None     # Network.log / histograms: device results and their pinned copy
-        self._events = None                         # the TensorBoard event file, opened by the first log()
+        self._hist_tags = summaries.histogram_tags(self._table)
 
     # ------------------------------------------------------------------ buffers
     def _alloc_io(self, rows: int):
-        with torch.cuda.device(self._tdev):
-            a = self.num_actions
-            self._hx = torch.empty((rows, STATE_DIM), dtype=torch.float32, pin_memory=True)
-            self._hyr = torch.empty((rows,), dtype=torch.float32, pin_memory=True)
-            self._ha = torch.empty((rows, a), dtype=torch.float32, pin_memory=True)
-            self._hp = torch.empty((rows, a), dtype=torch.float32, pin_memory=True)
-            self._hv = torch.empty((rows,), dtype=torch.float32, pin_memory=True)
-            self._dx = torch.empty((rows, STATE_DIM), dtype=torch.float32, device=self._tdev)
-            self._dyr = torch.empty((rows,), dtype=torch.float32, device=self._tdev)
-            self._da = torch.empty((rows, a), dtype=torch.float32, device=self._tdev)
-            self._dp_out = torch.empty((rows, a), dtype=torch.float32, device=self._tdev)
-            self._dv_out = torch.empty((rows,), dtype=torch.float32, device=self._tdev)
-        self._io_rows = rows
+        super()._alloc_io(rows)
         self._hx8 = self._dx8 = None          # uint8 frame staging, allocated on first use (F2 ingestion)
 
     def _io_u8(self):
@@ -239,13 +193,6 @@ class Network(ArenaNetworkMixin):
             if x.shape[1] != state_dim:
                 raise ValueError(f"x must be [B, {state_dim}], got {x.shape}")
         return x
-
-    def _ensure(self, rows: int):
-        if rows > self._max_batch:
-            _capi.check(self._lib.ga3c_reserve(self._h, rows), "ga3c_reserve")
-            self._max_batch = rows
-        if rows > self._io_rows:
-            self._alloc_io(rows)
 
     _CHUNK_BYTES = 8 << 20
 
@@ -294,14 +241,11 @@ class Network(ArenaNetworkMixin):
 
     def __del__(self):
         try:
-            if getattr(self, "_events", None) is not None:
-                self._events.close()
             if getattr(self, "_h", None):
                 self._lib.ga3c_dp_detach(self._h)
-                self._lib.ga3c_destroy(self._h)
-                self._h = None
         except Exception:
             pass
+        super().__del__()
 
     # ------------------------------------------------------------------ device-resident API
     def predict_device(self, x_dev: torch.Tensor, p_out: torch.Tensor = None, v_out: torch.Tensor = None, stream=None):
@@ -444,8 +388,7 @@ class Network(ArenaNetworkMixin):
             if self._dp_steps % 64 == 1:      # a timed-out cross-rank wait leaves garbage weights: fail, do not train on
                 self.dp_check()
         if fetch_losses:
-            c1, c2, cv = (float(v) for v in losses[:3])
-            self.last_losses = dict(cost_p_1=c1, cost_p_2=c2, cost_p=-(c1 + c2), cost_v=cv, cost_all=-(c1 + c2) + cv)
+            self.last_losses = self._loss_dict(losses)
             return self.last_losses
         return None
 
@@ -466,70 +409,31 @@ class Network(ArenaNetworkMixin):
                                self._loss_dev.data_ptr(), st.cuda_stream), "ga3c_forward_backward")
                 l = self._loss_dev.cpu()
             st.synchronize()
-        c1, c2, cv = (float(v) for v in l[:3])
-        return dict(cost_p_1=c1, cost_p_2=c2, cost_p=-(c1 + c2), cost_v=cv, cost_all=-(c1 + c2) + cv)
+        return self._loss_dict(l)
 
     # ------------------------------------------------------------------ TensorBoard summaries (NetworkVP.py:152-173, :259-265)
-    _HROW = 5 + summaries.BUCKETS
-
-    def _summaries(self, x, y_r, a):
-        """predict, forward_backward and ga3c_histograms on the same frames as ONE critical section of the handle (no trainer
-        thread can overwrite the activation workspace in between), then one device -> host copy.  predict goes first: it
-        rewrites n2 / d1 of the workspace, which forward_backward then leaves as the training forward computes them.  Weights,
-        slots and the step counter are not touched.  Returns (losses, {tag: (min, max, num, sum, sum_squares, counts)},
-        [tags of the histograms holding a NaN / Inf])."""
+    def _summary_pass(self, x, y_r, a, loss_ptr, st):
+        """predict, then forward_backward with the loss sums to loss_ptr, on st, for frames x (float32 or uint8); returns the
+        rows.  predict goes first: it rewrites n2 / d1 of the workspace, which forward_backward then leaves as the training
+        forward computes them.  Histogram tags: the 10 variables, then activation_n1, activation_n2, activation_d2 (dense1),
+        activation_v and activation_p; n1 and n2 are histogrammed as the network stores them (bf16)."""
         x = self._frames(x, self.state_dim)
         b = x.shape[0]
-        if b == 0:
-            raise ValueError("the summaries need at least one row")
         y_r = np.asarray(y_r, dtype=np.float32).reshape(b)
         a = np.asarray(a, dtype=np.float32).reshape(b, self.num_actions)
         u8 = x.dtype == np.uint8
-        tags = summaries.histogram_tags(self._table)
-        n_hist = len(tags) * self._HROW
-        if self._summ_dev is None:
-            # [histogram rows | 16 int32 non-finite flags | 4 fp32 loss sums] as doubles, so that one copy brings it all back
-            with torch.cuda.device(self._tdev):
-                self._summ_dev = torch.empty(n_hist + 10, dtype=torch.float64, device=self._tdev)
-                self._summ_host = torch.empty(n_hist + 10, dtype=torch.float64, pin_memory=True)
-        base = self._summ_dev.data_ptr()
-        bad_ptr, loss_ptr = base + 8 * n_hist, base + 8 * n_hist + 64
-        with self._lock:
-            self._ensure(b)
-            hx, dx = self._io_u8() if u8 else (self._hx, self._dx)
-            st = self._stream
-            with torch.cuda.stream(st):
-                self._h2d(x, hx, dx, b)
-                self._h2d(y_r, self._hyr, self._dyr, b)
-                self._h2d(a, self._ha, self._da, b)
-                pred = self._lib.ga3c_predict_u8 if u8 else self._lib.ga3c_predict
-                _capi.check(pred(self._h, dx.data_ptr(), b, self._dp_out.data_ptr(), self._dv_out.data_ptr(), st.cuda_stream),
-                            "ga3c_predict")
-                fb = self._lib.ga3c_forward_backward_u8 if u8 else self._lib.ga3c_forward_backward
-                _capi.check(fb(self._h, dx.data_ptr(), self._dyr.data_ptr(), self._da.data_ptr(), b, float(self.beta), loss_ptr,
-                               st.cuda_stream), "ga3c_forward_backward")
-                _capi.check(self._lib.ga3c_histograms(self._h, b, self._dp_out.data_ptr(), self._dv_out.data_ptr(), base, bad_ptr,
-                                                      st.cuda_stream), "ga3c_histograms")
-                self._summ_host.copy_(self._summ_dev, non_blocking=True)
-            st.synchronize()
-            host = self._summ_host.numpy().copy()
-        rows = host[:n_hist].reshape(len(tags), self._HROW)
-        stats = {t: (r[0], r[1], r[2], r[3], r[4], r[5:]) for t, r in zip(tags, rows)}
-        bad = host[n_hist:n_hist + 8].view(np.int32)[:len(tags)]
-        c1, c2, cv = (float(v) for v in host[n_hist + 8:].view(np.float32)[:3])
-        l = dict(cost_p_1=c1, cost_p_2=c2, cost_p=-(c1 + c2), cost_v=cv, cost_all=-(c1 + c2) + cv)
-        return l, stats, [t for t, f in zip(tags, bad) if f]
-
-    def histograms(self, x, y_r, a) -> dict:
-        """The 15 histograms `log` writes, for frames x (float32 or uint8) and targets y_r, a:
-        {tag: (min, max, num, sum, sum_squares, counts)}, TF's histogram::Histogram with its 1551 default buckets
-        (ga3c_b200.summaries.LIMITS), computed on the GPU.  Tags: weights_<variable name> (tf.summary's tag cleaning, e.g.
-        weights_conv11/w_0) in TF creation order, then activation_n1, activation_n2, activation_d2 (dense1), activation_v and
-        activation_p.  n1 and n2 are histogrammed as the network stores them (bf16).  Raises ValueError on a NaN / Inf."""
-        _, stats, bad = self._summaries(x, y_r, a)
-        if bad:
-            raise self._nonfinite(bad)
-        return stats
+        self._ensure(b)
+        hx, dx = self._io_u8() if u8 else (self._hx, self._dx)
+        self._h2d(x, hx, dx, b)
+        self._h2d(y_r, self._hyr, self._dyr, b)
+        self._h2d(a, self._ha, self._da, b)
+        pred = self._lib.ga3c_predict_u8 if u8 else self._lib.ga3c_predict
+        _capi.check(pred(self._h, dx.data_ptr(), b, self._dp_out.data_ptr(), self._dv_out.data_ptr(), st.cuda_stream),
+                    "ga3c_predict")
+        fb = self._lib.ga3c_forward_backward_u8 if u8 else self._lib.ga3c_forward_backward
+        _capi.check(fb(self._h, dx.data_ptr(), self._dyr.data_ptr(), self._da.data_ptr(), b, float(self.beta), loss_ptr,
+                       st.cuda_stream), "ga3c_forward_backward")
+        return b
 
     def log(self, x, y_r, a, training_step, feed_dict=None):
         """NetworkVP.py:259-265: appends the six scalars to logs/<model_name>/scalars.csv (as the MLP networks do) and writes
@@ -546,29 +450,15 @@ class Network(ArenaNetworkMixin):
         self._log_summaries(*self._summaries(x, y_r, a), training_step)
 
     # ------------------------------------------------------------------ variables / checkpoints
-    def get_global_step(self):              # NetworkVP.py:233-235
-        return int(self._lib.ga3c_global_step(self._h))
-
     def _download(self, which: int) -> np.ndarray:
         self.dp_check()
-        out = np.empty(self._arena_floats, dtype=np.float32)
-        with self._lock:
-            _capi.check(self._lib.ga3c_arena_download(self._h, which, out.ctypes.data, out.size), "ga3c_arena_download")
-        return out
-
-    def _upload(self, which: int, arena: np.ndarray):
-        arena = np.ascontiguousarray(arena, dtype=np.float32)
-        with self._lock:
-            _capi.check(self._lib.ga3c_arena_upload(self._h, which, arena.ctypes.data, arena.size), "ga3c_arena_upload")
+        return super()._download(which)
 
     def get_gradients(self):
         """Gradients left by the last forward_backward.  Data parallel: dp_mode 'nccl' leaves the allreduced gradient on every
         rank; dp_mode 'fused' leaves this rank's OWN contribution, except for the slice of dense1/w this rank owns, which
         holds the sum over ranks (the reduction happens on the owner; only the bf16 shadow of the new weights travels)."""
         return self._split(self._download(1))
-
-    def _set_global_step(self, step: int):
-        self._lib.ga3c_set_global_step(self._h, int(step))
 
     def _after_load(self):
         if self.dp_mode is not None:
@@ -584,20 +474,6 @@ class Network(ArenaNetworkMixin):
                                   "dp_exchange.cuh): replicas are out of sync")
 
     # ------------------------------------------------------------------ introspection (tests / profiling)
-    def launch_count(self) -> int:
-        return int(self._lib.ga3c_launch_count(self._h))
-
-    def kernel_timing(self, max_records: int):
-        """Bracket every kernel of the path with CUDA events on its launch stream (0 = off)."""
-        _capi.check(self._lib.ga3c_timing_enable(self._h, int(max_records)), "ga3c_timing_enable")
-
-    def kernel_times(self) -> dict:
-        """{kernel name: (total ms, launches)} since the last call; synchronises the device."""
-        n = self._lib.ga3c_kernel_count()
-        tot, cnt = (C.c_double * n)(), (C.c_int64 * n)()
-        _capi.check(self._lib.ga3c_timing_collect(self._h, tot, cnt, n), "ga3c_timing_collect")
-        return {self._lib.ga3c_kernel_name(k).decode(): (tot[k], cnt[k]) for k in range(n)}
-
     def trace_begin(self, stream=None):
         """Start a step timeline trace (ga3c_trace_begin): kernels stamp %globaltimer at launch / start / end."""
         st = stream if stream is not None else torch.cuda.current_stream(self._tdev)

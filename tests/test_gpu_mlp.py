@@ -388,13 +388,12 @@ def test_full_size_batch_and_reproducibility(mlp):
         assert err(g1[k], g_ref)[1] <= TOL_GRAD_REL, (k, err(g1[k], g_ref))
 
 
-def check_tensor_cores_against_oracle_and_fp32(mlp, monkeypatch, s, a, stream, batch, tc):
+def check_tensor_cores_against_oracle_and_fp32(mlp, monkeypatch, s, a, batch, tc):
     """fork_vp (s, a) with GA3C_MLP_TC = tc (None: unset, the default 4,096-row threshold) against the oracle and against a
     GA3C_MLP_TC=0 handle (fp32 FMA path): predictions, losses and gradients.  Predict streams (front, 3 GEMMs, heads) only for
-    one action and state_dim <= 4 with GA3C_MLP_STREAM=1; otherwise it is one fused launch."""
+    one action and state_dim <= 4; otherwise it is one fused launch."""
     kind = "fork_vp"
     params, x, y_r, act = make_mlp_case(kind, s, a, batch, seed=11)
-    monkeypatch.setenv("GA3C_MLP_STREAM", stream)
     out = {}
     for mode in ("1", "0"):
         if mode == "1" and tc is None:
@@ -409,7 +408,7 @@ def check_tensor_cores_against_oracle_and_fp32(mlp, monkeypatch, s, a, stream, b
         n1 = net.launch_count()
         out[mode] = (net.losses(x, y_r, act), net.get_gradients(), net.launch_count() - n1, pv, n1 - n0)
     assert out["1"][2] > out["0"][2] == 3, (out["1"][2], out["0"][2])      # the GEMM launches really ran
-    streamed = a == 1 and s <= 4 and stream == "1"
+    streamed = a == 1 and s <= 4
     assert out["0"][4] == 1 and out["1"][4] == (5 if streamed else 1), (out["1"][4], out["0"][4])
     p_ref, v_ref = om.forward(params, x, kind)
     for mode in ("1", "0"):
@@ -426,20 +425,20 @@ def check_tensor_cores_against_oracle_and_fp32(mlp, monkeypatch, s, a, stream, b
         assert r <= TOL_GRAD_REL or d <= 1e-6, ("vs fp32 path", k, d, r)
 
 
-@pytest.mark.parametrize("s,a,stream", [(3, 1, "1"), (3, 1, "0"), (4, 2, "1"), (5, 1, "1"), (8, 2, "1"), (24, 4, "1")])
+@pytest.mark.parametrize("s,a", [(3, 1), (4, 2), (5, 1), (8, 2), (24, 4)])
 @pytest.mark.parametrize("batch", [33, 128, 1000, 4097])
-def test_tensor_core_wide_layers_match_oracle_and_the_fp32_path(mlp, monkeypatch, s, a, stream, batch):
+def test_tensor_core_wide_layers_match_oracle_and_the_fp32_path(mlp, monkeypatch, s, a, batch):
     """The 256 -> 256, 256 -> 100 and 100 -> 64 layers of the fork NetworkVP as 3xTF32 tcgen05 GEMMs (mlp_tc.cu; taken from 4096
     rows on, forced here from 1 row): same tolerances against the oracle as the fp32 FMA path, and close to that path itself --
     predictions, losses and gradients.  With one action and state_dim <= 4 the narrow ends are the streaming kernels of
-    mlp_stream.cu (GA3C_MLP_STREAM=0: the fused kernel's phases); otherwise always the fused kernel's phases, and with
-    state_dim > 4 layer 0's weight gradient comes from the tile kernel (mlp_wgrad) instead of mlp_skinny_wgrad."""
-    check_tensor_cores_against_oracle_and_fp32(mlp, monkeypatch, s, a, stream, batch, tc="1")
+    mlp_stream.cu; otherwise the fused kernel's phases, and with state_dim > 4 layer 0's weight gradient comes from the tile
+    kernel (mlp_wgrad) instead of mlp_skinny_wgrad."""
+    check_tensor_cores_against_oracle_and_fp32(mlp, monkeypatch, s, a, batch, tc="1")
 
 
 def test_tensor_cores_from_the_default_threshold(mlp, monkeypatch):
     """GA3C_MLP_TC unset: a LunarLanderContinuous-sized NetworkVP (8, 2) crosses the default 4,096-row threshold at 5,000 rows."""
-    check_tensor_cores_against_oracle_and_fp32(mlp, monkeypatch, 8, 2, "1", 5000, tc=None)
+    check_tensor_cores_against_oracle_and_fp32(mlp, monkeypatch, 8, 2, 5000, tc=None)
 
 
 def test_batch_sum_is_additive(mlp):

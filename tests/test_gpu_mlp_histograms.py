@@ -61,19 +61,18 @@ def test_histograms_match_the_oracle(mlp, kind, s, a, b):
     check_against_the_network(net, kind, x, y_r, act)
 
 
-@pytest.mark.parametrize("stream", ["1", "0"])
-def test_histograms_on_the_tensor_core_path(mlp, monkeypatch, stream):
+@pytest.mark.parametrize("s,a", [(3, 1), (8, 2)])
+def test_histograms_on_the_tensor_core_path(mlp, monkeypatch, s, a):
     """GA3C_MLP_TC=1: the wide layers of the fork NetworkVP as tcgen05 GEMMs from one row on, the narrow ends as streaming
-    kernels (GA3C_MLP_STREAM=1) or as the fused kernel's phases (0); predict then also writes the layer workspace."""
+    kernels (one action, state_dim <= 4; predict then also writes the layer workspace) or as the fused kernel's phases."""
     monkeypatch.setenv("GA3C_MLP_TC", "1")
-    monkeypatch.setenv("GA3C_MLP_STREAM", stream)
-    kind, s, a, b = "fork_vp", 3, 1, 1000
+    kind, b = "fork_vp", 1000
     params, x, y_r, act = make_mlp_case(kind, s, a, b, seed=3)
     net = make_mlp_net(mlp, kind, s, a, max_batch=b)
     net.set_variables(params)
     n0 = net.launch_count()
     net.predict_p_and_v(x)
-    assert net.launch_count() - n0 == (5 if stream == "1" else 1)         # the path these env variables select
+    assert net.launch_count() - n0 == (5 if a == 1 and s <= 4 else 1)      # the path the shape selects
     check_against_the_network(net, kind, x, y_r, act)
 
 
