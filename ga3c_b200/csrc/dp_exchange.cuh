@@ -77,6 +77,21 @@ __device__ __forceinline__ float4 dp_ld_f4(const float4* p) {      // L2 (the ow
   return r;
 }
 
+// ---- RMSProp, TensorFlow semantics (tf.train.RMSPropOptimizer, NetworkVP_discrate.py:101-105) ----
+//   ms  <- rho*ms + (1-rho)*g^2 ; mom <- mu*mom + lr*g/sqrt(ms + eps) ; w <- w - mom       [TF-SEMANTICS]
+// The one element update of every optimizer kernel (elementwise.cu) and of the dense1/w exchange (dp_big_loop).  With mu == 0
+// (Config.RMSPROP_MOMENTUM) mom enters as zero and leaves as the step.
+__device__ __forceinline__ void rms_update(const float4& g, float4& w, float4& ms, float4& mo, float lr, float decay, float momentum,
+                                           float eps) {
+  const float one_m_rho = 1.f - decay;
+  auto one = [&](float gc, float& wc, float& msc, float& moc) {
+    msc = decay * msc + one_m_rho * gc * gc;
+    moc = momentum * moc + lr * gc / sqrtf(msc + eps);
+    wc -= moc;
+  };
+  one(g.x, w.x, ms.x, mo.x); one(g.y, w.y, ms.y, mo.y); one(g.z, w.z, ms.z, mo.z); one(g.w, w.w, ms.w, mo.w);
+}
+
 struct DpBigArgs {
   uint8_t* peer[DP_WORLD_MAX];      // slab bases: [params | grads | ms | mom | shadow | LL receive buffers | comm]
   int rank, world;
@@ -92,7 +107,7 @@ struct DpBigArgs {
 template <int W, int U>
 __device__ __forceinline__ void dp_big_loop(const DpBigArgs& d, long long lo, long long hi, long long first, long long stride) {
   const long long base4 = d.w1_offset >> 2;
-  const float one_m_rho = 1.f - d.decay;
+  const float lr = d.lr, decay = d.decay, momentum = d.momentum, eps = d.eps;     // read ahead of the loop: 4 B less spill
   float4* w_own = reinterpret_cast<float4*>(d.peer[d.rank]) + base4;
   float4* g_own = reinterpret_cast<float4*>(d.peer[d.rank] + d.arena_bytes) + base4;
   float4* ms_own = reinterpret_cast<float4*>(d.peer[d.rank] + 2 * d.arena_bytes) + base4;
@@ -119,12 +134,7 @@ __device__ __forceinline__ void dp_big_loop(const DpBigArgs& d, long long lo, lo
 #pragma unroll
       for (int r = 1; r < NW; ++r) { g.x += q[u][r].x; g.y += q[u][r].y; g.z += q[u][r].z; g.w += q[u][r].w; }   // rank order
       float4 mo = has_mom ? mom_own[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-#define GA3C_RMS(c)                                                          \
-  ms[u].c = d.decay * ms[u].c + one_m_rho * g.c * g.c;                       \
-  mo.c = d.momentum * mo.c + d.lr * g.c / sqrtf(ms[u].c + d.eps);            \
-  w[u].c -= mo.c;
-      GA3C_RMS(x) GA3C_RMS(y) GA3C_RMS(z) GA3C_RMS(w)
-#undef GA3C_RMS
+      rms_update(g, w[u], ms[u], mo, lr, decay, momentum, eps);
       ms_own[i] = ms[u];
       if (has_mom) mom_own[i] = mo;
       g_own[i] = g;                    // the reduced gradient of the owned slice (introspection); only this rank reads the slice

@@ -1,6 +1,8 @@
 // HBM-bound elementwise kernels: RMSProp over the flat arena, bf16 shadow refresh, discounted
 // returns, action sampling.
+#include <algorithm>
 #include <cstdlib>
+#include <type_traits>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -12,46 +14,59 @@ namespace ga3c {
 // The heads / conv12_bwd / conv11_wgrad kernels leave one slab of partial sums per CTA (a mirror of the small-tensor
 // prefix of the gradient arena + the loss sums).  512 threads = 16 slab lanes x 32 float4 columns: lane l adds slabs
 // l, l + 16, ... (independent 16-byte loads of L2-resident data), then the 16 lane sums are added in lane order.
-// The order is a function of the launch geometry only, so the gradients are bit-reproducible.
+// The order is a function of the launch geometry only, so the gradients are bit-reproducible.  Every kernel that sums the
+// slabs (grad_reduce_kernel, the slab blocks of rmsprop_reduce_kernel, dp_small_kernel) does it in slab_column_sum, so the
+// sum is the same whichever of them runs: ga3c_fb_tail leaves the gradient ga3c_train_step applies, and every data-parallel
+// rank computes its share of the small tensors alike.
 constexpr int GR_LANES = 16, GR_COLS = 32, GR_UNROLL = 10;     // 160 slabs (one per SM) in a single batch of loads
-__global__ void __launch_bounds__(GR_LANES * GR_COLS) grad_reduce_kernel(GradReduceArgs a) {
+
+// Floats j .. j + 3, j = (blockIdx.x * GR_COLS + col) * 4, summed over their slabs by the whole block (lane sl = threadIdx.x /
+// GR_COLS), after the dependency wait.  Lane 0 gets the sum (the other lanes a partial one); it stores the loss sums
+// (j >= out_floats) itself and leaves the gradient prefix to the caller.
+__device__ __forceinline__ float4 slab_column_sum(const GradReduceArgs& r, int col, int sl) {
   __shared__ float4 part[GR_LANES][GR_COLS];
-  const int col = threadIdx.x & (GR_COLS - 1), sl = threadIdx.x / GR_COLS;
   const int j = (blockIdx.x * GR_COLS + col) * 4;
   int count = 0;
-  if (j < a.n_floats) {
+  if (j < r.n_floats) {
 #pragma unroll
     for (int s = GR_MAX_SEG - 1; s >= 0; --s)
-      if (j < a.seg_end[s]) count = a.seg_count[s];
+      if (j < r.seg_end[s]) count = r.seg_count[s];
   }
-  griddep_launch();
-  griddep_wait(K_GRAD_REDUCE);  // the slabs come from the kernels that precede this one
   float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-  const float* src = a.part + j;
+  const float* src = r.part + j;
   for (int i0 = sl; i0 < count; i0 += GR_UNROLL * GR_LANES) {
     float4 q[GR_UNROLL];
 #pragma unroll
     for (int u = 0; u < GR_UNROLL; ++u) {
       const int i = i0 + u * GR_LANES;
-      q[u] = i < count ? __ldcg(reinterpret_cast<const float4*>(src + (int64_t)i * a.stride)) : make_float4(0.f, 0.f, 0.f, 0.f);
+      q[u] = i < count ? __ldcg(reinterpret_cast<const float4*>(src + (int64_t)i * r.stride)) : make_float4(0.f, 0.f, 0.f, 0.f);
     }
 #pragma unroll
     for (int u = 0; u < GR_UNROLL; ++u) { acc.x += q[u].x; acc.y += q[u].y; acc.z += q[u].z; acc.w += q[u].w; }
   }
   part[sl][col] = acc;
   __syncthreads();
-  if (sl == 0 && j < a.n_floats) {
+  if (sl == 0 && j < r.n_floats) {
 #pragma unroll
     for (int l = 1; l < GR_LANES; ++l) {
       const float4 q = part[l][col];
       acc.x += q.x; acc.y += q.y; acc.z += q.z; acc.w += q.w;
     }
-    if (j < a.out_floats) *reinterpret_cast<float4*>(a.out + j) = acc;
-    else if (a.out_tail != nullptr) {          // caller's buffer: no alignment assumed
-      float* t = a.out_tail + (j - a.out_floats);
+    if (j >= r.out_floats && r.out_tail != nullptr) {          // caller's buffer: no alignment assumed
+      float* t = r.out_tail + (j - r.out_floats);
       t[0] = acc.x; t[1] = acc.y; t[2] = acc.z; t[3] = acc.w;
     }
   }
+  return acc;
+}
+
+__global__ void __launch_bounds__(GR_LANES * GR_COLS) grad_reduce_kernel(GradReduceArgs a) {
+  const int col = threadIdx.x & (GR_COLS - 1), sl = threadIdx.x / GR_COLS;
+  const int j = (blockIdx.x * GR_COLS + col) * 4;
+  griddep_launch();
+  griddep_wait(K_GRAD_REDUCE);  // the slabs come from the kernels that precede this one
+  const float4 acc = slab_column_sum(a, col, sl);
+  if (sl == 0 && j < a.out_floats) *reinterpret_cast<float4*>(a.out + j) = acc;
   trace_mark(K_GRAD_REDUCE, 2);
 }
 
@@ -62,49 +77,51 @@ int launch_grad_reduce(const GradReduceArgs& a, cudaStream_t stream) {
   return launch_pdl(grad_reduce_kernel, dim3(grid), dim3(GR_LANES * GR_COLS), 0, stream, a);
 }
 
-// ---- RMSProp, TensorFlow semantics (tf.train.RMSPropOptimizer, NetworkVP_discrate.py:101-105) ----
-//   ms  <- rho*ms + (1-rho)*g^2 ; mom <- mu*mom + lr*g/sqrt(ms + eps) ; w <- w - mom       [TF-SEMANTICS]
-// One float4 per thread per iteration over the whole arena (all 10 variables in one launch instead
-// of TF's 10 ApplyRMSProp launches).  With mu == 0 (Config.RMSPROP_MOMENTUM) the mom slot is dead:
-// 20 B/param of traffic (read w,g,ms; write w,ms) + 2 B/param for the bf16 shadow of dense1/w.
+// ---- optimizer state ---------------------------------------------------------------------------------------
+// w, ms and mom of one float4 of an arena.  With mu == 0 (Config.RMSPROP_MOMENTUM, HAS_MOM = false) the mom slot is dead: it
+// reads as zero and is never written.
+// Preload rule.  w / ms (and mom) do not depend on the kernels that precede an optimizer launch, so the optimizer kernels of
+// the train step (rmsprop_reduce_kernel, dp_small_kernel) load them BEFORE the dependency wait and their latency hides under the
+// tail of the backward -- but only when a.preload says that this is safe: w / ms were last written by the optimizer launch of
+// the PREVIOUS step, and a prologue is ordered after that launch only if some kernel in between cannot become resident next to
+// it.  With batch >= num_sms the conv kernels of this step occupy every SM with a CTA that takes the SM's whole shared memory,
+// so every CTA of the previous optimizer launch has exited before this kernel can be launched; with smaller batches the whole
+// chain of a step can sit in its prologues while the previous optimizer is still running (back-to-back asynchronous calls),
+// and the loads move behind the wait.
+// e: the arena element of the float4, a multiple of 4
 template <bool HAS_MOM>
-__device__ __forceinline__ void rms_update(const RmsPropArgs& a, const float4& g, float4& w, float4& ms, float4& mo) {
-  const float one_m_rho = 1.f - a.decay;
-#define GA3C_RMS(c)                                                          \
-  ms.c = a.decay * ms.c + one_m_rho * g.c * g.c;                             \
-  mo.c = a.momentum * mo.c + a.lr * g.c / sqrtf(ms.c + a.eps);              \
-  w.c -= mo.c;
-  GA3C_RMS(x) GA3C_RMS(y) GA3C_RMS(z) GA3C_RMS(w)
-#undef GA3C_RMS
+__device__ __forceinline__ void load_slots(const float* ms, const float* mom, int64_t e, float4& ms_v, float4& mo_v) {
+  ms_v = *reinterpret_cast<const float4*>(ms + e);
+  mo_v = HAS_MOM ? *reinterpret_cast<const float4*>(mom + e) : make_float4(0.f, 0.f, 0.f, 0.f);
+}
+template <bool HAS_MOM>
+__device__ __forceinline__ void store_slots(float* ms, float* mom, int64_t e, const float4& ms_v, const float4& mo_v) {
+  *reinterpret_cast<float4*>(ms + e) = ms_v;
+  if (HAS_MOM) *reinterpret_cast<float4*>(mom + e) = mo_v;
+}
+template <bool HAS_MOM>
+__device__ __forceinline__ void load_state(const RmsPropArgs& a, int64_t e, float4& w, float4& ms, float4& mo) {
+  w = *reinterpret_cast<const float4*>(a.w + e);
+  load_slots<HAS_MOM>(a.ms, a.mom, e, ms, mo);
+}
+template <bool HAS_MOM>
+__device__ __forceinline__ void store_state(const RmsPropArgs& a, int64_t e, const float4& w, const float4& ms, const float4& mo) {
+  *reinterpret_cast<float4*>(a.w + e) = w;
+  store_slots<HAS_MOM>(a.ms, a.mom, e, ms, mo);
+}
+// the bf16 shadow of dense1/w, if the float4 lies in [w1_offset, w1_offset + w1_count) (one unsigned compare)
+__device__ __forceinline__ void store_shadow(const RmsPropArgs& a, int64_t e, const float4& w) {
+  if ((uint64_t)(e - a.w1_offset) < (uint64_t)a.w1_count)
+    reinterpret_cast<uint2*>(a.w1_shadow)[(e - a.w1_offset) >> 2] = make_uint2(pack_bf16(w.x, w.y), pack_bf16(w.z, w.w));
 }
 
-template <bool HAS_MOM>
-__global__ void __launch_bounds__(256) rmsprop_kernel(RmsPropArgs a) {
-  griddep_launch();
-  griddep_wait(K_RMSPROP);      // the gradients come from the backward kernels that precede this one
-  const int64_t n4 = a.n_floats >> 2;
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
-    const float4 g = reinterpret_cast<const float4*>(a.g)[i];
-    float4 w = reinterpret_cast<float4*>(a.w)[i];
-    float4 ms = reinterpret_cast<float4*>(a.ms)[i];
-    float4 mo = HAS_MOM ? reinterpret_cast<float4*>(a.mom)[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-    rms_update<HAS_MOM>(a, g, w, ms, mo);
-    reinterpret_cast<float4*>(a.w)[i] = w;
-    reinterpret_cast<float4*>(a.ms)[i] = ms;
-    if (HAS_MOM) reinterpret_cast<float4*>(a.mom)[i] = mo;
-    const int64_t e = i << 2;
-    if (e >= a.w1_offset && e < a.w1_offset + a.w1_count)
-      reinterpret_cast<uint2*>(a.w1_shadow)[(e - a.w1_offset) >> 2] = make_uint2(pack_bf16(w.x, w.y), pack_bf16(w.z, w.w));
-  }
-  trace_mark(K_RMSPROP, 2);
-}
+// grid of the grid-stride arena kernels: 256-thread blocks, at most 8 per SM of a 148-SM B200
+static int arena_grid(int64_t n4) { return (int)std::min<int64_t>((n4 + 255) / 256, 148 * 8); }
 
-int launch_rmsprop(const RmsPropArgs& a, cudaStream_t stream) {
-  const int64_t n4 = a.n_floats >> 2;
-  const int grid = (int)((n4 + 255) / 256 < 148 * 8 ? (n4 + 255) / 256 : 148 * 8);
-  if (a.momentum != 0.f) return launch_pdl(rmsprop_kernel<true>, dim3(grid), dim3(256), 0, stream, a);
-  return launch_pdl(rmsprop_kernel<false>, dim3(grid), dim3(256), 0, stream, a);
+// launch(std::true_type) when the optimizer has momentum (a live mom slot), launch(std::false_type) when it has none
+template <class F>
+static int by_momentum(float momentum, F&& launch) {
+  return momentum != 0.f ? launch(std::true_type{}) : launch(std::false_type{});
 }
 
 // ---- Config.USE_GRAD_CLIP: tf.clip_by_average_norm per variable (NetworkVP_discrate.py:118-121) --------------
@@ -147,50 +164,65 @@ __global__ void __launch_bounds__(32 * CLIP_MAX_TENSORS) clip_scale_kernel(ClipA
   if (lane == 0) c.scale[t] = c.clip / fmaxf(c.by_norm ? sqrtf(s) : sqrtf(s) / (float)c.count[t], c.clip);
 }
 
-template <bool HAS_MOM>
-__global__ void __launch_bounds__(256) rmsprop_clip_kernel(RmsPropArgs a, ClipArgs c) {
-  griddep_launch();
-  griddep_wait(K_RMSPROP);
-  const int64_t n4 = a.n_floats >> 2;
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
-    const int64_t e = i << 2;
-    float sc = 0.f;                       // alignment gaps between tensors hold zeros
+// the entry of `scale` (one per tensor of c) for arena element e, 0 in the alignment gaps between tensors (they hold zeros).
+// One scale per float4 is exact: tensors start 4-aligned, and when a count is not a multiple of 4 the rest of its last float4
+// lies in the gap.
+__device__ __forceinline__ float clip_scale_at(const ClipArgs& c, const float* scale, int64_t e) {
+  float sc = 0.f;
 #pragma unroll
-    for (int t = 0; t < CLIP_MAX_TENSORS; ++t)
-      if (t < c.n_tensors && e >= c.offset[t] && e < c.offset[t] + c.count[t]) sc = c.scale[t];
-    float4 g = reinterpret_cast<const float4*>(a.g)[i];
-    // a float4 never straddles two tensors' live elements with different scales unless a count is not a multiple of 4: then
-    // the tail elements belong to the gap (zeros), so one scale per float4 is exact
-    g.x *= sc; g.y *= sc; g.z *= sc; g.w *= sc;
-    float4 w = reinterpret_cast<float4*>(a.w)[i];
-    float4 ms = reinterpret_cast<float4*>(a.ms)[i];
-    float4 mo = HAS_MOM ? reinterpret_cast<float4*>(a.mom)[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-    rms_update<HAS_MOM>(a, g, w, ms, mo);
-    reinterpret_cast<float4*>(a.w)[i] = w;
-    reinterpret_cast<float4*>(a.ms)[i] = ms;
-    if (HAS_MOM) reinterpret_cast<float4*>(a.mom)[i] = mo;
-    if (a.w1_count > 0 && e >= a.w1_offset && e < a.w1_offset + a.w1_count)
-      reinterpret_cast<uint2*>(a.w1_shadow)[(e - a.w1_offset) >> 2] = make_uint2(pack_bf16(w.x, w.y), pack_bf16(w.z, w.w));
-  }
-  trace_mark(K_RMSPROP, 2);
+  for (int t = 0; t < CLIP_MAX_TENSORS; ++t)
+    if (t < c.n_tensors && e >= c.offset[t] && e < c.offset[t] + c.count[t]) sc = scale[t];
+  return sc;
 }
 
 int clip_chunks(int64_t max_count) { return (int)((max_count + CLIP_CHUNK - 1) / CLIP_CHUNK); }
 
-int launch_rmsprop_clipped(const RmsPropArgs& a, const ClipArgs& c, cudaStream_t stream) {
-  int r;
-  if ((r = launch_pdl(grad_sqnorm_kernel, dim3(c.max_chunks, c.n_tensors), dim3(256), 0, stream, c))) return r;
-  if ((r = launch_pdl(clip_scale_kernel, dim3(1), dim3(32 * CLIP_MAX_TENSORS), 0, stream, c))) return r;
+// c.scale of every tensor of c: 2 launches
+static int launch_clip_scales(const ClipArgs& c, cudaStream_t stream) {
+  if (int r = launch_pdl(grad_sqnorm_kernel, dim3(c.max_chunks, c.n_tensors), dim3(256), 0, stream, c)) return r;
+  return launch_pdl(clip_scale_kernel, dim3(1), dim3(32 * CLIP_MAX_TENSORS), 0, stream, c);
+}
+
+// ---- RMSProp over the arena ---------------------------------------------------------------------------------
+// One float4 per thread per iteration over the whole arena (all 10 variables in one launch instead of TF's 10 ApplyRMSProp
+// launches).  Without momentum: 20 B/param of traffic (read w,g,ms; write w,ms) + 2 B/param for the bf16 shadow of dense1/w.
+// CLIP: each gradient scaled by its tensor's clip scale (c.scale) first.
+template <bool HAS_MOM, bool CLIP>
+__global__ void __launch_bounds__(256) rmsprop_kernel(RmsPropArgs a, ClipArgs c) {
+  griddep_launch();
+  griddep_wait(K_RMSPROP);      // the gradients come from the kernels that precede this one
   const int64_t n4 = a.n_floats >> 2;
-  const int grid = (int)((n4 + 255) / 256 < 148 * 8 ? (n4 + 255) / 256 : 148 * 8);
-  if (a.momentum != 0.f) return launch_pdl(rmsprop_clip_kernel<true>, dim3(grid), dim3(256), 0, stream, a, c);
-  return launch_pdl(rmsprop_clip_kernel<false>, dim3(grid), dim3(256), 0, stream, a, c);
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
+    const int64_t e = i << 2;
+    float4 g = reinterpret_cast<const float4*>(a.g)[i];
+    if (CLIP) {
+      const float sc = clip_scale_at(c, c.scale, e);
+      g.x *= sc; g.y *= sc; g.z *= sc; g.w *= sc;
+    }
+    float4 w, ms, mo;
+    load_state<HAS_MOM>(a, e, w, ms, mo);
+    rms_update(g, w, ms, mo, a.lr, a.decay, a.momentum, a.eps);
+    store_state<HAS_MOM>(a, e, w, ms, mo);
+    store_shadow(a, e, w);
+  }
+  trace_mark(K_RMSPROP, 2);
+}
+
+int launch_rmsprop(const RmsPropArgs& a, const ClipArgs* c, cudaStream_t stream, int* kernels) {
+  *kernels = c != nullptr ? 3 : 1;
+  if (c != nullptr)
+    if (int r = launch_clip_scales(*c, stream)) return r;
+  const int grid = arena_grid(a.n_floats >> 2);
+  return by_momentum(a.momentum, [&](auto mom) {
+    return c != nullptr ? launch_pdl(rmsprop_kernel<mom, true>, dim3(grid), dim3(256), 0, stream, a, *c)
+                        : launch_pdl(rmsprop_kernel<mom, false>, dim3(grid), dim3(256), 0, stream, a, ClipArgs{});
+  });
 }
 
 // ---- Config.DUAL_RMSPROP (NetworkVP_discrate.py:87-98, :124-128) ---------------------------------------------
 template <bool HAS_MOM>
-__global__ void __launch_bounds__(256) rmsprop_dual_kernel(RmsPropDualArgs d) {
+__global__ void __launch_bounds__(256) rmsprop_dual_kernel(RmsPropDualArgs d, ClipArgs c) {
   const RmsPropArgs& a = d.a;
   griddep_launch();
   griddep_wait(K_RMSPROP);
@@ -203,127 +235,62 @@ __global__ void __launch_bounds__(256) rmsprop_dual_kernel(RmsPropDualArgs d) {
     const float4 w0 = reinterpret_cast<float4*>(a.w)[i];
     float4 w = w0;
     float s1 = 1.f, s2 = 1.f;
-    if (d.scale1 != nullptr) {           // one scale per float4 is exact: tensors start 4-aligned, gaps hold zeros
-      s1 = s2 = 0.f;
-#pragma unroll
-      for (int t = 0; t < CLIP_MAX_TENSORS; ++t)
-        if (t < d.n_tensors && e >= d.t_offset[t] && e < d.t_offset[t] + d.t_count[t]) { s1 = d.scale1[t]; s2 = d.scale2[t]; }
-    }
-    if (!skip1) {
-      float4 g = reinterpret_cast<const float4*>(a.g)[i];
-      g.x *= s1; g.y *= s1; g.z *= s1; g.w *= s1;
-      float4 ms = reinterpret_cast<float4*>(a.ms)[i];
-      float4 mo = HAS_MOM ? reinterpret_cast<float4*>(a.mom)[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-      float4 w1 = w0;
-      rms_update<HAS_MOM>(a, g, w1, ms, mo);
-      w.x -= w0.x - w1.x; w.y -= w0.y - w1.y; w.z -= w0.z - w1.z; w.w -= w0.w - w1.w;
-      reinterpret_cast<float4*>(a.ms)[i] = ms;
-      if (HAS_MOM) reinterpret_cast<float4*>(a.mom)[i] = mo;
-    }
-    if (!skip2) {
-      float4 g = reinterpret_cast<const float4*>(d.g2)[i];
-      g.x *= s2; g.y *= s2; g.z *= s2; g.w *= s2;
-      float4 ms = reinterpret_cast<float4*>(d.ms2)[i];
-      float4 mo = HAS_MOM ? reinterpret_cast<float4*>(d.mom2)[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-      float4 w2 = w0;
-      rms_update<HAS_MOM>(a, g, w2, ms, mo);
-      w.x -= w0.x - w2.x; w.y -= w0.y - w2.y; w.z -= w0.z - w2.z; w.w -= w0.w - w2.w;
-      reinterpret_cast<float4*>(d.ms2)[i] = ms;
-      if (HAS_MOM) reinterpret_cast<float4*>(d.mom2)[i] = mo;
-    }
+    if (d.scale1 != nullptr) { s1 = clip_scale_at(c, d.scale1, e); s2 = clip_scale_at(c, d.scale2, e); }
+    // one optimizer's step, taken at w0 and subtracted from w
+    auto step = [&](const float* g_arena, float* ms_arena, float* mom_arena, float s) {
+      float4 g = reinterpret_cast<const float4*>(g_arena)[i];
+      g.x *= s; g.y *= s; g.z *= s; g.w *= s;
+      float4 ms, mo;
+      load_slots<HAS_MOM>(ms_arena, mom_arena, e, ms, mo);
+      float4 wk = w0;
+      rms_update(g, wk, ms, mo, a.lr, a.decay, a.momentum, a.eps);
+      w.x -= w0.x - wk.x; w.y -= w0.y - wk.y; w.z -= w0.z - wk.z; w.w -= w0.w - wk.w;
+      store_slots<HAS_MOM>(ms_arena, mom_arena, e, ms, mo);
+    };
+    if (!skip1) step(a.g, a.ms, a.mom, s1);
+    if (!skip2) step(d.g2, d.ms2, d.mom2, s2);
     reinterpret_cast<float4*>(a.w)[i] = w;
-    if (a.w1_count > 0 && e >= a.w1_offset && e < a.w1_offset + a.w1_count)
-      reinterpret_cast<uint2*>(a.w1_shadow)[(e - a.w1_offset) >> 2] = make_uint2(pack_bf16(w.x, w.y), pack_bf16(w.z, w.w));
+    store_shadow(a, e, w);
   }
   trace_mark(K_RMSPROP, 2);
 }
 
-int launch_rmsprop_dual(const RmsPropDualArgs& d, cudaStream_t stream) {
-  const int64_t n4 = d.a.n_floats >> 2;
-  const int grid = (int)((n4 + 255) / 256 < 148 * 8 ? (n4 + 255) / 256 : 148 * 8);
-  if (d.a.momentum != 0.f) return launch_pdl(rmsprop_dual_kernel<true>, dim3(grid), dim3(256), 0, stream, d);
-  return launch_pdl(rmsprop_dual_kernel<false>, dim3(grid), dim3(256), 0, stream, d);
-}
-
-int launch_rmsprop_dual_clipped(RmsPropDualArgs d, const ClipArgs& c1, const ClipArgs& c2, cudaStream_t stream) {
-  int r;
-  for (const ClipArgs* c : {&c1, &c2}) {
-    if ((r = launch_pdl(grad_sqnorm_kernel, dim3(c->max_chunks, c->n_tensors), dim3(256), 0, stream, *c))) return r;
-    if ((r = launch_pdl(clip_scale_kernel, dim3(1), dim3(32 * CLIP_MAX_TENSORS), 0, stream, *c))) return r;
+int launch_rmsprop_dual(RmsPropDualArgs d, const ClipArgs* c1, const ClipArgs* c2, cudaStream_t stream, int* kernels) {
+  *kernels = c1 != nullptr ? 5 : 1;
+  if (c1 != nullptr) {
+    int r;
+    if ((r = launch_clip_scales(*c1, stream)) || (r = launch_clip_scales(*c2, stream))) return r;
+    d.scale1 = c1->scale; d.scale2 = c2->scale;
   }
-  d.scale1 = c1.scale; d.scale2 = c2.scale; d.n_tensors = c1.n_tensors;
-  for (int t = 0; t < c1.n_tensors; ++t) { d.t_offset[t] = c1.offset[t]; d.t_count[t] = c1.count[t]; }
-  return launch_rmsprop_dual(d, stream);
+  const ClipArgs table = c1 != nullptr ? *c1 : ClipArgs{};
+  const int grid = arena_grid(d.a.n_floats >> 2);
+  return by_momentum(d.a.momentum, [&](auto mom) {
+    return launch_pdl(rmsprop_dual_kernel<mom>, dim3(grid), dim3(256), 0, stream, d, table);
+  });
 }
 
 // ---- single-GPU step tail: grad_reduce + RMSProp in one launch -------------------------------------------
-// Blocks [0, n_red) sum the gradient-partial slabs of 32 float4 columns exactly like grad_reduce_kernel (same order,
-// same bits), store the reduced gradient and apply RMSProp to those columns; the remaining blocks update dense1/w,
-// one float4 per thread.  w / ms (and mom) do not depend on the preceding kernels, so they are loaded BEFORE the
-// dependency wait and their latency hides under the tail of the backward -- but only when a.preload says that this is safe:
-// w / ms were last written by the optimizer launch of the PREVIOUS step, and a prologue is ordered after that launch only if
-// some kernel in between cannot become resident next to it.  With batch >= num_sms the conv kernels of this step occupy every
-// SM with a CTA that takes the SM's whole shared memory, so every CTA of the previous optimizer launch has exited before this
-// kernel can be launched; with smaller batches the whole chain of a step can sit in its prologues while the previous
-// optimizer is still running (back-to-back asynchronous calls), and the loads move behind the wait.
+// Blocks [0, n_red) sum the gradient-partial slabs of 32 float4 columns (slab_column_sum), store the reduced gradient and
+// apply RMSProp to those columns; the remaining blocks update dense1/w, one float4 per thread.  Both load w / ms (and mom)
+// before the dependency wait when a.preload allows it (the preload rule above load_slots).
 constexpr int RR_U = 3;      // float4 per thread in the dense1/w blocks of rmsprop_reduce_kernel
 template <bool HAS_MOM>
 __global__ void __launch_bounds__(GR_LANES * GR_COLS, 2) rmsprop_reduce_kernel(RmsPropArgs a, GradReduceArgs r, int n_red) {
-  __shared__ float4 part[GR_LANES][GR_COLS];
   const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
   if ((int)blockIdx.x < n_red) {
     const int col = threadIdx.x & (GR_COLS - 1), sl = threadIdx.x / GR_COLS;
     const int j = (blockIdx.x * GR_COLS + col) * 4;
-    int count = 0;
-    if (j < r.n_floats) {
-#pragma unroll
-      for (int s = GR_MAX_SEG - 1; s >= 0; --s)
-        if (j < r.seg_end[s]) count = r.seg_count[s];
-    }
     const bool owner = sl == 0 && j < r.out_floats;
     float4 w = zero, ms = zero, mo = zero;
-    if (owner && a.preload) {
-      w = *reinterpret_cast<const float4*>(a.w + j);
-      ms = *reinterpret_cast<const float4*>(a.ms + j);
-      if (HAS_MOM) mo = *reinterpret_cast<const float4*>(a.mom + j);
-    }
+    if (owner && a.preload) load_state<HAS_MOM>(a, j, w, ms, mo);
     griddep_launch();
     griddep_wait(K_RMSPROP);      // the slabs come from the kernels that precede this one
-    if (owner && !a.preload) {
-      w = *reinterpret_cast<const float4*>(a.w + j);
-      ms = *reinterpret_cast<const float4*>(a.ms + j);
-      if (HAS_MOM) mo = *reinterpret_cast<const float4*>(a.mom + j);
-    }
-    float4 acc = zero;
-    const float* src = r.part + j;
-    for (int i0 = sl; i0 < count; i0 += GR_UNROLL * GR_LANES) {
-      float4 q[GR_UNROLL];
-#pragma unroll
-      for (int u = 0; u < GR_UNROLL; ++u) {
-        const int i = i0 + u * GR_LANES;
-        q[u] = i < count ? __ldcg(reinterpret_cast<const float4*>(src + (int64_t)i * r.stride)) : zero;
-      }
-#pragma unroll
-      for (int u = 0; u < GR_UNROLL; ++u) { acc.x += q[u].x; acc.y += q[u].y; acc.z += q[u].z; acc.w += q[u].w; }
-    }
-    part[sl][col] = acc;
-    __syncthreads();
-    if (sl == 0 && j < r.n_floats) {
-#pragma unroll
-      for (int l = 1; l < GR_LANES; ++l) {
-        const float4 q = part[l][col];
-        acc.x += q.x; acc.y += q.y; acc.z += q.z; acc.w += q.w;
-      }
-      if (owner) {
-        *reinterpret_cast<float4*>(r.out + j) = acc;                 // the reduced gradient (introspection, checkpoints)
-        rms_update<HAS_MOM>(a, acc, w, ms, mo);
-        *reinterpret_cast<float4*>(a.w + j) = w;
-        *reinterpret_cast<float4*>(a.ms + j) = ms;
-        if (HAS_MOM) *reinterpret_cast<float4*>(a.mom + j) = mo;
-      } else if (r.out_tail != nullptr) {
-        float* t = r.out_tail + (j - r.out_floats);
-        t[0] = acc.x; t[1] = acc.y; t[2] = acc.z; t[3] = acc.w;
-      }
+    if (owner && !a.preload) load_state<HAS_MOM>(a, j, w, ms, mo);
+    const float4 g = slab_column_sum(r, col, sl);
+    if (owner) {
+      *reinterpret_cast<float4*>(r.out + j) = g;                 // the reduced gradient (introspection, checkpoints)
+      rms_update(g, w, ms, mo, a.lr, a.decay, a.momentum, a.eps);
+      store_state<HAS_MOM>(a, j, w, ms, mo);
     }
   } else {
     // RR_U float4 per thread, a block apart (coalesced).  RR_U = 3 keeps the whole grid -- 113 slab blocks + 162 of these at
@@ -336,11 +303,7 @@ __global__ void __launch_bounds__(GR_LANES * GR_COLS, 2) rmsprop_reduce_kernel(R
     for (int u = 0; u < RR_U; ++u) {
       const int64_t i = i0 + u * blockDim.x;
       w[u] = ms[u] = mo[u] = zero;
-      if (i < n4 && a.preload) {
-        w[u] = reinterpret_cast<const float4*>(a.w)[i];
-        ms[u] = reinterpret_cast<const float4*>(a.ms)[i];
-        if (HAS_MOM) mo[u] = reinterpret_cast<const float4*>(a.mom)[i];
-      }
+      if (i < n4 && a.preload) load_state<HAS_MOM>(a, i << 2, w[u], ms[u], mo[u]);
     }
     griddep_launch();
     griddep_wait(K_RMSPROP);      // dense1/w's gradient comes from the wgrad GEMM
@@ -348,11 +311,7 @@ __global__ void __launch_bounds__(GR_LANES * GR_COLS, 2) rmsprop_reduce_kernel(R
 #pragma unroll
       for (int u = 0; u < RR_U; ++u) {
         const int64_t i = i0 + u * blockDim.x;
-        if (i < n4) {
-          w[u] = reinterpret_cast<const float4*>(a.w)[i];
-          ms[u] = reinterpret_cast<const float4*>(a.ms)[i];
-          if (HAS_MOM) mo[u] = reinterpret_cast<const float4*>(a.mom)[i];
-        }
+        if (i < n4) load_state<HAS_MOM>(a, i << 2, w[u], ms[u], mo[u]);
       }
     }
     float4 g[RR_U];
@@ -365,13 +324,9 @@ __global__ void __launch_bounds__(GR_LANES * GR_COLS, 2) rmsprop_reduce_kernel(R
     for (int u = 0; u < RR_U; ++u) {
       const int64_t i = i0 + u * blockDim.x;
       if (i < n4) {
-        rms_update<HAS_MOM>(a, g[u], w[u], ms[u], mo[u]);
-        reinterpret_cast<float4*>(a.w)[i] = w[u];
-        reinterpret_cast<float4*>(a.ms)[i] = ms[u];
-        if (HAS_MOM) reinterpret_cast<float4*>(a.mom)[i] = mo[u];
-        const int64_t e = i << 2;
-        if (e >= a.w1_offset && e < a.w1_offset + a.w1_count)
-          reinterpret_cast<uint2*>(a.w1_shadow)[(e - a.w1_offset) >> 2] = make_uint2(pack_bf16(w[u].x, w[u].y), pack_bf16(w[u].z, w[u].w));
+        rms_update(g[u], w[u], ms[u], mo[u], a.lr, a.decay, a.momentum, a.eps);
+        store_state<HAS_MOM>(a, i << 2, w[u], ms[u], mo[u]);
+        store_shadow(a, i << 2, w[u]);
       }
     }
   }
@@ -383,73 +338,37 @@ int launch_rmsprop_reduce(const RmsPropArgs& a, const GradReduceArgs& r, cudaStr
   const int n_red = (r.n_floats / 4 + GR_COLS - 1) / GR_COLS;
   const int64_t rest4 = (a.n_floats - r.out_floats) >> 2;
   const int grid = n_red + (int)((rest4 + RR_U * T - 1) / (RR_U * T));
-  if (a.momentum != 0.f) return launch_pdl(rmsprop_reduce_kernel<true>, dim3(grid), dim3(T), 0, stream, a, r, n_red);
-  return launch_pdl(rmsprop_reduce_kernel<false>, dim3(grid), dim3(T), 0, stream, a, r, n_red);
+  return by_momentum(a.momentum, [&](auto mom) {
+    return launch_pdl(rmsprop_reduce_kernel<mom>, dim3(grid), dim3(T), 0, stream, a, r, n_red);
+  });
 }
 
 GA3C_EVT_ATTACH(evt_attach_elementwise)
 
 // ---- data-parallel exchange, small tensors (dp_exchange.cuh) ---------------------------------------------
 // One block per 32-float4 column block of the small-tensor prefix (+ the loss sums).  Block cb sums this rank's per-CTA
-// slabs for its columns (same order and bits as grad_reduce_kernel); its 32 owner threads push the sums into every peer's
+// slabs for its columns (slab_column_sum); its 32 owner threads push the sums into every peer's
 // receive buffer in the LL wire format, collect the peers' contributions from this rank's own receive buffer, add them in
 // rank order (every rank computes the identical sum) and apply RMSProp to the local copy.  Receive buffers alternate with
 // the step parity: a peer pushes step s + 2 only after it has seen this rank's step s + 1, i.e. after this rank's step-s
 // launch has ended.
 template <bool HAS_MOM>
 __global__ void __launch_bounds__(GR_LANES * GR_COLS) dp_small_kernel(RmsPropDpArgs d, int64_t recv_offset) {
-  __shared__ float4 part[GR_LANES][GR_COLS];
   EvtLog evt_i = evt_open();
   const RmsPropArgs& a = d.base;
   const GradReduceArgs& r = d.red;
   const int col = threadIdx.x & (GR_COLS - 1), sl = threadIdx.x / GR_COLS;
   const int j = (blockIdx.x * GR_COLS + col) * 4;
   const bool owner = sl == 0 && j < r.out_floats;
-  int count = 0;
-  if (j < r.n_floats) {
-#pragma unroll
-    for (int s = GR_MAX_SEG - 1; s >= 0; --s)
-      if (j < r.seg_end[s]) count = r.seg_count[s];
-  }
   float4 w = make_float4(0.f, 0.f, 0.f, 0.f), ms = w, mo = w;
-  auto load_state = [&]() {
-    w = *reinterpret_cast<const float4*>(a.w + j);
-    ms = *reinterpret_cast<const float4*>(a.ms + j);
-    if (HAS_MOM) mo = *reinterpret_cast<const float4*>(a.mom + j);
-  };
-  // w / ms of the small prefix were last written by this kernel one step ago; see rmsprop_reduce_kernel for when the early
-  // loads are safe
-  if (owner && a.preload) load_state();
+  // w / ms of the small prefix were last written by this kernel one step ago: the preload rule above load_slots
+  if (owner && a.preload) load_state<HAS_MOM>(a, j, w, ms, mo);
   griddep_launch();
   evt_mark(evt_i, 60, 0);
   griddep_wait(K_RMSPROP);        // the slabs come from the conv backward launch that precedes this one
   evt_mark(evt_i, 61, 0);
-  if (owner && !a.preload) load_state();
-  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-  const float* src = r.part + j;
-  for (int i0 = sl; i0 < count; i0 += GR_UNROLL * GR_LANES) {
-    float4 q[GR_UNROLL];
-#pragma unroll
-    for (int u = 0; u < GR_UNROLL; ++u) {
-      const int i = i0 + u * GR_LANES;
-      q[u] = i < count ? __ldcg(reinterpret_cast<const float4*>(src + (int64_t)i * r.stride)) : make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-#pragma unroll
-    for (int u = 0; u < GR_UNROLL; ++u) { acc.x += q[u].x; acc.y += q[u].y; acc.z += q[u].z; acc.w += q[u].w; }
-  }
-  part[sl][col] = acc;
-  __syncthreads();
-  if (sl == 0 && j < r.n_floats) {
-#pragma unroll
-    for (int l = 1; l < GR_LANES; ++l) {
-      const float4 q = part[l][col];
-      acc.x += q.x; acc.y += q.y; acc.z += q.z; acc.w += q.w;
-    }
-    if (j >= r.out_floats && r.out_tail != nullptr) {
-      float* t = r.out_tail + (j - r.out_floats);
-      t[0] = acc.x; t[1] = acc.y; t[2] = acc.z; t[3] = acc.w;
-    }
-  }
+  if (owner && !a.preload) load_state<HAS_MOM>(a, j, w, ms, mo);
+  const float4 acc = slab_column_sum(r, col, sl);
   evt_mark(evt_i, 62, 0);
   if (owner) {
     // receive buffers: [parity][source rank][small prefix in LL format: 8 bytes per float]
@@ -472,10 +391,8 @@ __global__ void __launch_bounds__(GR_LANES * GR_COLS) dp_small_kernel(RmsPropDpA
         g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
       }
     evt_mark(evt_i, 63, 0);
-    rms_update<HAS_MOM>(a, g, w, ms, mo);
-    *reinterpret_cast<float4*>(a.w + j) = w;
-    *reinterpret_cast<float4*>(a.ms + j) = ms;
-    if (HAS_MOM) *reinterpret_cast<float4*>(a.mom + j) = mo;
+    rms_update(g, w, ms, mo, a.lr, a.decay, a.momentum, a.eps);
+    store_state<HAS_MOM>(a, j, w, ms, mo);
   }
   evt_mark(evt_i, 64, 0);
   trace_mark(K_RMSPROP, 2);
@@ -528,9 +445,9 @@ int configure_dp() {
 int launch_dp_small(const RmsPropDpArgs& d, int64_t recv_offset, cudaStream_t stream) {
   const int n_cb = (d.red.n_floats / 4 + GR_COLS - 1) / GR_COLS;
   if (n_cb > DP_MAX_CB) return (int)cudaErrorInvalidValue;
-  if (d.base.momentum != 0.f)
-    return launch_pdl(dp_small_kernel<true>, dim3(n_cb), dim3(GR_LANES * GR_COLS), 0, stream, d, recv_offset);
-  return launch_pdl(dp_small_kernel<false>, dim3(n_cb), dim3(GR_LANES * GR_COLS), 0, stream, d, recv_offset);
+  return by_momentum(d.base.momentum, [&](auto mom) {
+    return launch_pdl(dp_small_kernel<mom>, dim3(n_cb), dim3(GR_LANES * GR_COLS), 0, stream, d, recv_offset);
+  });
 }
 
 __global__ void __launch_bounds__(256) f32_to_bf16_kernel(const float* __restrict__ src, uint16_t* __restrict__ dst, int64_t n4) {
@@ -543,8 +460,7 @@ __global__ void __launch_bounds__(256) f32_to_bf16_kernel(const float* __restric
 
 int launch_f32_to_bf16(const float* src, uint16_t* dst, int64_t n, cudaStream_t stream) {
   const int64_t n4 = n >> 2;
-  const int grid = (int)((n4 + 255) / 256 < 148 * 8 ? (n4 + 255) / 256 : 148 * 8);
-  f32_to_bf16_kernel<<<grid, 256, 0, stream>>>(src, dst, n4);
+  f32_to_bf16_kernel<<<arena_grid(n4), 256, 0, stream>>>(src, dst, n4);
   return (int)cudaGetLastError();
 }
 

@@ -42,8 +42,10 @@ struct Handle {
   float *clip_ss2 = nullptr, *clip_scale2 = nullptr;      // ... of the second optimizer's gradient (DUAL_RMSPROP + USE_GRAD_CLIP)
   double* histo_part = nullptr;    // histograms: fp64 partial moments per block
   size_t histo_part_bytes = 0;
+  int64_t skip_lo[4] = {}, skip_hi[4] = {};     // Config.DUAL_RMSPROP: what each optimizer leaves alone (RmsPropDualArgs)
   int last_batch = 0;              // rows of the activation workspace written by the last forward
   int64_t global_step = 0;
+  int step_advance = 1;            // global_step per optimizer update, set at create from the reference's rules
   LaunchLog log;                   // launch counter + per-kernel CUDA-event timing
 };
 
@@ -219,6 +221,31 @@ ClipArgs clip_args(const Handle<C>* h, int which) {
   c.clip = h->cfg.grad_clip_norm;
   c.chunk_ss = which ? h->clip_ss2 : h->clip_ss; c.scale = which ? h->clip_scale2 : h->clip_scale;
   return c;
+}
+
+// The optimizer update of the arena the config selects -- RMSProp, with Config.USE_GRAD_CLIP, with Config.DUAL_RMSPROP, or
+// with both -- over the handle's first optimizer arguments `a`.  One timing record under K_RMSPROP, every kernel counted.
+template <class C>
+int launch_optimizer(Handle<C>* h, const RmsPropArgs& a, cudaStream_t st) {
+  const bool clip = h->cfg.use_grad_clip;
+  int kernels = 0;
+  ClipArgs c1{}, c2{};
+  if (h->cfg.dual_rmsprop) {
+    RmsPropDualArgs d{};
+    d.a = a;
+    d.g2 = h->g2; d.ms2 = h->ms2; d.mom2 = h->mom2;
+    for (int i = 0; i < 4; ++i) { d.skip_lo[i] = h->skip_lo[i]; d.skip_hi[i] = h->skip_hi[i]; }
+    // tf.clip_by_norm per variable and optimizer (NetworkVP.py:127-137, NetworkVP_discrate.py:107-117); the gradient-less
+    // variables' gradient is None there, which the reference filters and clip_args leaves out
+    if (clip) { c1 = clip_args(h, 0); c2 = clip_args(h, 1); c1.by_norm = c2.by_norm = 1; }
+    LAUNCH(h, K_RMSPROP, st, launch_rmsprop_dual(d, clip ? &c1 : nullptr, clip ? &c2 : nullptr, st, &kernels));
+  } else {
+    if (clip) c1 = clip_args(h, 0);
+    LAUNCH(h, K_RMSPROP, st, launch_rmsprop(a, clip ? &c1 : nullptr, st, &kernels));
+  }
+  h->log.launches += kernels - 1;        // LAUNCH counted one
+  h->global_step += h->step_advance;
+  return 0;
 }
 
 }  // namespace ga3c

@@ -25,7 +25,7 @@ __global__ void __launch_bounds__(HD_THREADS) heads_kernel(HeadsArgs p) {
   // The head weights are written by the optimizer launch of the previous step.  A prologue may run while a kernel two or more
   // launches back is still executing (only code after the wait is ordered transitively, common.cuh), so reading them before
   // the dependency wait is safe only when something in between cannot be resident next to that optimizer launch: p.preload
-  // (batch >= num_sms: the conv forward in front of this kernel fills every SM, see rmsprop_reduce_kernel).  Otherwise
+  // (batch >= num_sms: the conv forward in front of this kernel fills every SM, see the preload rule in elementwise.cu).  Otherwise
   // they are read after the wait.
   if (p.preload) heads_load_weights<A>(p, hs, tid, HD_THREADS);
   griddep_launch();

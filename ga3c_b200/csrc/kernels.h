@@ -116,12 +116,10 @@ struct RmsPropArgs {
   int64_t n_floats;        // arena size (multiple of 4)
   int64_t w1_offset, w1_count;
   float lr, decay, momentum, eps;
-  int preload;             // the optimizer kernels may load w / ms / mom before their dependency wait (rmsprop_reduce_kernel)
+  int preload;             // the optimizer kernels may load w / ms / mom before their dependency wait (elementwise.cu, preload rule)
 };
-int launch_rmsprop(const RmsPropArgs& a, cudaStream_t stream);
-// Config.USE_GRAD_CLIP: tf.clip_by_average_norm per variable, then RMSProp (3 launches: chunk sums of squares, per-tensor
-// scale, update).  offset / count: the variables' element ranges in the arena; chunk_ss: [n_tensors][max_chunks] scratch,
-// max_chunks = clip_chunks(largest count); scale: [n_tensors] scratch.
+// Config.USE_GRAD_CLIP: tf.clip_by_average_norm per variable before RMSProp.  offset / count: the variables' element ranges in
+// the arena; chunk_ss: [n_tensors][max_chunks] scratch, max_chunks = clip_chunks(largest count); scale: [n_tensors] scratch.
 constexpr int CLIP_MAX_TENSORS = 24;
 struct ClipArgs {
   const float* g;
@@ -132,7 +130,9 @@ struct ClipArgs {
   int by_norm;                      // 0: tf.clip_by_average_norm (||g|| / n against clip), 1: tf.clip_by_norm (||g|| against clip)
 };
 int clip_chunks(int64_t max_count);
-int launch_rmsprop_clipped(const RmsPropArgs& a, const ClipArgs& c, cudaStream_t stream);
+// RMSProp over the arena, its gradient clipped first unless c is null.  *kernels: the launches it enqueued (clipped: chunk sums
+// of squares, per-tensor scale, update).
+int launch_rmsprop(const RmsPropArgs& a, const ClipArgs* c, cudaStream_t stream, int* kernels);
 // Config.DUAL_RMSPROP: two optimizers with their own slots, both steps taken from the weights the call started with:
 // w <- w - step(g, ms, mom) - step(g2, ms2, mom2).  Elements inside [skip_lo[i], skip_hi[i]) are left alone by optimizer i / 2
 // (i = 0, 1: first optimizer; 2, 3: second): the variables its cost does not reach.
@@ -141,15 +141,11 @@ struct RmsPropDualArgs {
   const float* g2;
   float *ms2, *mom2;
   int64_t skip_lo[4], skip_hi[4];
-  // DUAL_RMSPROP + USE_GRAD_CLIP (NetworkVP_discrate.py:107-117): per-variable tf.clip_by_norm scales of g (scale1) and g2
-  // (scale2), indexed like the tensor table below; null = unclipped
-  const float *scale1, *scale2;
-  int n_tensors;
-  int64_t t_offset[CLIP_MAX_TENSORS], t_count[CLIP_MAX_TENSORS];
+  const float *scale1, *scale2;    // set by launch_rmsprop_dual when it clips
 };
-int launch_rmsprop_dual(const RmsPropDualArgs& d, cudaStream_t stream);
-// the same with both gradients clipped first: c1 describes g (d.a.g), c2 describes g2; both by_norm.  5 launches.
-int launch_rmsprop_dual_clipped(RmsPropDualArgs d, const ClipArgs& c1, const ClipArgs& c2, cudaStream_t stream);
+// DUAL_RMSPROP + USE_GRAD_CLIP (NetworkVP_discrate.py:107-117) unless c1 is null: c1 describes g (d.a.g), c2 describes g2, both
+// by_norm.  *kernels: 1, or 5 when clipped.
+int launch_rmsprop_dual(RmsPropDualArgs d, const ClipArgs* c1, const ClipArgs* c2, cudaStream_t stream, int* kernels);
 // grad_reduce + RMSProp in one launch (single-GPU step; r.out must be a.g, r.out_floats the small-tensor prefix)
 int launch_rmsprop_reduce(const RmsPropArgs& a, const GradReduceArgs& r, cudaStream_t stream);
 // data-parallel exchange over peer memory (dp_exchange.cuh), in two instalments.

@@ -13,7 +13,6 @@ struct ga3c_mlp : Handle<ga3c_mlp_config> {
   MlpNet net{};
   int64_t live_floats = 0;               // live tensors are packed first; [live_floats, arena_floats) is never updated
   float* part = nullptr;                 // [MLP_MAX_SPLITS][live_floats] weight-gradient partial arenas
-  int64_t skip_lo[2] = {}, skip_hi[2] = {};          // arena ranges of logits_v/* and of the policy head
   // workspace for max_batch rows; last_batch: rows of act[] written by the last forward (0: none since it was allocated)
   float* act[MLP_MAX_LAYERS] = {};
   float* dz[MLP_MAX_LAYERS] = {};
@@ -142,9 +141,14 @@ extern "C" int ga3c_mlp_create(const ga3c_mlp_config* cfg, ga3c_mlp** out) {
   net.wv_off = (int)n->params[pv].offset; net.bv_off = (int)n->params[pv + 1].offset;
   net.wp_off = (int)n->params[px].offset; net.bp_off = (int)n->params[px + 1].offset;
   if (py >= 0) { net.wy_off = (int)n->params[py].offset; net.by_off = (int)n->params[py + 1].offset; }
+  // DUAL_RMSPROP (NetworkVP.py:107-118): cost_p does not reach logits_v/*, cost_v not the policy head, whose variables are
+  // consecutive in the arena
   n->skip_lo[0] = n->params[pv].offset; n->skip_hi[0] = n->params[pv + 1].offset + n->params[pv + 1].count;
-  const int plast = py >= 0 ? py + 1 : px + 1;      // the policy head's variables are consecutive in the arena
-  n->skip_lo[1] = n->params[px].offset; n->skip_hi[1] = n->params[plast].offset + n->params[plast].count;
+  const int plast = py >= 0 ? py + 1 : px + 1;
+  n->skip_lo[2] = n->params[px].offset; n->skip_hi[2] = n->params[plast].offset + n->params[plast].count;
+  // opt.minimize(..., global_step=self.global_step) once per optimizer; clipped, the fork's NetworkVP still hands global_step to
+  // apply_gradients (NetworkVP.py:127-141) and NetworkVP_discrate does not (NetworkVP_discrate.py:107-121)
+  n->step_advance = cfg->use_grad_clip && cfg->kind != GA3C_MLP_FORK_VP ? 0 : cfg->dual_rmsprop ? 2 : 1;
   n->stream_ok = n->tc_hi > n->tc_lo && mlp_stream_ok(net, n->tc_lo, n->tc_hi);
 
   if (cfg->use_grad_clip) {
@@ -370,18 +374,10 @@ extern "C" int ga3c_mlp_forward_backward(ga3c_mlp* n, const float* x, const floa
 extern "C" int ga3c_mlp_apply_rmsprop(ga3c_mlp* n, float lr, void* stream) {
   if (!n) return set_error("ga3c_mlp_apply_rmsprop: null handle");
   CK(cudaSetDevice(n->cfg.device));
-  const RmsPropArgs a = rmsprop_args(n, lr);
   if (n->cfg.dual_rmsprop) return set_error("ga3c_mlp_apply_rmsprop: with DUAL_RMSPROP use ga3c_mlp_train_step (two backward passes)");
-  if (n->cfg.use_grad_clip) {            // tf.clip_by_average_norm per variable (NetworkVP.py:138-141, NetworkVP_discrate.py:118-121)
-    // every variable is live here (checked at create)
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_clipped(a, clip_args(n, 0), (cudaStream_t)stream));
-    n->log.launches += 2;
-    if (n->cfg.kind == GA3C_MLP_FORK_VP) n->global_step += 1;     // the fork's NetworkVP passes global_step, _discrate does not
-    return 0;
-  }
-  LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop(a, (cudaStream_t)stream));
-  n->global_step += 1;                   // opt.minimize(..., global_step=self.global_step)
-  return 0;
+  // USE_GRAD_CLIP: tf.clip_by_average_norm per variable (NetworkVP.py:138-141, NetworkVP_discrate.py:118-121); every variable
+  // is live then (checked at create)
+  return launch_optimizer(n, rmsprop_args(n, lr), (cudaStream_t)stream);
 }
 
 extern "C" int ga3c_mlp_train_step(ga3c_mlp* n, const float* x, const float* yr, const float* a, int32_t batch, float lr,
@@ -390,25 +386,7 @@ extern "C" int ga3c_mlp_train_step(ga3c_mlp* n, const float* x, const float* yr,
     // Config.DUAL_RMSPROP (NetworkVP.py:107-118, :143-147): cost_p into g, cost_v into g2, both steps from the same weights
     if (int r = mlp_fb_impl(n, x, yr, a, batch, beta, loss, stream, 1, n->g)) return r;
     if (int r = mlp_fb_impl(n, x, yr, a, batch, beta, nullptr, stream, 2, n->g2)) return r;
-    RmsPropDualArgs d{};
-    d.a = rmsprop_args(n, lr);
-    d.g2 = n->g2; d.ms2 = n->ms2; d.mom2 = n->mom2;
-    d.skip_lo[0] = n->skip_lo[0]; d.skip_hi[0] = n->skip_hi[0];        // cost_p: not logits_v
-    d.skip_lo[2] = n->skip_lo[1]; d.skip_hi[2] = n->skip_hi[1];        // cost_v: not the policy head
-    if (n->cfg.use_grad_clip) {
-      // tf.clip_by_norm per variable and optimizer (NetworkVP.py:127-137, NetworkVP_discrate.py:107-117); the fork's NetworkVP
-      // hands global_step to both apply_gradients calls, NetworkVP_discrate to neither
-      // (the gradient-less variables' gradient is None: the reference filters them, clip_args leaves them out)
-      ClipArgs c1 = clip_args(n, 0), c2 = clip_args(n, 1);
-      c1.by_norm = c2.by_norm = 1;
-      LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_dual_clipped(d, c1, c2, (cudaStream_t)stream));
-      n->log.launches += 4;
-      if (n->cfg.kind == GA3C_MLP_FORK_VP) n->global_step += 2;
-      return 0;
-    }
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_dual(d, (cudaStream_t)stream));
-    n->global_step += 2;
-    return 0;
+    return launch_optimizer(n, rmsprop_args(n, lr), (cudaStream_t)stream);
   }
   if (int r = ga3c_mlp_forward_backward(n, x, yr, a, batch, beta, loss, stream)) return r;
   return ga3c_mlp_apply_rmsprop(n, lr, stream);

@@ -107,6 +107,11 @@ extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
     cur = align_up(cur + n->params[order[k]].count);
   }
   n->arena_floats = cur;
+  const int skip[4] = {P_VW, P_VB, P_PW, P_PB};          // cost_p does not reach logits_v (stop_gradient), cost_v not logits_p
+  for (int i = 0; i < 4; ++i) { n->skip_lo[i] = n->off(skip[i]); n->skip_hi[i] = n->off(skip[i]) + n->params[skip[i]].count; }
+  // opt.minimize(..., global_step=self.global_step) once per optimizer (NetworkVP_discrate.py:130; DUAL_RMSPROP: both minimize
+  // calls, :125-126); clipped, apply_gradients is called without global_step (:107-117, :121) and the step counter stays put
+  n->step_advance = cfg->use_grad_clip ? 0 : cfg->dual_rmsprop ? 2 : 1;
 
   const size_t ab = (size_t)n->arena_floats * sizeof(float);
   const size_t shadow_bytes = (size_t)FLAT * FC * 2;
@@ -404,21 +409,14 @@ static RmsPropArgs rmsprop_args(ga3c_net* n, float lr) {
 static int apply_rmsprop_impl(ga3c_net* n, float lr, void* stream) {
   if (!n) return set_error("ga3c_apply_rmsprop: null handle");
   CK(cudaSetDevice(n->cfg.device));
-  RmsPropArgs a = rmsprop_args(n, lr);
   if (n->cfg.dual_rmsprop) return set_error("ga3c_apply_rmsprop: with DUAL_RMSPROP use ga3c_train_step (two backward passes)");
-  if (n->cfg.use_grad_clip) {
-    // clip_by_average_norm needs the whole (reduced) gradient of a variable: local arena only (single GPU, or after the
-    // host's NCCL allreduce in dp_mode 'nccl')
-    if (n->dp_world > 1) return set_error("ga3c_apply_rmsprop: USE_GRAD_CLIP is not available with the peer-memory exchange");
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_clipped(a, clip_args(n, 0), (cudaStream_t)stream));
-    n->log.launches += 2;
-    return 0;          // NetworkVP_discrate.py:121: apply_gradients without global_step -- the step counter stays put
-  }
+  // clip_by_average_norm needs the whole (reduced) gradient of a variable: local arena only (single GPU, or after the
+  // host's NCCL allreduce in dp_mode 'nccl')
+  if (n->cfg.use_grad_clip && n->dp_world > 1)
+    return set_error("ga3c_apply_rmsprop: USE_GRAD_CLIP is not available with the peer-memory exchange");
   // the peer-memory exchange is part of the train step (its dense1/w half starts behind dense_bwd, on a side stream)
   if (n->dp_world > 1) return set_error("ga3c_apply_rmsprop: not available on a peer-memory data-parallel handle; use ga3c_train_step");
-  LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop(a, (cudaStream_t)stream));
-  n->global_step += 1;   // opt.minimize(..., global_step=self.global_step), NetworkVP_discrate.py:130
-  return 0;
+  return launch_optimizer(n, rmsprop_args(n, lr), (cudaStream_t)stream);
 }
 
 extern "C" int ga3c_apply_rmsprop(ga3c_net* n, float lr, void* stream) { return apply_rmsprop_impl(n, lr, stream); }
@@ -537,22 +535,7 @@ static int dual_forward_backward_impl(ga3c_net* n, const void* x, bool x_u8, con
 static int dual_apply_impl(ga3c_net* n, float lr, void* stream) {
   if (!n || !n->cfg.dual_rmsprop) return set_error("ga3c_dual_apply: the handle was not created with dual_rmsprop");
   CK(cudaSetDevice(n->cfg.device));
-  RmsPropDualArgs d{};
-  d.a = rmsprop_args(n, lr);
-  d.g2 = n->g2; d.ms2 = n->ms2; d.mom2 = n->mom2;
-  const int skip[4] = {P_VW, P_VB, P_PW, P_PB};          // cost_p does not reach logits_v (stop_gradient), cost_v not logits_p
-  for (int i = 0; i < 4; ++i) { d.skip_lo[i] = n->off(skip[i]); d.skip_hi[i] = n->off(skip[i]) + n->params[skip[i]].count; }
-  if (n->cfg.use_grad_clip) {
-    // NetworkVP_discrate.py:107-117: tf.clip_by_norm per variable and optimizer, then apply_gradients WITHOUT global_step
-    ClipArgs c1 = clip_args(n, 0), c2 = clip_args(n, 1);
-    c1.by_norm = c2.by_norm = 1;
-    LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_dual_clipped(d, c1, c2, (cudaStream_t)stream));
-    n->log.launches += 4;
-    return 0;
-  }
-  LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_dual(d, (cudaStream_t)stream));
-  n->global_step += 2;      // both minimize calls advance it (NetworkVP_discrate.py:125-126)
-  return 0;
+  return launch_optimizer(n, rmsprop_args(n, lr), (cudaStream_t)stream);
 }
 extern "C" int ga3c_dual_forward_backward(ga3c_net* n, const float* x, const float* yr, const float* a, int32_t batch, float beta,
                                           float* loss, void* stream) {
@@ -576,7 +559,7 @@ static DpBigArgs dp_big_args(ga3c_net* n, float lr) {
 static RmsPropDpArgs dp_small_args(ga3c_net* n, float lr, int batch, const DpBigArgs& b) {
   RmsPropDpArgs d{};
   d.base = rmsprop_args(n, lr);
-  d.base.preload = batch >= n->num_sms;         // see rmsprop_reduce_kernel
+  d.base.preload = batch >= n->num_sms;         // the preload rule (elementwise.cu)
   for (int q = 0; q < n->dp_world; ++q) d.peer[q] = n->dp_peer[q];
   d.rank = n->dp_rank; d.world = n->dp_world; d.step = b.step;
   d.arena_bytes = b.arena_bytes; d.comm_offset = n->comm_off;
@@ -600,7 +583,7 @@ static int train_step_empty(ga3c_net* n, float lr, float* loss, void* stream) {
   const DpBigArgs b = dp_big_args(n, lr);
   if (int r = enqueue_dp_big(n, b, st)) return r;                  // behind the zeroed gradient
   LAUNCH(n, K_RMSPROP, st, launch_dp_small(dp_small_args(n, lr, 0, b), n->xbuf_off, st));
-  n->global_step += 1;
+  n->global_step += n->step_advance;
   return 0;
 }
 
@@ -626,15 +609,15 @@ static int train_step_impl(ga3c_net* n, const void* x, bool x_u8, const float* y
     const DpBigArgs b = dp_big_args(n, lr);
     if (int r = fb_tail_impl(n, x, x_u8, batch, stream, true, false, &b)) return r;
     LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_dp_small(dp_small_args(n, lr, batch, b), n->xbuf_off, (cudaStream_t)stream));
-    n->global_step += 1;
+    n->global_step += n->step_advance;
     return 0;
   }
   // single GPU: the slab reduction rides in the optimizer launch
   if (int r = fb_tail_impl(n, x, x_u8, batch, stream, true, false)) return r;
   RmsPropArgs ra = rmsprop_args(n, lr);
-  ra.preload = batch >= n->num_sms;               // see rmsprop_reduce_kernel
+  ra.preload = batch >= n->num_sms;               // the preload rule (elementwise.cu)
   LAUNCH(n, K_RMSPROP, (cudaStream_t)stream, launch_rmsprop_reduce(ra, reduce_args(n, batch), (cudaStream_t)stream));
-  n->global_step += 1;   // opt.minimize(..., global_step=self.global_step), NetworkVP_discrate.py:130
+  n->global_step += n->step_advance;
   return 0;
 }
 extern "C" int ga3c_train_step(ga3c_net* n, const float* x, const float* yr, const float* a, int32_t batch, float lr,
