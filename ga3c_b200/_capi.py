@@ -15,7 +15,8 @@ _CONFIG_TAIL = [("rmsprop_decay", C.c_float), ("rmsprop_momentum", C.c_float), (
 
 
 class ga3c_config(C.Structure):
-    _fields_ = [("device", C.c_int32), ("num_actions", C.c_int32), ("max_batch", C.c_int32)] + _CONFIG_TAIL
+    _fields_ = [("device", C.c_int32), ("num_actions", C.c_int32), ("max_batch", C.c_int32)] + _CONFIG_TAIL + [
+        ("image_height", C.c_int32), ("image_width", C.c_int32), ("stacked_frames", C.c_int32)]
 
 
 class ga3c_mlp_config(C.Structure):

@@ -207,6 +207,9 @@ __device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.
 // trace_attach_<file>(); detached (the default) it costs one predicated load per CTA.
 enum KernelId { K_CONV_FWD = 0, K_DENSE_FWD, K_HEADS, K_DENSE_WGRAD, K_DENSE_DGRAD, K_CONV12_BWD, K_CONV11_WGRAD, K_RMSPROP,
                 K_GRAD_REDUCE, K_MLP_FUSED, K_MLP_WGRAD, K_MLP_REDUCE, K_DP_BIG, K_MLP_TC, K_HISTO,
+                // the generic conv trunk (conv_gen.cu)
+                K_GEN_WPREP, K_GEN_IM2COL1, K_GEN_CONV11, K_GEN_IM2COL2, K_GEN_CONV12, K_GEN_CONV12_DGRAD, K_GEN_COL2IM,
+                K_GEN_CONV12_WGRAD, K_GEN_CONV11_WGRAD,
                 K_COUNT };
 constexpr int TRACE_SLOTS = 6;
 static __device__ unsigned long long* g_trace = nullptr;

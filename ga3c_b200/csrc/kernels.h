@@ -12,6 +12,7 @@ int trace_attach_conv_bwd_fused(unsigned long long* buf);
 int trace_attach_dense_tc(unsigned long long* buf);
 int trace_attach_heads(unsigned long long* buf);
 int trace_attach_elementwise(unsigned long long* buf);
+int trace_attach_conv_gen(unsigned long long* buf);
 
 // pipeline event log of CTA 0 (debug): attach a zeroed [16 warps][1024][2] uint64 buffer (or nullptr)
 int evt_attach_conv_fwd(unsigned long long* buf);
@@ -33,6 +34,7 @@ inline int l2_hints(bool train, bool x_u8) {
 int configure_conv_fwd();
 int configure_conv_bwd_fused();
 int configure_dense_tc();
+int configure_conv_gen();
 
 // conv_fwd.cu -- x fp32 (or uint8, x_u8: k/128 - 1 applied on the fly) [B,28224] -> n2 bf16 [B,3872]; when training also n1 (bf16, in
 // the Blk2 operand layout) and xblk (the bf16 block matrix of the frame): both are read back by the conv backward (common.cuh)
@@ -40,8 +42,9 @@ int launch_conv_fwd(const void* x, bool x_u8, const float* w11, const float* b11
                     uint8_t* n1_out, uint8_t* xblk_out, uint16_t* n2_out, int batch, int num_sms, cudaStream_t stream);
 
 // dense_tc.cu -- the three dense1 GEMMs (NetworkDNav.py:90 and its autodiff) on tcgen05 / TMEM / TMA.  fwd leaves `splits` raw fp32 partial tiles
-// in d1_part[splits][B][256]; the heads kernel sums them, adds the bias and applies the ReLU.
-int dense_fwd_splits(int batch, int num_sms);
+// in d1_part[splits][B][256]; the heads kernel sums them, adds the bias and applies the ReLU.  kdim: dense1's K (FLAT = 3872 at
+// 84x84x4, H2 * W2 * 32 on the generic trunk).
+int dense_fwd_splits(int batch, int num_sms, int kdim);
 // data parallel, side-stream exchange: flags = this rank's comm block + DPC_BIGDONE ([world] x 64 B, u64 step numbers), see
 // gemm_tc_body (dense_tc.cu).  flags == nullptr: no gate.
 struct DpGate {
@@ -50,14 +53,54 @@ struct DpGate {
   unsigned long long step;          // every flag must have reached this step
   int world;
 };
-int launch_dense_fwd_tc(const uint16_t* n2, const uint16_t* w1bf, float* d1_part, int batch, int splits, cudaStream_t stream,
-                        const DpGate* gate = nullptr);
+int launch_dense_fwd_tc(const uint16_t* n2, const uint16_t* w1bf, float* d1_part, int batch, int kdim, int splits,
+                        cudaStream_t stream, const DpGate* gate = nullptr);
 int launch_dense_dgrad_tc(const uint16_t* dd1, const uint16_t* w1bf, const uint16_t* n2, uint8_t* dn2, int batch,
                           cudaStream_t stream);       // dn2 in the G operand layout (common.cuh), borders untouched
-int launch_dense_wgrad_tc(const uint16_t* n2, const uint16_t* dd1, float* g_w1, int batch, cudaStream_t stream);
+int launch_dense_wgrad_tc(const uint16_t* n2, const uint16_t* dd1, float* g_w1, int batch, int kdim, cudaStream_t stream);
 // dgrad + wgrad tiles in one grid (both only need dd1): the train step uses this one
 int launch_dense_bwd_tc(const uint16_t* dd1, const uint16_t* w1bf, const uint16_t* n2, uint8_t* dn2, float* g_w1, int batch,
                         cudaStream_t stream);
+// the generic trunk's forms of the two: dn2 row-major [B][kdim], like n2
+int launch_dense_dgrad_rows_tc(const uint16_t* dd1, const uint16_t* w1bf, const uint16_t* n2, uint16_t* dn2, int batch,
+                               int kdim, cudaStream_t stream);
+int launch_dense_bwd_rows_tc(const uint16_t* dd1, const uint16_t* w1bf, const uint16_t* n2, uint16_t* dn2, float* g_w1,
+                             int batch, int kdim, cudaStream_t stream);
+
+// conv_gen.cu -- the conv trunk for any input geometry (H, W, C) other than 84x84x4: im2col gathers and GEMMs on the tcgen05
+// core of dense_tc.cu.  All activations are row-major: X1 [B*H1*W1][ld1 = 64C + 8] (the im2col of the frames, column 64C = 1,
+// the rest of the pad 0), n1 [B*H1*W1][16], X2 [B*H2*W2][GEN_LD2] (the im2col of n1, column 256 = 1), n2 = [B*H2*W2][32].
+constexpr int GEN_LD2 = 264;
+struct GenGeom {
+  int h, w, c;                 // input
+  int h1, w1, pt1, pl1;        // conv11 output size and SAME padding before (top, left)
+  int h2, w2, pt2, pl2;        // conv12
+  int k1, ld1;                 // conv11 K = 64C and X1's row length
+  int kdim;                    // dense1 K = h2 * w2 * 32
+};
+GenGeom gen_geom(int h, int w, int c);
+struct GenBufs {
+  uint16_t *x1, *n1, *x2, *n2, *dn2, *dn1;
+  float* dx2;                  // [B*H2*W2][256] fp32: conv12's data gradient before col2im
+  uint16_t *w11t, *w12t, *w12; // bf16 GEMM operands: conv11/w^T [16][64C], conv12/w^T [32][256], conv12/w [256][32]
+};
+// forward, one launch each: weights -> bf16 operands, im2col of the frames, conv11 GEMM (bias + ReLU) -> n1, im2col of n1,
+// conv12 GEMM (bias + ReLU) -> n2
+int launch_gen_wprep(const GenGeom& g, const GenBufs& b, const float* w11, const float* w12, cudaStream_t st);
+int launch_gen_im2col1(const GenGeom& g, const GenBufs& b, const void* x, bool x_u8, int batch, cudaStream_t st);
+int launch_gen_conv11(const GenGeom& g, const GenBufs& b, const float* b11, int batch, cudaStream_t st);
+int launch_gen_im2col2(const GenGeom& g, const GenBufs& b, int batch, cudaStream_t st);
+int launch_gen_conv12(const GenGeom& g, const GenBufs& b, const float* b12, int batch, cudaStream_t st);
+// backward from dn2: conv12 data gradient -> dx2, col2im + the n1 > 0 mask -> dn1, and the weight / bias gradients of conv12
+// and conv11 as `slabs` partial sums (slab s = k-block range s of the GEMM over positions) into the gradient-partial slabs,
+// gp_stride floats apart, that launch_grad_reduce sums in a fixed order
+int gen_wgrad_slabs(const GenGeom& g, int batch, int num_sms);
+int launch_gen_conv12_dgrad(const GenGeom& g, const GenBufs& b, int batch, cudaStream_t st);
+int launch_gen_col2im(const GenGeom& g, const GenBufs& b, int batch, cudaStream_t st);
+int launch_gen_conv12_wgrad(const GenGeom& g, const GenBufs& b, float* g_w12, float* g_b12, int64_t gp_stride, int slabs,
+                            int batch, cudaStream_t st);
+int launch_gen_conv11_wgrad(const GenGeom& g, const GenBufs& b, float* g_w11, float* g_b11, int64_t gp_stride, int slabs,
+                            int batch, cudaStream_t st);
 
 // heads.cu -- value / policy heads, softmax, A3C loss and its backward (NetworkVP_discrate.py:60-85)
 struct HeadsArgs {

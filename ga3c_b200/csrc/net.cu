@@ -49,15 +49,24 @@ struct ga3c_net : Handle<ga3c_config> {
   std::mutex mtx;                  // ga3c_lock / ga3c_unlock
   unsigned long long* evt = nullptr;       // pipeline event log of CTA 0 (ga3c_evt_*), device memory
   unsigned long long* trace = nullptr;     // [K_COUNT][TRACE_SLOTS] globaltimer stamps (ga3c_trace_*), device memory
+  // input geometry: 84x84x4 runs the specialised trunk (conv_fwd.cu, conv_bwd_fused.cu), every other one the generic trunk
+  // (conv_gen.cu) on the row-major buffers in gen (gen.n2 / gen.dn2 alias n2 / dn2 above)
+  GenGeom geo{};
+  bool generic = false;
+  GenBufs gen{};
+  int conv_slabs = 0;              // gradient-partial slabs the conv backward of the current step wrote
 
   int64_t off(int i) const { return params[i].offset; }
+  int64_t w1_count() const { return (int64_t)geo.kdim * FC; }
 };
 
 
 static const char* const kKernelNames[K_COUNT] = {"conv_fwd", "dense_fwd", "heads", "dense_wgrad", "dense_bwd",
                                                   "conv_bwd", "conv11_wgrad", "rmsprop", "grad_reduce",
                                                   "mlp_fused", "mlp_wgrad", "mlp_reduce", "dp_big", "mlp_tc",
-                                                  "histograms"};
+                                                  "histograms", "gen_wprep", "gen_im2col11", "gen_conv11",
+                                                  "gen_im2col12", "gen_conv12", "gen_conv12_dgrad", "gen_col2im",
+                                                  "gen_conv12_wgrad", "gen_conv11_wgrad"};
 
 enum { P_C11W = 0, P_C11B, P_C12W, P_C12B, P_D1W, P_D1B, P_VW, P_VB, P_PW, P_PB, P_COUNT };
 
@@ -70,24 +79,32 @@ int set_error(const std::string& m) { g_err = m; return -1; }     // for the oth
 const char* kernel_name(int kid) { return (kid >= 0 && kid < K_COUNT) ? kKernelNames[kid] : nullptr; }
 }
 extern "C" const char* ga3c_last_error(void) { return g_err.c_str(); }
-extern "C" int ga3c_abi_version(void) { return 9; }
+extern "C" int ga3c_abi_version(void) { return 10; }
 
 extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
   if (!cfg || !out) return set_error("ga3c_create: null argument");
   *out = nullptr;
   if (cfg->num_actions < 1 || cfg->num_actions > MAX_ACTIONS) return set_error("ga3c_create: num_actions must be 1..18");
   if (cfg->max_batch < 1) return set_error("ga3c_create: max_batch must be >= 1");
+  const int ih = cfg->image_height ? cfg->image_height : IMG, iw = cfg->image_width ? cfg->image_width : IMG;
+  const int ic = cfg->stacked_frames ? cfg->stacked_frames : IMG_C;
+  if (ih < 1 || ih > 256) return set_error("ga3c_create: image_height (Config.IMAGE_HEIGHT) must be 1..256");
+  if (iw < 1 || iw > 256) return set_error("ga3c_create: image_width (Config.IMAGE_WIDTH) must be 1..256");
+  if (ic < 1 || ic > 8) return set_error("ga3c_create: stacked_frames (Config.STACKED_FRAMES) must be 1..8");
   int num_sms = 0;
   if (int r = open_device(cfg->device, "ga3c_create", &num_sms)) return r;
   ga3c_net* n = new ga3c_net();
   n->cfg = *cfg;
+  n->cfg.image_height = ih; n->cfg.image_width = iw; n->cfg.stacked_frames = ic;
+  n->geo = gen_geom(ih, iw, ic);
+  n->generic = !(ih == IMG && iw == IMG && ic == IMG_C);
   n->num_sms = num_sms;
   const int A = cfg->num_actions;
   // TF creation order (NetworkVP.py:284-285 would list them so); offsets pack the small tensors first
   struct { const char* name; int nd; int64_t s[4]; } spec[P_COUNT] = {
-      {"conv11/w:0", 4, {8, 8, 4, 16}}, {"conv11/b:0", 1, {16, 0, 0, 0}},
+      {"conv11/w:0", 4, {8, 8, ic, 16}}, {"conv11/b:0", 1, {16, 0, 0, 0}},
       {"conv12/w:0", 4, {4, 4, 16, 32}}, {"conv12/b:0", 1, {32, 0, 0, 0}},
-      {"dense1/w:0", 2, {FLAT, FC, 0, 0}}, {"dense1/b:0", 1, {FC, 0, 0, 0}},
+      {"dense1/w:0", 2, {n->geo.kdim, FC, 0, 0}}, {"dense1/b:0", 1, {FC, 0, 0, 0}},
       {"logits_v/w:0", 2, {FC, 1, 0, 0}}, {"logits_v/b:0", 1, {1, 0, 0, 0}},
       {"logits_p/w:0", 2, {FC, A, 0, 0}}, {"logits_p/b:0", 1, {A, 0, 0, 0}}};
   n->params.resize(P_COUNT);
@@ -114,7 +131,7 @@ extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
   n->step_advance = cfg->use_grad_clip ? 0 : cfg->dual_rmsprop ? 2 : 1;
 
   const size_t ab = (size_t)n->arena_floats * sizeof(float);
-  const size_t shadow_bytes = (size_t)FLAT * FC * 2;
+  const size_t shadow_bytes = (size_t)n->w1_count() * 2;
   n->xbuf_off = (int64_t)(4 * ab + shadow_bytes);
   n->comm_off = n->xbuf_off + 2 * (int64_t)DP_MAX_WORLD * n->small_floats * 8;
   if (int r = alloc_arenas(n, (size_t)n->comm_off + DP_COMM_BYTES - 4 * ab)) { ga3c_destroy(n); return r; }
@@ -125,7 +142,7 @@ extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
   cudaMemset(n->gpart, 0, (size_t)2 * n->num_sms * n->gp_stride * sizeof(float));
   if (int r = alloc_workspace(n, cfg->max_batch)) { ga3c_destroy(n); return r; }
   int r;
-  if ((r = configure_conv_fwd()) || (r = configure_conv_bwd_fused()) || (r = configure_dense_tc())) {
+  if ((r = configure_conv_fwd()) || (r = configure_conv_bwd_fused()) || (r = configure_dense_tc()) || (r = configure_conv_gen())) {
     ga3c_destroy(n);
     return fail_cuda("cudaFuncSetAttribute", (cudaError_t)r);
   }
@@ -138,16 +155,37 @@ extern "C" int ga3c_create(const ga3c_config* cfg, ga3c_net** out) {
 static void free_workspace(ga3c_net* n) {
   cudaFree(n->n1); cudaFree(n->n2); cudaFree(n->d1); cudaFree(n->dd1); cudaFree(n->dn2); cudaFree(n->dn1); cudaFree(n->xblk);
   cudaFree(n->d1_part);
+  cudaFree(n->gen.x1); cudaFree(n->gen.n1); cudaFree(n->gen.x2); cudaFree(n->gen.dx2); cudaFree(n->gen.dn1); cudaFree(n->gen.w11t);
   n->n2 = n->dd1 = n->dn1 = nullptr; n->n1 = n->dn2 = n->xblk = nullptr; n->d1 = n->d1_part = nullptr;
+  n->gen = GenBufs{};
+}
+
+// the generic trunk's buffers (DESIGN.md, "The generic conv trunk": X1 and dx2 dominate)
+static int alloc_workspace_generic(ga3c_net* n, size_t mb) {
+  const GenGeom& g = n->geo;
+  const size_t p1 = mb * g.h1 * g.w1, p2 = mb * g.h2 * g.w2;
+  GenBufs& b = n->gen;
+  CK(cudaMalloc((void**)&b.x1, p1 * g.ld1 * 2)); CK(cudaMalloc((void**)&b.n1, p1 * 16 * 2));
+  CK(cudaMalloc((void**)&b.x2, p2 * GEN_LD2 * 2)); CK(cudaMalloc((void**)&b.dx2, p2 * 256 * 4));
+  CK(cudaMalloc((void**)&b.dn1, p1 * 16 * 2));
+  CK(cudaMalloc((void**)&b.w11t, ((size_t)16 * g.k1 + 2 * 32 * 256) * 2));
+  b.w12t = b.w11t + (size_t)16 * g.k1; b.w12 = b.w12t + 32 * 256;
+  CK(cudaMalloc((void**)&n->n2, mb * g.kdim * 2)); CK(cudaMalloc((void**)&n->dn2, mb * g.kdim * 2));
+  b.n2 = n->n2; b.dn2 = reinterpret_cast<uint16_t*>(n->dn2);
+  return 0;
 }
 
 static int alloc_workspace(ga3c_net* n, int max_batch) {
   const size_t mb = (size_t)max_batch;
-  CK(cudaMalloc((void**)&n->n1, mb * B2_BYTES)); CK(cudaMalloc((void**)&n->n2, mb * FLAT * 2));
+  if (n->generic) {
+    if (int r = alloc_workspace_generic(n, mb)) return r;
+  } else {
+    CK(cudaMalloc((void**)&n->n1, mb * B2_BYTES)); CK(cudaMalloc((void**)&n->n2, mb * FLAT * 2));
+    CK(cudaMalloc((void**)&n->dn2, mb * G_BYTES)); CK(cudaMalloc((void**)&n->dn1, mb * N1_POS * C1_OUT * 2));
+    CK(cudaMalloc((void**)&n->xblk, mb * XB_FRAME_BYTES));
+    CK(cudaMemset(n->n1, 0, mb * B2_BYTES)); CK(cudaMemset(n->dn2, 0, mb * G_BYTES)); CK(cudaMemset(n->xblk, 0, mb * XB_FRAME_BYTES));
+  }
   CK(cudaMalloc((void**)&n->d1, mb * FC * 4)); CK(cudaMalloc((void**)&n->dd1, mb * FC * 2));
-  CK(cudaMalloc((void**)&n->dn2, mb * G_BYTES)); CK(cudaMalloc((void**)&n->dn1, mb * N1_POS * C1_OUT * 2));
-  CK(cudaMalloc((void**)&n->xblk, mb * XB_FRAME_BYTES));
-  CK(cudaMemset(n->n1, 0, mb * B2_BYTES)); CK(cudaMemset(n->dn2, 0, mb * G_BYTES)); CK(cudaMemset(n->xblk, 0, mb * XB_FRAME_BYTES));
   // splits * batch <= max(batch, 64 * num_sms) rows for every batch (dense_fwd_splits)
   const size_t part_rows = mb > (size_t)64 * n->num_sms ? mb : (size_t)64 * n->num_sms;
   CK(cudaMalloc((void**)&n->d1_part, part_rows * FC * 4));
@@ -161,7 +199,7 @@ extern "C" int ga3c_reserve(ga3c_net* n, int32_t max_batch) {
   CK(cudaSetDevice(n->cfg.device));
   CK(cudaDeviceSynchronize());
   free_workspace(n);
-  if (int r = alloc_workspace(n, max_batch)) { n->cfg.max_batch = 0; return r; }
+  if (int r = alloc_workspace(n, max_batch)) { free_workspace(n); cudaGetLastError(); n->cfg.max_batch = 0; return r; }
   return 0;
 }
 
@@ -215,7 +253,7 @@ extern "C" int ga3c_arena_ptr(ga3c_net* n, int which, float** ptr_dev) {
 extern "C" int ga3c_arena_upload(ga3c_net* n, int which, const float* host, int64_t nf) {
   if (int r = arena_upload(n, which, host, nf, "ga3c_arena_upload")) return r;
   if (which == 0) {
-    CKL(launch_f32_to_bf16(n->w + n->off(P_D1W), n->w1_shadow, (int64_t)FLAT * FC, 0));
+    CKL(launch_f32_to_bf16(n->w + n->off(P_D1W), n->w1_shadow, n->w1_count(), 0));
     n->log.launches++;
     CK(cudaDeviceSynchronize());
   }
@@ -227,7 +265,7 @@ extern "C" int ga3c_arena_download(ga3c_net* n, int which, float* host, int64_t 
   if (n->dp_world > 1 && (which == 0 || which == 2 || which == 3)) {
     // peer-memory exchange: the fp32 master copy and the RMSProp slots of a dense1/w slice live on its owner (only the bf16
     // shadow travels).  A peer's slice is stable here: it changes only inside a step this rank takes part in.
-    const int64_t n4 = (int64_t)FLAT * FC / 4, per = (n4 + n->dp_world - 1) / n->dp_world;
+    const int64_t n4 = n->w1_count() / 4, per = (n4 + n->dp_world - 1) / n->dp_world;
     for (int q = 0; q < n->dp_world; ++q) {
       if (q == n->dp_rank) continue;
       const int64_t lo = per * q, hi = lo + per < n4 ? lo + per : n4;
@@ -267,19 +305,35 @@ static DpGate dp_gate(const ga3c_net* n) {
   return g;
 }
 
+// the generic trunk's forward: n1 and n2 (and X1, X2 for the backward) from the frames
+static int gen_forward(ga3c_net* n, const void* x, bool x_u8, int batch, cudaStream_t st) {
+  const GenGeom& g = n->geo;
+  const float* w = n->w;
+  LAUNCH(n, K_GEN_WPREP, st, launch_gen_wprep(g, n->gen, w + n->off(P_C11W), w + n->off(P_C12W), st));
+  LAUNCH(n, K_GEN_IM2COL1, st, launch_gen_im2col1(g, n->gen, x, x_u8, batch, st));
+  LAUNCH(n, K_GEN_CONV11, st, launch_gen_conv11(g, n->gen, w + n->off(P_C11B), batch, st));
+  LAUNCH(n, K_GEN_IM2COL2, st, launch_gen_im2col2(g, n->gen, batch, st));
+  LAUNCH(n, K_GEN_CONV12, st, launch_gen_conv12(g, n->gen, w + n->off(P_C12B), batch, st));
+  return 0;
+}
+
 static int predict_impl(ga3c_net* n, const void* x, bool x_u8, int32_t batch, float* p_out, float* v_out, void* stream) {
   if (int r = check_batch(n, batch, "ga3c_predict")) return r;
   if (!x || !p_out || !v_out) return set_error("ga3c_predict: null buffer");
   CK(cudaSetDevice(n->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
   const float* w = n->w;
-  LAUNCH(n, K_CONV_FWD, st, launch_conv_fwd(x, x_u8, w + n->off(P_C11W), w + n->off(P_C11B), w + n->off(P_C12W),
-                                            w + n->off(P_C12B), nullptr, nullptr, n->n2, batch, n->num_sms, st));
+  if (n->generic) {
+    if (int r = gen_forward(n, x, x_u8, batch, st)) return r;
+  } else {
+    LAUNCH(n, K_CONV_FWD, st, launch_conv_fwd(x, x_u8, w + n->off(P_C11W), w + n->off(P_C11B), w + n->off(P_C12W),
+                                              w + n->off(P_C12B), nullptr, nullptr, n->n2, batch, n->num_sms, st));
+  }
   const DpGate gate = dp_gate(n);
-  const int splits = dense_fwd_splits(batch, n->num_sms);
+  const int splits = dense_fwd_splits(batch, n->num_sms, n->geo.kdim);
   HeadsArgs h = heads_args(n, batch, splits);
   h.p_out = p_out; h.v_out = v_out; h.train = 0;
-  LAUNCH(n, K_DENSE_FWD, st, launch_dense_fwd_tc(n->n2, n->w1_shadow, n->d1_part, batch, splits, st, &gate));
+  LAUNCH(n, K_DENSE_FWD, st, launch_dense_fwd_tc(n->n2, n->w1_shadow, n->d1_part, batch, n->geo.kdim, splits, st, &gate));
   LAUNCH(n, K_HEADS, st, launch_heads(h, n->num_sms, st));
   n->last_batch = batch;
   return 0;
@@ -304,12 +358,16 @@ static int fb_head_impl(ga3c_net* n, const void* x, bool x_u8, const float* yr, 
   const float* w = n->w;
   float* g = n->g;
   float* gp = n->gpart;       // small-tensor gradients: per-CTA partial slabs, summed at the end of ga3c_fb_tail
-  const int splits = dense_fwd_splits(batch, n->num_sms);
+  const int splits = dense_fwd_splits(batch, n->num_sms, n->geo.kdim);
   if (!skip_forward) {        // the second DUAL_RMSPROP pass reuses n1 / n2 / the dense1 partials of the first
-    LAUNCH(n, K_CONV_FWD, st, launch_conv_fwd(x, x_u8, w + n->off(P_C11W), w + n->off(P_C11B), w + n->off(P_C12W),
-                                              w + n->off(P_C12B), n->n1, n->xblk, n->n2, batch, n->num_sms, st));
+    if (n->generic) {
+      if (int r = gen_forward(n, x, x_u8, batch, st)) return r;
+    } else {
+      LAUNCH(n, K_CONV_FWD, st, launch_conv_fwd(x, x_u8, w + n->off(P_C11W), w + n->off(P_C11B), w + n->off(P_C12W),
+                                                w + n->off(P_C12B), n->n1, n->xblk, n->n2, batch, n->num_sms, st));
+    }
     const DpGate gate = dp_gate(n);
-    LAUNCH(n, K_DENSE_FWD, st, launch_dense_fwd_tc(n->n2, n->w1_shadow, n->d1_part, batch, splits, st, &gate));
+    LAUNCH(n, K_DENSE_FWD, st, launch_dense_fwd_tc(n->n2, n->w1_shadow, n->d1_part, batch, n->geo.kdim, splits, st, &gate));
   }
   HeadsArgs h = heads_args(n, batch, splits);
   h.yr = yr; h.a = a; h.beta = beta; h.train = 1; h.dd1 = n->dd1; h.part = part;
@@ -319,7 +377,7 @@ static int fb_head_impl(ga3c_net* n, const void* x, bool x_u8, const float* yr, 
   n->loss_out = loss;
   LAUNCH(n, K_HEADS, st, launch_heads(h, n->num_sms, st));
   (void)g;
-  if (with_wgrad) LAUNCH(n, K_DENSE_WGRAD, st, launch_dense_wgrad_tc(n->n2, n->dd1, n->g + n->off(P_D1W), batch, st));
+  if (with_wgrad) LAUNCH(n, K_DENSE_WGRAD, st, launch_dense_wgrad_tc(n->n2, n->dd1, n->g + n->off(P_D1W), batch, n->geo.kdim, st));
   n->last_batch = batch;
   return 0;
 }
@@ -336,7 +394,7 @@ static GradReduceArgs reduce_args(ga3c_net* n, int batch, float* g_dst = nullptr
   r.part = n->gpart; r.stride = n->gp_stride; r.out = g_dst ? g_dst : n->g; r.out_tail = n->loss_out;
   r.out_floats = (int)n->small_floats; r.n_floats = (int)n->small_floats + 4;
   for (int s = 0; s < GR_MAX_SEG; ++s) { r.seg_end[s] = r.n_floats; r.seg_count[s] = n->gp_heads_grid; }
-  r.seg_end[0] = (int)n->off(P_D1B); r.seg_count[0] = conv_bwd_grid(batch, n->num_sms);
+  r.seg_end[0] = (int)n->off(P_D1B); r.seg_count[0] = n->generic ? n->conv_slabs : conv_bwd_grid(batch, n->num_sms);
   return r;
 }
 
@@ -362,15 +420,31 @@ static int fb_tail_impl(ga3c_net* n, const void* x, bool x_u8, int32_t batch, vo
   cudaStream_t st = (cudaStream_t)stream;
   const float* w = n->w;
   float* gp = n->gpart;
-  if (with_wgrad)   // dgrad + wgrad tiles of dense1 in one grid
-    LAUNCH(n, K_DENSE_DGRAD, st, launch_dense_bwd_tc(n->dd1, n->w1_shadow, n->n2, n->dn2, (g_dst ? g_dst : n->g) + n->off(P_D1W), batch, st));
-  else
-    LAUNCH(n, K_DENSE_DGRAD, st, launch_dense_dgrad_tc(n->dd1, n->w1_shadow, n->n2, n->dn2, batch, st));
-  if (dp != nullptr)
-    if (int r = enqueue_dp_big(n, *dp, st)) return r;
-  LAUNCH(n, K_CONV12_BWD, st, launch_conv_bwd(n->xblk, n->n1, n->dn2, w + n->off(P_C12W), n->keep_dn1 ? n->dn1 : nullptr,
-                                              gp + n->off(P_C11W), gp + n->off(P_C11B), gp + n->off(P_C12W),
-                                              gp + n->off(P_C12B), n->gp_stride, batch, n->num_sms, x_u8, st));
+  float* const g_w1 = (g_dst ? g_dst : n->g) + n->off(P_D1W);
+  if (n->generic) {
+    const GenGeom& ge = n->geo;
+    if (with_wgrad)
+      LAUNCH(n, K_DENSE_DGRAD, st, launch_dense_bwd_rows_tc(n->dd1, n->w1_shadow, n->n2, n->gen.dn2, g_w1, batch, ge.kdim, st));
+    else
+      LAUNCH(n, K_DENSE_DGRAD, st, launch_dense_dgrad_rows_tc(n->dd1, n->w1_shadow, n->n2, n->gen.dn2, batch, ge.kdim, st));
+    n->conv_slabs = gen_wgrad_slabs(ge, batch, n->num_sms);
+    LAUNCH(n, K_GEN_CONV12_DGRAD, st, launch_gen_conv12_dgrad(ge, n->gen, batch, st));
+    LAUNCH(n, K_GEN_COL2IM, st, launch_gen_col2im(ge, n->gen, batch, st));
+    LAUNCH(n, K_GEN_CONV12_WGRAD, st, launch_gen_conv12_wgrad(ge, n->gen, gp + n->off(P_C12W), gp + n->off(P_C12B), n->gp_stride,
+                                                              n->conv_slabs, batch, st));
+    LAUNCH(n, K_GEN_CONV11_WGRAD, st, launch_gen_conv11_wgrad(ge, n->gen, gp + n->off(P_C11W), gp + n->off(P_C11B), n->gp_stride,
+                                                              n->conv_slabs, batch, st));
+  } else {
+    if (with_wgrad)   // dgrad + wgrad tiles of dense1 in one grid
+      LAUNCH(n, K_DENSE_DGRAD, st, launch_dense_bwd_tc(n->dd1, n->w1_shadow, n->n2, n->dn2, g_w1, batch, st));
+    else
+      LAUNCH(n, K_DENSE_DGRAD, st, launch_dense_dgrad_tc(n->dd1, n->w1_shadow, n->n2, n->dn2, batch, st));
+    if (dp != nullptr)
+      if (int r = enqueue_dp_big(n, *dp, st)) return r;
+    LAUNCH(n, K_CONV12_BWD, st, launch_conv_bwd(n->xblk, n->n1, n->dn2, w + n->off(P_C12W), n->keep_dn1 ? n->dn1 : nullptr,
+                                                gp + n->off(P_C11W), gp + n->off(P_C11B), gp + n->off(P_C12W),
+                                                gp + n->off(P_C12B), n->gp_stride, batch, n->num_sms, x_u8, st));
+  }
   if (reduce) LAUNCH(n, K_GRAD_REDUCE, st, launch_grad_reduce(reduce_args(n, batch, g_dst), st));
   return 0;
 }
@@ -402,7 +476,7 @@ extern "C" int ga3c_fb_tail_u8(ga3c_net* n, const uint8_t* x, int32_t batch, voi
 
 static RmsPropArgs rmsprop_args(ga3c_net* n, float lr) {
   RmsPropArgs a = rmsprop_base(n, lr, n->arena_floats);
-  a.w1_shadow = n->w1_shadow; a.w1_offset = n->off(P_D1W); a.w1_count = (int64_t)FLAT * FC;
+  a.w1_shadow = n->w1_shadow; a.w1_offset = n->off(P_D1W); a.w1_count = n->w1_count();
   return a;
 }
 
@@ -450,6 +524,7 @@ extern "C" int ga3c_dp_detach(ga3c_net* n) {
 
 extern "C" int ga3c_dp_attach(ga3c_net* n, int32_t rank, int32_t world, const void* handles) {
   if (!n || !handles) return set_error("ga3c_dp_attach: null argument");
+  if (n->generic) return set_error("ga3c_dp_attach: the peer-memory exchange needs the 84x84x4 geometry (use dp_mode 'nccl')");
   if (world < 1 || world > DP_MAX_WORLD || rank < 0 || rank >= world)
     return set_error("ga3c_dp_attach: world must be 1.." + std::to_string(DP_MAX_WORLD) + " and 0 <= rank < world");
   CK(cudaSetDevice(n->cfg.device));
@@ -474,6 +549,7 @@ extern "C" int ga3c_dp_attach(ga3c_net* n, int32_t rank, int32_t world, const vo
 // device pointers, no IPC handles involved.  peers[r] is rank r's handle (peers[rank] == net).
 extern "C" int ga3c_dp_attach_local(ga3c_net* n, int32_t rank, int32_t world, ga3c_net* const* peers) {
   if (!n || !peers) return set_error("ga3c_dp_attach_local: null argument");
+  if (n->generic) return set_error("ga3c_dp_attach_local: the peer-memory exchange needs the 84x84x4 geometry (use dp_mode 'nccl')");
   if (world < 1 || world > DP_MAX_WORLD || rank < 0 || rank >= world || peers[rank] != n)
     return set_error("ga3c_dp_attach_local: need 0 <= rank < world <= 8 and peers[rank] == net");
   CK(cudaSetDevice(n->cfg.device));
@@ -552,7 +628,7 @@ static DpBigArgs dp_big_args(ga3c_net* n, float lr) {
   for (int r = 0; r < n->dp_world; ++r) b.peer[r] = n->dp_peer[r];
   b.rank = n->dp_rank; b.world = n->dp_world; b.step = ++n->dp_step;
   b.arena_bytes = (int64_t)n->arena_floats * 4; b.shadow_off = 4 * b.arena_bytes; b.comm_offset = n->comm_off;
-  b.w1_offset = n->off(P_D1W); b.w1_count = (int64_t)FLAT * FC;
+  b.w1_offset = n->off(P_D1W); b.w1_count = n->w1_count();
   b.lr = lr; b.decay = n->cfg.rmsprop_decay; b.momentum = n->cfg.rmsprop_momentum; b.eps = n->cfg.rmsprop_epsilon;
   return b;
 }
@@ -579,7 +655,7 @@ static int train_step_empty(ga3c_net* n, float lr, float* loss, void* stream) {
   n->loss_out = loss;
   n->last_batch = 0;
   // the exchange publishes "gradient final" itself; dp_small sums zero slabs
-  CK(cudaMemsetAsync(n->g + n->off(P_D1W), 0, (size_t)FLAT * FC * 4, st));
+  CK(cudaMemsetAsync(n->g + n->off(P_D1W), 0, (size_t)n->w1_count() * 4, st));
   const DpBigArgs b = dp_big_args(n, lr);
   if (int r = enqueue_dp_big(n, b, st)) return r;                  // behind the zeroed gradient
   LAUNCH(n, K_RMSPROP, st, launch_dp_small(dp_small_args(n, lr, 0, b), n->xbuf_off, st));
@@ -651,6 +727,18 @@ extern "C" int ga3c_select_actions(const float* p, const double* u, int32_t batc
 extern "C" int ga3c_workspace_ptr(ga3c_net* n, int which, void** ptr, int64_t* bytes) {
   if (!n || !ptr) return set_error("ga3c_workspace_ptr: null argument");
   const int64_t b = n->last_batch;
+  if (n->generic) {          // row-major: n1 / dn1 [B,H1,W1,16], n2 / dn2 [B,K] bf16, 7 = X1 [B*H1*W1][64C + 8] bf16
+    const GenGeom& g = n->geo;
+    const int64_t p1 = b * g.h1 * g.w1;
+    switch (which) {
+      case 0: *ptr = n->gen.n1; if (bytes) *bytes = p1 * 32; return 0;
+      case 1: *ptr = n->n2; if (bytes) *bytes = b * g.kdim * 2; return 0;
+      case 4: *ptr = n->dn2; if (bytes) *bytes = b * g.kdim * 2; return 0;
+      case 5: *ptr = n->gen.dn1; if (bytes) *bytes = p1 * 32; return 0;
+      case 6: *ptr = n->w1_shadow; if (bytes) *bytes = n->w1_count() * 2; return 0;
+      case 7: *ptr = n->gen.x1; if (bytes) *bytes = p1 * g.ld1 * 2; return 0;
+    }
+  }
   switch (which) {
     case 0: *ptr = n->n1; if (bytes) *bytes = b * B2_BYTES; break;
     case 1: *ptr = n->n2; if (bytes) *bytes = b * FLAT * 2; break;
@@ -676,8 +764,13 @@ extern "C" int ga3c_histograms(ga3c_net* n, int32_t batch, const float* p, const
   HistoArgs a{};
   for (int i = 0; i < P_COUNT; ++i) a.src[i] = HistoSrc{n->w + n->off(i), n->params[i].count, 0, 0};
   const long long b = batch;
-  a.src[P_COUNT + 0] = HistoSrc{n->n1, b * B2_BYTES / 2, 1, 1};
-  a.src[P_COUNT + 1] = HistoSrc{n->n2, b * FLAT, 1, 0};
+  if (n->generic) {
+    a.src[P_COUNT + 0] = HistoSrc{n->gen.n1, b * n->geo.h1 * n->geo.w1 * C1_OUT, 1, 0};
+    a.src[P_COUNT + 1] = HistoSrc{n->n2, b * n->geo.kdim, 1, 0};
+  } else {
+    a.src[P_COUNT + 0] = HistoSrc{n->n1, b * B2_BYTES / 2, 1, 1};
+    a.src[P_COUNT + 1] = HistoSrc{n->n2, b * FLAT, 1, 0};
+  }
   a.src[P_COUNT + 2] = HistoSrc{n->d1, b * FC, 0, 0};
   a.src[P_COUNT + 3] = HistoSrc{v, b, 0, 0};
   a.src[P_COUNT + 4] = HistoSrc{p, b * n->cfg.num_actions, 0, 0};
@@ -702,7 +795,7 @@ extern "C" const char* ga3c_kernel_name(int kid) { return (kid >= 0 && kid < K_C
 static int trace_attach_all(unsigned long long* buf) {
   int r;
   if ((r = trace_attach_conv_fwd(buf)) || (r = trace_attach_conv_bwd_fused(buf)) || (r = trace_attach_dense_tc(buf)) ||
-      (r = trace_attach_heads(buf)) || (r = trace_attach_elementwise(buf)) || (r = trace_attach_mlp(buf)) || (r = trace_attach_mlp_tc(buf)) || (r = trace_attach_mlp_stream(buf)))
+      (r = trace_attach_heads(buf)) || (r = trace_attach_elementwise(buf)) || (r = trace_attach_conv_gen(buf)) || (r = trace_attach_mlp(buf)) || (r = trace_attach_mlp_tc(buf)) || (r = trace_attach_mlp_stream(buf)))
     return r;
   return 0;
 }

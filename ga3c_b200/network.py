@@ -30,6 +30,18 @@ from .config import Config as _DefaultConfig
 STATE_DIM = 84 * 84 * 4
 
 
+def geometry(cfg):
+    """(IMAGE_HEIGHT, IMAGE_WIDTH, STACKED_FRAMES) of a Config, 84 / 84 / 4 where it has no such attribute (Config.py:90-92).
+    Raises ValueError naming the knob outside 1..256 / 1..256 / 1..8."""
+    out = []
+    for knob, default, hi in (("IMAGE_HEIGHT", 84, 256), ("IMAGE_WIDTH", 84, 256), ("STACKED_FRAMES", 4, 8)):
+        v = int(getattr(cfg, knob, default))
+        if not 1 <= v <= hi:
+            raise ValueError(f"Config.{knob} must be 1..{hi}, got {v}")
+        out.append(v)
+    return tuple(out)
+
+
 class _DevArray:
     """Exposes a raw device allocation owned by the C library through __cuda_array_interface__."""
 
@@ -60,9 +72,10 @@ class _TrainSlot:
     slot, on that slot's own stream, while call k's kernels run and its caller waits for them -- PCIe never idles between
     steps.  Slot = trainer_id % 2; a slot is used by one call at a time (its lock)."""
 
-    def __init__(self, tdev):
+    def __init__(self, tdev, state_dim):
         self.lock = threading.Lock()
         self.tdev = tdev
+        self.state_dim = state_dim
         self.rows = 0
         self.rows8 = 0
         with torch.cuda.device(tdev):
@@ -76,25 +89,31 @@ class _TrainSlot:
                 self.ha = torch.empty((rows, num_actions), dtype=torch.float32, pin_memory=True)
                 self.dyr = torch.empty((rows,), dtype=torch.float32, device=self.tdev)
                 self.da = torch.empty((rows, num_actions), dtype=torch.float32, device=self.tdev)
-                self.hx = torch.empty((rows, STATE_DIM), dtype=torch.float32, pin_memory=True)
-                self.dx = torch.empty((rows, STATE_DIM), dtype=torch.float32, device=self.tdev)
+                self.hx = torch.empty((rows, self.state_dim), dtype=torch.float32, pin_memory=True)
+                self.dx = torch.empty((rows, self.state_dim), dtype=torch.float32, device=self.tdev)
                 self.rows = rows
             if u8 and rows > self.rows8:
-                self.hx8 = torch.empty((rows, STATE_DIM), dtype=torch.uint8, pin_memory=True)
-                self.dx8 = torch.empty((rows, STATE_DIM), dtype=torch.uint8, device=self.tdev)
+                self.hx8 = torch.empty((rows, self.state_dim), dtype=torch.uint8, pin_memory=True)
+                self.dx8 = torch.empty((rows, self.state_dim), dtype=torch.uint8, device=self.tdev)
                 self.rows8 = rows
         return (self.hx8, self.dx8) if u8 else (self.hx, self.dx)
 
 
 class Network(ArenaNetworkMixin):
-    def __init__(self, device, model_name, num_actions, state_dim=STATE_DIM, *, config=None, max_batch=None,
+    def __init__(self, device, model_name, num_actions, state_dim=None, *, config=None, max_batch=None,
                  seed=None, data_parallel=None, dp_mode=None):
+        """state_dim (default: the Config's H*W*C) must equal IMAGE_HEIGHT * IMAGE_WIDTH * STACKED_FRAMES of `config`."""
         cfg = config or _DefaultConfig
+        if state_dim is None:
+            state_dim = int(np.prod(geometry(cfg)))
         sd = int(np.prod(state_dim)) if not isinstance(state_dim, int) else state_dim
-        if sd != STATE_DIM:
-            raise ValueError(f"conv NetworkVP expects state_dim = 84*84*4 = {STATE_DIM}, got {sd}")
+        h, w, nc = self.geometry = geometry(cfg)
+        if sd != h * w * nc:
+            raise ValueError(f"conv NetworkVP expects state_dim = IMAGE_HEIGHT*IMAGE_WIDTH*STACKED_FRAMES = {h}*{w}*{nc} = "
+                             f"{h * w * nc}, got {sd}")
         fields = self._setup(device, model_name, num_actions, sd, cfg, max_batch)
-        c = _capi.ga3c_config(device=self._ordinal, num_actions=self.num_actions, max_batch=self._max_batch, **fields)
+        c = _capi.ga3c_config(device=self._ordinal, num_actions=self.num_actions, max_batch=self._max_batch,
+                              image_height=h, image_width=w, stacked_frames=nc, **fields)
         h = C.c_void_p()
         _capi.check(self._lib.ga3c_create(C.byref(c), C.byref(h)), "ga3c_create")
         self._h = h
@@ -117,11 +136,12 @@ class Network(ArenaNetworkMixin):
             self._stream = torch.cuda.Stream(device=self._tdev)
             self._loss_dev = torch.zeros(4, dtype=torch.float32, device=self._tdev)
         self._alloc_io(self._max_batch)
-        self._train_slots = [_TrainSlot(self._tdev) for _ in range(2)]     # staging per trainer thread, allocated on first use
+        self._train_slots = [_TrainSlot(self._tdev, self.state_dim) for _ in range(2)]     # staging per trainer thread, allocated on first use
 
         # variable init: U(-d, d), d = 1/sqrt(fan_in)  (NetworkVP.py:214-217, NetworkDNav.py:258-261)
         rng = np.random.default_rng(seed)
-        fan_in = {"conv11": 8 * 8 * 4, "conv12": 4 * 4 * 16, "dense1": 3872, "logits_v": 256, "logits_p": 256}
+        fan_in = {"conv11": 8 * 8 * self.geometry[2], "conv12": 4 * 4 * 16, "dense1": self._table["dense1/w:0"][1][0],
+                  "logits_v": 256, "logits_p": 256}
         init = {}
         for name, (_, shape) in self._table.items():
             d = 1.0 / np.sqrt(fan_in[name.split("/")[0]])
@@ -143,9 +163,9 @@ class Network(ArenaNetworkMixin):
             self.dp_mode = dp_mode or os.environ.get("GA3C_DP", "fused")
             if self.dp_mode not in ("fused", "nccl"):
                 raise ValueError(f"dp_mode must be 'fused' or 'nccl', got {self.dp_mode!r}")
-        if self.dp_mode == "fused" and (getattr(cfg, "USE_GRAD_CLIP", False) or self._dual):
+        if self.dp_mode == "fused" and (getattr(cfg, "USE_GRAD_CLIP", False) or self._dual or self.geometry != (84, 84, 4)):
             # the per-variable norms need the whole reduced gradient, and DUAL_RMSPROP has two gradient arenas: allreduce
-            # first (NCCL), then clip / update locally
+            # first (NCCL), then clip / update locally; the peer-memory exchange is built around the 84x84x4 arena
             self.dp_mode = "nccl"
         if self._allreduce.enabled and self._dual:
             g2 = C.c_void_p()
@@ -177,8 +197,8 @@ class Network(ArenaNetworkMixin):
     def _io_u8(self):
         if self._hx8 is None or self._hx8.shape[0] < self._io_rows:
             with torch.cuda.device(self._tdev):
-                self._hx8 = torch.empty((self._io_rows, STATE_DIM), dtype=torch.uint8, pin_memory=True)
-                self._dx8 = torch.empty((self._io_rows, STATE_DIM), dtype=torch.uint8, device=self._tdev)
+                self._hx8 = torch.empty((self._io_rows, self.state_dim), dtype=torch.uint8, pin_memory=True)
+                self._dx8 = torch.empty((self._io_rows, self.state_dim), dtype=torch.uint8, device=self._tdev)
         return self._hx8, self._dx8
 
     @staticmethod
@@ -498,7 +518,8 @@ class Network(ArenaNetworkMixin):
         """Activation workspace of the last call as float32 numpy (bf16 buffers are widened), flat in the LOGICAL order of the
         reference tensors: n1 (0) and dn2 (4) live in HBM in the tcgen05 operand layouts the conv backward consumes
         (include/ga3c_b200.h, ga3c_workspace_ptr) and are unscrambled here to [B, 21*21*16] / [B, 11*11*32]; 7 = the bf16 copy of
-        the frames, unscrambled to the padded image [B, 88, 88, 4]."""
+        the frames, unscrambled to the padded image [B, 88, 88, 4].  Any other geometry than 84x84x4 keeps them row-major: n1 and
+        dn1 [B, H1*W1*16], n2 and dn2 [B, H2*W2*32], 7 the im2col matrix of the frames [B*H1*W1, 64C + 8]."""
         ptr, nbytes = C.c_void_p(), C.c_int64()
         _capi.check(self._lib.ga3c_workspace_ptr(self._h, which, C.byref(ptr), C.byref(nbytes)), "ga3c_workspace_ptr")
         torch.cuda.synchronize(self._tdev)
@@ -509,6 +530,8 @@ class Network(ArenaNetworkMixin):
         holder = type("H", (), {"__cuda_array_interface__": iface})()
         t = torch.as_tensor(holder, device=self._tdev).view(torch.bfloat16)
         flat = t.float().cpu().numpy().copy()
+        if self.geometry != (84, 84, 4):
+            return flat
         if which == 0:            # Blk2: [B][plane = ((Y&1)*2 + (X&1))*2 + h][row = (Y>>1)*13 + (X>>1)][8], Y = y + 1, X = x + 1
             raw = flat.reshape(-1, 8, 160, 8)
             y, x, h = np.meshgrid(np.arange(21), np.arange(21), np.arange(2), indexing="ij")

@@ -56,9 +56,19 @@ typedef struct ga3c_config {
                               * both steps are subtracted; global_step advances by 2.  With USE_GRAD_CLIP each optimizer's
                               * gradients go through tf.clip_by_norm per variable and global_step stays put
                               * (NetworkVP_discrate.py:107-117).  Data parallel: dp_mode 'nccl' only (two allreduces).       */
+  /* Input geometry (ABI 10), appended so that a caller that zero-fills the struct keeps 84 x 84 x 4.  0 = the default.
+   * Frames are NHWC [B, H, W, C] flattened, H * W * C floats (or bytes, _u8) per row.  84 x 84 x 4 runs the specialised
+   * trunk; every other geometry a generic one (im2col + tcgen05 GEMMs, same layers, same bf16 rounding points), whose
+   * activations lie row-major in the workspace (ga3c_workspace_ptr).  Derived sizes (TF SAME): H1 = ceil(H/4), W1 = ceil(W/4),
+   * H2 = ceil(H1/2), W2 = ceil(W1/2); dense1/w is [K = H2 * W2 * 32, 256] and conv11/w [8, 8, C, 16] (ga3c_param_info).
+   * Generic handles cannot attach the peer-memory exchange (ga3c_dp_attach fails; dp_mode 'nccl' works). */
+  int32_t image_height;      /* Config.IMAGE_HEIGHT     (84): 1..256                          */
+  int32_t image_width;       /* Config.IMAGE_WIDTH      (84): 1..256                          */
+  int32_t stacked_frames;    /* Config.STACKED_FRAMES   (4):  1..8                            */
 } ga3c_config;
 
 const char* ga3c_last_error(void);
+/* 10: ga3c_config gained image_height, image_width, stacked_frames (input geometry) */
 int ga3c_abi_version(void);
 
 int ga3c_create(const ga3c_config* cfg, ga3c_net** out);
@@ -307,7 +317,11 @@ int ga3c_stage_h2d(void* dst_dev, void* staging, const void* src, int64_t bytes,
  *        3 dd1 [B,256] bf16, 4 dn2 bf16 in the G operand layout [B][4 planes][172 rows][8] (channels 8j.. of position (oy, ox) in
  *          plane j, row (oy+1)*13 + ox+1; zero borders), 5 dn1 [B,441,16] bf16 (only with ga3c_keep_dn1), 7 xblk: the bf16
  *          block matrix of the frames [B][4 quarters][8 planes][128 rows][8] that the conv backward reads instead of x, 6 the bf16 shadow of dense1/w [3872,256] (what the dense1 GEMMs read; in a
- *        data-parallel job the copy every rank holds, so comparing it across ranks checks the exchange) */
+ *        data-parallel job the copy every rank holds, so comparing it across ranks checks the exchange).
+ * A handle of any other geometry than 84x84x4 (the generic trunk) keeps its activations row-major: 0 n1 [B,H1,W1,16] bf16,
+ * 1 n2 [B,K] bf16, 4 dn2 [B,K] bf16, 5 dn1 [B,H1,W1,16] bf16 (always stored), 7 X1 [B*H1*W1][64C + 8] bf16, the im2col
+ * matrix of the frames (columns (kh, kw, c), then a column of ones and 7 zero columns), which the backward reads instead of x;
+ * 2, 3 and 6 as above with K = H2*W2*32 for 3872. */
 int ga3c_workspace_ptr(ga3c_net* net, int which, void** ptr_dev, int64_t* bytes);
 /* dn1 (the conv12 data gradient) normally never leaves the SM: the fused conv backward kernel consumes it from shared
  * memory.  on != 0 makes that kernel also store it to the workspace (id 5 above) so that tests can compare it. */
