@@ -19,6 +19,9 @@ Three arithmetic modes:
   quant='bf16'                   -- operands rounded to bfloat16 at exactly the points where
                                     the CUDA path rounds them (see DESIGN.md "Rounding points");
                                     accumulation stays in `dtype`.
+
+The input geometry (Config.IMAGE_HEIGHT, IMAGE_WIDTH, STACKED_FRAMES) is the keyword `geom=`, a Geometry; None means
+the reference's 84x84x4, whose sizes are also the module constants below.
 """
 from __future__ import annotations
 
@@ -54,31 +57,66 @@ H2, P2_LO, P2_HI = same_pad(H1, C2_K, C2_S)   # 11, 1, 2
 FLAT = H2 * H2 * C2_OUT                       # 3872
 
 
-def param_shapes(num_actions: int):
+class Geometry:
+    """Derived sizes of an h x w x c input under TF SAME padding (SURVEY A.1): conv11's output h1 x w1 with top / left pads
+    pt1 / pl1, conv12's h2 x w2 with pt2 / pl2, and dense1's fan-in flat = h2 * w2 * 32."""
+
+    def __init__(self, h: int, w: int, c: int):
+        self.h, self.w, self.c = h, w, c
+        self.h1, self.pt1, _ = same_pad(h, C1_K, C1_S)
+        self.w1, self.pl1, _ = same_pad(w, C1_K, C1_S)
+        self.h2, self.pt2, _ = same_pad(self.h1, C2_K, C2_S)
+        self.w2, self.pl2, _ = same_pad(self.w1, C2_K, C2_S)
+        self.state_dim = h * w * c
+        self.flat = self.h2 * self.w2 * C2_OUT
+
+    def __repr__(self):
+        return f"{self.h}x{self.w}x{self.c}"
+
+
+DEFAULT_GEOMETRY = Geometry(H, W, C)
+
+
+def _geom(geom):
+    return DEFAULT_GEOMETRY if geom is None else geom
+
+
+def param_shapes(num_actions: int, *, geom=None):
+    g = _geom(geom)
     return {
-        "conv11/w:0": (C1_K, C1_K, C, C1_OUT), "conv11/b:0": (C1_OUT,),
+        "conv11/w:0": (C1_K, C1_K, g.c, C1_OUT), "conv11/b:0": (C1_OUT,),
         "conv12/w:0": (C2_K, C2_K, C1_OUT, C2_OUT), "conv12/b:0": (C2_OUT,),
-        "dense1/w:0": (FLAT, FC), "dense1/b:0": (FC,),
+        "dense1/w:0": (g.flat, FC), "dense1/b:0": (FC,),
         "logits_v/w:0": (FC, 1), "logits_v/b:0": (1,),
         "logits_p/w:0": (FC, num_actions), "logits_p/b:0": (num_actions,),
     }
 
 
-def init_params(rng: np.random.Generator, num_actions: int = 6):
+def init_params(rng: np.random.Generator, num_actions: int = 6, *, geom=None):
     """U(-d, d) with d = 1/sqrt(fan_in): NetworkVP.py:214-217 (conv), NetworkDNav.py:258-261 (dense)."""
-    fan_in = {"conv11": C1_K * C1_K * C, "conv12": C2_K * C2_K * C1_OUT, "dense1": FLAT,
+    g = _geom(geom)
+    fan_in = {"conv11": C1_K * C1_K * g.c, "conv12": C2_K * C2_K * C1_OUT, "dense1": g.flat,
               "logits_v": FC, "logits_p": FC}
     out = {}
-    for name, shp in param_shapes(num_actions).items():
+    for name, shp in param_shapes(num_actions, geom=g).items():
         d = 1.0 / np.sqrt(fan_in[name.split("/")[0]])
         out[name] = rng.uniform(-d, d, size=shp).astype(np.float32)
     return out
 
 
-def synth_frames(rng: np.random.Generator, batch: int):
-    """Frames exactly as Environment.py:57-61 produces them: uint8 k -> k/128 - 1 (float32)."""
-    k = rng.integers(0, 256, size=(batch, STATE_DIM), dtype=np.int64)
+def normalise(k):
+    """Environment.py:57-61: uint8 k -> k/128 - 1 (float32)."""
     return (k.astype(np.float32) / np.float32(128.0) - np.float32(1.0)).astype(np.float32)
+
+
+def synth_frames(rng: np.random.Generator, batch: int, *, geom=None):
+    """Frames exactly as Environment.py produces them, drawn as int64."""
+    return normalise(rng.integers(0, 256, size=(batch, _geom(geom).state_dim), dtype=np.int64))
+
+
+def synth_frames_u8(rng: np.random.Generator, batch: int, *, geom=None):
+    """The uint8 frames themselves (a different draw from synth_frames'); normalise() gives their float32 form."""
+    return rng.integers(0, 256, size=(batch, _geom(geom).state_dim), dtype=np.uint8)
 
 
 def synth_targets(rng: np.random.Generator, batch: int, num_actions: int = 6):
@@ -108,42 +146,49 @@ def _q(x, quant, dtype):
 # --------------------------------------------------------------------------------------
 # conv as im2col (cross-correlation, NHWC x HWIO, SAME) -- NetworkVP.py:224
 # --------------------------------------------------------------------------------------
-def _im2col(x, k, s, lo, hi, n_out):
+def _im2col(x, k, s):
+    """x [B, H, W, C] -> [B*OH*OW, k*k*C] for a k x k / stride s conv with SAME zero padding."""
     b, h, w, c = x.shape
-    xp = np.zeros((b, h + lo + hi, w + lo + hi, c), dtype=x.dtype)
-    xp[:, lo:lo + h, lo:lo + w, :] = x
+    oh, t, bo = same_pad(h, k, s)
+    ow, l, r = same_pad(w, k, s)
+    xp = np.zeros((b, h + t + bo, w + l + r, c), dtype=x.dtype)
+    xp[:, t:t + h, l:l + w, :] = x
     sb, sh, sw, sc = xp.strides
     cols = np.lib.stride_tricks.as_strided(
-        xp, shape=(b, n_out, n_out, k, k, c), strides=(sb, sh * s, sw * s, sh, sw, sc), writeable=False)
-    return cols.reshape(b * n_out * n_out, k * k * c)     # K order (kh, kw, cin)
+        xp, shape=(b, oh, ow, k, k, c), strides=(sb, sh * s, sw * s, sh, sw, sc), writeable=False)
+    return cols.reshape(b * oh * ow, k * k * c)     # K order (kh, kw, cin)
 
 
 def _col2im(dcols, b, h, k, s, lo, hi, n_out, c):
-    dxp = np.zeros((b, h + lo + hi, h + lo + hi, c), dtype=dcols.dtype)
-    d6 = dcols.reshape(b, n_out, n_out, k, k, c)
+    """The adjoint of _im2col: dcols [B*OH*OW, k*k*c] summed back onto the unpadded [B, H, W, c] input.  The input size h,
+    the SAME pads lo / hi and the output size n_out are one int each for a square input, else (vertical, horizontal) pairs."""
+    (h, w), (t, l), (bo, r), (oh, ow) = (np.broadcast_to(v, 2) for v in (h, lo, hi, n_out))
+    dxp = np.zeros((b, h + t + bo, w + l + r, c), dtype=dcols.dtype)
+    d6 = dcols.reshape(b, oh, ow, k, k, c)
     for kh in range(k):
         for kw in range(k):
-            dxp[:, kh:kh + s * n_out:s, kw:kw + s * n_out:s, :] += d6[:, :, :, kh, kw, :]
-    return dxp[:, lo:lo + h, lo:lo + h, :]
+            dxp[:, kh:kh + s * oh:s, kw:kw + s * ow:s, :] += d6[:, :, :, kh, kw, :]
+    return dxp[:, t:t + h, l:l + w, :]
 
 
 # --------------------------------------------------------------------------------------
 # forward
 # --------------------------------------------------------------------------------------
-def forward(params, x, *, dtype=np.float64, quant=None, min_policy=0.0, keep=False, use_log_softmax=False):
-    """A2/A3/A4 forward.  x: [B, 28224] (flat NHWC).  Returns (p [B,A], v [B]) or a cache dict."""
+def forward(params, x, *, geom=None, dtype=np.float64, quant=None, min_policy=0.0, keep=False, use_log_softmax=False):
+    """A2/A3/A4 forward.  x: [B, H*W*C] (flat NHWC).  Returns (p [B,A], v [B]) or a cache dict."""
+    g = _geom(geom)
     b = x.shape[0]
-    xq = _q(x.reshape(b, H, W, C), quant, dtype)
+    xq = _q(x.reshape(b, g.h, g.w, g.c), quant, dtype)
     w11 = _q(params["conv11/w:0"], quant, dtype).reshape(-1, C1_OUT)
     w12 = _q(params["conv12/w:0"], quant, dtype).reshape(-1, C2_OUT)
     w1 = _q(params["dense1/w:0"], quant, dtype)
-    col1 = _im2col(xq, C1_K, C1_S, P1_LO, P1_HI, H1)
+    col1 = _im2col(xq, C1_K, C1_S)
     n1 = np.maximum(col1 @ w11 + params["conv11/b:0"].astype(dtype), 0)
-    n1 = _q(n1, quant, dtype).reshape(b, H1, H1, C1_OUT)
-    col2 = _im2col(n1, C2_K, C2_S, P2_LO, P2_HI, H2)
+    n1 = _q(n1, quant, dtype).reshape(b, g.h1, g.w1, C1_OUT)
+    col2 = _im2col(n1, C2_K, C2_S)
     n2 = np.maximum(col2 @ w12 + params["conv12/b:0"].astype(dtype), 0)
     n2 = _q(n2, quant, dtype)
-    flat = n2.reshape(b, FLAT)                                # (h, w, c) order, NetworkDNav.py:86-89
+    flat = n2.reshape(b, g.flat)                              # (h, w, c) order, NetworkDNav.py:86-89
     d1 = np.maximum(flat @ w1 + params["dense1/b:0"].astype(dtype), 0)   # stays in `dtype`
     v = (d1 @ params["logits_v/w:0"].astype(dtype) + params["logits_v/b:0"].astype(dtype))[:, 0]
     z = d1 @ params["logits_p/w:0"].astype(dtype) + params["logits_p/b:0"].astype(dtype)
@@ -151,9 +196,10 @@ def forward(params, x, *, dtype=np.float64, quant=None, min_policy=0.0, keep=Fal
     e = np.exp(zs)
     s = e / e.sum(axis=1, keepdims=True)
     a_n = z.shape[1]
-    p = (s + dtype(min_policy)) / (dtype(1.0) + dtype(min_policy) * a_n)  # NetworkVP_discrate.py:73-74
     if use_log_softmax:
         p = s                                                              # NetworkVP_discrate.py:65 (no MIN_POLICY mix)
+    else:
+        p = (s + dtype(min_policy)) / (dtype(1.0) + dtype(min_policy) * a_n)  # NetworkVP_discrate.py:73-74
     if not keep:
         return p, v
     return dict(x=xq, col1=col1, n1=n1, col2=col2, n2=n2, flat=flat, d1=d1, v=v, z=z, s=s, p=p, lsm=zs - np.log(e.sum(axis=1, keepdims=True)),
@@ -188,11 +234,13 @@ def losses_from_log_softmax(lsm, s, v, y_r, a, beta, v_stop=None):
     return dict(cost_p_1=cost_p_1_agg, cost_p_2=cost_p_2_agg, cost_p=cost_p, cost_v=cost_v, cost_all=cost_p + cost_v)
 
 
-def loss_and_grads(params, x, y_r, a, *, beta=0.01, log_eps=1e-6, min_policy=0.0,
-                   dtype=np.float64, quant=None, keep=False, use_log_softmax=False, part="all"):
+def loss_and_grads(params, x, y_r, a, *, geom=None, beta=0.01, log_eps=1e-6, min_policy=0.0,
+                   dtype=np.float64, quant=None, keep=False, use_log_softmax=False, part="all", v_stop=None):
     """A5 minus the optimizer: returns (losses dict, grads dict keyed like params); with keep=True
-    also the forward cache extended by the backward intermediates dd1 / dn2 / dn1 / dz / dv."""
-    f = forward(params, x, dtype=dtype, quant=quant, min_policy=min_policy, keep=True, use_log_softmax=use_log_softmax)
+    also the forward cache extended by the backward intermediates dd1 / dn2 / dn1 / dz / dv.
+    `v_stop` (finite-difference tests only) freezes the value inside the advantage, as in losses_from_heads."""
+    g = _geom(geom)
+    f = forward(params, x, geom=g, dtype=dtype, quant=quant, min_policy=min_policy, keep=True, use_log_softmax=use_log_softmax)
     b = x.shape[0]
     y_r = np.asarray(y_r, dtype=dtype)
     a = np.asarray(a, dtype=dtype)
@@ -200,21 +248,22 @@ def loss_and_grads(params, x, y_r, a, *, beta=0.01, log_eps=1e-6, min_policy=0.0
     log_eps = dtype(log_eps)
     p, v, s, d1 = f["p"], f["v"], f["s"], f["d1"]
     a_n = p.shape[1]
-    losses = losses_from_heads(p, v, y_r, a, beta, log_eps)
 
     # heads backward
-    sel = (p * a).sum(axis=1)
-    adv = y_r - v                                            # stop_gradient on v here
+    adv = y_r - (v if v_stop is None else v_stop)            # stop_gradient on v here
     dv = v - y_r                                             # from cost_v only
-    g = (-a * ((sel >= log_eps) * adv / np.where(sel >= log_eps, sel, 1))[:, None]
-         + beta * (np.log(np.maximum(p, log_eps)) + (p >= log_eps)))
-    h = g / (dtype(1.0) + dtype(min_policy) * a_n)
-    dz = s * (h - (s * h).sum(axis=1, keepdims=True))
     if use_log_softmax:
         # d/dz of -(sum_a lsm a) adv - (-beta sum lsm s):  -adv (a - s sum(a)) + beta s (lsm - sum(lsm s))
         lsm = f["lsm"]
-        losses = losses_from_log_softmax(lsm, s, v, y_r, a, beta)
+        losses = losses_from_log_softmax(lsm, s, v, y_r, a, beta, v_stop=v_stop)
         dz = -adv[:, None] * (a - s * a.sum(axis=1, keepdims=True)) + beta * s * (lsm - (lsm * s).sum(axis=1, keepdims=True))
+    else:
+        losses = losses_from_heads(p, v, y_r, a, beta, log_eps, v_stop=v_stop)
+        sel = (p * a).sum(axis=1)
+        gz = (-a * ((sel >= log_eps) * adv / np.where(sel >= log_eps, sel, 1))[:, None]
+              + beta * (np.log(np.maximum(p, log_eps)) + (p >= log_eps)))
+        h = gz / (dtype(1.0) + dtype(min_policy) * a_n)
+        dz = s * (h - (s * h).sum(axis=1, keepdims=True))
     # Config.DUAL_RMSPROP minimises cost_p and cost_v separately (NetworkVP_discrate.py:87-98, :124-128): part = "p" is the
     # gradient of cost_p alone (nothing reaches logits_v: stop_gradient), part = "v" that of cost_v alone (nothing reaches logits_p)
     if part == "p":
@@ -234,13 +283,13 @@ def loss_and_grads(params, x, y_r, a, *, beta=0.01, log_eps=1e-6, min_policy=0.0
     grads["dense1/w:0"] = f["flat"].T @ dd1
     grads["dense1/b:0"] = dd1.sum(axis=0)
     dflat = (dd1 @ f["w1"].T) * (f["flat"] > 0)
-    dn2 = _q(dflat, quant, dtype).reshape(b * H2 * H2, C2_OUT)
-    grads["conv12/w:0"] = (f["col2"].T @ dn2).reshape(C2_K, C2_K, C1_OUT, C2_OUT)
+    dn2 = _q(dflat, quant, dtype).reshape(-1, C2_OUT)
+    grads["conv12/w:0"] = f["col2"].T @ dn2
     grads["conv12/b:0"] = dn2.sum(axis=0)
-    dcol2 = dn2 @ f["w12"].T
-    dn1 = _col2im(dcol2, b, H1, C2_K, C2_S, P2_LO, P2_HI, H2, C1_OUT) * (f["n1"] > 0)
-    dn1 = _q(dn1, quant, dtype).reshape(b * H1 * H1, C1_OUT)
-    grads["conv11/w:0"] = (f["col1"].T @ dn1).reshape(C1_K, C1_K, C, C1_OUT)
+    n_out, lo, hi = zip(same_pad(g.h1, C2_K, C2_S), same_pad(g.w1, C2_K, C2_S))
+    dn1 = _col2im(dn2 @ f["w12"].T, b, (g.h1, g.w1), C2_K, C2_S, lo, hi, n_out, C1_OUT) * (f["n1"] > 0)
+    dn1 = _q(dn1, quant, dtype).reshape(-1, C1_OUT)
+    grads["conv11/w:0"] = f["col1"].T @ dn1
     grads["conv11/b:0"] = dn1.sum(axis=0)
     for k in grads:
         grads[k] = grads[k].reshape(params[k].shape)
@@ -248,7 +297,7 @@ def loss_and_grads(params, x, y_r, a, *, beta=0.01, log_eps=1e-6, min_policy=0.0
         for k in (("logits_v/w:0", "logits_v/b:0") if part == "p" else ("logits_p/w:0", "logits_p/b:0")):
             del grads[k]
     if keep:
-        f.update(dd1=dd1, dn2=dn2.reshape(b, FLAT), dn1=dn1.reshape(b, H1 * H1 * C1_OUT), dz=dz, dv=dv)
+        f.update(dd1=dd1, dn2=dn2.reshape(b, -1), dn1=dn1.reshape(b, -1), dz=dz, dv=dv)
         return losses, grads, f
     return losses, grads
 

@@ -1,11 +1,41 @@
 """Shared helpers of the GPU parity tests: run the CUDA path and the oracle on the same seeded
-inputs and report per-tensor error figures.  The oracle is the checker, never the thing measured."""
+inputs and report per-tensor error figures.  The oracle is the checker, never the thing measured.
+
+Tolerances of the conv network (SURVEY A.8, calibrated on B200 and frozen here).  The CUDA path rounds
+operands to bf16 at fixed points (x, conv weights, n1, n2, w1, dd1, dn2, dn1) and accumulates in fp32;
+the oracle is run in its `quant='bf16'` mode, which rounds at the same points and accumulates in fp64.
+Residual differences are fp32-vs-fp64 accumulation order, which now and then flips a bf16 rounding
+(1 ulp = 2^-8 relative) of a stored activation:
+    p        |d| <= 2e-5          v        |d| <= 2e-4
+    stored bf16 activations      |d| <= 2^-7 * max|ref|  and  <= 1% of elements off by > 1e-5 * max|ref|
+    loss sums                    rel <= 1e-4
+    gradients                    |d| <= 2e-3 * max|ref| per tensor
+    weights after RMSProp        |d| <= 2e-6   (lr 3e-4 scales the gradient error)
+Against the un-quantised fp64 oracle (the irreducible bf16 gap): |dp| <= 1e-2, |dv| <= 2e-2.
+"""
 from __future__ import annotations
 
 import numpy as np
+import pytest
 
 from oracle import oracle_mlp as om
 from oracle import oracle_np as onp
+
+TOL_P, TOL_V = 2e-5, 2e-4
+TOL_ACT_REL = 2.0 ** -7
+TOL_LOSS_REL = 1e-4
+TOL_GRAD_REL = 2e-3
+TOL_W_ABS = 2e-6
+
+
+@pytest.fixture(scope="module")
+def ga3c():
+    """The package, for a test module that imports this fixture; fails (never skips) without a CUDA device."""
+    import torch
+    if not torch.cuda.is_available():
+        pytest.fail("GPU tests need a CUDA device; there is no CPU fallback")
+    import ga3c_b200
+    return ga3c_b200
 
 
 def make_case(batch: int, num_actions: int = 6, seed: int = 12345):
@@ -67,15 +97,16 @@ def err(got, ref):
     return d, d / max(s, 1e-30)
 
 
-def layer_report(net, params, x, y_r, a, *, beta=0.01, log_eps=1e-6, min_policy=0.0, use_log_softmax=False):
-    """Runs predict + forward_backward on `net` (weights := params) and compares every stored
-    activation, every gradient and the loss sums with the bf16-rounding-point oracle (fp64 accumulate).
-    Returns {name: (abs_err, rel_err)}."""
+def layer_report(net, params, x, y_r, a, *, geom=None, beta=0.01, log_eps=1e-6, min_policy=0.0, use_log_softmax=False):
+    """Runs predict + forward_backward on the conv `net` (weights := params) and compares every stored
+    activation, every gradient and the loss sums with the bf16-rounding-point oracle (fp64 accumulate) at
+    input geometry `geom` (None: 84x84x4).  Returns {name: (abs_err, rel_err)}."""
+    g = onp.DEFAULT_GEOMETRY if geom is None else geom
     net.set_variables(params)
     net.beta = beta
     rep = {}
     p, v = net.predict_p_and_v(x)
-    losses_ref, grads_ref, f = onp.loss_and_grads(params, x, y_r, a, beta=beta, log_eps=log_eps,
+    losses_ref, grads_ref, f = onp.loss_and_grads(params, x, y_r, a, geom=g, beta=beta, log_eps=log_eps,
                                                   min_policy=min_policy, quant="bf16", keep=True,
                                                   use_log_softmax=use_log_softmax)
     rep["p"] = err(p, f["p"])
@@ -84,33 +115,52 @@ def layer_report(net, params, x, y_r, a, *, beta=0.01, log_eps=1e-6, min_policy=
     losses = net.losses(x, y_r, a)
     net.keep_dn1(False)
     b = x.shape[0]
-    rep["n1"] = err(net.workspace(0), f["n1"].reshape(b, -1))
-    rep["n2"] = err(net.workspace(1), f["n2"].reshape(b, -1))
-    rep["d1"] = err(net.workspace(2), f["d1"])
-    rep["dd1"] = err(net.workspace(3), f["dd1"])
-    rep["dn2"] = err(net.workspace(4), f["dn2"])
-    rep["dn1"] = err(net.workspace(5), f["dn1"])
+    ws = [net.workspace(i) for i in range(6)]
+    rep["n1"] = err(ws[0], f["n1"].reshape(b, -1))
+    rep["n2"] = err(ws[1], f["n2"].reshape(b, -1))
+    rep["d1"] = err(ws[2], f["d1"])
+    rep["dd1"] = err(ws[3], f["dd1"])
+    rep["dn2"] = err(ws[4], f["dn2"])
+    rep["dn1"] = err(ws[5], f["dn1"])
     # Layer-local view of the two masked data gradients: the same oracle arithmetic applied to the CUDA path's OWN stored inputs
     # (dd1 / dn2 and the activation masks).  A stored activation that sits within an fp32-vs-fp64 accumulation difference of
     # the ReLU boundary flips its mask bit; the global comparison above then shows that element's whole gradient (and what
     # it spreads to upstream) as an error although every kernel did its arithmetic right.  At full-size batches (millions of
     # activations) a handful of such flips is certain; the local view is immune, and `outliers` says how few elements differ.
-    w12q = f["w12"]
-    n1_mask = (net.workspace(0).reshape(b, -1) > 0)
-    n2_mask = (net.workspace(1).reshape(b, -1) > 0)
-    dn2_cuda = net.workspace(4).astype(np.float64).reshape(b * onp.H2 * onp.H2, onp.C2_OUT)
-    dd1_cuda = net.workspace(3).astype(np.float64).reshape(b, -1)
+    n1_mask = ws[0].reshape(b, -1) > 0
+    n2_mask = ws[1].reshape(b, -1) > 0
+    dn2_cuda = ws[4].astype(np.float64).reshape(-1, onp.C2_OUT)
+    dd1_cuda = ws[3].astype(np.float64).reshape(b, -1)
     dn2_local = onp.bf16_round((dd1_cuda @ f["w1"].T) * n2_mask)
-    dn1_local = onp._col2im(dn2_cuda @ w12q.T, b, onp.H1, onp.C2_K, onp.C2_S, onp.P2_LO, onp.P2_HI, onp.H2, onp.C1_OUT)
+    n_out, lo, hi = zip(onp.same_pad(g.h1, onp.C2_K, onp.C2_S), onp.same_pad(g.w1, onp.C2_K, onp.C2_S))
+    dn1_local = onp._col2im(dn2_cuda @ f["w12"].T, b, (g.h1, g.w1), onp.C2_K, onp.C2_S, lo, hi, n_out, onp.C1_OUT)
     dn1_local = onp.bf16_round(dn1_local.reshape(b, -1) * n1_mask)
-    rep["dn2_local"] = err(net.workspace(4), dn2_local)
-    rep["dn1_local"] = err(net.workspace(5), dn1_local)
-    for k in ("dn1", "dn2"):
-        got, ref = net.workspace(5 if k == "dn1" else 4).ravel(), np.asarray(f[k], dtype=np.float64).ravel()
-        rep[k + "_outliers"] = (float((np.abs(got - ref) > 2.0 ** -7 * np.abs(ref).max()).mean()), 0.0)
+    rep["dn2_local"] = err(ws[4], dn2_local)
+    rep["dn1_local"] = err(ws[5], dn1_local)
+    for k, got in (("dn1", ws[5]), ("dn2", ws[4])):
+        ref = np.asarray(f[k], dtype=np.float64).ravel()
+        rep[k + "_outliers"] = (float((np.abs(got.ravel() - ref) > 2.0 ** -7 * np.abs(ref).max()).mean()), 0.0)
     for k in ("cost_p_1", "cost_p_2", "cost_v", "cost_all"):
         rep["loss/" + k] = err([losses[k]], [losses_ref[k]])
     grads = net.get_gradients()
     for k in grads_ref:
         rep["grad/" + k] = err(grads[k], grads_ref[k])
     return rep
+
+
+def check_report(rep):
+    """layer_report's figures against the tolerances above."""
+    assert rep["p"][0] <= TOL_P and rep["v"][0] <= TOL_V, rep
+    for k in ("n1", "n2", "dd1"):
+        assert rep[k][1] <= TOL_ACT_REL, (k, rep[k])
+    for k in ("dn2", "dn1"):
+        # masked data gradients: exact against the oracle fed the same stored inputs; against the end-to-end oracle either
+        # within tolerance everywhere, or off only at the rare elements behind a ReLU-boundary flip (layer_report)
+        assert rep[k + "_local"][1] <= TOL_ACT_REL, (k, rep[k + "_local"])
+        assert rep[k][1] <= TOL_ACT_REL or rep[k + "_outliers"][0] <= 1e-4, (k, rep[k], rep[k + "_outliers"])
+    assert rep["d1"][1] <= 1e-3, rep["d1"]
+    for k, (d, r) in rep.items():
+        if k.startswith("loss/"):
+            assert r <= TOL_LOSS_REL or d <= 1e-5, (k, d, r)
+        if k.startswith("grad/"):
+            assert r <= TOL_GRAD_REL, (k, d, r)

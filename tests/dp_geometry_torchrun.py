@@ -18,7 +18,6 @@ dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 import ga3c_b200
 from ga3c_b200.dataparallel import shard_rows
 from oracle import oracle_np as onp        # checker only
-import _geometry_oracle as go              # checker only
 
 HWC = (42, 42, 4)
 
@@ -27,21 +26,22 @@ class Cfg(ga3c_b200.Config):
     IMAGE_HEIGHT, IMAGE_WIDTH, STACKED_FRAMES = HWC
 
 
-g = go.Geometry(*HWC)
+g = onp.Geometry(*HWC)
 B = 16 * world
 rng = np.random.default_rng(4242)
-params = go.init_params(rng, g, 6)
+params = onp.init_params(rng, 6, geom=g)
 net = ga3c_b200.Network(f"gpu:{local}", "dpgeo", 6, config=Cfg, max_batch=64)
 assert net.dp_mode == "nccl", net.dp_mode
 net.set_variables(params)
 ref = {k: v.astype(np.float64) for k, v in params.items()}
 ms, mom = onp.rmsprop_init(ref)
 for step in range(3):
-    x = go.normalise(go.synth_frames_u8(rng, g, B))
+    x = onp.normalise(onp.synth_frames_u8(rng, B, geom=g))
     y_r, a = onp.synth_targets(rng, B, 6)
     lo, hi = shard_rows(B, rank, world)
     net.train(x[lo:hi], y_r[lo:hi], a[lo:hi], None, None, 0)
-    _, grads = go.loss_and_grads(g, {k: v.astype(np.float32) for k, v in ref.items()}, x, y_r, a, quant="bf16", beta=net.beta)
+    _, grads = onp.loss_and_grads({k: v.astype(np.float32) for k, v in ref.items()}, x, y_r, a, geom=g, quant="bf16",
+                               beta=net.beta)
     ref, ms, mom = onp.rmsprop_update(ref, grads, ms, mom, lr=net.learning_rate, dtype=np.float64)
 got = net.get_variables()
 flat = torch.from_numpy(np.concatenate([got[k].ravel() for k in sorted(got)])).cuda()

@@ -1,5 +1,5 @@
-"""CPU checks of the input-geometry support (Config.IMAGE_HEIGHT, IMAGE_WIDTH, STACKED_FRAMES): the geometry-parameterised
-oracle (tests/_geometry_oracle.py) against finite differences, torch and oracle_np, and the C ABI's ga3c_config mirror."""
+"""CPU checks of the input-geometry support (Config.IMAGE_HEIGHT, IMAGE_WIDTH, STACKED_FRAMES): the oracle at non-default
+geometries against finite differences and torch, and the C ABI's ga3c_config mirror."""
 import ctypes as C
 import os
 import re
@@ -10,15 +10,14 @@ import numpy as np
 import pytest
 
 from oracle import oracle_np as onp
-import _geometry_oracle as go
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _case(g, b, seed=7, num_actions=5):
     rng = np.random.default_rng(seed)
-    params = go.init_params(rng, g, num_actions)
-    x = go.normalise(go.synth_frames_u8(rng, g, b))
+    params = onp.init_params(rng, num_actions, geom=g)
+    x = onp.normalise(onp.synth_frames_u8(rng, b, geom=g))
     y_r, a = onp.synth_targets(rng, b, num_actions)
     return params, x, y_r, a
 
@@ -27,10 +26,10 @@ def _case(g, b, seed=7, num_actions=5):
 def test_oracle_backward_matches_finite_differences(hwc):
     """Non-square, one with C = 1: the analytic fp64 gradients of cost_all against central differences, on a sample of entries
     of every variable (v held fixed inside the advantage, as tf.stop_gradient does)."""
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, x, y_r, a = _case(g, 3)
     params = {k: v.astype(np.float64) for k, v in params.items()}
-    _, grads, f = go.loss_and_grads(g, params, x, y_r, a, keep=True)
+    _, grads, f = onp.loss_and_grads(params, x, y_r, a, geom=g, keep=True)
     v_stop = f["v"]
     rng = np.random.default_rng(1)
     eps = 1e-6
@@ -39,8 +38,8 @@ def test_oracle_backward_matches_finite_differences(hwc):
             hi, lo = {**params}, {**params}
             hi[name] = val.copy(); hi[name][idx] += eps
             lo[name] = val.copy(); lo[name][idx] -= eps
-            lh, _ = go.loss_and_grads(g, hi, x, y_r, a, v_stop=v_stop)
-            ll, _ = go.loss_and_grads(g, lo, x, y_r, a, v_stop=v_stop)
+            lh, _ = onp.loss_and_grads(hi, x, y_r, a, geom=g, v_stop=v_stop)
+            ll, _ = onp.loss_and_grads(lo, x, y_r, a, geom=g, v_stop=v_stop)
             num = (lh["cost_all"] - ll["cost_all"]) / (2 * eps)
             assert abs(num - grads[name][idx]) <= 1e-6 + 1e-5 * abs(num), (name, idx, num, grads[name][idx])
 
@@ -51,9 +50,9 @@ def test_same_padding_matches_torch_conv2d_after_explicit_pad(hwc):
     input (F.pad with the (before, after) split TF uses)."""
     torch = pytest.importorskip("torch")
     F = torch.nn.functional
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, x, _, _ = _case(g, 2)
-    f = go.forward(g, params, x, keep=True)
+    f = onp.forward(params, x, geom=g, keep=True)
 
     def conv(inp, w, b, k, s):
         _, _, h, wd = inp.shape
@@ -70,26 +69,10 @@ def test_same_padding_matches_torch_conv2d_after_explicit_pad(hwc):
     np.testing.assert_allclose(f["n2"].reshape(2, g.h2, g.w2, 32), n2.permute(0, 2, 3, 1).numpy(), rtol=1e-12, atol=1e-12)
 
 
-def test_oracle_equals_oracle_np_at_84x84x4():
-    """At the default geometry the parameterised oracle computes what oracle_np does, bf16 mode included."""
-    g = go.Geometry(84, 84, 4)
-    rng = np.random.default_rng(3)
-    params = onp.init_params(rng, 6)
-    x = onp.synth_frames(rng, 2)
-    y_r, a = onp.synth_targets(rng, 2, 6)
-    for quant in (None, "bf16"):
-        l1, g1 = onp.loss_and_grads(params, x, y_r, a, quant=quant)
-        l2, g2 = go.loss_and_grads(g, params, x, y_r, a, quant=quant)
-        for k in l1:
-            assert l1[k] == pytest.approx(l2[k], rel=1e-12)
-        for k in g1:
-            np.testing.assert_allclose(g2[k], g1[k], rtol=1e-10, atol=1e-12)
-
-
 @pytest.mark.parametrize("h,w,c", [(1, 1, 1), (256, 256, 8), (1, 256, 1), (256, 1, 8), (84, 84, 4), (105, 80, 4), (100, 100, 2)])
 def test_derived_sizes_follow_the_formula(h, w, c):
     """H1 = ceil(H/4), H2 = ceil(H1/2) (likewise W), K = H2*W2*32, at the ends of the accepted range; padding low side smaller."""
-    g = go.Geometry(h, w, c)
+    g = onp.Geometry(h, w, c)
     assert (g.h1, g.w1) == (-(-h // 4), -(-w // 4))
     assert (g.h2, g.w2) == (-(-g.h1 // 2), -(-g.w1 // 2))
     assert g.flat == g.h2 * g.w2 * 32

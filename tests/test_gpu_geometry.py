@@ -1,35 +1,20 @@
 """GPU tests (`-m gpu`) of the conv network at input geometries other than 84x84x4 (Config.IMAGE_HEIGHT, IMAGE_WIDTH,
-STACKED_FRAMES), which run the generic trunk (conv_gen.cu), against the geometry-parameterised bf16 oracle
-(tests/_geometry_oracle.py) with the tolerances of test_gpu_parity.py."""
+STACKED_FRAMES), which run the generic trunk (conv_gen.cu), against the bf16 oracle at that geometry with the tolerances of
+tests/_parity.py."""
 import numpy as np
 import pytest
 
 from oracle import oracle_np as onp
 from oracle import histogram_np as hnp
-import _geometry_oracle as go
-from _parity import err
+from _parity import TOL_GRAD_REL, TOL_LOSS_REL, TOL_P, TOL_V, TOL_W_ABS, check_report, err, layer_report
+from _parity import ga3c  # noqa: F401  (pytest fixture)
 
 pytestmark = pytest.mark.gpu
-
-TOL_P, TOL_V = 2e-5, 2e-4
-TOL_ACT_REL = 2.0 ** -7
-TOL_LOSS_REL = 1e-4
-TOL_GRAD_REL = 2e-3
-TOL_W_ABS = 2e-6
 
 GEOMETRIES = [(84, 84, 1), (84, 84, 3), (42, 42, 4), (105, 80, 4), (100, 100, 2), (8, 8, 1), (128, 128, 4)]
 IDS = [f"{h}x{w}x{c}" for h, w, c in GEOMETRIES]
 GEN_KERNELS = {"gen_wprep", "gen_im2col11", "gen_conv11", "gen_im2col12", "gen_conv12", "gen_conv12_dgrad", "gen_col2im",
                "gen_conv12_wgrad", "gen_conv11_wgrad"}
-
-
-@pytest.fixture(scope="module")
-def ga3c():
-    import torch
-    if not torch.cuda.is_available():
-        pytest.fail("GPU tests need a CUDA device; there is no CPU fallback")
-    import ga3c_b200
-    return ga3c_b200
 
 
 def config(hwc, **kw):
@@ -49,84 +34,39 @@ def make_net(ga3c, hwc, max_batch, num_actions=6, **kw):
 
 def case(g, b, seed=12345, num_actions=6):
     rng = np.random.default_rng(seed)
-    params = go.init_params(rng, g, num_actions)
-    k = go.synth_frames_u8(rng, g, b)
+    params = onp.init_params(rng, num_actions, geom=g)
+    k = onp.synth_frames_u8(rng, b, geom=g)
     y_r, a = onp.synth_targets(rng, b, num_actions)
-    return params, k, go.normalise(k), y_r, a
-
-
-def layer_report(net, g, params, x, y_r, a, **kw):
-    net.set_variables(params)
-    p, v = net.predict_p_and_v(x)
-    losses_ref, grads_ref, f = go.loss_and_grads(g, params, x, y_r, a, quant="bf16", keep=True, **kw)
-    rep = {"p": err(p, f["p"]), "v": err(v, f["v"])}
-    losses = net.losses(x, y_r, a)
-    b = x.shape[0]
-    ws = {i: net.workspace(i) for i in (0, 1, 2, 3, 4, 5)}
-    rep["n1"] = err(ws[0], f["n1"].reshape(b, -1))
-    rep["n2"] = err(ws[1], f["n2"].reshape(b, -1))
-    rep["d1"] = err(ws[2], f["d1"])
-    rep["dd1"] = err(ws[3], f["dd1"])
-    # layer-local data gradients: the oracle's arithmetic on the CUDA path's own stored inputs (see tests/_parity.py)
-    n1_mask, n2_mask = ws[0].reshape(b, -1) > 0, ws[1].reshape(b, -1) > 0
-    dn2_local = onp.bf16_round((ws[3].astype(np.float64).reshape(b, -1) @ f["w1"].T) * n2_mask)
-    dn1_local = go.col2im(ws[4].astype(np.float64).reshape(-1, 32) @ f["w12"].T, b, g.h1, g.w1, 4, 2, g.h2, g.w2, 16)
-    dn1_local = onp.bf16_round(dn1_local.reshape(b, -1) * n1_mask)
-    rep["dn2"], rep["dn2_local"] = err(ws[4], f["dn2"]), err(ws[4], dn2_local)
-    rep["dn1"], rep["dn1_local"] = err(ws[5], f["dn1"]), err(ws[5], dn1_local)
-    for k, i in (("dn1", 5), ("dn2", 4)):
-        ref = np.asarray(f[k], dtype=np.float64).ravel()
-        rep[k + "_outliers"] = (float((np.abs(ws[i].ravel() - ref) > 2.0 ** -7 * np.abs(ref).max()).mean()), 0.0)
-    for k in ("cost_p_1", "cost_p_2", "cost_v", "cost_all"):
-        rep["loss/" + k] = err([losses[k]], [losses_ref[k]])
-    grads = net.get_gradients()
-    for k in grads_ref:
-        rep["grad/" + k] = err(grads[k], grads_ref[k])
-    return rep
-
-
-def check_report(rep):
-    assert rep["p"][0] <= TOL_P and rep["v"][0] <= TOL_V, rep
-    for k in ("n1", "n2", "dd1"):
-        assert rep[k][1] <= TOL_ACT_REL, (k, rep[k])
-    for k in ("dn2", "dn1"):
-        assert rep[k + "_local"][1] <= TOL_ACT_REL, (k, rep[k + "_local"])
-        assert rep[k][1] <= TOL_ACT_REL or rep[k + "_outliers"][0] <= 1e-4, (k, rep[k], rep[k + "_outliers"])
-    assert rep["d1"][1] <= 1e-3, rep["d1"]
-    for k, (d, r) in rep.items():
-        if k.startswith("loss/"):
-            assert r <= TOL_LOSS_REL or d <= 1e-5, (k, d, r)
-        if k.startswith("grad/"):
-            assert r <= TOL_GRAD_REL, (k, d, r)
+    return params, k, onp.normalise(k), y_r, a
 
 
 @pytest.mark.parametrize("hwc", GEOMETRIES, ids=IDS)
 def test_predict_matches_oracle(ga3c, hwc):
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     net = make_net(ga3c, hwc, 300)
     for b in (1, 37, 300):
         params, _, x, _, _ = case(g, b, seed=b)
         net.set_variables(params)
         p, v = net.predict_p_and_v(x)
-        pr, vr = go.forward(g, params, x, quant="bf16")
+        pr, vr = onp.forward(params, x, geom=g, quant="bf16")
         assert np.abs(p - pr).max() <= TOL_P and np.abs(v - vr).max() <= TOL_V, (b, np.abs(p - pr).max(), np.abs(v - vr).max())
 
 
 @pytest.mark.parametrize("hwc", GEOMETRIES, ids=IDS)
 def test_layers_and_gradients_match_oracle(ga3c, hwc):
     """The 4 loss sums, all 10 gradients and the layer-local n1 / n2 / d1 / dd1 / dn2 / dn1 (row-major workspace)."""
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, _, x, y_r, a = case(g, 37)
     net = make_net(ga3c, hwc, 64)
     assert net._table["dense1/w:0"][1] == (g.flat, 256) and net._table["conv11/w:0"][1] == (8, 8, hwc[2], 16)
-    check_report(layer_report(net, g, params, x, y_r, a))
+    check_report(layer_report(net, params, x, y_r, a, geom=g))
 
 
 @pytest.mark.parametrize("hwc", GEOMETRIES, ids=IDS)
 def test_train_steps_uint8_and_reruns(ga3c, hwc):
     """Three RMSProp steps: weights and slots against the oracle; uint8 frames give bit-identical results to their normalised
     fp32 copy; a second network fed the same steps ends bit-identical (fixed-order reductions)."""
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, k, x, y_r, a = case(g, 29, seed=5)
     lr = 3e-4
     results = []
@@ -140,7 +80,7 @@ def test_train_steps_uint8_and_reruns(ga3c, hwc):
     p_ref = {kk: v.astype(np.float64) for kk, v in params.items()}
     ms, mom = onp.rmsprop_init(p_ref)
     for _ in range(3):
-        _, grads = go.loss_and_grads(g, {kk: v.astype(np.float32) for kk, v in p_ref.items()}, x, y_r, a, quant="bf16")
+        _, grads = onp.loss_and_grads({kk: v.astype(np.float32) for kk, v in p_ref.items()}, x, y_r, a, geom=g, quant="bf16")
         p_ref, ms, mom = onp.rmsprop_update(p_ref, grads, ms, mom, lr=lr, dtype=np.float64)
     w, (gms, gmom) = results[0]
     for kk in params:
@@ -155,7 +95,7 @@ def test_train_steps_uint8_and_reruns(ga3c, hwc):
 
 def test_predict_uint8_bit_identical(ga3c):
     hwc = (105, 80, 4)
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, k, x, _, _ = case(g, 41)
     net = make_net(ga3c, hwc, 64)
     net.set_variables(params)
@@ -166,27 +106,27 @@ def test_predict_uint8_bit_identical(ga3c):
 
 def test_b1024_training_matches_oracle(ga3c):
     hwc = (42, 42, 4)
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, _, x, y_r, a = case(g, 1024, seed=1024)
     net = make_net(ga3c, hwc, 1024)
-    check_report(layer_report(net, g, params, x, y_r, a))
+    check_report(layer_report(net, params, x, y_r, a, geom=g))
     net.train(x, y_r, a)
     assert all(np.isfinite(v).all() for v in net.get_variables().values())
 
 
 def test_log_softmax_min_policy(ga3c):
     hwc = (84, 84, 3)
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, _, x, y_r, a = case(g, 33)
     net = make_net(ga3c, hwc, 64, USE_LOG_SOFTMAX=True)
-    check_report(layer_report(net, g, params, x, y_r, a, use_log_softmax=True))
+    check_report(layer_report(net, params, x, y_r, a, geom=g, use_log_softmax=True))
     net = make_net(ga3c, hwc, 64, MIN_POLICY=0.05)
-    check_report(layer_report(net, g, params, x, y_r, a, min_policy=0.05))
+    check_report(layer_report(net, params, x, y_r, a, geom=g, min_policy=0.05))
 
 
 def test_grad_clip_and_dual_rmsprop(ga3c):
     hwc = (100, 100, 2)
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, _, x, y_r, a = case(g, 20)
     lr = 3e-4
     # USE_GRAD_CLIP: clip_by_average_norm per variable before RMSProp
@@ -194,7 +134,7 @@ def test_grad_clip_and_dual_rmsprop(ga3c):
     net.set_variables(params)
     net.learning_rate = lr
     net.train(x, y_r, a)
-    _, grads = go.loss_and_grads(g, params, x, y_r, a, quant="bf16")
+    _, grads = onp.loss_and_grads(params, x, y_r, a, geom=g, quant="bf16")
     ref = {k: v.astype(np.float64) for k, v in params.items()}
     ms, mom = onp.rmsprop_init(ref)
     p2, _, _ = onp.rmsprop_update(ref, {k: onp.clip_by_average_norm(v, 0.05) for k, v in grads.items()}, ms, mom, lr=lr,
@@ -209,7 +149,7 @@ def test_grad_clip_and_dual_rmsprop(ga3c):
     net.train(x, y_r, a)
     new = {k: v.astype(np.float64) for k, v in params.items()}
     for part in ("p", "v"):
-        _, gp = go.loss_and_grads(g, params, x, y_r, a, quant="bf16", part=part)
+        _, gp = onp.loss_and_grads(params, x, y_r, a, geom=g, quant="bf16", part=part)
         sub = {k: params[k].astype(np.float64) for k in gp}
         ms, mom = onp.rmsprop_init(sub)
         p2, _, _ = onp.rmsprop_update(sub, gp, ms, mom, lr=lr, dtype=np.float64)
@@ -222,7 +162,7 @@ def test_grad_clip_and_dual_rmsprop(ga3c):
 
 def test_histograms_match_oracle(ga3c):
     hwc = (105, 80, 4)
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, _, x, y_r, a = case(g, 24)
     net = make_net(ga3c, hwc, 32)
     net.set_variables(params)
@@ -243,7 +183,7 @@ def test_histograms_match_oracle(ga3c):
 def test_save_load_roundtrip_and_cross_geometry_load(ga3c, tmp_path, monkeypatch):
     monkeypatch.chdir(tmp_path)
     hwc = (8, 8, 1)
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, _, x, y_r, a = case(g, 9)
     net = make_net(ga3c, hwc, 16)
     net.set_variables(params)
@@ -316,11 +256,11 @@ def test_predictors_and_trainer_over_the_slab_transport(ga3c):
     from ga3c_b200.transport import SlabPredictionQueue, SlabTrainingQueue
     from test_gpu_parity import _Server
     hwc, n = (42, 42, 4), 24
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, k, x, y_r, a = case(g, n)
     net = make_net(ga3c, hwc, 64)
     net.set_variables(params)
-    pr, vr = go.forward(g, params, x, quant="bf16")
+    pr, vr = onp.forward(params, x, geom=g, quant="bf16")
     for native in (False, True):
         net.set_variables(params)             # the trainer of the previous round moved them
         pq = SlabPredictionQueue(n, g.state_dim, 6, dtype=np.uint8)
@@ -372,7 +312,7 @@ def test_fb_head_and_fb_tail_match_oracle(ga3c, u8):
     import torch
     from ga3c_b200 import _capi
     hwc = (105, 80, 4)
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, k, x, y_r, a = case(g, 45, seed=9)
     net = make_net(ga3c, hwc, 64)
     net.set_variables(params)
@@ -386,7 +326,7 @@ def test_fb_head_and_fb_tail_match_oracle(ga3c, u8):
     torch.cuda.synchronize()
     split = net.get_gradients()
     losses = net._loss_dict(loss.cpu())
-    losses_ref, grads_ref = go.loss_and_grads(g, params, x, y_r, a, quant="bf16", beta=net.beta)
+    losses_ref, grads_ref = onp.loss_and_grads(params, x, y_r, a, geom=g, quant="bf16", beta=net.beta)
     for kk in ("cost_p_1", "cost_p_2", "cost_v", "cost_all"):
         d, r = err([losses[kk]], [losses_ref[kk]])
         assert r <= TOL_LOSS_REL or d <= 1e-5, (kk, d, r)
@@ -403,7 +343,7 @@ def test_reserve_failure_leaves_a_usable_handle(ga3c):
     the handle then refuses every batch, and a later reserve that fits brings it back."""
     import ctypes as C
     hwc = (256, 256, 8)
-    g = go.Geometry(*hwc)
+    g = onp.Geometry(*hwc)
     params, _, x, _, _ = case(g, 3)
     net = make_net(ga3c, hwc, 4)
     net.set_variables(params)
@@ -417,7 +357,7 @@ def test_reserve_failure_leaves_a_usable_handle(ga3c):
     assert net._lib.ga3c_reserve(net._h, 8) == 0
     assert net._lib.ga3c_predict(net._h, xd.data_ptr(), 3, p.data_ptr(), v.data_ptr(), None) == 0
     torch.cuda.synchronize()
-    pr, vr = go.forward(g, params, x, quant="bf16")
+    pr, vr = onp.forward(params, x, geom=g, quant="bf16")
     assert np.abs(p.cpu().numpy() - pr).max() <= TOL_P and np.abs(v.cpu().numpy() - vr).max() <= TOL_V
 
 

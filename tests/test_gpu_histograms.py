@@ -6,19 +6,11 @@ import pytest
 
 from oracle import histogram_np as oh
 from oracle import oracle_np as onp
+from _parity import ga3c  # noqa: F401  (pytest fixture)
 
 pytestmark = pytest.mark.gpu
 
 ROW = 5 + 1551
-
-
-@pytest.fixture(scope="module")
-def ga3c():
-    import torch
-    if not torch.cuda.is_available():
-        pytest.fail("GPU tests need a CUDA device; there is no CPU fallback")
-    import ga3c_b200
-    return ga3c_b200
 
 
 def device_histogram(t):
@@ -122,8 +114,8 @@ def test_kernel_flags_nan_and_inf(ga3c):
 def _net(ga3c, b, seed=7):
     rng = np.random.default_rng(seed)
     params = onp.init_params(rng, 6)
-    k = rng.integers(0, 256, size=(b, onp.STATE_DIM), dtype=np.uint8)
-    x = (k.astype(np.float32) / np.float32(128.0) - np.float32(1.0)).astype(np.float32)
+    k = onp.synth_frames_u8(rng, b)
+    x = onp.normalise(k)
     y_r, a = onp.synth_targets(rng, b)
     net = ga3c.Network("gpu:0", "histtest", 6, max_batch=max(b, 32))
     net.set_variables(params)

@@ -1,17 +1,6 @@
 """GPU parity tests (`-m gpu`): the CUDA path, called through the C-ABI library, against the oracle.
 
-Tolerances (SURVEY A.8, calibrated on B200 and frozen here).  The CUDA path rounds operands to
-bf16 at fixed points (x, conv weights, n1, n2, w1, dd1, dn2, dn1) and accumulates in fp32; the
-oracle is run in its `quant='bf16'` mode, which rounds at the same points and accumulates in fp64.
-Residual differences are fp32-vs-fp64 accumulation order, which now and then flips a bf16 rounding
-(1 ulp = 2^-8 relative) of a stored activation:
-    p        |d| <= 2e-5          v        |d| <= 2e-4
-    stored bf16 activations      |d| <= 2^-7 * max|ref|  and  <= 1% of elements off by > 1e-5 * max|ref|
-    loss sums                    rel <= 1e-4
-    gradients                    |d| <= 2e-3 * max|ref| per tensor
-    weights after RMSProp        |d| <= 2e-6   (lr 3e-4 scales the gradient error)
-Against the un-quantised fp64 oracle (the irreducible bf16 gap): |dp| <= 1e-2, |dv| <= 2e-2.
-Integer / fp64 work (returns, sampling) is bit-exact.
+Tolerances: tests/_parity.py.  Integer / fp64 work (returns, sampling) is bit-exact.
 """
 import json
 import os
@@ -22,41 +11,10 @@ import numpy as np
 import pytest
 
 from oracle import oracle_np as onp
-from _parity import make_case, layer_report, err
+from _parity import TOL_GRAD_REL, TOL_LOSS_REL, TOL_P, TOL_V, TOL_W_ABS, check_report, err, layer_report, make_case
+from _parity import ga3c  # noqa: F401  (pytest fixture)
 
 pytestmark = pytest.mark.gpu
-
-TOL_P, TOL_V = 2e-5, 2e-4
-TOL_ACT_REL = 2.0 ** -7
-TOL_LOSS_REL = 1e-4
-TOL_GRAD_REL = 2e-3
-TOL_W_ABS = 2e-6
-
-
-@pytest.fixture(scope="module")
-def ga3c():
-    import torch
-    if not torch.cuda.is_available():
-        pytest.fail("GPU tests need a CUDA device; there is no CPU fallback")
-    import ga3c_b200
-    return ga3c_b200
-
-
-def check_report(rep):
-    assert rep["p"][0] <= TOL_P and rep["v"][0] <= TOL_V, rep
-    for k in ("n1", "n2", "dd1"):
-        assert rep[k][1] <= TOL_ACT_REL, (k, rep[k])
-    for k in ("dn2", "dn1"):
-        # masked data gradients: exact against the oracle fed the same stored inputs; against the end-to-end oracle either
-        # within tolerance everywhere, or off only at the rare elements behind a ReLU-boundary flip (tests/_parity.py)
-        assert rep[k + "_local"][1] <= TOL_ACT_REL, (k, rep[k + "_local"])
-        assert rep[k][1] <= TOL_ACT_REL or rep[k + "_outliers"][0] <= 1e-4, (k, rep[k], rep[k + "_outliers"])
-    assert rep["d1"][1] <= 1e-3, rep["d1"]
-    for k, (d, r) in rep.items():
-        if k.startswith("loss/"):
-            assert r <= TOL_LOSS_REL or d <= 1e-5, (k, d, r)
-        if k.startswith("grad/"):
-            assert r <= TOL_GRAD_REL, (k, d, r)
 
 
 # ------------------------------------------------------------------------------------------------
