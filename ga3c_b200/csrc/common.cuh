@@ -286,6 +286,8 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+__device__ __forceinline__ float sigmoid(float z) { return 1.f / (1.f + expf(-z)); }
+
 // ---- swizzles shared by producer and consumer kernels -----------------------------------------
 // padded conv11 output (n1p): pixel (py, px) in 24x24, 32 B per pixel, two 16-B chunks.
 //   slot(px): rotate the low 3 bits of px right by one, so px, px+2, px+4, px+6 land in four

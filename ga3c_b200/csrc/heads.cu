@@ -1,9 +1,6 @@
 // Value / policy heads, softmax, A3C loss and its backward, fused.  All fp32.
 //
-// Reference graph (NetworkVP_discrate.py:60-85, :100; SURVEY Appendix A.3/A.4):
-//   v = d1.Wv + bv ; z = d1.Wp + bp ; s = softmax(z) ; p = (s + MIN_POLICY) / (1 + MIN_POLICY*A)
-//   cost_p_1 = log(max(sum(p*a), eps)) * (R - stop_gradient(v)) ; cost_p_2 = -beta * sum(log(max(p, eps)) * p)
-//   cost_v = 0.5 * (R - v)^2 ; every batch reduction is a SUM.
+// v = d1.Wv + bv, z = d1.Wp + bp; the loss of a3c_loss.cuh (reference graph there).
 // The kernel is also the tail of dense1 (NetworkDNav.py:90): it sums the split-K partial tiles the
 // tcgen05 GEMM left in d1_part (fixed order => deterministic), adds the bias and applies the ReLU.
 // Phase 1: one warp per sample, warp-shuffle reductions for the A+1 dot products, then the whole
@@ -35,7 +32,7 @@ __global__ void __launch_bounds__(HD_THREADS) heads_kernel(HeadsArgs p) {
 
   HeadsAcc<A> ac;
   ac.clear();
-  const float inv_mix = 1.f / (1.f + p.min_policy * (float)A);
+  const float inv_mix = policy_inv_mix(p.la, A);
 
   const int n_chunks = (p.batch + HD_CHUNK - 1) / HD_CHUNK;
   for (int c = blockIdx.x; c < n_chunks; c += gridDim.x) {

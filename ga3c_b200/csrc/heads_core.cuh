@@ -1,8 +1,9 @@
-// The fused value / policy heads, softmax, A3C loss and its backward (NetworkVP_discrate.py:60-85, :100; SURVEY A.3 / A.4) as device
-// functions, run by heads_kernel (heads.cu: behind the split-K dense1 GEMM, summing its partial tiles from L2).  All fp32.
+// The fused value / policy heads of the conv net, with the A3C loss and its backward of a3c_loss.cuh, as device functions, run by
+// heads_kernel (heads.cu: behind the split-K dense1 GEMM, summing its partial tiles from L2).  All fp32.
 #pragma once
 #include "common.cuh"
 #include "kernels.h"
+#include "a3c_loss.cuh"
 
 namespace ga3c {
 
@@ -24,11 +25,12 @@ template <int A>
 struct HeadsAcc {
   float acc[A + 1];        // thread j: dWp[j][0..A-1], dWv[j]
   float acc_b1, acc_bh;    // thread j: db1[j]; thread k <= A: dbp[k] / dbv
-  float l1, l2, lv;        // lane 0 of each warp: loss partial sums
+  A3cSums loss;            // lane 0 of each warp: loss partial sums
   __device__ __forceinline__ void clear() {
 #pragma unroll
     for (int k = 0; k <= A; ++k) acc[k] = 0.f;
-    acc_b1 = acc_bh = l1 = l2 = lv = 0.f;
+    acc_b1 = acc_bh = 0.f;
+    loss = A3cSums{};
   }
 };
 
@@ -50,9 +52,6 @@ template <int A>
 __device__ __forceinline__ void heads_sample(const HeadsArgs& p, HeadsSmem<A>& hs, HeadsAcc<A>& ac, int b, int sl, int lane,
                                              const float4& fa, const float4& fb, float inv_mix) {
   constexpr int A1 = A + 1;
-  float& l1 = ac.l1;
-  float& l2 = ac.l2;
-  float& lv = ac.lv;
   *reinterpret_cast<float4*>(p.d1 + (size_t)b * FC + 4 * lane) = fa;
   *reinterpret_cast<float4*>(p.d1 + (size_t)b * FC + 128 + 4 * lane) = fb;
   if (p.train) {
@@ -70,79 +69,30 @@ __device__ __forceinline__ void heads_sample(const HeadsArgs& p, HeadsSmem<A>& h
     z[k] = warp_sum(s) + hs.bias_s[k];
   }
   const float v = z[A];
-  float mx = z[0];
-#pragma unroll
-  for (int k = 1; k < A; ++k) mx = fmaxf(mx, z[k]);
-  float sm[A], den = 0.f;
-#pragma unroll
-  for (int k = 0; k < A; ++k) { sm[k] = expf(z[k] - mx); den += sm[k]; }
-  const float inv_den = 1.f / den;
-  float pr[A];
-#pragma unroll
-  for (int k = 0; k < A; ++k) { sm[k] *= inv_den; pr[k] = p.log_softmax ? sm[k] : (sm[k] + p.min_policy) * inv_mix; }
-  if (p.p_out != nullptr) {
-#pragma unroll
-    for (int k = 0; k < A; ++k) if (lane == k) p.p_out[(size_t)b * A + k] = pr[k];
-    if (lane == 0) p.v_out[b] = v;
-  }
+  const LossArgs la = p.la;
+  float dz[A];
+  const float* arow = p.a + (size_t)b * A;
+  if (p.p_out != nullptr && lane == 0) p.v_out[b] = v;
+  const float yr = p.train ? p.yr[b] : 0.f;
+  const A3cTerms t = softmax_policy_row(
+      z, A, v, yr, la, inv_mix, p.train, [&](int k) { return arow[k]; },
+      [&](int k, float pk) { if (p.p_out != nullptr && lane == k) p.p_out[(size_t)b * A + k] = pk; },
+      [&](int k, float dzk) { dz[k] = dzk; });
   if (p.train) {
-    const float yr = p.yr[b];
-    float av[A], sel = 0.f;
-#pragma unroll
-    for (int k = 0; k < A; ++k) { av[k] = p.a[(size_t)b * A + k]; sel = fmaf(pr[k], av[k], sel); }
-    const float adv = yr - v, dv = v - yr;
-    float dz[A], ent = 0.f, c1;
-    if (p.log_softmax) {
-      // Config.USE_LOG_SOFTMAX (NetworkVP_discrate.py:64-71): lsm = z - max - log(den); cost_p_1 = sum(lsm a) adv,
-      // cost_p_2 = -beta sum(lsm s);  dz_k = -adv (a_k - s_k sum(a)) + beta s_k (lsm_k - sum(lsm s))
-      const float lden = logf(den);
-      float lsm[A], sa = 0.f, sla = 0.f;
-#pragma unroll
-      for (int k = 0; k < A; ++k) {
-        lsm[k] = (z[k] - mx) - lden;
-        ent = fmaf(lsm[k], sm[k], ent);
-        sa += av[k];
-        sla = fmaf(lsm[k], av[k], sla);
-      }
-#pragma unroll
-      for (int k = 0; k < A; ++k) dz[k] = -adv * (av[k] - sm[k] * sa) + p.beta * sm[k] * (lsm[k] - ent);
-      c1 = sla * adv;
-    } else {
-      const float coef = (sel >= p.log_eps) ? adv / sel : 0.f;
-      float h[A], sh = 0.f;
-#pragma unroll
-      for (int k = 0; k < A; ++k) {
-        const float lg = logf(fmaxf(pr[k], p.log_eps));
-        ent = fmaf(lg, pr[k], ent);
-        const float gk = -av[k] * coef + p.beta * (lg + (pr[k] >= p.log_eps ? 1.f : 0.f));
-        h[k] = gk * inv_mix;
-        sh = fmaf(sm[k], h[k], sh);
-      }
-#pragma unroll
-      for (int k = 0; k < A; ++k) dz[k] = sm[k] * (h[k] - sh);
-      c1 = logf(fmaxf(sel, p.log_eps)) * adv;
-    }
-    // Config.DUAL_RMSPROP: part 1 = gradient of cost_p alone, part 2 = of cost_v alone (0: cost_all)
-    const float dvv = p.part == 1 ? 0.f : dv;
-    if (p.part == 2) {
-#pragma unroll
-      for (int k = 0; k < A; ++k) dz[k] = 0.f;
-    }
+    const float dv = t.dv;
     if (lane == 0) {
-      l1 += c1;
-      l2 += -p.beta * ent;
-      lv += 0.5f * (yr - v) * (yr - v);
+      t.add_to(p.la.beta, ac.loss);
 #pragma unroll
       for (int k = 0; k < A; ++k) hs.dzs[sl][k] = dz[k];
-      hs.dzs[sl][A] = dvv;
+      hs.dzs[sl][A] = dv;
     }
     // dd1[j] = relu'(d1[j]) * (sum_k dz_k Wp[j][k] + dv Wv[j]) for this lane's 8 features
     float da[4], db[4];
     {
       const float4 wa = *reinterpret_cast<const float4*>(&hs.wt[A][4 * lane]);
       const float4 wb = *reinterpret_cast<const float4*>(&hs.wt[A][128 + 4 * lane]);
-      da[0] = dvv * wa.x; da[1] = dvv * wa.y; da[2] = dvv * wa.z; da[3] = dvv * wa.w;
-      db[0] = dvv * wb.x; db[1] = dvv * wb.y; db[2] = dvv * wb.z; db[3] = dvv * wb.w;
+      da[0] = dv * wa.x; da[1] = dv * wa.y; da[2] = dv * wa.z; da[3] = dv * wa.w;
+      db[0] = dv * wb.x; db[1] = dv * wb.y; db[2] = dv * wb.z; db[3] = dv * wb.w;
     }
 #pragma unroll
     for (int k = 0; k < A; ++k) {
@@ -201,7 +151,7 @@ __device__ __forceinline__ void heads_store_slab(const HeadsArgs& p, HeadsSmem<A
   p.g_b1[slab + jx] = ac.acc_b1;
   if (jx < A) p.g_bp[slab + jx] = ac.acc_bh;
   if (jx == A) p.g_bv[slab] = ac.acc_bh;
-  if (lane == 0) { hs.loss_s[warp][0] = ac.l1; hs.loss_s[warp][1] = ac.l2; hs.loss_s[warp][2] = ac.lv; }
+  if (lane == 0) { hs.loss_s[warp][0] = ac.loss.l1; hs.loss_s[warp][1] = ac.loss.l2; hs.loss_s[warp][2] = ac.loss.lv; }
   __syncthreads();
   if (jx < 4) {
     float t = 0.f;

@@ -102,7 +102,15 @@ int launch_gen_conv12_wgrad(const GenGeom& g, const GenBufs& b, float* g_w12, fl
 int launch_gen_conv11_wgrad(const GenGeom& g, const GenBufs& b, float* g_w11, float* g_b11, int64_t gp_stride, int slabs,
                             int batch, cudaStream_t st);
 
-// heads.cu -- value / policy heads, softmax, A3C loss and its backward (NetworkVP_discrate.py:60-85)
+// The knobs of the A3C loss (a3c_loss.cuh), for the conv heads and the MLP kernels alike
+struct LossArgs {
+  float beta;                  // entropy weight of the call
+  float log_eps, min_policy;   // Config.LOG_EPSILON, Config.MIN_POLICY
+  int log_softmax;             // Config.USE_LOG_SOFTMAX
+  int part;                    // Config.DUAL_RMSPROP passes: 0 gradient of cost_all, 1 of cost_p alone, 2 of cost_v alone
+};
+
+// heads.cu -- value / policy heads, softmax, A3C loss and its backward (a3c_loss.cuh)
 struct HeadsArgs {
   const float* d1_part; // [n_split][B,256] raw split-K partial sums of dense1 (no bias, no ReLU)
   int n_split;
@@ -111,7 +119,7 @@ struct HeadsArgs {
   const float *wp, *bp, *wv, *bv;
   const float *yr, *a;  // train only
   int batch, num_actions;
-  float beta, log_eps, min_policy;
+  LossArgs la;
   float *p_out, *v_out;        // may be null in train mode
   uint16_t* dd1;               // [B,256] bf16, train only
   // train only: this CTA's partial sums go to slab blockIdx.x of the gradient-partial workspace (pointers are
@@ -120,8 +128,6 @@ struct HeadsArgs {
   float* loss;                 // [4] (cost_p_1, cost_p_2, cost_v, 0) partial sums, same slab scheme
   int64_t gp_stride;
   int train;
-  int log_softmax;             // Config.USE_LOG_SOFTMAX
-  int part;                    // Config.DUAL_RMSPROP passes: 0 gradient of cost_all, 1 of cost_p alone, 2 of cost_v alone
   int preload;                 // the head weights may be read before the dependency wait (heads.cu)
 };
 int heads_grid(int batch, int num_sms);          // CTAs (= slabs written) of a training launch

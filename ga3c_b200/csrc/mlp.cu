@@ -14,6 +14,7 @@
 #include "common.cuh"
 #include "kernels.h"
 #include "mlp.cuh"
+#include "a3c_loss.cuh"
 
 namespace ga3c {
 
@@ -26,14 +27,12 @@ constexpr int HLD = 49;              // row pitch of the head matrix / logits ti
 constexpr int NT = 256;              // threads of the weight-gradient / reduce kernels
 constexpr int FT = 512;              // threads of the fused kernel: 16 warps x 4 rows = one 64-row tile
 constexpr int HW = 48;               // head matrix columns held in shared memory (>= MLP_MAX_OUT, zero padded)
-constexpr float PI_F = 3.14159265358979323846f;
 
 constexpr size_t FUSED_SMEM =
     (size_t)(2 * MLP_TM * LD + WS * RC * LD + MLP_MAX_HID * HLD + MLP_TM * HLD + 48 + 32) * sizeof(float);
 static_assert(FUSED_SMEM <= 232448, "shared memory budget of one CTA per SM");
 
 __device__ __forceinline__ int round_up16(int v) { return (v + 15) & ~15; }
-__device__ __forceinline__ float sigmoidf_(float z) { return 1.f / (1.f + expf(-z)); }
 
 // element (k, j) of the head matrix [hid][n_out]: column 0 = logits_v, then logits_p (discrate) or out_x | out_y (fork_vp)
 __device__ __forceinline__ int head_w_index(const MlpNet& net, int k, int j) {
@@ -283,7 +282,7 @@ __global__ void __launch_bounds__(FT, 1) mlp_fused_kernel(const MlpNet net, cons
           float z = 0.f;
           if (c < L.n) {
             z = v[e] + __ldg(bias + c);
-            if (L.act == MLP_ACT_SIGMOID) z = sigmoidf_(z);
+            if (L.act == MLP_ACT_SIGMOID) z = sigmoid(z);
           }
           v[e] = z;
         }
@@ -317,108 +316,41 @@ __global__ void __launch_bounds__(FT, 1) mlp_fused_kernel(const MlpNet net, cons
     }
     __syncthreads();
 
-    // ---- per row: p, v, loss terms, dlogits ----
-    float l1 = 0.f, l2 = 0.f, lv = 0.f;
+    // ---- per row: p, v, loss terms, dlogits (a3c_loss.cuh) ----
+    A3cSums sums;
     if (tid < TM) {
       const int r = tid;
       const bool valid = row0 + r < B;
       float* z = lg + r * HLD;
       const float v = z[0];
-      float yr = 0.f, adv = 0.f, dv = 0.f;
-      if (TRAIN && valid) {
-        yr = s.yr[row0 + r];
-        adv = yr - v;                     // stop_gradient(v) inside cost_p_1
-        dv = v - yr;
-        lv = 0.5f * (yr - v) * (yr - v);
-      }
+      const float yr = TRAIN && valid ? s.yr[row0 + r] : 0.f;
       if (valid && s.v_out != nullptr) s.v_out[row0 + r] = v;
+      A3cTerms t{};
       if (net.kind == MLP_KIND_FORK_VP) {
-        // p = atan2(sigmoid(out_y) - 0.5, sigmoid(out_x) - 0.5) / pi; softmax_p = log_softmax_p = p  (NetworkVP.py:175-192, :95-101)
         float sel = 0.f, sq = 0.f;
         for (int j = 0; j < A; ++j) {
-          const float ox = sigmoidf_(z[1 + j]), oy = sigmoidf_(z[1 + A + j]);
-          const float X = ox - 0.5f, Y = oy - 0.5f;
-          const float p = atan2f(Y, X) / PI_F;
-          if (valid && s.p_out != nullptr) s.p_out[(size_t)(row0 + r) * A + j] = p;
+          const float av = TRAIN && valid ? s.a[(size_t)(row0 + r) * A + j] : 0.f;
+          const ForkAction f = fork_policy(z[1 + j], z[1 + A + j], av, v, yr, s.la, sel, sq);
+          if (valid && s.p_out != nullptr) s.p_out[(size_t)(row0 + r) * A + j] = f.p;
           if (TRAIN) {
-            float dzx = 0.f, dzy = 0.f;
-            if (valid) {
-              const float av = s.a[(size_t)(row0 + r) * A + j];
-              sel = fmaf(p, av, sel);
-              sq = fmaf(p, p, sq);
-              const float dp = -av * adv + 2.f * s.beta * p;
-              const float inv = 1.f / (PI_F * (X * X + Y * Y));
-              dzx = dp * (-Y * inv) * ox * (1.f - ox);
-              dzy = dp * (X * inv) * oy * (1.f - oy);
-            }
-            z[1 + j] = dzx;
-            z[1 + A + j] = dzy;
+            z[1 + j] = valid ? f.dzx : 0.f;
+            z[1 + A + j] = valid ? f.dzy : 0.f;
           }
         }
-        if (TRAIN && valid) { l1 = sel * adv; l2 = -s.beta * sq; }
+        t = fork_policy_terms(sel, sq, v, yr, s.la);
       } else {
-        // softmax (+ MIN_POLICY mix), log(max(., eps)) loss terms and their backward  (NetworkVP_discrate.py:66-85)
-        const float inv_mix = 1.f / (1.f + net.min_policy * (float)A);
-        float mx = z[1];
-        for (int j = 1; j < A; ++j) mx = fmaxf(mx, z[1 + j]);
-        float den = 0.f;
-        for (int j = 0; j < A; ++j) den += expf(z[1 + j] - mx);
-        const float inv_den = 1.f / den;
-        float sel = 0.f, ent = 0.f, sh = 0.f;
-        for (int j = 0; j < A; ++j) {
-          const float sm = expf(z[1 + j] - mx) * inv_den;
-          const float p = net.log_softmax ? sm : (sm + net.min_policy) * inv_mix;
-          if (valid && s.p_out != nullptr) s.p_out[(size_t)(row0 + r) * A + j] = p;
-          if (TRAIN && valid) sel = fmaf(p, s.a[(size_t)(row0 + r) * A + j], sel);
-        }
-        if (TRAIN && net.log_softmax) {
-          // Config.USE_LOG_SOFTMAX (NetworkVP_discrate.py:64-71): dz_j = -adv (a_j - s_j sum(a)) + beta s_j (lsm_j - sum(lsm s))
-          const float lden = logf(den);
-          float sa = 0.f, sla = 0.f;
-          for (int j = 0; j < A; ++j) {
-            const float lsm = (z[1 + j] - mx) - lden;
-            const float av = valid ? s.a[(size_t)(row0 + r) * A + j] : 0.f;
-            ent = fmaf(lsm, expf(z[1 + j] - mx) * inv_den, ent);
-            sa += av;
-            sla = fmaf(lsm, av, sla);
-          }
-          for (int j = 0; j < A; ++j) {
-            const float lsm = (z[1 + j] - mx) - lden;
-            const float sm = expf(z[1 + j] - mx) * inv_den;
-            const float av = valid ? s.a[(size_t)(row0 + r) * A + j] : 0.f;
-            z[1 + j] = valid ? -adv * (av - sm * sa) + s.beta * sm * (lsm - ent) : 0.f;
-          }
-          if (valid) { l1 = sla * adv; l2 = -s.beta * ent; }
-        } else if (TRAIN) {
-          const float coef = (valid && sel >= net.log_eps) ? adv / sel : 0.f;
-          // two sweeps: sh = sum_j sm_j h_j first, then dz_j = sm_j (h_j - sh)
-          for (int j = 0; j < A; ++j) {
-            const float sm = expf(z[1 + j] - mx) * inv_den;
-            const float p = (sm + net.min_policy) * inv_mix;
-            const float lgp = logf(fmaxf(p, net.log_eps));
-            const float av = valid ? s.a[(size_t)(row0 + r) * A + j] : 0.f;
-            const float gk = -av * coef + s.beta * (lgp + (p >= net.log_eps ? 1.f : 0.f));
-            ent = fmaf(lgp, p, ent);
-            sh = fmaf(sm, gk * inv_mix, sh);
-          }
-          float dzj[MLP_MAX_OUT];
-          for (int j = 0; j < A; ++j) {
-            const float sm = expf(z[1 + j] - mx) * inv_den;
-            const float p = (sm + net.min_policy) * inv_mix;
-            const float lgp = logf(fmaxf(p, net.log_eps));
-            const float av = valid ? s.a[(size_t)(row0 + r) * A + j] : 0.f;
-            const float gk = -av * coef + s.beta * (lgp + (p >= net.log_eps ? 1.f : 0.f));
-            dzj[j] = valid ? sm * (gk * inv_mix - sh) : 0.f;
-          }
-          for (int j = 0; j < A; ++j) z[1 + j] = dzj[j];
-          if (valid) { l1 = logf(fmaxf(sel, net.log_eps)) * adv; l2 = -s.beta * ent; }
-        }
+        // a row beyond the batch takes zero actions; its p is not stored and its gradients are zero
+        const float* arow = s.a + (size_t)(row0 + r) * A;
+        float* prow = s.p_out + (size_t)(row0 + r) * A;
+        t = softmax_policy_row(
+            z + 1, A, v, yr, s.la, policy_inv_mix(s.la, A), TRAIN, [&](int j) { return valid ? arow[j] : 0.f; },
+            [&](int j, float pj) { if (valid && s.p_out != nullptr) prow[j] = pj; },
+            [&](int j, float dzj) { z[1 + j] = valid ? dzj : 0.f; });
       }
       if (TRAIN) {
-        z[0] = s.part == 1 ? 0.f : dv;                     // Config.DUAL_RMSPROP: cost_p alone does not reach the value head ...
-        if (s.part == 2)
-          for (int j = 1; j < n_out; ++j) z[j] = 0.f;      // ... and cost_v alone not the policy head
+        z[0] = valid ? t.dv : 0.f;
         if (valid) {
+          t.add_to(s.la.beta, sums);
           float* dl = s.dlogits + (size_t)(row0 + r) * net.n_out_ld;
           for (int j = 0; j < n_out; ++j) dl[j] = z[j];
         }
@@ -429,7 +361,7 @@ __global__ void __launch_bounds__(FT, 1) mlp_fused_kernel(const MlpNet net, cons
     // loss sums of the tile, fixed order: warp tree, then warp 0 + warp 1
     constexpr int RW = (TM + 31) / 32;     // warps that hold rows (threads beyond TM contribute zeros)
     if (tid < 32 * RW) {
-      l1 = warp_sum(l1); l2 = warp_sum(l2); lv = warp_sum(lv);
+      const float l1 = warp_sum(sums.l1), l2 = warp_sum(sums.l2), lv = warp_sum(sums.lv);
       if ((tid & 31) == 0) { red[(tid >> 5) * 4 + 0] = l1; red[(tid >> 5) * 4 + 1] = l2; red[(tid >> 5) * 4 + 2] = lv; }
     }
     __syncthreads();                       // dlogits tile + loss partials visible

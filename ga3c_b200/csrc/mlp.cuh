@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "kernels.h"
+
 namespace ga3c {
 
 constexpr int MLP_MAX_LAYERS = 8;     // live hidden layers
@@ -30,8 +32,6 @@ struct MlpNet {
   int wv_off, bv_off;   // logits_v
   int wp_off, bp_off;   // logits_p   (fork_vp: logits_p/out_x)
   int wy_off, by_off;   // fork_vp: logits_p/out_y
-  float log_eps, min_policy;
-  int log_softmax;      // DISCRATE: Config.USE_LOG_SOFTMAX
 };
 
 struct MlpStepArgs {
@@ -39,8 +39,7 @@ struct MlpStepArgs {
   const float* x;                       // [B, state_dim]
   const float *yr, *a;                  // train: [B], [B, A]
   int batch, train;
-  int part;                             // Config.DUAL_RMSPROP passes: 0 gradient of cost_all, 1 of cost_p alone, 2 of cost_v alone
-  float beta;
+  LossArgs la;                          // log_softmax, min_policy: DISCRATE only
   float *p_out, *v_out;                 // may be null in train mode
   float* act[MLP_MAX_LAYERS];           // train: layer outputs [B, n_l]
   float* dz[MLP_MAX_LAYERS];            // train: gradients w.r.t. the pre-activations [B, n_l]

@@ -75,7 +75,6 @@ extern "C" int ga3c_mlp_create(const ga3c_mlp_config* cfg, ga3c_mlp** out) {
   const int S = cfg->state_dim, A = cfg->num_actions;
   MlpNet& net = n->net;
   net.kind = cfg->kind; net.state_dim = S; net.num_actions = A;
-  net.log_eps = cfg->log_epsilon; net.min_policy = cfg->min_policy; net.log_softmax = cfg->use_log_softmax != 0;
 
   auto add = [&](const std::string& scope, int k, int width, int live) {    // dense_layer: 'w' [k, width] then 'b' [width]
     Param w{scope + "/w:0", 0, (int64_t)k * width, 2, {k, width, 0, 0}, live};
@@ -266,9 +265,10 @@ static RmsPropArgs rmsprop_args(ga3c_mlp* n, float lr) {
   return a;
 }
 
-static MlpStepArgs step_args(ga3c_mlp* n, const float* x, int batch) {
+static MlpStepArgs step_args(ga3c_mlp* n, const float* x, int batch, float beta = 0.f, int part = 0) {
   MlpStepArgs s{};
   s.w = n->w; s.x = x; s.batch = batch;
+  s.la = LossArgs{beta, n->cfg.log_epsilon, n->cfg.min_policy, n->cfg.use_log_softmax != 0, part};
   for (int l = 0; l < n->net.n_layers; ++l) { s.act[l] = n->act[l]; s.dz[l] = n->dz[l]; }
   s.dlogits = n->dlogits; s.loss_part = n->loss_part;
   return s;
@@ -303,8 +303,8 @@ static int mlp_fb_impl(ga3c_mlp* n, const float* x, const float* yr, const float
   if (!x || !yr || !a) return set_error("ga3c_mlp_forward_backward: null buffer");
   CK(cudaSetDevice(n->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
-  MlpStepArgs s = step_args(n, x, batch);
-  s.yr = yr; s.a = a; s.beta = beta; s.train = 1; s.part = part;
+  MlpStepArgs s = step_args(n, x, batch, beta, part);
+  s.yr = yr; s.a = a; s.train = 1;
   n->last_batch = batch;
   const int tm = mlp_tile_rows(batch, n->num_sms);
   if (n->tc_hi > n->tc_lo && batch >= n->tc_min_batch) {

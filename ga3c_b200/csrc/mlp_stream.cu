@@ -13,20 +13,14 @@
 #include "common.cuh"
 #include "kernels.h"
 #include "mlp.cuh"
+#include "a3c_loss.cuh"
 
 namespace ga3c {
 
 namespace {
 
-constexpr float PI_F = 3.14159265358979323846f;
 constexpr int ST_THREADS = 256, ST_WARPS = ST_THREADS / 32;
-__device__ __forceinline__ float sigmoid_(float z) { return 1.f / (1.f + expf(-z)); }
-__device__ __forceinline__ float act_(float z, int act) { return act == MLP_ACT_SIGMOID ? sigmoid_(z) : z; }
-__device__ __forceinline__ float warp_allsum(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
+__device__ __forceinline__ float act_(float z, int act) { return act == MLP_ACT_SIGMOID ? sigmoid(z) : z; }
 
 // ---- front, forward ---------------------------------------------------------------------------------------------------------------
 // 64 threads per row (N1 = 256: four columns each), 4 rows per block and iteration.  W1's four columns (x N0 <= 4 rows) and the
@@ -115,7 +109,7 @@ __global__ void __launch_bounds__(ST_THREADS) mlp_heads_kernel(const MlpNet net,
   }
   bh[0] = __ldg(s.w + net.bv_off); bh[1] = __ldg(s.w + net.bp_off); bh[2] = __ldg(s.w + net.by_off);
   const int my = lane & (HU - 1);                                  // the row of the group whose scalar part this lane computes
-  float l1 = 0.f, l2 = 0.f, lv = 0.f;                             // loss terms of the rows this lane owns (lanes 0 .. HU-1 count)
+  A3cSums sums;                                                   // loss terms of the rows this lane owns (lanes 0 .. HU-1 count)
   for (int r0 = warp * HU; r0 < B; r0 += nwarps * HU) {
     float hv[HU][KMAX];
 #pragma unroll
@@ -137,29 +131,21 @@ __global__ void __launch_bounds__(ST_THREADS) mlp_heads_kernel(const MlpNet net,
       for (int i = 0; i < KMAX; ++i) {
         a0 = fmaf(hv[u][i], wh[i][0], a0); a1 = fmaf(hv[u][i], wh[i][1], a1); a2 = fmaf(hv[u][i], wh[i][2], a2);
       }
-      a0 = warp_allsum(a0); a1 = warp_allsum(a1); a2 = warp_allsum(a2);
+      a0 = warp_sum(a0); a1 = warp_sum(a1); a2 = warp_sum(a2);
       if (u == my) { z0 = a0 + bh[0]; z1 = a1 + bh[1]; z2 = a2 + bh[2]; }
     }
     const float v = z0;
-    const float ox = sigmoid_(z1), oy = sigmoid_(z2);
-    const float X = ox - 0.5f, Y = oy - 0.5f;
-    const float p = atan2f(Y, X) / PI_F;
+    float sel = 0.f, sq = 0.f;
+    const ForkAction f = fork_policy(z1, z2, av, v, yr, s.la, sel, sq);
     if (lane < HU && valid) {
       if (s.v_out != nullptr) s.v_out[r] = v;
-      if (s.p_out != nullptr) s.p_out[r] = p;
+      if (s.p_out != nullptr) s.p_out[r] = f.p;
     }
     if (TRAIN) {
-      const float adv = yr - v;                                    // stop_gradient(v) inside cost_p_1
-      const float dp = -av * adv + 2.f * s.beta * p;
-      const float inv = 1.f / (PI_F * (X * X + Y * Y));
-      float d0 = s.part == 1 ? 0.f : v - yr;                       // Config.DUAL_RMSPROP: cost_p alone does not reach the value head ...
-      float d1 = dp * (-Y * inv) * ox * (1.f - ox);
-      float d2 = dp * (X * inv) * oy * (1.f - oy);
-      if (s.part == 2) { d1 = 0.f; d2 = 0.f; }                     // ... and cost_v alone not the policy head
+      const A3cTerms t = fork_policy_terms(sel, sq, v, yr, s.la);
+      const float d0 = t.dv, d1 = f.dzx, d2 = f.dzy;
       if (lane < HU && valid) {
-        l1 += (p * av) * adv;
-        l2 += -s.beta * (p * p);
-        lv += 0.5f * (yr - v) * (yr - v);
+        t.add_to(s.la.beta, sums);
         *reinterpret_cast<float4*>(s.dlogits + (size_t)r * net.n_out_ld) = make_float4(d0, d1, d2, 0.f);
       }
 #pragma unroll
@@ -183,10 +169,10 @@ __global__ void __launch_bounds__(ST_THREADS) mlp_heads_kernel(const MlpNet net,
   }
   if (TRAIN) {                                                  // one row of loss_part per block: lanes 0 .. HU-1 of a warp in lane
     __shared__ float red[ST_WARPS][3];                          // order, then the warps in warp order
-    float t1 = l1, t2 = l2, tv = lv;
+    float t1 = sums.l1, t2 = sums.l2, tv = sums.lv;
 #pragma unroll
     for (int u = 1; u < HU; ++u) {
-      t1 += __shfl_sync(0xffffffffu, l1, u); t2 += __shfl_sync(0xffffffffu, l2, u); tv += __shfl_sync(0xffffffffu, lv, u);
+      t1 += __shfl_sync(0xffffffffu, sums.l1, u); t2 += __shfl_sync(0xffffffffu, sums.l2, u); tv += __shfl_sync(0xffffffffu, sums.lv, u);
     }
     if (lane == 0) { red[threadIdx.x >> 5][0] = t1; red[threadIdx.x >> 5][1] = t2; red[threadIdx.x >> 5][2] = tv; }
     __syncthreads();
@@ -241,7 +227,7 @@ __global__ void __launch_bounds__(ST_THREADS) mlp_front_bwd_kernel(const MlpNet 
         float a = 0.f;
         a = fmaf(d[u][0].x, w1[k][0], a); a = fmaf(d[u][0].y, w1[k][1], a); a = fmaf(d[u][0].z, w1[k][2], a); a = fmaf(d[u][0].w, w1[k][3], a);
         a = fmaf(d[u][1].x, w1[k][4], a); a = fmaf(d[u][1].y, w1[k][5], a); a = fmaf(d[u][1].z, w1[k][6], a); a = fmaf(d[u][1].w, w1[k][7], a);
-        t[k] = warp_allsum(a);
+        t[k] = warp_sum(a);
       }
       if (lane < N0) {
         float g = lane == 0 ? t[0] : lane == 1 ? t[1] : lane == 2 ? t[2] : t[3];

@@ -78,7 +78,7 @@ struct Epi3Fwd {         // out = act(acc + b)
   __device__ __forceinline__ void operator()(int, int m, int n, float4 v, const float4 b) const {
     v.x += b.x; v.y += b.y; v.z += b.z; v.w += b.w;
     if (act == MLP_ACT_SIGMOID) {
-      v.x = 1.f / (1.f + expf(-v.x)); v.y = 1.f / (1.f + expf(-v.y)); v.z = 1.f / (1.f + expf(-v.z)); v.w = 1.f / (1.f + expf(-v.w));
+      v.x = sigmoid(v.x); v.y = sigmoid(v.y); v.z = sigmoid(v.z); v.w = sigmoid(v.w);
     }
     *reinterpret_cast<float4*>(out + (size_t)m * N + n) = v;
   }

@@ -281,13 +281,13 @@ extern "C" int ga3c_arena_download(ga3c_net* n, int which, float* host, int64_t 
 extern "C" int64_t ga3c_global_step(const ga3c_net* n) { return n ? n->global_step : -1; }
 extern "C" int ga3c_set_global_step(ga3c_net* n, int64_t s) { if (!n) return -1; n->global_step = s; return 0; }
 
-static HeadsArgs heads_args(ga3c_net* n, int batch, int splits) {
+static HeadsArgs heads_args(ga3c_net* n, int batch, int splits, float beta = 0.f, int part = 0) {
   HeadsArgs h{};
   h.d1 = n->d1; h.d1_part = n->d1_part; h.n_split = splits; h.b1 = n->w + n->off(P_D1B);
   h.wp = n->w + n->off(P_PW); h.bp = n->w + n->off(P_PB);
   h.wv = n->w + n->off(P_VW); h.bv = n->w + n->off(P_VB);
   h.batch = batch; h.num_actions = n->cfg.num_actions;
-  h.log_eps = n->cfg.log_epsilon; h.min_policy = n->cfg.min_policy; h.log_softmax = n->cfg.use_log_softmax != 0;
+  h.la = LossArgs{beta, n->cfg.log_epsilon, n->cfg.min_policy, n->cfg.use_log_softmax != 0, part};
   h.preload = batch >= n->num_sms;
   return h;
 }
@@ -369,8 +369,8 @@ static int fb_head_impl(ga3c_net* n, const void* x, bool x_u8, const float* yr, 
     const DpGate gate = dp_gate(n);
     LAUNCH(n, K_DENSE_FWD, st, launch_dense_fwd_tc(n->n2, n->w1_shadow, n->d1_part, batch, n->geo.kdim, splits, st, &gate));
   }
-  HeadsArgs h = heads_args(n, batch, splits);
-  h.yr = yr; h.a = a; h.beta = beta; h.train = 1; h.dd1 = n->dd1; h.part = part;
+  HeadsArgs h = heads_args(n, batch, splits, beta, part);
+  h.yr = yr; h.a = a; h.train = 1; h.dd1 = n->dd1;
   h.g_wp = gp + n->off(P_PW); h.g_bp = gp + n->off(P_PB); h.g_wv = gp + n->off(P_VW); h.g_bv = gp + n->off(P_VB);
   h.g_b1 = gp + n->off(P_D1B); h.loss = gp + n->small_floats; h.gp_stride = n->gp_stride;
   n->gp_heads_grid = heads_grid(batch, n->num_sms);
